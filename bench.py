@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the stralg hot path on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 N = 1  -> workload "build": SA + BWT + C + sampled O of a 3 Gbp synthetic DNA text (BASELINE.json
           configs[2]; the text is resident in HBM before the timed region).  value = Mchars/s.
@@ -23,6 +23,11 @@ headline is the search metric as well (build nested as `build`), so that efficie
 is computable from the lines of one series.
 --impl reference times the reference's own CPU implementation (oracle/_ref, else the oracle
 port) on a bounded sample of the same workload; rank 0 only.
+--dump-outputs DIR (rank 0) writes, after the timed steps, a fixed seeded sample of what the last timed step
+computed: the build's suffix array, C table and O table, and the (L, R) intervals of the timed search.  The
+inputs are generated from fixed seeds, so two builds of the project can be compared file by file.  The one
+difference in what is timed: the last build step's index is released after the timed region instead of inside it
+(one host-side release of its device buffers per run), so that its tables can be read afterwards.
 
 One JSON line on stdout (rank 0).  Timing: W >= 3 warm-up steps, CUDA events on the launching
 stream, barrier + synchronize on both sides, max over ranks; inputs are far larger than L2.
@@ -49,11 +54,53 @@ READ_LEN = 100
 MISS_PER_1024 = 102  # ~10 % of the reads are uniform random (SURVEY 8d, C4)
 SEED = 88172645463325252
 CPU_SAMPLE = 1 << 24
+DUMP_ROWS = 1 << 19  # rows per sampled array of --dump-outputs: all of them come to about 32 MB in float64
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SEED = 20261020
 
 
 def env_int(name, dflt):
     v = os.environ.get(name)
     return int(v) if v else dflt
+
+
+def dump_rows(count, seed):
+    """The fixed, seeded, sorted rows of an output of `count` rows that --dump-outputs writes (all rows when the
+    output is small), so that two builds of the project dump the same entries."""
+    if count <= DUMP_ROWS:
+        return np.arange(count, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).integers(0, count, DUMP_ROWS, dtype=np.int64))
+
+
+def build_outputs(idx, torch, device):
+    """What a caller of the timed build receives, sampled: SA rows, the C table and O(a, i) (the sampled O table
+    answers through the library's occ query)."""
+    from stralg_b200 import texts as T
+    rows = dump_rows(idx.length, DUMP_SEED)
+    sa = T.device_view(idx.device_ptr("sa"), idx.length, 4, device)
+    sa_rows = sa[torch.from_numpy(rows).to(sa.device)].cpu().numpy().view(np.uint32)
+    occ_i = dump_rows(idx.length + 1, DUMP_SEED + 1).astype(np.uint32)
+    occ_a = np.random.default_rng(DUMP_SEED + 2).integers(0, idx.sigma, len(occ_i)).astype(np.uint8)
+    return {"build_sa_rows": rows, "build_sa": sa_rows, "build_c_table": idx.c_table(),
+            "build_occ_i": occ_i, "build_occ_a": occ_a, "build_occ": idx.occ(occ_a, occ_i)}
+
+
+def search_outputs(L, R, torch):
+    """(L, R) of the timed search's last step (int32 tensors holding uint32 values), sampled by read."""
+    rows = dump_rows(L.numel(), DUMP_SEED + 3)
+    sel = torch.from_numpy(rows).to(L.device)
+    return {"search_read_rows": rows, "search_L": L[sel].cpu().numpy().view(np.uint32),
+            "search_R": R[sel].cpu().numpy().view(np.uint32)}
+
+
+def write_outputs(out_dir, arrays):
+    """DIR/<name>.npy in float64 (every value here is an integer below 2^53, so the conversion is exact)."""
+    arrays = {k: np.asarray(v).astype(np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peak():
@@ -577,6 +624,7 @@ def gpu_arm(args, rank, local_rank, world):
 
     sampler = ClockSampler(local_rank)
     out = {}
+    dump = {} if (args.dump_outputs and rank == 0) else None  # name -> array of the last timed step
 
     if workload == "build":
         # ------------------------------------------------------------------ device-resident build
@@ -590,7 +638,7 @@ def gpu_arm(args, rank, local_rank, world):
         t_wall0 = time.time()
         ev0.record()
         stats = None
-        for _ in range(args.steps):
+        for step in range(args.steps):
             idx = build(profile=True)
             for name, ms, by in idx.profile():
                 a = stage_ms.setdefault(name, [0, 0.0, 0.0])
@@ -598,11 +646,15 @@ def gpu_arm(args, rank, local_rank, world):
                 a[1] += ms
                 a[2] += by
             stats = idx.stats()
-            idx.close()
+            if not (dump is not None and step == args.steps - 1):  # --dump-outputs reads the last index below
+                idx.close()
         ev1.record()
         barrier()
         t_wall1 = time.time()
         sampler.stop()
+        if dump is not None:
+            dump.update(build_outputs(idx, torch, local_rank))
+            idx.close()
         launches = lib.b200sa_launch_count() - launches0
         ms_total = max_over_ranks(ev0.elapsed_time(ev1))
         ms_step = ms_total / args.steps
@@ -821,7 +873,7 @@ def gpu_arm(args, rank, local_rank, world):
                 out["compat"] = {"error": str(ex)[:300]}
         if not args.no_search:
             out["search"] = search_bench(args, lib, stralg_b200, torch, dev, local_rank, stream, text, n, None, 0, 1,
-                                         peak, peak_src, build)
+                                         peak, peak_src, build, dump=dump)
             # BASELINE.json's metric has two parts: the build on 1 GPU (this line's `value`) and the search at
             # 1/2/4/8 GPUs (the `value` of the N > 1 lines).  The N = 1 point of the SEARCH series is repeated
             # here at the top level so that a scaling table can be read off the lines of one run.
@@ -843,7 +895,7 @@ def gpu_arm(args, rank, local_rank, world):
             nested_build = {"metric": METRIC_BUILD, "value": n / (bms / 1e3) / 1e6, "unit": "Mchars/s", "ms_per_step": bms,
                             "n": n, "note": "the full build line is what `python bench.py --gpus 1` prints"}
         res = search_bench(args, lib, stralg_b200, torch, dev, local_rank, stream, text, n, dist, rank, world, peak,
-                           peak_src, build)
+                           peak_src, build, dump=dump)
         out = res
         if nested_build:
             out["build"] = nested_build
@@ -852,13 +904,15 @@ def gpu_arm(args, rank, local_rank, world):
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if rank == 0:
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(out) + "\n").encode())
 
 
 def search_bench(args, lib, stralg_b200, torch, dev, local_rank, stream, text, n, dist, rank, world, peak, peak_src,
-                 build):
+                 build, dump=None):
     """Replicated index, reads split over ranks, (L, R) delivered on rank 0 in the timed region.  The reads are
     2-bit packed (b200sa_search_device_packed / _batch_packed; VERDICT r1 item 3); the one-byte-per-base entry
     points are measured beside them (`byte_api`)."""
@@ -916,6 +970,8 @@ def search_bench(args, lib, stralg_b200, torch, dev, local_rank, stream, text, n
     barrier()
     tw1 = time.time()
     sampler.stop()
+    if dump is not None:
+        dump.update(search_outputs(*ss.result(), torch))
     ms_total = ev0.elapsed_time(ev1)
     if dist is not None:
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
@@ -1176,7 +1232,12 @@ def main():
     ap.add_argument("--sa-rate", type=int, default=32)
     ap.add_argument("--approx-reads", type=int, default=200_000)
     ap.add_argument("--approx-d2", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed, seeded sample of what the last step computed (suffix "
+                         "array rows, C table, O(a, i), search intervals) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     args.warmup_ref = min(args.warmup, 1)
     rank = int(os.environ.get("RANK", "0"))

@@ -175,24 +175,6 @@ cudaMemPool_t library_pool() {
 }
 }  // namespace b200sa
 
-static void use_device(int device) {
-    CUDA_CHECK(cudaSetDevice(device));
-    static std::mutex mu;
-    static bool once[64] = {};
-    std::lock_guard<std::mutex> lock(mu);
-    if (device >= 0 && device < 64 && !once[device]) {
-        if (const char *g = getenv("B200SA_L2_FETCH")) {  // measurement aid
-            size_t before = 0;
-            cudaDeviceGetLimit(&before, cudaLimitMaxL2FetchGranularity);
-            cudaError_t e = cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(g));
-            size_t after = 0;
-            cudaDeviceGetLimit(&after, cudaLimitMaxL2FetchGranularity);
-            fprintf(stderr, "b200sa: L2 fetch granularity %zu -> %zu (%s)\n", before, after, cudaGetErrorString(e));
-        }
-        once[device] = true;
-    }
-}
-
 // Restores the caller's current device when an entry point returns (ADVICE r1: the library must not
 // silently switch the device of the process that hosts it).
 struct DeviceGuard {
@@ -356,7 +338,6 @@ static int build_into(b200sa_index *h, const uint8_t *codes, uint64_t n, uint32_
                       void *stream, enum b200sa_error *err) {
     API_GUARD_BEGIN
     DeviceGuard guard(device);
-    use_device(device);
     DeviceIndex &ix = h->ix;
     ix.stream = (cudaStream_t)stream;
     ix.device = device;
@@ -466,7 +447,6 @@ int b200sa_extend(b200sa_index *idx, const uint8_t *codes, uint32_t flags) {
     mail_server_release(idx);  // (the resident one-pattern search was launched with the tables as they were)
     API_GUARD_BEGIN
     DeviceGuard guard(ix.device);
-    use_device(ix.device);
     cudaStream_t st = ix.stream;
     std::lock_guard<std::mutex> arena_lock(g_arena_mu[ix.device & 63]);
     Arena &arena = g_arena[ix.device & 63];
@@ -1108,7 +1088,6 @@ b200sa_index *b200sa_replicate(const b200sa_index *src, int device, void *stream
             CUDA_CHECK(cudaStreamSynchronize(src->ix.stream));  // the source tables are complete
         }
         DeviceGuard guard(device);
-        use_device(device);
         const DeviceIndex &a = src->ix;
         DeviceIndex &ix = h->ix;
         cudaStream_t st = (cudaStream_t)stream;
@@ -1311,7 +1290,6 @@ int b200sa_sample_sa(b200sa_index *idx, uint32_t rate, int drop_sa) {
     if (ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "the sampled suffix array needs the O table (B200SA_BUILD_OCC)", nullptr);
     API_GUARD_BEGIN
     DeviceGuard guard(ix.device);
-    use_device(ix.device);
     build_sampled_sa(ix, rate);
     if (drop_sa && !(idx->flags & B200SA_BUILD_TEXTCMP)) ix.sa.release();
     CUDA_CHECK(cudaStreamSynchronize(ix.stream));
@@ -1420,7 +1398,6 @@ b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200s
     }
     try {
         DeviceGuard guard(device);
-        use_device(device);
         IndexFileHeader fh;
         if (fread(&fh, sizeof fh, 1, f) != 1 || memcmp(fh.magic, "B200SAIX", 8) != 0)
             throw std::invalid_argument("not a b200sa index file");

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <cstdlib>
 #include <mutex>
 #include <stdexcept>
 #include <string>
@@ -233,6 +234,12 @@ struct Arena {
 };
 
 static inline unsigned div_up_u(u64 a, u64 b) { return (unsigned)((a + b - 1) / b); }
+
+// integer value of environment variable `name`; `dflt` when it is unset or empty
+static inline int env_int(const char *name, int dflt) {
+    const char *v = getenv(name);
+    return v && *v ? atoi(v) : dflt;
+}
 
 // cudaFuncSetAttribute (the opt-in for more than 48 KB of dynamic shared memory) is per device, i.e.
 // per context: a process that builds on several devices has to repeat it on each one.  first()

@@ -158,24 +158,11 @@ struct BlockRegs {
     u64 w0, w1;
 };
 
-template <int LM>
 __device__ __forceinline__ BlockRegs load_dna_block(const u8 *blocks, u32 b) {
     u64 a, bb, c, d;
     const u8 *p = blocks + (size_t)b * 32;
-    if (LM == 0) {
-        asm volatile("ld.global.nc.L1::no_allocate.v4.u64 {%0,%1,%2,%3}, [%4];"
-                     : "=l"(a), "=l"(bb), "=l"(c), "=l"(d) : "l"(p));
-    } else if (LM == 1) {
-        uint4 x = __ldg((const uint4 *)p), y = __ldg((const uint4 *)p + 1);
-        a = ((u64)x.y << 32) | x.x; bb = ((u64)x.w << 32) | x.z;
-        c = ((u64)y.y << 32) | y.x; d = ((u64)y.w << 32) | y.z;
-    } else if (LM == 2) {
-        asm volatile("ld.global.v4.u64 {%0,%1,%2,%3}, [%4];"
-                     : "=l"(a), "=l"(bb), "=l"(c), "=l"(d) : "l"(p));
-    } else {
-        asm volatile("ld.global.nc.L1::no_allocate.L2::64B.v4.u64 {%0,%1,%2,%3}, [%4];"
-                     : "=l"(a), "=l"(bb), "=l"(c), "=l"(d) : "l"(p));
-    }
+    asm volatile("ld.global.nc.L1::no_allocate.L2::64B.v4.u64 {%0,%1,%2,%3}, [%4];"
+                 : "=l"(a), "=l"(bb), "=l"(c), "=l"(d) : "l"(p));
     BlockRegs r;
     r.c0 = (u32)a; r.c1 = (u32)(a >> 32); r.c2 = (u32)bb; r.c3 = (u32)(bb >> 32);
     r.w0 = c; r.w1 = d;
@@ -222,7 +209,7 @@ __global__ void __launch_bounds__(256) ktable_build_kernel(OccView ov, CTable5 c
 }
 
 // one pattern: pat[begin .. begin + m), readable in aligned 8-byte words; (L, R) = the interval of bwt.c:171-198
-template <int LM, bool SC, bool STATS>
+template <bool SC, bool STATS>
 __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTable5 &c5, const TextCmp &tc, const KTable &kt,
                                                   u32 len, const u8 *__restrict__ pat, u64 begin, u64 m, u32 &Lout, u32 &Rout,
                                                   u32 &n_blk, u32 &n_pw, u32 &n_tw, u32 &n_sa) {
@@ -274,9 +261,9 @@ __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTabl
             break;
         }
         const u32 bL = L >> 6, bR = R >> 6;
-        BlockRegs kL = load_dna_block<LM>(ov.blocks, bL);
+        BlockRegs kL = load_dna_block(ov.blocks, bL);
         BlockRegs kR = kL;
-        if (bR != bL) kR = load_dna_block<LM>(ov.blocks, bR);
+        if (bR != bL) kR = load_dna_block(ov.blocks, bR);
         if (STATS) n_blk += bR != bL ? 2u : 1u;
         const u32 ca = c5.c[a];
         L = ca + rank_in_block(kL, a, L, ov.primary);
@@ -383,9 +370,9 @@ __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTabl
         } else {
             // the step that fails: BWT[Lk] != a, so both ranks coincide and the interval is empty
             const u32 Lk = k ? tc.isa[s - (u32)k] : L;
-            BlockRegs kb = load_dna_block<LM>(ov.blocks, Lk >> 6);
+            BlockRegs kb = load_dna_block(ov.blocks, Lk >> 6);
             BlockRegs kb2 = kb;
-            if (((Lk + 1) >> 6) != (Lk >> 6)) kb2 = load_dna_block<LM>(ov.blocks, (Lk + 1) >> 6);
+            if (((Lk + 1) >> 6) != (Lk >> 6)) kb2 = load_dna_block(ov.blocks, (Lk + 1) >> 6);
             if (STATS) {
                 n_sa += k ? 1u : 0u;
                 n_blk += 1u + ((((Lk + 1) >> 6) != (Lk >> 6)) ? 1u : 0u);
@@ -398,7 +385,7 @@ __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTabl
     Rout = R;
 }
 
-template <int LM, bool SC, bool STATS>
+template <bool SC, bool STATS>
 __global__ void __launch_bounds__(256) fm_search_dna_kernel(OccView ov, CTable5 c5, TextCmp tc, KTable kt, u32 len,
                                                             const u8 *__restrict__ pat,
                                                             const u64 *__restrict__ off, u32 fixed_len, u64 npat,
@@ -410,7 +397,7 @@ __global__ void __launch_bounds__(256) fm_search_dna_kernel(OccView ov, CTable5 
     u64 begin = off ? off[q] : q * (u64)fixed_len;
     u64 m = off ? off[q + 1] - begin : (u64)fixed_len;
     u32 L, R;
-    fm_search_dna_one<LM, SC, STATS>(ov, c5, tc, kt, len, pat, begin, m, L, R, n_blk, n_pw, n_tw, n_sa);
+    fm_search_dna_one<SC, STATS>(ov, c5, tc, kt, len, pat, begin, m, L, R, n_blk, n_pw, n_tw, n_sa);
     outL[q] = L;
     outR[q] = R;
     if (STATS) {
@@ -476,7 +463,7 @@ __global__ void __launch_bounds__(32) fm_mailbox_server_kernel(OccView ov, CTabl
             u32 L, R, c0 = 0, c1 = 0, c2 = 0, c3 = 0;
             u64 t0, t1;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-            fm_search_dna_one<3, SC, false>(ov, c5, tc, kt, len, spat, 0, (u64)m, L, R, c0, c1, c2, c3);
+            fm_search_dna_one<SC, false>(ov, c5, tc, kt, len, spat, 0, (u64)m, L, R, c0, c1, c2, c3);
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
             st_sys_u64(resp + 2, t1 - t0);  // (nanoseconds inside the search: B200SA_MAIL_DEBUG)
             st_sys_u64(resp, (u64)L | ((u64)expect << 48));
@@ -541,13 +528,12 @@ __device__ __forceinline__ u64 bits_ending(const u64 *__restrict__ words, u64 en
     return nbits >= 64 ? v : (v & ((1ull << nbits) - 1ull));
 }
 
-// MINB: resident CTAs per SM the register allocation aims at (8: 32 registers, every thread slot of the SM in use)
-template <bool SC, bool STATS, bool PF = false, int MINB = 1>
-__global__ void __launch_bounds__(256, MINB) fm_search_dna_packed_kernel(OccView ov, CTable5 c5, TextCmp tc, KTable kt, u32 len,
-                                                                   const u64 *__restrict__ pw, u32 m, u32 stride,
-                                                                   u64 npat, u32 *__restrict__ outL,
-                                                                   u32 *__restrict__ outR,
-                                                                   unsigned long long *__restrict__ stats) {
+template <bool SC, bool STATS>
+__global__ void __launch_bounds__(256, 1) fm_search_dna_packed_kernel(OccView ov, CTable5 c5, TextCmp tc, KTable kt, u32 len,
+                                                                      const u64 *__restrict__ pw, u32 m, u32 stride,
+                                                                      u64 npat, u32 *__restrict__ outL,
+                                                                      u32 *__restrict__ outR,
+                                                                      unsigned long long *__restrict__ stats) {
     const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= npat) return;
     u32 n_blk = 0, n_pw = 0, n_tw = 0, n_sa = 0;
@@ -578,9 +564,9 @@ __global__ void __launch_bounds__(256, MINB) fm_search_dna_packed_kernel(OccView
             break;
         }
         const u32 bL = L >> 6, bR = R >> 6;
-        BlockRegs kL = load_dna_block<3>(ov.blocks, bL);
+        BlockRegs kL = load_dna_block(ov.blocks, bL);
         BlockRegs kR = kL;
-        if (bR != bL) kR = load_dna_block<3>(ov.blocks, bR);
+        if (bR != bL) kR = load_dna_block(ov.blocks, bR);
         if (STATS) n_blk += bR != bL ? 2u : 1u;
         const u32 ca = c5.c[a];
         L = ca + rank_in_block(kL, a, L, ov.primary);
@@ -591,9 +577,6 @@ __global__ void __launch_bounds__(256, MINB) fm_search_dna_packed_kernel(OccView
         const u32 s = tc.sa[L];
         if (STATS) ++n_sa;
         const u32 rem = (u32)i + 1u;
-        // nine reads in ten match to the end and then ask for ISA[s - rem]; starting that fetch here, behind the
-        // text comparison, measured SLOWER (B200SA_SEARCH_ISA_PREFETCH=1 turns it on)
-        if (PF && s >= rem) asm volatile("prefetch.global.L2 [%0];" ::"l"(tc.isa + (s - rem)));
         u32 k = 0;  // bases matched so far, from pattern[i] / text[s-1] downwards
         u64 t_idx = ~0ull, t_word = 0;
         bool mismatch = false;
@@ -625,9 +608,9 @@ __global__ void __launch_bounds__(256, MINB) fm_search_dna_packed_kernel(OccView
             } else {
                 // the step that fails: BWT[Lk] != a, so both ranks coincide and the interval is empty
                 const u32 Lk = k ? tc.isa[s - k] : L;
-                BlockRegs kb = load_dna_block<3>(ov.blocks, Lk >> 6);
+                BlockRegs kb = load_dna_block(ov.blocks, Lk >> 6);
                 BlockRegs kb2 = kb;
-                if (((Lk + 1) >> 6) != (Lk >> 6)) kb2 = load_dna_block<3>(ov.blocks, (Lk + 1) >> 6);
+                if (((Lk + 1) >> 6) != (Lk >> 6)) kb2 = load_dna_block(ov.blocks, (Lk + 1) >> 6);
                 if (STATS) {
                     n_sa += k ? 1u : 0u;
                     n_blk += 1u + ((((Lk + 1) >> 6) != (Lk >> 6)) ? 1u : 0u);
@@ -681,22 +664,15 @@ void fm_search_packed(const DeviceIndex &ix, const u8 *d_packed, u32 m, u32 stri
     CTable5 c5;
     for (int i = 0; i < 8; ++i) c5.c[i] = ix.c_host[i];
     const unsigned blocks = div_up_u(npat, 256);
-    static const bool no_sc = getenv("B200SA_SEARCH_NO_TEXTCMP") != nullptr;
-    static const bool no_kt = getenv("B200SA_SEARCH_NO_KTABLE") != nullptr;
     TextCmp tc{ix.sa.ptr, ix.isa.ptr, ix.text_packed.ptr};
-    KTable kt{no_kt ? nullptr : ix.ktable.ptr, ix.ktable_k};
-    const bool sc = tc.sa && tc.isa && tc.packed && ix.pk.bits == 2 && !no_sc;
+    KTable kt{ix.ktable.ptr, ix.ktable_k};
+    const bool sc = tc.sa && tc.isa && tc.packed && ix.pk.bits == 2;
     const u64 *pw = (const u64 *)d_packed;
     if (d_stats) {
         if (sc) fm_search_dna_packed_kernel<true, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, d_stats);
         else fm_search_dna_packed_kernel<false, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, d_stats);
     } else if (sc) {
-        // (measured, 3 Gbp / 10^8 reads: 15.7 ms with the prefetch against 13.6 ms without -- off unless asked for)
-        static const bool pf = getenv("B200SA_SEARCH_ISA_PREFETCH") && atoi(getenv("B200SA_SEARCH_ISA_PREFETCH")) != 0;
-        static const int occ8 = getenv("B200SA_SEARCH_OCC8") ? atoi(getenv("B200SA_SEARCH_OCC8")) : 0;
-        if (pf) fm_search_dna_packed_kernel<true, false, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, nullptr);
-        else if (occ8) fm_search_dna_packed_kernel<true, false, false, 8><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, nullptr);
-        else fm_search_dna_packed_kernel<true, false, false><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, nullptr);
+        fm_search_dna_packed_kernel<true, false><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, nullptr);
     } else {
         fm_search_dna_packed_kernel<false, false><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, pw, m, stride, npat, d_L, d_R, nullptr);
     }
@@ -713,38 +689,25 @@ void fm_search(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fix
     static const bool force_generic = getenv("B200SA_SEARCH_GENERIC") != nullptr;
     if (ix.occ_layout == OCC_DNA32 && (((uintptr_t)d_pat) & 7) == 0 && !force_generic)
     {
-        static const int lm = getenv("B200SA_SEARCH_LM") ? atoi(getenv("B200SA_SEARCH_LM")) : 3;
-        static const bool no_sc = getenv("B200SA_SEARCH_NO_TEXTCMP") != nullptr;
         TextCmp tc{ix.sa.ptr, ix.isa.ptr, ix.text_packed.ptr};
-        static const bool no_kt = getenv("B200SA_SEARCH_NO_KTABLE") != nullptr;
-        KTable kt{no_kt ? nullptr : ix.ktable.ptr, ix.ktable_k};
-        const bool sc = tc.sa && tc.isa && tc.packed && ix.pk.bits == 2 && !no_sc;
-#define LAUNCH_DNA(LM_, SC_) fm_search_dna_kernel<LM_, SC_, false><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, nullptr)
+        KTable kt{ix.ktable.ptr, ix.ktable_k};
+        const bool sc = tc.sa && tc.isa && tc.packed && ix.pk.bits == 2;
         if (d_stats) {
-            // counting variant of the default configuration
-            if (sc) fm_search_dna_kernel<3, true, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, d_stats);
-            else fm_search_dna_kernel<3, false, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, d_stats);
+            if (sc) fm_search_dna_kernel<true, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, d_stats);
+            else fm_search_dna_kernel<false, true><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, d_stats);
         } else if (sc) {
-            if (lm == 0) LAUNCH_DNA(0, true); else LAUNCH_DNA(3, true);
+            fm_search_dna_kernel<true, false><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, nullptr);
         } else {
-            switch (lm) {
-                case 0: LAUNCH_DNA(0, false); break;
-                case 1: LAUNCH_DNA(1, false); break;
-                case 2: LAUNCH_DNA(2, false); break;
-                default: LAUNCH_DNA(3, false); break;
-            }
+            fm_search_dna_kernel<false, false><<<blocks, 256, 0, st>>>(ov, c5, tc, kt, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, nullptr);
         }
-#undef LAUNCH_DNA
     }
     else if (ix.occ_layout == OCC_DNA32)
         fm_search_kernel<1><<<blocks, 256, 0, st>>>(ov, c5, ix.c_table.ptr, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R);
     else {
-        static const bool no_sc2 = getenv("B200SA_SEARCH_NO_TEXTCMP") != nullptr;
         TextCmp tc{ix.sa.ptr, ix.isa.ptr, ix.text_packed.ptr};
-        static const bool no_kt2 = getenv("B200SA_SEARCH_NO_KTABLE") != nullptr;
-        KTable kt{no_kt2 ? nullptr : ix.ktable.ptr, ix.ktable_k, ix.sigma - 1};
+        KTable kt{ix.ktable.ptr, ix.ktable_k, ix.sigma - 1};
         const bool al = (((uintptr_t)d_pat) & 7) == 0 && !force_generic;
-        const bool sc2 = tc.sa && tc.isa && tc.packed && !no_sc2;
+        const bool sc2 = tc.sa && tc.isa && tc.packed;
 #define LAUNCH_GEN(SC_, AL_) fm_search_kernel<2, SC_, AL_><<<blocks, 256, 0, st>>>(ov, c5, ix.c_table.ptr, ix.len, d_pat, d_off, fixed_len, npat, d_L, d_R, tc, ix.pk.bits, kt)
         if (sc2 && al) LAUNCH_GEN(true, true);
         else if (sc2) LAUNCH_GEN(true, false);

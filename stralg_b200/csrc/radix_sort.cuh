@@ -9,7 +9,6 @@
 // scatters of stralg/sa_is.c:203-263; none of that code is reused.
 #pragma once
 #include "common.cuh"
-#include <cstdlib>
 
 namespace b200sa {
 namespace rs {
@@ -296,42 +295,11 @@ struct SortPlan {
 template <int RB>
 struct Sorter {
     static constexpr int BINS = 1 << RB;
+    // pass-kernel shape
+    static constexpr int PASS_NT = 256, PASS_IPT = 12;
+    typedef PassCfg<RB, PASS_NT, PASS_IPT> Cfg;
 
-    // pass-kernel shape: selectable with B200SA_PASS_CFG for tuning runs
-    static int cfg_id() {
-        static int id = -1;
-        if (id < 0) {
-            const char *e = getenv("B200SA_PASS_CFG");
-            id = e && *e ? atoi(e) : 0;
-            if (id < 0 || id > 3) id = 0;
-        }
-        return id;
-    }
-    static int tile_size() {
-        switch (cfg_id()) {
-            case 1: return 512 * 12;
-            case 2: return 256 * 16;
-            case 3: return 384 * 12;
-            default: return 256 * 12;
-        }
-    }
-    static size_t lookback_words(u32 n) { return (size_t)div_up_u(n, 256 * 12) * BINS; }
-
-    template <int NT, int IPT>
-    static void launch_pass(const u64 *kin, const u32 *vin, u64 *kout, u32 *vout, u32 n, int shift, u32 mask,
-                            const u32 *digit_base, u64 *lookback, u32 *ticket, cudaStream_t st) {
-        typedef PassCfg<RB, NT, IPT> Cfg;
-        static PerDeviceOnce once;
-        if (once.first())
-            CUDA_CHECK(cudaFuncSetAttribute(onesweep_pass_kernel<RB, NT, IPT>,
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
-        unsigned tiles = div_up_u(n, Cfg::TILE);
-        CUDA_CHECK(cudaMemsetAsync(lookback, 0, (size_t)tiles * BINS * 8, st));
-        CUDA_CHECK(cudaMemsetAsync(ticket, 0, 4, st));
-        onesweep_pass_kernel<RB, NT, IPT><<<tiles, NT, Cfg::SMEM, st>>>(kin, vin, kout, vout, n, shift, mask,
-                                                                         digit_base, lookback, ticket);
-        KERNEL_CHECK();
-    }
+    static size_t lookback_words(u32 n) { return (size_t)div_up_u(n, Cfg::TILE) * BINS; }
 
     static void configure() {
         static PerDeviceOnce once;
@@ -361,12 +329,16 @@ struct Sorter {
     static void pass(const u64 *kin, const u32 *vin, u64 *kout, u32 *vout, u32 n, int shift, int bits,
                      const u32 *digit_base, u64 *lookback, u32 *ticket, cudaStream_t st) {
         u32 mask = bits >= RB ? (u32)(BINS - 1) : ((1u << bits) - 1u);
-        switch (cfg_id()) {
-            case 1: launch_pass<512, 12>(kin, vin, kout, vout, n, shift, mask, digit_base, lookback, ticket, st); break;
-            case 2: launch_pass<256, 16>(kin, vin, kout, vout, n, shift, mask, digit_base, lookback, ticket, st); break;
-            case 3: launch_pass<384, 12>(kin, vin, kout, vout, n, shift, mask, digit_base, lookback, ticket, st); break;
-            default: launch_pass<256, 12>(kin, vin, kout, vout, n, shift, mask, digit_base, lookback, ticket, st); break;
-        }
+        static PerDeviceOnce once;
+        if (once.first())
+            CUDA_CHECK(cudaFuncSetAttribute(onesweep_pass_kernel<RB, PASS_NT, PASS_IPT>,
+                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
+        unsigned tiles = div_up_u(n, Cfg::TILE);
+        CUDA_CHECK(cudaMemsetAsync(lookback, 0, (size_t)tiles * BINS * 8, st));
+        CUDA_CHECK(cudaMemsetAsync(ticket, 0, 4, st));
+        onesweep_pass_kernel<RB, PASS_NT, PASS_IPT><<<tiles, PASS_NT, Cfg::SMEM, st>>>(kin, vin, kout, vout, n, shift, mask,
+                                                                                     digit_base, lookback, ticket);
+        KERNEL_CHECK();
     }
 };
 

@@ -58,11 +58,6 @@ static unsigned sm_count(int device) {
     return (unsigned)c;
 }
 
-static int env_int2(const char *name, int dflt) {
-    const char *v = getenv(name);
-    return v && *v ? atoi(v) : dflt;
-}
-
 // ---------------------------------------------------------------------------------------------
 // Planning
 // ---------------------------------------------------------------------------------------------
@@ -80,8 +75,8 @@ static u64 pow_u64(u64 x, int k) {
 // Dense keys (see DenseKey): digits are not tied to symbol boundaries, a partly used top digit is
 // accounted for when the bucket bits are chosen.
 static bool msd_make_plan_dense(u32 len, u32 nsym, int b, MsdPlan &pl, const u64 *sym_counts) {
-    const int dmax = std::max(4, std::min(10, env_int2("B200SA_MSD_DMAX", 10)));
-    const int target = std::max(1, env_int2("B200SA_MSD_AVG", 3000));
+    const int dmax = std::max(4, std::min(10, env_int("B200SA_MSD_DMAX", 10)));
+    const int target = std::max(1, env_int("B200SA_MSD_AVG", 3000));
     int log2len = 0;
     while ((1ull << log2len) < (u64)len) ++log2len;
     // bits a symbol really carries: the order-0 entropy of the text when the letter counts are known (a rare
@@ -97,12 +92,12 @@ static bool msd_make_plan_dense(u32 len, u32 nsym, int b, MsdPlan &pl, const u64
             }
         if (tot > 0.0) eff = std::min(eff, std::max(0.25, H));
     }
-    const int margin = env_int2("B200SA_KEY_MARGIN", 8);
+    const int margin = env_int("B200SA_KEY_MARGIN", 8);
     const int k_wanted = std::max(1, (int)std::ceil((log2len + margin) / eff));
     int best_K = 0;
     for (int pb = b; pb >= 0; pb -= b) {
         int K = std::min(k_wanted, 128 / b - (pb ? 1 : 0));  // a 128-bit window holds prev + K symbols
-        const int kf = env_int2("B200SA_MSD_K", 0);
+        const int kf = env_int("B200SA_MSD_K", 0);
         if (kf > 0) K = std::min(K, kf);
         for (; K >= 1; --K) {
             const u64 span = pow_u64(nsym, K);            // keys are 0 .. span - 1
@@ -112,7 +107,7 @@ static bool msd_make_plan_dense(u32 len, u32 nsym, int b, MsdPlan &pl, const u64
             int BB = 1;
             auto used = [&](int bb) { return bb >= KB ? span : ((span - 1) >> (KB - bb)) + 1; };
             while ((u64)len / used(BB) > (u64)target && BB + 1 <= 3 * dmax && BB + 1 <= KB) ++BB;
-            const int forced = env_int2("B200SA_MSD_BB", 0);
+            const int forced = env_int("B200SA_MSD_BB", 0);
             if (forced > 0) BB = std::max(1, std::min(std::min(3 * dmax, KB), forced));
             const int nl = (BB + dmax - 1) / dmax;
             int D[3] = {0, 0, 0};
@@ -154,7 +149,7 @@ bool msd_make_plan(u32 len, u32 sigma, int bits, MsdPlan &pl, const u64 *sym_cou
     {
         // alphabets that use less than 9/10 of the codes of their symbol width: dense keys
         const u32 nsym = sigma > 1 ? sigma - 1 : 1;
-        const int dk = env_int2("B200SA_DENSE_KEYS", -1);
+        const int dk = env_int("B200SA_DENSE_KEYS", -1);
         const bool sparse_alphabet = b >= 2 && nsym >= 2 && (u64)nsym * 10 <= (9ull << b);
         if (dk != 0 && b >= 2 && nsym >= 2 && (sparse_alphabet || dk > 0) && msd_make_plan_dense(len, nsym, b, pl, sym_counts)) return true;
         pl.dense = DenseKey{0, 0, 0, 0, 0};
@@ -163,12 +158,12 @@ bool msd_make_plan(u32 len, u32 sigma, int bits, MsdPlan &pl, const u64 *sym_cou
     // their b bits the leading bits of a symbol carry no information), until an average bucket
     // holds <= `target` suffixes.  At most 10 bits per level.
     int dmax = (b == 4 || b == 8) ? 8 : 10;
-    dmax = env_int2("B200SA_MSD_DMAX", dmax);
+    dmax = env_int("B200SA_MSD_DMAX", dmax);
     dmax = std::max(b, std::min(10, dmax / b * b));
-    const int target = std::max(1, env_int2("B200SA_MSD_AVG", 3000));
+    const int target = std::max(1, env_int("B200SA_MSD_AVG", 3000));
     int BB = b;
     while (((u64)len >> BB) > (u64)target && BB + b <= 3 * dmax) BB += b;
-    int forced = env_int2("B200SA_MSD_BB", 0);
+    int forced = env_int("B200SA_MSD_BB", 0);
     if (forced > 0) BB = std::max(b, std::min(3 * dmax, forced / b * b));
     const int nl = (BB + dmax - 1) / dmax;
     const int syms = BB / b;
@@ -182,7 +177,7 @@ bool msd_make_plan(u32 len, u32 sigma, int bits, MsdPlan &pl, const u64 *sym_cou
     while ((1ull << log2len) < (u64)len) ++log2len;
     double eff = std::log2((double)(sigma > 2 ? sigma - 1 : 1));
     if (eff < 0.5) eff = 0.5;
-    const int margin = env_int2("B200SA_KEY_MARGIN", 8);
+    const int margin = env_int("B200SA_KEY_MARGIN", 8);
     const int k_wanted = std::max(1, (int)std::ceil((log2len + margin) / eff));
     const int k_min = (BB + b - 1) / b;
     auto kcap = [&](int pb) {
@@ -199,7 +194,7 @@ bool msd_make_plan(u32 len, u32 sigma, int bits, MsdPlan &pl, const u64 *sym_cou
         K = kn;
         pb = 0;
     }
-    int kf = env_int2("B200SA_MSD_K", 0);
+    int kf = env_int("B200SA_MSD_K", 0);
     if (kf > 0) K = std::min(kf, kcap(pb));
     if (K < k_min) {
         K = k_min;
@@ -428,28 +423,6 @@ __device__ __forceinline__ u32 block_exclusive(u32 v, u32 *wsum) {
     return wbase + incl - v;
 }
 
-// exclusive prefix of `v` over a 512-thread block (wsum: 16 words of shared memory)
-__device__ __forceinline__ u32 block512_exclusive(u32 v, u32 *wsum) {
-    const u32 lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-    u32 incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (unsigned)o) incl += t;
-    }
-    if (lane == 31) wsum[warp] = incl;
-    __syncthreads();
-    u32 ws = lane < 16 ? wsum[lane] : 0u;
-    u32 wi = ws;
-#pragma unroll
-    for (int o = 1; o < 16; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, wi, o);
-        if (lane >= (unsigned)o) wi += t;
-    }
-    const u32 wbase = __shfl_sync(0xffffffffu, wi - ws, warp);
-    return wbase + incl - v;
-}
-
 // ---------------------------------------------------------------------------------------------
 // Partition of a level >= 2: a tile of <= P_TILE elements written by the previous level is split
 // by the digit at element bit `dshift`.  Persistent CTAs (two per SM): while a tile is being
@@ -469,9 +442,7 @@ struct PartArgs {
 static constexpr int P_INB = P_TILE + 2;  // landing buffer: the copy starts at a 16-byte boundary
 static constexpr size_t P_SMEM = (size_t)P_INB * 8 * 2 + (size_t)P_TILE * 8 + (size_t)P_MAXBINS * 4 * 2 + 32 * 4 + 2 * 8;
 
-template <int NT = P_NT>
-__global__ void __launch_bounds__(NT, 2) msd_partition_kernel(PartArgs a) {
-    constexpr int IPT = P_TILE / NT;
+__global__ void __launch_bounds__(P_NT, 2) msd_partition_kernel(PartArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     u64 *inb = (u64 *)smem_raw;                   // [2][P_INB] landing buffers
     u64 *buf = inb + 2 * P_INB;                   // [P_TILE] elements grouped by digit
@@ -512,15 +483,15 @@ __global__ void __launch_bounds__(NT, 2) msd_partition_kernel(PartArgs a) {
         const u64 *in = inb + stage * P_INB + (ds.x & 1u);
         // the other landing buffer was last read before the barrier that ended the previous iteration
         if (tid == 0 && tile + gridDim.x < ntiles) issue(tile + gridDim.x, stage ^ 1u);
-        for (u32 i = tid; i < B; i += NT) hist[i] = 0;
+        for (u32 i = tid; i < B; i += P_NT) hist[i] = 0;
         __syncthreads();
         mbar_wait_parity(&mbar[stage], (it >> 1) & 1u);
 
         // ---- digits and slots inside the tile's digit groups (arbitrary order: MSD) ----
-        u32 dsl[IPT];
+        u32 dsl[P_IPT];
 #pragma unroll
-        for (int j = 0; j < IPT; ++j) {
-            const u32 i = (u32)j * NT + tid;
+        for (int j = 0; j < P_IPT; ++j) {
+            const u32 i = (u32)j * P_NT + tid;
             dsl[j] = 0;
             if (i < count) {
                 const u32 d = (u32)(in[i] >> a.dshift) & (B - 1);
@@ -531,7 +502,7 @@ __global__ void __launch_bounds__(NT, 2) msd_partition_kernel(PartArgs a) {
 
         // ---- exclusive scan of the digit counts; reserve the runs in the child buckets ----
         {
-            constexpr int DPT = P_MAXBINS / NT;
+            constexpr int DPT = P_MAXBINS / P_NT;
             const u32 d0 = tid * DPT;
             u32 c[DPT], g[DPT];
             u32 sum = 0;
@@ -545,7 +516,7 @@ __global__ void __launch_bounds__(NT, 2) msd_partition_kernel(PartArgs a) {
                 g[q] = 0;
                 if (c[q]) g[q] = atomicAdd(&a.cursor[(size_t)parent * B + d0 + q], c[q]);
             }
-            u32 run = block_exclusive<NT>(sum, wsum);
+            u32 run = block_exclusive<P_NT>(sum, wsum);
 #pragma unroll
             for (int q = 0; q < DPT; ++q) {
                 if (d0 + q < B) {
@@ -559,15 +530,15 @@ __global__ void __launch_bounds__(NT, 2) msd_partition_kernel(PartArgs a) {
 
         // ---- group the tile by digit in shared memory ----
 #pragma unroll
-        for (int j = 0; j < IPT; ++j) {
-            const u32 i = (u32)j * NT + tid;
+        for (int j = 0; j < P_IPT; ++j) {
+            const u32 i = (u32)j * P_NT + tid;
             if (i < count) buf[hist[dsl[j] & 1023u] + (dsl[j] >> 10)] = in[i];
         }
         __syncthreads();
 
         // ---- consecutive threads write consecutive slots of a digit run ----
 #pragma unroll 4
-        for (u32 i = tid; i < count; i += NT) {
+        for (u32 i = tid; i < count; i += P_NT) {
             const u64 v = buf[i];
             a.out[gofs[(u32)(v >> a.dshift) & (B - 1)] + i] = v;
         }
@@ -630,41 +601,40 @@ __device__ __forceinline__ u64 dense_key_q(u64 H, u64 L, u64 M, int sh, const De
 }
 
 // BITS = symbol width, HAS_PREV = the preceding symbol is carried in the element (pb == BITS):
-// compile-time so that every per-symbol shift is an immediate.
-template <int BITS, bool HAS_PREV, int NT = T1_NT, int IPT = T1_IPT, int CTAS = 2, bool DENSE = false>
-__global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args a) {
-    constexpr int TILE = NT * IPT;
-    constexpr int STAGE_MAX = TILE * 8 / 64 + 5;
+// compile-time so that every per-symbol shift is an immediate.  DENSE = the key is a.dense's
+// base-nsym number of the K symbols.
+template <int BITS, bool HAS_PREV, bool DENSE>
+__global__ void __launch_bounds__(T1_NT, 2) msd_partition_text_kernel(Text1Args a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    u64 *buf = (u64 *)smem_raw;                   // [TILE] elements grouped by digit
-    u64 *stage = buf + TILE;                   // [STAGE_MAX] packed text of the tile (one word of lead-in)
-    u32 *hist = (u32 *)(stage + STAGE_MAX);    // [MAXBINS] counts, then tile-local offsets
+    u64 *buf = (u64 *)smem_raw;                   // [T1_TILE] elements grouped by digit
+    u64 *stage = buf + T1_TILE;                   // [T1_STAGE_MAX] packed text of the tile (one word of lead-in)
+    u32 *hist = (u32 *)(stage + T1_STAGE_MAX);    // [MAXBINS] counts, then tile-local offsets
     u32 *gofs = hist + MSD_MAXBINS;               // [MAXBINS] global slot of the digit's run minus its tile offset
     u32 *wsum = gofs + MSD_MAXBINS;               // [32]
-    static_assert(TILE <= (1 << 14) && MSD_MAXBINS <= (1 << 10), "tile-local low word: 14 bits of position, 10 of digit");
+    static_assert(T1_TILE <= (1 << 14) && MSD_MAXBINS <= (1 << 10), "tile-local low word: 14 bits of position, 10 of digit");
 
     constexpr int b = BITS;
     constexpr u32 lead = HAS_PREV ? (u32)BITS : 0u;
     const u32 tid = threadIdx.x;
     const u32 B = 1u << a.D;
-    const u64 begin = (u64)blockIdx.x * TILE;
-    const u32 count = (u32)min((u64)TILE, (u64)a.len - begin);
+    const u64 begin = (u64)blockIdx.x * T1_TILE;
+    const u32 count = (u32)min((u64)T1_TILE, (u64)a.len - begin);
 
     // ---- stage the tile's text: word k of `stage` is packed[begin*b/64 - 1 + k] ----
     {
-        constexpr u32 nstage = (u32)(TILE / 64) * b + 5;
+        constexpr u32 nstage = (u32)(T1_TILE / 64) * b + 5;
         const u64 w0 = begin * (u64)b / 64;
-        for (u32 k = tid; k < nstage; k += NT) {
+        for (u32 k = tid; k < nstage; k += T1_NT) {
             const u64 w = w0 + k;  // index + 1
             stage[k] = (w >= 1 && w - 1 < a.nwords) ? a.packed[w - 1] : 0ull;
         }
-        for (u32 i = tid; i < B; i += NT) hist[i] = 0;
+        for (u32 i = tid; i < B; i += T1_NT) hist[i] = 0;
     }
     __syncthreads();
 
     // bit offset (inside `stage`) of the window of the thread's first position: it starts at the
     // preceding symbol when that symbol is carried in the element, else at the position itself
-    const u32 i0 = tid * IPT;
+    const u32 i0 = tid * T1_IPT;
     const u32 off0 = 64u + i0 * (u32)b - lead;
     const int kshift = 64 - a.KB;
     const int dsh = 32 - a.D;                           // digit = leading D bits of the key
@@ -673,9 +643,9 @@ __global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args 
     // ---- digits and slots inside the tile's digit groups (arbitrary order: MSD) ----
     u64 dkey = 0;
     const u32 dK = a.dense.Khi + a.dense.Klo;
-    u32 ds[IPT];
+    u32 ds[T1_IPT];
 #pragma unroll
-    for (int g = 0; g < IPT / 8; ++g) {
+    for (int g = 0; g < T1_IPT / 8; ++g) {
         u64 H, L, M = 0;
         if (DENSE) stage_window3(stage, off0 + (u32)(8 * g * b), H, L, M);
         else stage_window(stage, off0 + (u32)(8 * g * b), H, L);
@@ -701,9 +671,9 @@ __global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args 
     __syncthreads();
 
     // ---- exclusive scan of the digit counts; reserve the runs in the level-1 buckets ----
-    u32 gsub[MSD_MAXBINS / NT], gres[MSD_MAXBINS / NT];
+    u32 gsub[MSD_MAXBINS / T1_NT], gres[MSD_MAXBINS / T1_NT];
     {
-        constexpr int DPT = MSD_MAXBINS / NT;
+        constexpr int DPT = MSD_MAXBINS / T1_NT;
         const u32 d0 = tid * DPT;
         u32 c[DPT], g[DPT];
         u32 sum = 0;
@@ -717,7 +687,7 @@ __global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args 
             g[q] = 0;
             if (c[q]) g[q] = atomicAdd(&a.cursor[d0 + q], c[q]);
         }
-        u32 run = block_exclusive<NT>(sum, wsum);
+        u32 run = block_exclusive<T1_NT>(sum, wsum);
 #pragma unroll
         for (int q = 0; q < DPT; ++q) {
             if (d0 + q < B) hist[d0 + q] = run;
@@ -731,7 +701,7 @@ __global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args 
     // ---- form the elements (again from the staged text) and group the tile by digit.  An
     // element is two 32-bit words: [rest of key | preceding symbol] and the suffix start ----
 #pragma unroll
-    for (int g = 0; g < IPT / 8; ++g) {
+    for (int g = 0; g < T1_IPT / 8; ++g) {
         u64 H, L, M = 0;
         if (DENSE) stage_window3(stage, off0 + (u32)(8 * g * b), H, L, M);
         else stage_window(stage, off0 + (u32)(8 * g * b), H, L);
@@ -759,9 +729,9 @@ __global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args 
     // the reserved global slots are first needed now: the round trip of the reservation (a global
     // atomic per digit) ran behind the grouping above
     {
-        const u32 d0 = tid * (MSD_MAXBINS / NT);
+        const u32 d0 = tid * (MSD_MAXBINS / T1_NT);
 #pragma unroll
-        for (int q = 0; q < MSD_MAXBINS / NT; ++q)
+        for (int q = 0; q < MSD_MAXBINS / T1_NT; ++q)
             if (d0 + q < B) gofs[d0 + q] = gres[q] - gsub[q];
     }
     __syncthreads();
@@ -769,7 +739,7 @@ __global__ void __launch_bounds__(NT, CTAS) msd_partition_text_kernel(Text1Args 
     // ---- consecutive threads write consecutive slots of a digit run ----
     const u32 begin32 = (u32)begin;
 #pragma unroll 4
-    for (u32 i = tid; i < count; i += NT) {
+    for (u32 i = tid; i < count; i += T1_NT) {
         const u64 v = buf[i];
         const u32 lo = (u32)v;
         a.out[gofs[lo >> 14] + i] = (v & 0xffffffff00000000ull) | (u64)(begin32 + (lo & 16383u));
@@ -1591,17 +1561,13 @@ static void launch_hist_text(const DeviceIndex &ix, u64 nwords_data, int D, u32 
     KERNEL_CHECK();
 }
 
-template <int NT, int IPT>
-static constexpr size_t t1_smem() {
-    return (size_t)NT * IPT * 8 + (size_t)MSD_MAXBINS * 4 * 2 + (size_t)(NT * IPT * 8 / 64 + 5) * 8 + 32 * 4;
-}
-template <int NT, int IPT, int CTAS>
-static void launch_t1_variant(const Text1Args &ta, u32 len, cudaStream_t st) {
+template <int BITS, bool HAS_PREV, bool DENSE>
+static void launch_part_text(const Text1Args &ta, int device, cudaStream_t st) {
     static PerDeviceOnce once;
-    if (once.first())
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<2, true, NT, IPT, CTAS>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t1_smem<NT, IPT>()));
-    msd_partition_text_kernel<2, true, NT, IPT, CTAS><<<div_up_u(len, NT * IPT), NT, t1_smem<NT, IPT>(), st>>>(ta);
+    if (once.first(device))
+        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<BITS, HAS_PREV, DENSE>,
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
+    msd_partition_text_kernel<BITS, HAS_PREV, DENSE><<<div_up_u(ta.len, T1_TILE), T1_NT, T1_SMEM, st>>>(ta);
 }
 
 bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
@@ -1613,22 +1579,7 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
 
     static PerDeviceOnce once;
     if (once.first(ix.device)) {
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<2, true, T1_NT, T1_IPT, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<4, true, T1_NT, T1_IPT, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<8, true, T1_NT, T1_IPT, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<2, false, T1_NT, T1_IPT, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<4, false, T1_NT, T1_IPT, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_text_kernel<8, false, T1_NT, T1_IPT, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T1_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P_SMEM));
-        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_kernel<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P_SMEM));
+        CUDA_CHECK(cudaFuncSetAttribute(msd_partition_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P_SMEM));
         CUDA_CHECK(cudaFuncSetAttribute(msd_local_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L3_SMEM));
         CUDA_CHECK(cudaFuncSetAttribute(msd_local_sort_robust_kernel<RB_N, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RB_SMEM));
         CUDA_CHECK(cudaFuncSetAttribute(msd_local_sort_robust_kernel<RB_N_SMALL, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rb_smem<RB_N_SMALL>()));
@@ -1668,20 +1619,20 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
     auto decide = [&](const u32 *final_start, u64 nbuckets) -> int {
         u32 maxbucket = 0;
         read_back(&maxbucket, d_misc, 4, st);
-        if (env_int2("B200SA_DEBUG_PLAN", 0))
+        if (env_int("B200SA_DEBUG_PLAN", 0))
             fprintf(stderr, "[b200sa] round-0 plan: levels %d D %d/%d/%d BB %d K %d KB %d pb %d R %d dense %u (%u+%u, powlo %u) max bucket %u\n",
                     pl.nlevels, pl.D[0], pl.D[1], pl.D[2], pl.BB, pl.K, pl.KB, pl.pb, pl.R, pl.dense.nsym, pl.dense.Khi,
                     pl.dense.Klo, pl.dense.powlo, maxbucket);
         if (maxbucket <= (u32)L3_MAXB) return GO;
-        if (env_int2("B200SA_MSD_NO_OVERSIZE", 0)) return FALLBACK;
+        if (env_int("B200SA_MSD_NO_OVERSIZE", 0)) return FALLBACK;
         CUDA_CHECK(cudaMemsetAsync(d_over, 0, 16, st));
         msd_count_oversize_kernel<<<div_up_u(nbuckets, 256), 256, 0, st>>>(final_start, nbuckets, (u32)L3_MAXB, d_over);
         KERNEL_CHECK();
         unsigned long long h[2];
         read_back(h, d_over, 16, st);
-        if (env_int2("B200SA_DEBUG_PLAN", 0)) fprintf(stderr, "[b200sa] oversize buckets: %llu with %llu suffixes\n", h[0], h[1]);
-        const int more_frac = std::max(1, env_int2("B200SA_MSD_MORE_FRAC", 64));
-        const int bbmax = env_int2("B200SA_MSD_BBMAX", 26);
+        if (env_int("B200SA_DEBUG_PLAN", 0)) fprintf(stderr, "[b200sa] oversize buckets: %llu with %llu suffixes\n", h[0], h[1]);
+        const int more_frac = std::max(1, env_int("B200SA_MSD_MORE_FRAC", 64));
+        const int bbmax = env_int("B200SA_MSD_BBMAX", 26);
         const int bq = pl.dense.nsym ? 1 : b;  // (dense keys: digits are not tied to symbol boundaries)
         int room = std::min(std::min(pl.dmax, pl.R), bbmax - pl.BB) / bq * bq;
         if (h[1] > (unsigned long long)len / (unsigned)more_frac && pl.nlevels < 3 && room >= bq) {
@@ -1692,7 +1643,7 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
             CUDA_CHECK(cudaMemsetAsync(d_misc, 0, 4, st));
             return MORE;
         }
-        const int frac = std::max(1, env_int2("B200SA_MSD_OVER_FRAC", 8));
+        const int frac = std::max(1, env_int("B200SA_MSD_OVER_FRAC", 8));
         if (h[1] > (unsigned long long)len / (unsigned)frac) return FALLBACK;
         if (pl.dense.nsym) {
             // what the members of an oversize bucket of dense keys are known to share
@@ -1701,7 +1652,7 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
                                                                            (u32)pl.K, pow_u64(pl.dense.nsym, pl.K), d_misc + 2);
             KERNEL_CHECK();
             read_back(&dense_d0, d_misc + 2, 4, st);
-            if (env_int2("B200SA_DEBUG_PLAN", 0)) fprintf(stderr, "[b200sa] dense keys: oversize buckets share %u symbols\n", dense_d0);
+            if (env_int("B200SA_DEBUG_PLAN", 0)) fprintf(stderr, "[b200sa] dense keys: oversize buckets share %u symbols\n", dense_d0);
             // (a bucket that straddles a change of a leading symbol shares little: rare)
             if (dense_d0 < (u32)std::max(2, pl.K / 4) || dense_d0 > 32) return FALLBACK;
         }
@@ -1728,7 +1679,7 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
         case 4: launch_hist_text<4>(ix, nwords_data, pl.D[0], cursor[0], st, pl); break;
         default: launch_hist_text<8>(ix, nwords_data, pl.D[0], cursor[0], st, pl); break;
     }
-    if (pl.dense.nsym && !env_int2("B200SA_MSD_BB", 0)) {
+    if (pl.dense.nsym && !env_int("B200SA_MSD_BB", 0)) {
         // Dense keys spread evenly when the letters are equally likely.  The level-1 histogram tells how far the text
         // is from that (a rare letter -- N in DNA --, skewed amino-acid frequencies): with H1 bits of entropy in its
         // D1 leading key bits, a key bit carries h = (H1 - log2 fill) / D1 bits (fill: the used part of the top
@@ -1762,7 +1713,7 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
             pl.BB = BBn;
             pl.R = pl.KB - BBn;
         }
-        if (env_int2("B200SA_DEBUG_PLAN", 0))
+        if (env_int("B200SA_DEBUG_PLAN", 0))
             fprintf(stderr, "[b200sa] dense keys: level-1 entropy %.2f of %d bits, %.3f per key bit -> %d bucket bits\n", H1, pl.D[0], h, pl.BB);
     }
     {
@@ -1786,38 +1737,22 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
         ta.rest_shift = 32 + pl.pb;
         ta.cursor = cursor[0];
         t = ix.timer.begin("msd_part1", (double)len * (8.0 + b / 8.0));
-        const unsigned g1 = div_up_u(len, T1_TILE);
         ta.dense = pl.dense;
-        const int which = pl.dense.nsym ? 100 + (b == 2 ? 0 : b == 4 ? 1 : 2) * 2 + (pl.pb ? 1 : 0)
-                                        : (b == 1 ? 0 : b == 2 ? 1 : b == 4 ? 2 : 3) * 2 + (pl.pb ? 1 : 0);
-        switch (which) {
-            case 100: msd_partition_text_kernel<2, false, T1_NT, T1_IPT, 2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 101: msd_partition_text_kernel<2, true, T1_NT, T1_IPT, 2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 102: msd_partition_text_kernel<4, false, T1_NT, T1_IPT, 2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 103: msd_partition_text_kernel<4, true, T1_NT, T1_IPT, 2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 104: msd_partition_text_kernel<8, false, T1_NT, T1_IPT, 2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 105: msd_partition_text_kernel<8, true, T1_NT, T1_IPT, 2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 0: msd_partition_text_kernel<1, false><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 1: msd_partition_text_kernel<1, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 2: msd_partition_text_kernel<2, false><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 3: {
-                static const int variant = env_int2("B200SA_T1_VARIANT", 0);
-                switch (variant) {
-                    case 1: launch_t1_variant<512, 8, 3>(ta, len, st); break;
-                    case 2: launch_t1_variant<256, 16, 4>(ta, len, st); break;
-                    case 3: launch_t1_variant<1024, 8, 2>(ta, len, st); break;
-                    case 4: launch_t1_variant<512, 8, 4>(ta, len, st); break;
-                    case 5: launch_t1_variant<256, 8, 7>(ta, len, st); break;
-                    case 6: launch_t1_variant<1024, 16, 1>(ta, len, st); break;
-                    case 7: launch_t1_variant<512, 16, 3>(ta, len, st); break;
-                    default: msd_partition_text_kernel<2, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-                }
-                break;
+        const int dev = ix.device;
+        const bool prev = pl.pb != 0;
+        if (pl.dense.nsym) {  // (dense keys: 2, 4 or 8 bits per symbol)
+            switch (b) {
+                case 2: prev ? launch_part_text<2, true, true>(ta, dev, st) : launch_part_text<2, false, true>(ta, dev, st); break;
+                case 4: prev ? launch_part_text<4, true, true>(ta, dev, st) : launch_part_text<4, false, true>(ta, dev, st); break;
+                default: prev ? launch_part_text<8, true, true>(ta, dev, st) : launch_part_text<8, false, true>(ta, dev, st); break;
             }
-            case 4: msd_partition_text_kernel<4, false><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 5: msd_partition_text_kernel<4, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            case 6: msd_partition_text_kernel<8, false><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
-            default: msd_partition_text_kernel<8, true><<<g1, T1_NT, T1_SMEM, st>>>(ta); break;
+        } else {
+            switch (b) {
+                case 1: prev ? launch_part_text<1, true, false>(ta, dev, st) : launch_part_text<1, false, false>(ta, dev, st); break;
+                case 2: prev ? launch_part_text<2, true, false>(ta, dev, st) : launch_part_text<2, false, false>(ta, dev, st); break;
+                case 4: prev ? launch_part_text<4, true, false>(ta, dev, st) : launch_part_text<4, false, false>(ta, dev, st); break;
+                default: prev ? launch_part_text<8, true, false>(ta, dev, st) : launch_part_text<8, false, false>(ta, dev, st); break;
+            }
         }
         KERNEL_CHECK();
         ix.timer.end(t);
@@ -1856,9 +1791,7 @@ bool round0_msd(DeviceIndex &ix, bool want_bwt, Round0Msd &r) {
         pa.cursor = cursor[l];
         pa.desc = desc; pa.d_ntiles = d_misc + 1;
         t = ix.timer.begin("msd_part", (double)len * 16.0);
-        static const int p_variant = env_int2("B200SA_P_VARIANT", 0);
-        if (p_variant == 1) msd_partition_kernel<1024><<<std::min(grid, 2u * sm_count(ix.device)), 1024, P_SMEM, st>>>(pa);
-        else msd_partition_kernel<512><<<std::min(grid, 2u * sm_count(ix.device)), 512, P_SMEM, st>>>(pa);
+        msd_partition_kernel<<<std::min(grid, 2u * sm_count(ix.device)), P_NT, P_SMEM, st>>>(pa);
         KERNEL_CHECK();
         ix.timer.end(t);
         std::swap(cur, other);

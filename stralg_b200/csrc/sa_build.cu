@@ -2016,11 +2016,6 @@ __global__ void __launch_bounds__(256) count_heads_kernel(const u32 *__restrict_
 // ---------------------------------------------------------------------------------------------
 // Host orchestration
 // ---------------------------------------------------------------------------------------------
-static int env_int(const char *name, int dflt) {
-    const char *v = getenv(name);
-    return v && *v ? atoi(v) : dflt;
-}
-
 size_t build_workspace_estimate(u32 len, int bits) {
     // packed text + round-0 keys (2 x 8) + one value buffer + ranks + look-back + bitmaps, with slack
     size_t l = len;

@@ -1,6 +1,6 @@
 """A/B timing of build-stage variants selected by environment variables that the library reads per
 build (not cached): alternates the settings inside one process and prints per-stage medians.
-    python tools/ab_probe.py B200SA_P_VARIANT 0,2 msd_part [n] [reps]"""
+    python tools/ab_probe.py B200SA_MSD_AVG 3000,1500 msd_part [n] [reps]"""
 import ctypes as C
 import os
 import statistics

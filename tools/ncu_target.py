@@ -54,7 +54,7 @@ else:
             fn()
         e1.record()
         torch.cuda.synchronize()
-        print(f"{name} kernel: {e0.elapsed_time(e1) / 5:.3f} ms for {reads_n} reads (L2_FETCH={os.environ.get('B200SA_L2_FETCH')})")
+        print(f"{name} kernel: {e0.elapsed_time(e1) / 5:.3f} ms for {reads_n} reads")
     idx.close()
 torch.cuda.synchronize()
 print("done", what, n)

@@ -27,9 +27,7 @@ __global__ void __launch_bounds__(256) bwt_gather_kernel(const u32 *__restrict__
             if (s == 0) {
                 *primary = (u32)(r0 + q);
             } else {
-                u64 bitpos = (u64)(s - 1) * bits;
-                u64 w = packed[bitpos >> 6];
-                code = (u32)((w >> (64 - bits - (unsigned)(bitpos & 63))) & ((1u << bits) - 1u)) + 1u;
+                code = sym_at(packed, s - 1, bits) + 1u;
             }
         }
         out |= code << (8 * q);

@@ -264,6 +264,12 @@ struct PerDeviceOnce {
 // for it every time it looks at a counter.  Defined in api.cu.
 void read_back(void *dst, const void *dev_src, size_t bytes, cudaStream_t st);
 
+// packed symbol t (its code - 1) of the big-endian packed text
+__device__ __forceinline__ u32 sym_at(const u64 *__restrict__ packed, u32 t, int bits) {
+    u64 bitpos = (u64)t * bits;
+    return (u32)((packed[bitpos >> 6] >> (64 - bits - (unsigned)(bitpos & 63))) & ((1u << bits) - 1u));
+}
+
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31u; }
 __device__ __forceinline__ unsigned lanemask_lt() {
     unsigned m;

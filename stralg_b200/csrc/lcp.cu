@@ -29,11 +29,6 @@ __device__ __forceinline__ u64 lcp_window(const u64 *__restrict__ packed, u64 sy
     return (hi << o) | (packed[wi + 1] >> (64 - o));
 }
 
-__device__ __forceinline__ u32 sym_at(const u64 *__restrict__ packed, u32 t, int bits) {
-    u64 bitpos = (u64)t * bits;
-    return (u32)((packed[bitpos >> 6] >> (64 - bits - (unsigned)(bitpos & 63))) & ((1u << bits) - 1u));
-}
-
 __global__ void __launch_bounds__(256) phi_kernel(const u32 *__restrict__ sa, u32 len, u32 *__restrict__ phi) {
     u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= len) return;

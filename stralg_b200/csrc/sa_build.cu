@@ -2093,6 +2093,12 @@ static void scatter_active(const u8 *bits, const u32 *vals, const u32 *grp_in, u
                                                                                    out, grp_out);
     KERNEL_CHECK();
 }
+static void scatter_pairs(const u8 *bits, const u64 *keys, const u32 *vals, u32 m, const u32 *tile_offsets, u64 *kout,
+                          u32 *vout, cudaStream_t st) {
+    const u32 sub = compaction_sub(m);
+    scatter_pairs_kernel<<<div_up_u(m, (u64)CP_TILE * sub), CP_NT, 0, st>>>(bits, keys, vals, m, sub, tile_offsets, kout, vout);
+    KERNEL_CHECK();
+}
 
 // LSD round 0: rows that are not singletons, from the head bitmap (one thread per 64 rows)
 __global__ void __launch_bounds__(256) heads_to_actbits_kernel(const u8 *__restrict__ headbits, u32 m,
@@ -2104,12 +2110,8 @@ __global__ void __launch_bounds__(256) heads_to_actbits_kernel(const u8 *__restr
 // BWT rows (stralg/bwt.c:13-20) of the rows that were active after round 0, from the final suffix
 // array: the doubling rounds over large active sets do not maintain them (one gather per moved row and
 // round); their rows are exactly the rows whose bit is set here.
-// dense bitmaps (periodic texts: every row): one thread per row
-__global__ void __launch_bounds__(256) bwt_fix_rows_kernel(const u32 *__restrict__ actbits, const u32 *__restrict__ sa, u32 len,
-                                                           const u64 *__restrict__ packed, int bits, u8 *__restrict__ bwt,
-                                                           u32 *__restrict__ primary) {
-    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= len || !((actbits[r >> 5] >> (r & 31u)) & 1u)) return;
+__device__ __forceinline__ void bwt_fix_row(u64 r, const u32 *__restrict__ sa, const u64 *__restrict__ packed, int bits,
+                                            u8 *__restrict__ bwt, u32 *__restrict__ primary) {
     const u32 s = sa[r];
     if (s == 0) {
         bwt[r] = 0;
@@ -2119,6 +2121,15 @@ __global__ void __launch_bounds__(256) bwt_fix_rows_kernel(const u32 *__restrict
         const u64 w = packed[bitpos >> 6];
         bwt[r] = (u8)(((w >> (64 - bits - (unsigned)(bitpos & 63))) & ((1u << bits) - 1u)) + 1u);
     }
+}
+
+// dense bitmaps (periodic texts: every row): one thread per row
+__global__ void __launch_bounds__(256) bwt_fix_rows_kernel(const u32 *__restrict__ actbits, const u32 *__restrict__ sa, u32 len,
+                                                           const u64 *__restrict__ packed, int bits, u8 *__restrict__ bwt,
+                                                           u32 *__restrict__ primary) {
+    const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= len || !((actbits[r >> 5] >> (r & 31u)) & 1u)) return;
+    bwt_fix_row(r, sa, packed, bits, bwt, primary);
 }
 
 // sparse bitmaps (one thread per 32 rows: few rows are left once the pair path has taken its rows out)
@@ -2133,15 +2144,7 @@ __global__ void __launch_bounds__(256) bwt_fix_kernel(const u32 *__restrict__ ac
         w &= w - 1u;
         const u64 r = wi * 32 + bit;
         if (r >= len) break;
-        const u32 s = sa[r];
-        if (s == 0) {
-            bwt[r] = 0;
-            *primary = (u32)r;
-        } else {
-            const u64 bitpos = (u64)(s - 1) * bits;
-            const u64 pw = packed[bitpos >> 6];
-            bwt[r] = (u8)(((pw >> (64 - bits - (unsigned)(bitpos & 63))) & ((1u << bits) - 1u)) + 1u);
-        }
+        bwt_fix_row(r, sa, packed, bits, bwt, primary);
     }
 }
 
@@ -2271,18 +2274,825 @@ __global__ void __launch_bounds__(256) bytes_to_bits_kernel(const u8 *__restrict
     bits64[w] = v;
 }
 
+// environment knobs of the build (DESIGN.md §10), read once at its start
+struct BuildKnobs {
+    int radix_bits, key_margin;
+    bool passes0_set;  // LSD round 0 makes `passes0` passes (clamped), not the number computed from the text
+    int passes0;
+    int pairs;         // 0: off, 1: on large active sets, 2: on lists of any size (tests)
+    bool ext_tiebreak, chain, small_path, pivot;
+    bool pivot_force;  // (tests: every round, whatever it finds)
+    int bwt_round_frac, chain_min_frac, chain_use_frac, dense_factor;
+    u32 pivot_min;
+};
+
+static BuildKnobs read_build_knobs() {
+    BuildKnobs k;
+    k.radix_bits = env_int("B200SA_RADIX_BITS", 8);
+    k.key_margin = env_int("B200SA_KEY_MARGIN", 8);
+    const char *p0 = getenv("B200SA_PASSES0");
+    k.passes0_set = p0 && *p0;
+    k.passes0 = k.passes0_set ? atoi(p0) : 0;
+    k.pairs = env_int("B200SA_PAIRS", 1);
+    k.ext_tiebreak = env_int("B200SA_NO_EXT_TIEBREAK", 0) == 0;
+    k.chain = env_int("B200SA_CHAIN", 1) != 0;
+    k.small_path = env_int("B200SA_SMALL_PATH", 1) != 0;
+    k.pivot = env_int("B200SA_PIVOT", 1) != 0;
+    k.pivot_force = env_int("B200SA_PIVOT_FORCE", 0) != 0;
+    k.bwt_round_frac = std::max(1, env_int("B200SA_BWT_ROUND_FRAC", 32));
+    k.chain_min_frac = std::max(1, env_int("B200SA_CHAIN_MIN_FRAC", 64));
+    k.chain_use_frac = std::max(1, env_int("B200SA_CHAIN_USE_FRAC", 2));
+    k.dense_factor = std::max(1, env_int("B200SA_DENSE_FACTOR", 12));
+    k.pivot_min = (u32)std::max(2, env_int("B200SA_PIVOT_MIN", 1 << 16));
+    return k;
+}
+
+// what the stages of one build share
+struct BuildCtx {
+    DeviceIndex &ix;
+    const BuildKnobs &kn;
+    Arena &ar;
+    cudaStream_t st;
+    bool want_bwt;
+    u32 n, len;
+    int b;                   // bits per packed symbol
+    int log2len, lo_bits, key_bits;  // doubling rounds: bits of the rank half of a key, bits of a key
+    u32 *sa, *d_primary;
+    // workspace; actbits: bit per row, active after round 0
+    u64 *keysA, *keysB, *lookback;
+    u32 *valsV, *rank, *actbits, *hist, *uniform, *ticket, *tile_counts, *d_lazy;
+    u8 *headbits;
+    unsigned long long *d_total;
+    u8 *bwt_rows = nullptr;     // BWT output while the sort writes its rows as it goes
+    bool need_bwt_fix = false;  // a path moved rows without writing their BWT rows
+
+    BuildCtx(DeviceIndex &ix_, const BuildKnobs &kn_, bool want_bwt_, u32 *d_primary_)
+        : ix(ix_), kn(kn_), ar(*ix_.arena), st(ix_.stream), want_bwt(want_bwt_), n(ix_.n), len(ix_.len), b(ix_.pk.bits),
+          sa(ix_.sa.ptr), d_primary(d_primary_) {
+        log2len = 0;
+        while ((1ull << log2len) < (u64)len) ++log2len;
+        lo_bits = std::max(1, log2len);
+        key_bits = std::min(64, 2 * lo_bits);
+    }
+};
+
+// the active list: suffixes whose key is shared with another suffix, in suffix-array order, each with the first row of
+// its group; and what round 0 tells the rounds about it
+struct ActiveList {
+    bool bucketed = false;            // round 0 was the bucket sort (else the LSD passes)
+    u32 m = 0;
+    u32 *act = nullptr, *grp = nullptr;
+    int K = 0;                        // symbols in a round-0 key
+    u32 depth0 = 0;                   // symbols every active group shares after round 0 (0: K)
+    const u32 *short_rank = nullptr;  // bucketed round 0: ranks of the short suffixes of oversize buckets
+    bool bwt_in_sort = true;          // BWT rows ride along with the sort (else: gathered from the final SA)
+    u64 *rk_free[2] = {nullptr, nullptr};  // large buffers that are dead after round 0 (round keys go there)
+    LazyRank lr{};
+};
+
+// bucketed round 0: the list rank[] is scattered from for the suffixes active after it (round0_msd.cu writes no
+// ranks); marked: rank[] has been set to "not materialised" (and holds the ranks of decided suffixes)
+struct RankSource {
+    const u32 *act, *row;
+    u32 m;
+    bool marked;
+};
+
+// the tie-break's permuted list with a "stays" byte per element, when the pair path follows it and one compaction
+// serves both (act == nullptr: none); nres elements leave it
+struct PendingList {
+    u32 *act = nullptr, *row = nullptr;
+    u8 *keep = nullptr;
+    u32 nres = 0;
+};
+
+// rank_kernel's arguments for a doubling round ((group, rank) keys, moved suffixes stored into the SA), or for round 0
+// (K0 > 0: keys of K0 symbols under `keymask`, the preceding symbol at `prev_shift`, the SA already in place)
+static RankArgs rank_args(const BuildCtx &c, const u64 *keys, const u32 *vals, u32 m, u32 *newgrp, u8 *headbits, u8 *bwt,
+                          int always_write, int K0 = 0, u64 keymask = ~0ull, int prev_shift = 0) {
+    RankArgs a{};
+    a.keys = keys; a.vals = vals; a.m = m; a.gs = K0 ? 64 : c.lo_bits; a.keymask = keymask; a.K0 = K0; a.n = c.n;
+    a.rank = c.rank; a.newgrp = newgrp; a.scatter_all = 0; a.sa_out = K0 ? nullptr : c.sa; a.headbits = headbits;
+    a.bwt = bwt; a.prev_shift = prev_shift; a.packed = c.ix.packed; a.bits = c.b; a.primary = c.d_primary;
+    a.always_write = always_write;
+    return a;
+}
+
+// One list of a doubling round: radix sort of its (group, rank) keys over the digits that are not uniform, then new
+// ranks, the head bitmap and the new group of every element by sorted index (`newgrp`).  (keys, vals) hold the list,
+// (keys_other, vals_other) are the other buffer pair; returns the value buffer that holds the sorted list.
 template <int RB>
-static void build_sa_impl(DeviceIndex &ix, bool want_bwt) {
+static u32 *sort_and_rank(BuildCtx &c, u64 *keys, u32 *vals, u64 *keys_other, u32 *vals_other, u32 m, u32 *newgrp,
+                          u8 *headbits, u8 *bwt, int always_write) {
+    typedef rs::Sorter<RB> S;
+    const int npass = (c.key_bits + RB - 1) / RB;
+    u32 huniform[8];
+    int t = c.ix.timer.begin("round_hist", (double)m * 8.0);
+    S::histogram(keys, m, 0, c.key_bits, npass, c.hist, c.st);
+    S::scan(c.hist, m, npass, c.uniform, c.st);
+    read_back(huniform, c.uniform, (size_t)npass * 4, c.st);
+    c.ix.timer.end(t);
+    for (int p = 0; p < npass; ++p) {
+        if (huniform[p]) continue;
+        const int bits_here = std::min(RB, c.key_bits - p * RB);
+        t = c.ix.timer.begin("radix_pass", (double)m * 24.0);
+        S::pass(keys, vals, keys_other, vals_other, m, p * RB, bits_here, c.hist + (size_t)p * (1 << RB), c.lookback,
+                c.ticket, c.st);
+        c.ix.timer.end(t);
+        c.ix.stats.passes_elems += m;
+        std::swap(keys, keys_other);
+        std::swap(vals, vals_other);
+    }
+    t = c.ix.timer.begin("round_rank", (double)m * 20.0);
+    CUDA_CHECK(cudaMemsetAsync(headbits, 0, (((size_t)m + 63) / 64 + 2) * 8, c.st));
+    rank_kernel<<<div_up_u(m, RK_TILE), RK_NT, 0, c.st>>>(rank_args(c, keys, vals, m, newgrp, headbits, bwt, always_write));
+    KERNEL_CHECK();
+    c.ix.timer.end(t);
+    return vals;
+}
+
+// the list elements whose keep byte is set, (act, row) -> (act_out, row_out) in list order; returns their number
+static u32 compact_kept(BuildCtx &c, const u8 *keep8, u32 m, const u32 *act, const u32 *row, u32 *act_out, u32 *row_out) {
+    const u64 kw = ((u64)m + 63) / 64;
+    CUDA_CHECK(cudaMemsetAsync(c.headbits, 0, (kw + 2) * 8, c.st));
+    bytes_to_bits_kernel<<<div_up_u(kw, 256), 256, 0, c.st>>>(keep8, m, (u64 *)c.headbits, kw);
+    KERNEL_CHECK();
+    const u32 m2 = count_active<true>(c.headbits, m, c.tile_counts, c.d_total, c.st);
+    if (m2) scatter_active<true>(c.headbits, act, row, m, c.tile_counts, act_out, row_out, c.st);
+    return m2;
+}
+
+// ---- round 0, preferred: MSD bucket sort of 8-byte elements (round0_msd.cu); false when it does not apply ----
+static bool round0_bucketed(BuildCtx &c, ActiveList &L) {
+    DeviceIndex &ix = c.ix;
+    Round0Msd r0{};
+    if (!msd_make_plan(c.len, ix.sigma, c.b, r0.plan, ix.sym_counts_host)) return false;
+    Arena::Mark mk = c.ar.mark();
+    r0.bufA = c.keysA; r0.bufB = c.keysB; r0.actbits = c.actbits;
+    r0.d_primary = c.d_primary;
+    if (!round0_msd(ix, c.want_bwt, r0)) {
+        c.ar.release_to(mk);
+        return false;
+    }
+    L.bucketed = true;
+    L.K = r0.plan.K;
+    L.bwt_in_sort = r0.bwt_written;
+    L.lr.keys0 = nullptr; L.lr.bstart = r0.bucket_start; L.lr.BB = r0.plan.BB; L.lr.K = L.K;
+    L.lr.kb = r0.plan.KB; L.lr.dense = r0.plan.dense;
+    ix.stats.dense_keys = r0.plan.dense.nsym;
+    L.lr.keymask = (L.K * c.b >= 64) ? ~0ull : ((1ull << (L.K * c.b)) - 1ull);
+    ix.stats.k0 = L.K;
+    ix.stats.radix_bits = r0.plan.D[0];
+    ix.stats.passes0 = r0.plan.nlevels;
+    ix.stats.round0_mode = 1;
+    ix.stats.bucket_bits = r0.plan.BB;
+    ix.stats.passes_elems = (u64)c.len * r0.plan.nlevels;
+    ix.stats.shallow_buckets = r0.shallow_buckets;
+    ix.stats.shallow_elems = r0.shallow_buckets ? r0.shallow_elems : 0;
+    L.depth0 = r0.depth0;
+    L.short_rank = r0.short_rank;
+    // the active rows, in row order, with their group heads
+    int t = ix.timer.begin("compact0", (double)c.len * 0.125);
+    L.m = count_active<true>((const u8 *)c.actbits, c.len, c.tile_counts, c.d_total, c.st);
+    if (L.m) {
+        L.grp = c.ar.get<u32>(L.m);
+        scatter_active<true>((const u8 *)c.actbits, c.sa, r0.grow, c.len, c.tile_counts, L.act, L.grp, c.st);
+    }
+    ix.timer.end(t);
+    L.rk_free[0] = c.keysA;
+    L.rk_free[1] = c.keysB;
+    return true;
+}
+
+// ---- round 0, general: LSD radix passes over (u64 key, u32 suffix) pairs ----
+template <int RB>
+static void round0_lsd(BuildCtx &c, ActiveList &L) {
+    typedef rs::Sorter<RB> S;
+    constexpr int BINS = 1 << RB;
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 len = c.len;
+    const int b = c.b;
+    const int spd = RB / b;  // symbols per digit
+    const int pshift = prev_shift_for(b);
+    const int maxP = pshift / RB;  // the preceding-symbol field sits above the sorted digits
+    double eff = std::log2((double)(ix.sigma > 2 ? ix.sigma - 1 : 1));
+    if (eff < 0.5) eff = 0.5;
+    int P0 = c.kn.passes0_set ? c.kn.passes0 : (int)std::ceil((c.log2len + c.kn.key_margin) / (spd * eff));
+    P0 = std::max(1, std::min(P0, maxP));
+    L.K = spd * P0;
+    const u64 keymask0 = (L.K * b >= 64) ? ~0ull : ((1ull << (L.K * b)) - 1ull);
+    ix.stats.k0 = L.K;
+    ix.stats.radix_bits = RB;
+    ix.stats.passes0 = P0;
+    ix.stats.passes_elems = (u64)len * P0;
+    u32 *bases0 = c.ar.get<u32>((size_t)P0 * BINS);
+
+    u64 nwords_data = ((u64)len + ix.pk.cpw - 1) / ix.pk.cpw;
+    int t = ix.timer.begin("cmer_hist", (double)len * b / 8.0);
+    CUDA_CHECK(cudaMemsetAsync(c.hist, 0, (size_t)BINS * 4, st));
+    launch_cmer_hist<RB>(ix, nwords_data, c.hist, st);
+    round0_bases_kernel<RB><<<P0, 256, 0, st>>>(c.hist, ix.packed, c.n, L.K, b, bases0);
+    KERNEL_CHECK();
+    ix.timer.end(t);
+
+    // the value ping-pong is arranged so that the last pass writes straight into the SA output
+    u64 *kin = c.keysA, *kout = c.keysB;
+    u32 *vin = (P0 % 2) ? c.valsV : c.sa;
+    u32 *vout = (P0 % 2) ? c.sa : c.valsV;
+    t = ix.timer.begin("make_keys0", (double)len * 12.0);
+    make_keys0_kernel<<<div_up_u(len, 256 * 4), 256, 0, st>>>(ix.packed, c.n, len, L.K, b, kin, vin);
+    KERNEL_CHECK();
+    ix.timer.end(t);
+    for (int p = 0; p < P0; ++p) {
+        t = ix.timer.begin("radix_pass0", (double)len * 24.0);
+        S::pass(kin, vin, kout, vout, len, p * RB, RB, bases0 + (size_t)p * BINS, c.lookback, c.ticket, st);
+        ix.timer.end(t);
+        std::swap(kin, kout);
+        std::swap(vin, vout);
+    }
+    const u64 *keys0 = kin;  // vin == sa
+    u32 *newgrp0 = (u32 *)kout;  // (the other key buffer is free: new ranks by sorted index)
+
+    t = ix.timer.begin("rank0", (double)len * 16.0);
+    CUDA_CHECK(cudaMemsetAsync(c.headbits, 0, (((size_t)len + 63) / 64 + 2) * 8, st));
+    CUDA_CHECK(cudaMemsetAsync(c.rank, 0xff, (size_t)len * 4, st));  // nothing materialised yet
+    rank_kernel<<<div_up_u(len, RK_TILE), RK_NT, 0, st>>>(
+        rank_args(c, keys0, c.sa, len, newgrp0, c.headbits, c.want_bwt ? ix.bwt.ptr : nullptr, 0, L.K, keymask0, pshift));
+    KERNEL_CHECK();
+    ix.timer.end(t);
+
+    t = ix.timer.begin("compact0", (double)len * 0.125);
+    L.m = count_active<false>(c.headbits, len, c.tile_counts, c.d_total, st);
+    if (L.m) {
+        L.grp = c.ar.get<u32>(L.m);
+        scatter_active<false>(c.headbits, c.sa, newgrp0, len, c.tile_counts, L.act, L.grp, st);  // valsV is free once the sort is done
+        const size_t act_words = ((size_t)len + 63) / 64;
+        heads_to_actbits_kernel<<<div_up_u(act_words, 256), 256, 0, st>>>(c.headbits, len, (u64 *)c.actbits, act_words);
+        KERNEL_CHECK();
+    }
+    ix.timer.end(t);
+    L.lr.keys0 = keys0; L.lr.keymask = keymask0; L.lr.K = L.K; L.lr.kb = L.K * b;
+    L.rk_free[0] = kout;  // (keys0 stays: lazy ranks are looked up in it)
+}
+
+// the pair path takes the list after round 0
+static bool pair_path_applies(const BuildCtx &c, const ActiveList &L) {
+    return L.bucketed && c.kn.pairs && ((u64)L.m * 64 >= (u64)c.len || c.kn.pairs == 2);
+}
+
+// ---- groups of two to four equal keys are ordered by the next 64 bits of text (pairs only while the active set is
+// small: in a large one they are copies of repeats) ----
+static void text_tiebreak(BuildCtx &c, ActiveList &L, RankSource &rsrc, PendingList &pend) {
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 m = L.m;
+    int t = ix.timer.begin("resolve_small", (double)m * 40.0);
+    u32 *d_nres = c.ar.get<u32>(2);
+    CUDA_CHECK(cudaMemsetAsync(d_nres, 0, 8, st));
+    const int skip_pairs = (u64)m * 64 > (u64)c.len ? 1 : 0;
+    // (when most suffixes are active the groups are usually giant -- periodic texts: a cheap look first)
+    u32 nsmall = 1;
+    if ((u64)m * 2 > (u64)c.len) {
+        count_small_groups_kernel<<<div_up_u(m, 256), 256, 0, st>>>(L.grp, m, skip_pairs, d_nres + 1);
+        KERNEL_CHECK();
+        read_back(&nsmall, d_nres + 1, 4, st);
+        if ((u64)nsmall * 64 < (u64)m) nsmall = 0;  // (a trip over the whole list for a sprinkle of small groups: the rounds take them)
+    }
+    if (nsmall) {
+        // the permuted list goes into a buffer that is dead until the rounds write their keys (both m <= len words)
+        u8 *keep8 = c.ar.get<u8>((size_t)m + 64);
+        u32 *act_p = (u32 *)L.rk_free[0], *row_p = act_p + (((size_t)m + 3) & ~(size_t)3);  // (vector stores: 16-byte aligned)
+        resolve_small_groups_kernel<<<div_up_u(m, 256), 256, 0, st>>>(L.act, L.grp, m, ix.packed, c.b, L.K, c.n, skip_pairs,
+                                                                      c.sa, L.bucketed ? nullptr : c.rank, act_p, row_p,
+                                                                      c.bwt_rows, c.d_primary, keep8, d_nres);
+        KERNEL_CHECK();
+        u32 nres = 0;
+        read_back(&nres, d_nres, 4, st);
+        ix.stats.resolved_small = nres;
+        // (the permuted list replaces the old one even when nothing was decided: sub-groups may have formed)
+        rsrc.act = act_p;
+        rsrc.row = row_p;
+        // the list the rounds start from goes back into the buffers of the old one (dead now); the rank source stays
+        // where it is until the ranks have been scattered
+        if (nres && L.bucketed && nres < m) {
+            // the suffixes decided here are final but their rows still count as "active after round 0": when rounds
+            // follow, their ranks are materialised now (the pair path below may replace the list the other ranks
+            // are scattered from)
+            CUDA_CHECK(cudaMemsetAsync(c.rank, 0xff, (size_t)c.len * 4, st));
+            scatter_ranks_left_kernel<<<div_up_u(m, 256), 256, 0, st>>>(act_p, row_p, keep8, m, c.rank);
+            KERNEL_CHECK();
+            rsrc.marked = true;
+        }
+        if (nres && nres < m && pair_path_applies(c, L)) {
+            pend.act = act_p; pend.row = row_p; pend.keep = keep8; pend.nres = nres;
+        } else if (nres) {
+            L.m = compact_kept(c, keep8, m, act_p, row_p, L.act, L.grp);
+        } else {
+            CUDA_CHECK(cudaMemcpyAsync(L.act, act_p, (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
+            CUDA_CHECK(cudaMemcpyAsync(L.grp, row_p, (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
+        }
+    }
+    ix.timer.end(t);
+}
+
+// ---- pairs of a text with long exact repeats: decided by one comparison per copied segment (pair_runs_kernel).  It
+// also finishes the compaction the tie-break left pending ----
+static void pair_path(BuildCtx &c, ActiveList &L, RankSource &rsrc, const PendingList &pend) {
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 m = L.m, len = c.len;
+    // (the list the pair path reads: the permuted one when the tie-break left its compaction to this path)
+    const u32 *pl_act = pend.act ? pend.act : L.act, *pl_grp = pend.act ? pend.row : L.grp;
+    bool placed = false;
+    int t = ix.timer.begin("pair_partner", (double)m * 16.0 + (double)len * 4.0);
+    const size_t pt_entries = (size_t)len + PR_CAP + 2 * PR_TILE + 16;
+    const size_t pt_padded = (pt_entries + 127) & ~(size_t)127;
+    const size_t ord_bytes = (((size_t)len + PR_TILE) / PR_TILE + 1) * PR_TILE;
+    // (in the round-key buffer that is free now when the text is long enough for the padding to fit, else carved)
+    u32 *partner = pt_padded * 4 + ord_bytes <= ((size_t)len + 2) * 8 ? (u32 *)L.rk_free[1]
+                                                                    : (u32 *)c.ar.get<u8>(pt_padded * 4 + ord_bytes);
+    u8 *ord = (u8 *)(partner + pt_padded);
+    u32 *d_pr = c.ar.get<u32>(2);
+    CUDA_CHECK(cudaMemsetAsync(partner, 0xff, pt_entries * 4, st));
+    CUDA_CHECK(cudaMemsetAsync(d_pr, 0, 8, st));
+    pair_partner_kernel<<<div_up_u(m, 256 * PQ), 256, 0, st>>>(pl_act, pl_grp, m, partner, d_pr);
+    KERNEL_CHECK();
+    u32 npairs = 0;
+    read_back(&npairs, d_pr, 4, st);
+    ix.timer.end(t);
+    if (npairs && ((u64)npairs * 8 >= (u64)m || c.kn.pairs == 2)) {  // (two members each: at least a quarter of the list)
+        t = ix.timer.begin("pair_runs", (double)len * 5.0);
+        CUDA_CHECK(cudaMemsetAsync(ord, 0, ord_bytes, st));
+        pair_runs_kernel<<<div_up_u(len, PR_TILE), PR_NT, 0, st>>>(partner, c.n, ix.packed, c.b, L.K, ord);
+        KERNEL_CHECK();
+        ix.timer.end(t);
+        t = ix.timer.begin("pair_place", (double)m * 14.0);
+        u8 *keep8 = c.ar.get<u8>((size_t)m + 64);
+        pair_place_kernel<<<div_up_u(m, 256 * PQ), 256, 0, st>>>(pl_act, pl_grp, m, ord, c.sa, c.bwt_rows, c.actbits,
+                                                                c.d_primary, pend.keep, keep8, d_pr + 1);
+        KERNEL_CHECK();
+        u32 nplaced = 0;
+        read_back(&nplaced, d_pr + 1, 4, st);
+        ix.stats.pair_placed = nplaced;
+        ix.timer.end(t);
+        t = ix.timer.begin("pair_compact", (double)m * 10.0);
+        if (nplaced) {
+            // the rest of the list (its ranks are the only ones that are needed: only suffixes that stay active get
+            // one).  From the tie-break's permuted list it goes straight into the list's own buffers; else through
+            // the buffer that held the list round 0 left
+            u32 *tmpA = (u32 *)L.rk_free[0], *tmpB = tmpA + m;
+            const u32 m2 = pend.act ? compact_kept(c, keep8, m, pend.act, pend.row, L.act, L.grp)
+                                    : compact_kept(c, keep8, m, L.act, L.grp, tmpA, tmpB);
+            if (m2 != m - nplaced - pend.nres)
+                throw std::runtime_error("pair path: list accounting is inconsistent (internal error)");
+            if (m2 && !pend.act) {
+                CUDA_CHECK(cudaMemcpyAsync(L.act, tmpA, (size_t)m2 * 4, cudaMemcpyDeviceToDevice, st));
+                CUDA_CHECK(cudaMemcpyAsync(L.grp, tmpB, (size_t)m2 * 4, cudaMemcpyDeviceToDevice, st));
+            }
+            L.m = m2;
+            rsrc.act = L.act;
+            rsrc.row = L.grp;
+            rsrc.m = m2;
+            placed = true;
+        }
+        ix.timer.end(t);
+    }
+    if (pend.act && !placed) {
+        // the pair path placed nothing: the tie-break's own compaction after all
+        t = ix.timer.begin("resolve_small", (double)m * 16.0);
+        L.m = compact_kept(c, pend.keep, m, pend.act, pend.row, L.act, L.grp);
+        ix.timer.end(t);
+    }
+}
+
+// ---- bucketed round 0: ranks of the suffixes that were active after it (first row of their group, or their final
+// row where the text decided); everything else is marked "not materialised" first.  A text without repeats never gets
+// here: its few chance collisions are all decided above.  (LSD round 0: rank_kernel wrote the ranks, the tie-break
+// kept them up to date.) ----
+static void scatter_round0_ranks(BuildCtx &c, const ActiveList &L, const RankSource &rsrc) {
+    int t = c.ix.timer.begin("rank_scatter", (double)rsrc.m * 12.0 + (double)c.len * 4.0);
+    if (!rsrc.marked) CUDA_CHECK(cudaMemsetAsync(c.rank, 0xff, (size_t)c.len * 4, c.st));
+    scatter_ranks_kernel<<<div_up_u(rsrc.m, 256), 256, 0, c.st>>>(rsrc.act, rsrc.row, rsrc.m, L.short_rank, c.rank);
+    KERNEL_CHECK();
+    c.ix.timer.end(t);
+}
+
+// complete ranks ("dense"): ranks of retired suffixes are no longer recovered on demand
+static void go_dense(BuildCtx &c, LazyRank &lr) {
+    int t = c.ix.timer.begin("rank0_fill", (double)c.len * 16.0);
+    fill_singleton_ranks(c.ix, c.actbits, c.rank);
+    c.ix.timer.end(t);
+    lr.sparse = false;
+}
+
+// the list and the buffers of the doubling rounds
+struct RoundState {
+    u32 m;
+    u32 *act, *grp, *act2, *grp2;  // the list and the buffers of the next one
+    u64 *rkA, *rkB;                // round keys and the other key buffer of the sort
+    u64 h;                         // symbols every active group shares
+    u32 bwt_small;                 // active sets up to this size maintain their BWT rows in the rounds
+    // One region serves the chain arrays (live from chain_flags to make_keys) and the outputs of the small-group path
+    // (live from there to the end of the round).
+    size_t cont_bytes;
+    u8 *cont8, *cslot, *notdone, *headB;
+    u32 *chainkey, *d_ncont, *d_handled, *d_nheads;
+    // three list-sized buffers of the split paths; `r0` changes places with the list when the pivot path has
+    // assembled the next one there (every list buffer holds m_init words) -- from then on the region holds a
+    // list and the chain arrays, which share it, are not used any more
+    u32 *r0, *newgrpT, *bvals;
+    // pivot path: per-group tables by (head row) / 2, E bitmap, per-tile counts
+    u8 *ebits8, *rbits8;
+    u32 *pv_tile_e, *pv_piv;
+    unsigned long long *d_pvtot, *pv_cnt;
+    bool chain_on, small_on, pivot_on;
+    bool prefer_pivot;            // large groups or small ones?  (decides which of the two split paths a round tries first)
+    bool ids_are_heads = true;    // rank[] of an active suffix is the first row of its group (until the pivot path runs)
+    int small_pause = 0, small_fails = 0;  // rounds the small-group path sits out after finding almost nothing
+    int pivot_pause = 0, pivot_fails = 0;  // the same for the pivot path
+};
+
+// ---- chain offsets (see chain_flags_kernel): tried while the active set is a noticeable part of the text, dropped for
+// good once a round finds few groups that continue.  True when this round's keys use them ----
+static bool chain_offsets(BuildCtx &c, RoundState &R, const LazyRank &lr) {
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 m = R.m;
+    if (!R.chain_on || R.h > (u64)CHAIN_CAP || (u64)m * (u64)c.kn.chain_min_frac < (u64)c.len) return false;
+    int t = ix.timer.begin("chain_flags", (double)m * 13.0 + (double)c.len);
+    CUDA_CHECK(cudaMemsetAsync(R.cont8, 0, R.cont_bytes, st));
+    CUDA_CHECK(cudaMemsetAsync(R.cslot, 0, m, st));
+    CUDA_CHECK(cudaMemsetAsync(R.d_ncont, 0, 4, st));
+    const u32 cf_tiles = div_up_u(m, CF_STEP);
+    u32 ncont = 0;
+    bool worth = true;
+    if (cf_tiles > 16384) {
+        // a sample of 2 048 tiles first: a list whose groups do not continue (diverged copies, periodic
+        // texts) is not worth the full pass (what the sample marks is what the full pass would mark)
+        const u32 mul = cf_tiles / 2048;
+        chain_flags_kernel<<<2048, CF_NT, 0, st>>>(R.act, R.grp, m, c.rank, R.cslot, R.cont8, R.d_ncont, mul);
+        KERNEL_CHECK();
+        read_back(&ncont, R.d_ncont, 4, st);
+        worth = (u64)ncont * (u64)c.kn.chain_use_frac * 2 >= (u64)2048 * CF_STEP;
+        CUDA_CHECK(cudaMemsetAsync(R.d_ncont, 0, 4, st));
+        ncont = 0;
+    }
+    if (worth) {
+        chain_flags_kernel<<<cf_tiles, CF_NT, 0, st>>>(R.act, R.grp, m, c.rank, R.cslot, R.cont8, R.d_ncont, 1);
+        KERNEL_CHECK();
+        read_back(&ncont, R.d_ncont, 4, st);
+    }
+    ix.timer.end(t);
+    // worth it when most groups continue (copies of long segments); texts whose groups are large and
+    // shallow (many diverged copies) gain nothing from it
+    if ((u64)ncont * (u64)c.kn.chain_use_frac < (u64)m) {
+        R.chain_on = false;
+        return false;
+    }
+    t = ix.timer.begin("chain_keys", (double)c.len + (double)ncont * 4.0);
+    chain_keys_kernel<<<div_up_u(c.len, CK_TILE), CK_NT, 0, st>>>(R.cont8, c.len, lr, R.h, R.chainkey, c.d_lazy);
+    KERNEL_CHECK();
+    ix.timer.end(t);
+    ix.stats.chain_rounds++;
+    ix.stats.chain_elems += ncont;
+    return true;
+}
+
+// ---- large groups that mostly stay together: split around a pivot key (pivot_classify_kernel).  The E part of
+// every group goes straight into the next list; its L members and its R members, each compacted into a list of their
+// own, are split again the same way (a group whose members carry two or three distinct second keys -- a Fibonacci
+// string -- never reaches the radix sort); lists that are small, or whose groups scatter, are sorted.  True when the
+// round was done this way: the next list is in (R.act, R.grp2), `m2` long ----
+template <int RB>
+static bool pivot_round(BuildCtx &c, RoundState &R, u32 &m2) {
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 m = R.m;
+    const bool pivot_force = c.kn.pivot_force;
+    const u32 pivot_sub_min = std::max(2u, c.kn.pivot_min / 16u);  // lists of the pivot path that are split again
+    PivotArgs base{};
+    base.lo_bits = c.lo_bits; base.piv = R.pv_piv; base.cnt64 = R.pv_cnt; base.ebits8 = R.ebits8; base.lbits8 = R.notdone;
+    base.rbits8 = R.rbits8; base.tile_e = R.pv_tile_e; base.totals = R.d_pvtot; base.sa = c.sa; base.rank = c.rank;
+    base.primary = c.d_primary; base.singles = R.d_nheads;
+    u32 out_n = 0;           // entries of the next list (r0 / grp2) written so far
+    u64 pv_e = 0, pv_sorted = 0;
+    auto classify = [&](u64 *kx, const u32 *vx, u32 n, bool publish, u32 &ne, u32 &nl) {
+        PivotArgs pv = base;
+        pv.keys = kx; pv.act = vx; pv.m = n;
+        const u32 ntl = div_up_u(n, PV_TILE);
+        const u64 kw = ((u64)n + 63) / 64;
+        CUDA_CHECK(cudaMemsetAsync(R.ebits8 + kw * 8, 0, 16, st));
+        CUDA_CHECK(cudaMemsetAsync(R.notdone + kw * 8, 0, 16, st));
+        CUDA_CHECK(cudaMemsetAsync(R.rbits8 + kw * 8, 0, 16, st));
+        CUDA_CHECK(cudaMemsetAsync(R.d_pvtot, 0, 16, st));
+        if (publish) {
+            pivot_heads_kernel<<<div_up_u(n, PV_TILE), PV_NT, 0, st>>>(kx, n, c.lo_bits, R.pv_piv, R.pv_cnt);
+            KERNEL_CHECK();
+        }
+        pivot_classify_kernel<<<ntl, PV_NT, 0, st>>>(pv);
+        KERNEL_CHECK();
+        scan_tiles_kernel<<<1, 1024, 0, st>>>(R.pv_tile_e, ntl, R.d_pvtot);
+        KERNEL_CHECK();
+        unsigned long long tot[2] = {0, 0};
+        read_back(tot, R.d_pvtot, 16, st);
+        ne = (u32)tot[0];
+        nl = (u32)tot[1];
+    };
+    // radix sort of one list, new ranks, survivors appended to the next list
+    auto sort_list = [&](u64 *kx, u32 *vx, u32 n, u64 *ky, u32 *vy, u32 *ng) {
+        const u32 *sorted = sort_and_rank<RB>(c, kx, vx, ky, vy, n, ng, R.headB, nullptr, 1);
+        int tt = ix.timer.begin("compact", (double)n * 4.0);
+        const u32 mB = count_active<false>(R.headB, n, c.tile_counts, c.d_total, st);
+        if (mB) scatter_active<false>(R.headB, sorted, ng, n, c.tile_counts, R.r0 + out_n, R.grp2 + out_n, st);
+        out_n += mB;
+        pv_sorted += n;
+        ix.timer.end(tt);
+    };
+    // one list: keys / values in (kx, vx); (ky, vy) = the other buffer pair over the same index range;
+    // ng = as many free words (new ranks by sorted index)
+    std::function<void(int, u64 *, u32 *, u32, u64 *, u32 *, u32 *, u32, u32)> process;
+    process = [&](int level, u64 *kx, u32 *vx, u32 n, u64 *ky, u32 *vy, u32 *ng, u32 ne, u32 nl) {
+        // (level 0 arrives classified)
+        bool go = level == 0;
+        if (level > 0 && level < 8 && n >= pivot_sub_min) {
+            int tt = ix.timer.begin("pivot_classify", (double)n * 16.0);
+            classify(kx, vx, n, true, ne, nl);
+            ix.timer.end(tt);
+            go = (u64)ne * 3 >= (u64)n || pivot_force;
+        }
+        if (!go) {
+            sort_list(kx, vx, n, ky, vy, ng);
+            return;
+        }
+        int tt = ix.timer.begin("pivot_apply", (double)n * 24.0);
+        PivotArgs pv = base;
+        pv.keys = kx; pv.act = vx; pv.m = n;
+        pv.out_act = R.r0 + out_n; pv.out_grp = R.grp2 + out_n; pv.out_base = out_n; pv.dropbits = (u32 *)c.headbits;
+        pivot_apply_kernel<<<div_up_u(n, PV_TILE), PV_NT, 0, st>>>(pv);
+        KERNEL_CHECK();
+        ix.timer.end(tt);
+        out_n += ne;
+        pv_e += ne;
+        const u32 nr = n - ne - nl;
+        if (nl | nr) {
+            tt = ix.timer.begin("compact_big", (double)n * 0.25 + (double)(nl + nr) * 24.0);
+            if (nl) {
+                const u32 cnt = count_active<true>(R.notdone, n, c.tile_counts, c.d_total, st);
+                if (cnt != nl) throw std::runtime_error("pivot path: L members miscounted (internal error)");
+                scatter_pairs(R.notdone, kx, vx, n, c.tile_counts, ky, vy, st);
+            }
+            if (nr) {
+                const u32 cnt = count_active<true>(R.rbits8, n, c.tile_counts, c.d_total, st);
+                if (cnt != nr) throw std::runtime_error("pivot path: R members miscounted (internal error)");
+                scatter_pairs(R.rbits8, kx, vx, n, c.tile_counts, ky + nl, vy + nl, st);
+            }
+            ix.timer.end(tt);
+            if (nl) process(level + 1, ky, vy, nl, kx, vx, ng, 0, 0);
+            if (nr) process(level + 1, ky + nl, vy + nl, nr, kx + nl, vx + nl, ng + nl, 0, 0);
+        }
+    };
+    int t = ix.timer.begin("pivot_classify", (double)m * 16.0);
+    u32 n_e = 0, n_l = 0;
+    classify(R.rkA, R.act, m, false, n_e, n_l);
+    ix.timer.end(t);
+    if ((u64)n_e * 3 < (u64)m && !pivot_force) {
+        // the groups scatter: nothing was changed, the round goes on as usual; back off 2, 4, 8 ... rounds
+        R.pivot_pause = 2 << std::min(R.pivot_fails, 4);
+        ++R.pivot_fails;
+        return false;
+    }
+    R.ids_are_heads = false;
+    R.chain_on = false;
+    R.pivot_fails = 0;
+    CUDA_CHECK(cudaMemsetAsync(R.d_nheads, 0, 4, st));
+    CUDA_CHECK(cudaMemsetAsync(c.headbits, 0, (((size_t)m + 63) / 64 + 2) * 8, st));  // (no entry of the next list is dropped)
+    // (the old list is dead once its L and R members have been copied out: its value buffer is the
+    // scratch of the deeper levels; the old group heads are dead already, the keys carry them)
+    process(0, R.rkA, R.act, m, R.rkB, R.bvals, R.grp, n_e, n_l);
+    ix.stats.sorted_total -= (u64)m - pv_sorted;
+    ix.stats.pivot_rounds++;
+    ix.stats.pivot_elems += pv_e;
+    if (c.bwt_rows) c.need_bwt_fix = true;  // (this path does not write BWT rows)
+    // E groups of one member are final: out of the list (rare; through two buffers that are free now)
+    u32 n_single = 0;
+    read_back(&n_single, R.d_nheads, 4, st);
+    m2 = out_n;
+    if (n_single) {
+        // the survivors are copied to the old list's buffers (free now), which stay the list
+        t = ix.timer.begin("compact", (double)out_n * 16.0);
+        const u64 kw = ((u64)out_n + 63) / 64;
+        pivot_keep_kernel<<<div_up_u(kw, 256), 256, 0, st>>>((u64 *)c.headbits, out_n, kw);
+        KERNEL_CHECK();
+        m2 = count_active<true>(c.headbits, out_n, c.tile_counts, c.d_total, st);
+        if (m2 != out_n - n_single) throw std::runtime_error("pivot path: single-member groups miscounted (internal error)");
+        if (m2) scatter_active<true>(c.headbits, R.r0, R.grp2, out_n, c.tile_counts, R.act, R.newgrpT, st);
+        std::swap(R.grp2, R.newgrpT);
+        ix.timer.end(t);
+    } else {
+        std::swap(R.act, R.r0);
+    }
+    return true;
+}
+
+// ---- groups of up to RS_GMAX members are ordered where they stand (round_small_kernel); returns how many list
+// elements it placed ----
+static u32 small_groups_round(BuildCtx &c, RoundState &R) {
+    if (R.small_pause > 0) {
+        --R.small_pause;
+        return 0;
+    }
+    if (!R.small_on) return 0;
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 m = R.m;
+    int t = ix.timer.begin("round_small", (double)m * 28.0);
+    const u64 kw = ((u64)m + 63) / 64;
+    CUDA_CHECK(cudaMemsetAsync(c.headbits + kw * 8, 0, 16, st));
+    CUDA_CHECK(cudaMemsetAsync(R.notdone + kw * 8, 0, 16, st));
+    CUDA_CHECK(cudaMemsetAsync(R.d_handled, 0, 4, st));
+    SmallArgs sm{};
+    sm.act = R.act; sm.grp = R.grp; sm.keys = R.rkA; sm.m = m; sm.lo_bits = c.lo_bits; sm.sa = c.sa; sm.rank = c.rank;
+    sm.vals_out = R.r0; sm.newgrp_out = R.newgrpT; sm.headbits64 = (u64 *)c.headbits; sm.notdone64 = (u64 *)R.notdone;
+    sm.primary = c.d_primary; sm.handled = R.d_handled; sm.always_write = R.ids_are_heads ? 0 : 1;
+    round_small_kernel<<<div_up_u(m, RS_STEP), RS_NT, 0, st>>>(sm);
+    KERNEL_CHECK();
+    u32 handled = 0;
+    read_back(&handled, R.d_handled, 4, st);
+    ix.timer.end(t);
+    ix.stats.small_path_elems += handled;
+    if ((u64)handled * 32 < (u64)m) {  // (periodic texts: a few giant groups) -- back off 3, 6, 12 ... rounds
+        R.small_pause = 3 << std::min(R.small_fails, 4);
+        ++R.small_fails;
+        R.prefer_pivot = true;  // (large groups: the pivot path is the one to try)
+    }
+    if (handled && c.bwt_rows) c.need_bwt_fix = true;  // (this path does not write BWT rows)
+    return handled;
+}
+
+// ---- everything the small-group path left: radix sort of (group, rank) keys, new ranks from the sorted list; then
+// the next active set, the survivors of both paths one after the other (groups stay contiguous).  Returns its
+// length ----
+template <int RB>
+static u32 sort_round(BuildCtx &c, RoundState &R, u32 handled) {
+    DeviceIndex &ix = c.ix; const cudaStream_t st = c.st;
+    const u32 m = R.m, mb = m - handled;
+    u64 *bk = R.rkA, *k_other = R.rkB;  // keys / values of the elements that go through the sort
+    u32 *bv = R.act;
+    if (handled && mb) {
+        int t = ix.timer.begin("compact_big", (double)m * 0.125 + (double)mb * 24.0);
+        const u32 cnt = count_active<true>(R.notdone, m, c.tile_counts, c.d_total, st);
+        if (cnt != mb) throw std::runtime_error("split paths: slot accounting is inconsistent (internal error)");
+        scatter_pairs(R.notdone, R.rkA, R.act, m, c.tile_counts, R.rkB, R.bvals, st);
+        ix.timer.end(t);
+        bk = R.rkB; bv = R.bvals; k_other = R.rkA;
+    }
+    u8 *hb_big = handled ? R.headB : c.headbits;
+    const u32 *sorted_vals = nullptr;
+    if (mb) {
+        // BWT rows of moved suffixes: one gather per element and round -- kept in the rounds while the
+        // active set is small, otherwise one pass over the rows of round 0's active set at the end
+        u8 *bwt = m <= R.bwt_small ? c.bwt_rows : nullptr;
+        if (c.bwt_rows && !bwt) c.need_bwt_fix = true;
+        // (newgrp: the old heads are dead, the keys carry them)
+        sorted_vals = sort_and_rank<RB>(c, bk, bv, k_other, R.act2, mb, R.grp, hb_big, bwt, R.ids_are_heads ? 0 : 1);
+    }
+    int t = ix.timer.begin("compact", (double)m * 4.0);
+    // (`act` was read for the last time by the sort or by the compaction of its part; the survivors go to the value
+    // buffer the sort left free)
+    u32 *dst = sorted_vals == R.act ? R.act2 : R.act;
+    u32 mA = 0, mB = 0;
+    if (handled) {
+        mA = count_active<false>(c.headbits, m, c.tile_counts, c.d_total, st);
+        if (mA) scatter_active<false>(c.headbits, R.r0, R.newgrpT, m, c.tile_counts, dst, R.grp2, st);
+    }
+    if (mb) {
+        mB = count_active<false>(hb_big, mb, c.tile_counts, c.d_total, st);
+        if (mB) scatter_active<false>(hb_big, sorted_vals, R.grp, mb, c.tile_counts, dst + mA, R.grp2 + mA, st);
+    }
+    if (dst == R.act2) std::swap(R.act, R.act2);
+    ix.timer.end(t);
+    return mA + mB;
+}
+
+// ---- doubling rounds over the active set ----
+template <int RB>
+static void doubling_rounds(BuildCtx &c, ActiveList &L) {
+    DeviceIndex &ix = c.ix;
+    Arena &ar = c.ar;
+    const cudaStream_t st = c.st;
+    const u32 len = c.len;
+    LazyRank &lr = L.lr;
+    const u32 m = L.m;
+    // complete ranks ("dense") from the start when most suffixes are active; otherwise ranks of
+    // retired suffixes are recovered on demand, until a round needs many of them
+    if ((u64)m * 2 > (u64)len) {
+        go_dense(c, lr);
+        if (!L.bucketed) L.rk_free[1] = const_cast<u64 *>(lr.keys0);  // the sorted round-0 keys are dead now
+    }
+    RoundState R;
+    R.m = m; R.act = L.act; R.grp = L.grp;
+    R.rkA = L.rk_free[0] ? L.rk_free[0] : ar.get<u64>(m);
+    R.rkB = L.rk_free[1] ? L.rk_free[1] : ar.get<u64>(m);
+    R.act2 = ar.get<u32>(m); R.grp2 = ar.get<u32>(m);
+    R.h = L.depth0 ? (u64)L.depth0 : (u64)L.K;
+    R.bwt_small = std::max(1u, len / (u32)c.kn.bwt_round_frac);
+    R.chain_on = c.kn.chain && (u64)m * (u64)c.kn.chain_min_frac >= (u64)len;
+    R.small_on = c.kn.small_path; R.pivot_on = c.kn.pivot;
+    R.cont_bytes = ((size_t)len + 2 * (size_t)CHAIN_CAP + 8192 + 511) & ~(size_t)511;
+    const size_t m_init = m;
+    const size_t third = (m_init * 4 + 64 + 511) & ~(size_t)511;
+    size_t chain_bytes = R.chain_on ? R.cont_bytes + (size_t)len * 4 + ((m_init + 511) & ~(size_t)511) : 0;
+    size_t split_bytes = (R.small_on || R.pivot_on) ? 3 * third : 0;
+    // the optional paths are dropped, the larger first, rather than running the device out of memory
+    const size_t mem_margin = (size_t)2 << 30;
+    if (split_bytes > chain_bytes && !ar.can_fit(split_bytes, mem_margin)) {
+        split_bytes = 0;
+        R.small_on = R.pivot_on = false;
+    }
+    if (chain_bytes && !ar.can_fit(std::max(chain_bytes, split_bytes), mem_margin)) {
+        chain_bytes = 0;
+        R.chain_on = false;
+        if (split_bytes && !ar.can_fit(split_bytes, mem_margin)) {
+            split_bytes = 0;
+            R.small_on = R.pivot_on = false;
+        }
+    }
+    u8 *region = ar.get<u8>(std::max<size_t>(std::max(chain_bytes, split_bytes), 512));
+    R.cont8 = region; R.cslot = region + R.cont_bytes + (size_t)len * 4; R.chainkey = (u32 *)(region + R.cont_bytes);
+    R.r0 = (u32 *)region; R.newgrpT = (u32 *)(region + third); R.bvals = (u32 *)(region + 2 * third);
+    R.d_ncont = ar.get<u32>(4); R.d_handled = R.d_ncont + 1; R.d_nheads = R.d_ncont + 2;
+    const size_t bm_bytes = ((m_init + 63) / 64 + 2) * 8;
+    R.notdone = ar.get<u8>(bm_bytes); R.headB = ar.get<u8>(bm_bytes);
+    const size_t pv_entries = (size_t)len / 2 + 2;
+    if (R.pivot_on && !ar.can_fit(pv_entries * 12 + 2 * bm_bytes, mem_margin)) R.pivot_on = false;
+    R.ebits8 = R.pivot_on ? ar.get<u8>(bm_bytes) : nullptr;
+    R.pv_tile_e = R.pivot_on ? ar.get<u32>((size_t)div_up_u(m_init, PV_TILE) + 2) : nullptr;
+    R.rbits8 = R.pivot_on ? ar.get<u8>(bm_bytes) : nullptr;
+    R.d_pvtot = ar.get<unsigned long long>(2);
+    R.pv_cnt = R.pivot_on ? ar.get<unsigned long long>(pv_entries) : nullptr;
+    R.pv_piv = R.pivot_on ? ar.get<u32>(pv_entries) : nullptr;
+    R.prefer_pivot = c.kn.pivot_force;
+    if (R.pivot_on && !c.kn.pivot_force && m >= c.kn.pivot_min) {
+        CUDA_CHECK(cudaMemsetAsync(R.d_nheads, 0, 4, st));
+        count_heads_kernel<<<std::max(1u, std::min(div_up_u(m, 256 * 8), 148u * 8u)), 256, 0, st>>>(R.grp, m, R.d_nheads);
+        KERNEL_CHECK();
+        u32 nheads = 0;
+        read_back(&nheads, R.d_nheads, 4, st);
+        R.prefer_pivot = (u64)nheads * 64 <= (u64)m;
+    }
+    while (R.m > 0) {
+        ix.stats.rounds++;
+        ix.stats.sorted_total += R.m;
+        CUDA_CHECK(cudaMemsetAsync(c.d_lazy, 0, 4, st));
+        const bool use_chain = chain_offsets(c, R, lr);
+        int t = ix.timer.begin("round_keys", (double)R.m * 16.0);
+        const bool try_pivot = R.pivot_on && R.prefer_pivot && R.pivot_pause == 0 && R.m >= c.kn.pivot_min;
+        const unsigned kgrid = std::max(1u, std::min(div_up_u(R.m, 256 * 4), 148u * 16u));
+        if (lr.sparse)
+            make_keys_round_kernel<<<kgrid, 256, 0, st>>>(R.act, R.grp, R.m, lr, R.h, c.lo_bits, use_chain ? R.cslot : nullptr,
+                                                          R.chainkey, R.rkA, c.d_lazy, try_pivot ? R.pv_piv : nullptr, R.pv_cnt);
+        else
+            make_keys_dense_kernel<<<kgrid, 256, 0, st>>>(R.act, R.grp, R.m, c.rank, R.h, len, c.lo_bits,
+                                                          use_chain ? R.cslot : nullptr, R.chainkey, R.rkA,
+                                                          try_pivot ? R.pv_piv : nullptr, R.pv_cnt);
+        KERNEL_CHECK();
+        ix.timer.end(t);
+
+        u32 m2 = 0;
+        bool pivoted = false;
+        if (try_pivot) pivoted = pivot_round<RB>(c, R, m2);
+        else if (R.pivot_pause > 0) --R.pivot_pause;
+        if (!pivoted) m2 = sort_round<RB>(c, R, small_groups_round(c, R));
+
+        u32 nlazy = 0;
+        read_back(&nlazy, c.d_lazy, 4, st);
+        ix.stats.lazy_lookups += nlazy;
+        std::swap(R.grp, R.grp2);
+        R.m = m2;
+        R.h *= 2;
+        if (R.h > (u64)len * 2 + 2 && R.m > 0)
+            throw std::runtime_error("prefix doubling failed to converge (internal error)");
+        // a lookup costs several random accesses, completing the ranks one random store per suffix
+        if (R.m > 0 && lr.sparse && (u64)nlazy * (u64)c.kn.dense_factor > (u64)len) go_dense(c, lr);
+    }
+}
+
+// ---- BWT rows the rounds did not maintain, from the final SA ----
+static void bwt_fix(BuildCtx &c, u32 m_round0) {
+    int t = c.ix.timer.begin("bwt_fix", (double)c.len * 0.125);
+    // rows still marked: those round 0 left active minus the ones the pair path made final
+    const u64 marked = (u64)m_round0 - (u64)c.ix.stats.pair_placed;
+    if (marked * 8 > (u64)c.len)
+        bwt_fix_rows_kernel<<<div_up_u(c.len, 256), 256, 0, c.st>>>(c.actbits, c.sa, c.len, c.ix.packed, c.b, c.ix.bwt.ptr,
+                                                                    c.d_primary);
+    else
+        bwt_fix_kernel<<<div_up_u(div_up_u(c.len, 32), 256), 256, 0, c.st>>>(c.actbits, c.sa, c.len, c.ix.packed, c.b,
+                                                                            c.ix.bwt.ptr, c.d_primary);
+    KERNEL_CHECK();
+    c.ix.timer.end(t);
+}
+
+template <int RB>
+static void build_sa_impl(DeviceIndex &ix, const BuildKnobs &kn, bool want_bwt) {
     typedef rs::Sorter<RB> S;
     constexpr int BINS = 1 << RB;
     cudaStream_t st = ix.stream;
-    Arena &ar = *ix.arena;
-    const u32 n = ix.n, len = ix.len;
-    const int b = ix.pk.bits, cpw = ix.pk.cpw;
-    const int c = RB / b;  // symbols per digit
-
-    int log2len = 0;
-    while ((1ull << log2len) < (u64)len) ++log2len;
+    const u32 len = ix.len;
     ix.stats = BuildStats{};
     ix.stats.sorted_total = len;
 
@@ -2296,769 +3106,47 @@ static void build_sa_impl(DeviceIndex &ix, bool want_bwt) {
     DevBuf<u32> d_primary(1, st);
 
     // ---- workspace ----
+    BuildCtx c(ix, kn, want_bwt, d_primary.ptr);
+    Arena &ar = c.ar;
     // + 2: the bulk copies of round0_msd.cu read whole 16-byte units
-    u64 *keysA = ar.get<u64>((size_t)len + 2), *keysB = ar.get<u64>((size_t)len + 2);
-    u32 *valsV = ar.get<u32>(len);
-    u32 *rank = ar.get<u32>(len);
-    const size_t act_words64 = ((size_t)len + 63) / 64 + 2;
-    u32 *actbits = (u32 *)ar.get<u64>(act_words64);  // bit per row: active after round 0
-    u64 *lookback = ar.get<u64>(S::lookback_words(len));
-    u32 *hist = ar.get<u32>((size_t)8 * BINS), *uniform = ar.get<u32>(8), *ticket = ar.get<u32>(1);
-    size_t hb_bytes = (((size_t)len + 63) / 64 + 2) * 8;
-    u8 *headbits = ar.get<u8>(hb_bytes);
-    u32 *tile_counts = ar.get<u32>(div_up_u(len, CP_TILE) + 1);
-    unsigned long long *d_total = ar.get<unsigned long long>(1);
-    u32 *d_lazy = ar.get<u32>(1);
+    c.keysA = ar.get<u64>((size_t)len + 2); c.keysB = ar.get<u64>((size_t)len + 2);
+    c.valsV = ar.get<u32>(len);
+    c.rank = ar.get<u32>(len);
+    c.actbits = (u32 *)ar.get<u64>(((size_t)len + 63) / 64 + 2);
+    c.lookback = ar.get<u64>(S::lookback_words(len));
+    c.hist = ar.get<u32>((size_t)8 * BINS); c.uniform = ar.get<u32>(8); c.ticket = ar.get<u32>(1);
+    c.headbits = ar.get<u8>((((size_t)len + 63) / 64 + 2) * 8);
+    c.tile_counts = ar.get<u32>(div_up_u(len, CP_TILE) + 1);
+    c.d_total = ar.get<unsigned long long>(1);
+    c.d_lazy = ar.get<u32>(1);
 
-    u32 *sa = ix.sa.ptr;
-    u32 m = 0;           // suffixes whose round-0 key is shared with another suffix
-    u32 *act = valsV;    // ... listed here, in suffix-array order, each with the first row of its group
-    u32 *grp = nullptr;
-    int K = 0;
-    bool bwt_in_sort = true;  // BWT rows ride along with the sort (else: gathered from the final SA)
-    LazyRank lr{};
-    lr.rank = rank; lr.sparse = true; lr.sa0 = sa; lr.packed = ix.packed; lr.n = n; lr.len = len; lr.bits = b;
-    int t;
+    ActiveList L;
+    L.act = c.valsV;
+    L.lr.rank = c.rank; L.lr.sparse = true; L.lr.sa0 = c.sa; L.lr.packed = ix.packed; L.lr.n = c.n; L.lr.len = len;
+    L.lr.bits = c.b;
+    if (!round0_bucketed(c, L)) round0_lsd<RB>(c, L);
+    const u32 m_round0 = L.m;  // rows round 0 left active (their bits are set in `actbits`)
+    c.bwt_rows = (want_bwt && L.bwt_in_sort) ? ix.bwt.ptr : nullptr;
 
-    // ---- round 0, preferred: MSD bucket sort of 8-byte elements (round0_msd.cu) ----
-    bool done0 = false;
-    const u32 *short_rank = nullptr;  // bucketed round 0: ranks of the short suffixes of oversize buckets
-    u32 depth0 = 0;  // symbols every active group shares after round 0 (0: K)
-    u64 *rk_free[2] = {nullptr, nullptr};  // large buffers that are dead after round 0 (round keys go there)
-    {
-        Round0Msd r0{};
-        if (msd_make_plan(len, ix.sigma, b, r0.plan, ix.sym_counts_host)) {
-            Arena::Mark mk = ar.mark();
-            r0.bufA = keysA; r0.bufB = keysB; r0.actbits = actbits;
-            r0.d_primary = d_primary.ptr;
-            done0 = round0_msd(ix, want_bwt, r0);
-            if (done0) {
-                K = r0.plan.K;
-                bwt_in_sort = r0.bwt_written;
-                lr.keys0 = nullptr; lr.bstart = r0.bucket_start; lr.BB = r0.plan.BB; lr.K = K;
-                lr.kb = r0.plan.KB; lr.dense = r0.plan.dense;
-                ix.stats.dense_keys = r0.plan.dense.nsym;
-                lr.keymask = (K * b >= 64) ? ~0ull : ((1ull << (K * b)) - 1ull);
-                ix.stats.k0 = K;
-                ix.stats.radix_bits = r0.plan.D[0];
-                ix.stats.passes0 = r0.plan.nlevels;
-                ix.stats.round0_mode = 1;
-                ix.stats.bucket_bits = r0.plan.BB;
-                ix.stats.passes_elems = (u64)len * r0.plan.nlevels;
-                ix.stats.shallow_buckets = r0.shallow_buckets;
-                ix.stats.shallow_elems = r0.shallow_buckets ? r0.shallow_elems : 0;
-                depth0 = r0.depth0;
-                short_rank = r0.short_rank;
-                // the active rows, in row order, with their group heads
-                t = ix.timer.begin("compact0", (double)len * 0.125);
-                m = count_active<true>((const u8 *)actbits, len, tile_counts, d_total, st);
-                if (m) {
-                    grp = ar.get<u32>(m);
-                    scatter_active<true>((const u8 *)actbits, sa, r0.grow, len, tile_counts, act, grp, st);
-                }
-                ix.timer.end(t);
-                rk_free[0] = keysA;
-                rk_free[1] = keysB;
-            } else {
-                ar.release_to(mk);
-            }
-        }
-    }
-
-    // ---- round 0, general: LSD radix passes over (u64 key, u32 suffix) pairs ----
-    RankArgs ra{};
-    if (!done0) {
-        double eff = std::log2((double)(ix.sigma > 2 ? ix.sigma - 1 : 1));
-        if (eff < 0.5) eff = 0.5;
-        int margin = env_int("B200SA_KEY_MARGIN", 8);
-        int P0 = (int)std::ceil((log2len + margin) / (c * eff));
-        const int pshift = prev_shift_for(b);
-        int maxP = pshift / RB;  // the preceding-symbol field sits above the sorted digits
-        P0 = std::max(1, std::min(P0, maxP));
-        P0 = env_int("B200SA_PASSES0", P0);
-        P0 = std::max(1, std::min(P0, maxP));
-        K = c * P0;
-        const u64 keymask0 = (K * b >= 64) ? ~0ull : ((1ull << (K * b)) - 1ull);
-        ix.stats.k0 = K;
-        ix.stats.radix_bits = RB;
-        ix.stats.passes0 = P0;
-        ix.stats.passes_elems = (u64)len * P0;
-        u32 *bases0 = ar.get<u32>((size_t)P0 * BINS);
-
-        u64 nwords_data = ((u64)len + cpw - 1) / cpw;
-        t = ix.timer.begin("cmer_hist", (double)len * b / 8.0);
-        CUDA_CHECK(cudaMemsetAsync(hist, 0, (size_t)BINS * 4, st));
-        launch_cmer_hist<RB>(ix, nwords_data, hist, st);
-        round0_bases_kernel<RB><<<P0, 256, 0, st>>>(hist, ix.packed, n, K, b, bases0);
-        KERNEL_CHECK();
-        ix.timer.end(t);
-
-        // the value ping-pong is arranged so that the last pass writes straight into the SA output
-        u64 *kin = keysA, *kout = keysB;
-        u32 *vin = (P0 % 2) ? valsV : ix.sa.ptr;
-        u32 *vout = (P0 % 2) ? ix.sa.ptr : valsV;
-        t = ix.timer.begin("make_keys0", (double)len * 12.0);
-        make_keys0_kernel<<<div_up_u(len, 256 * 4), 256, 0, st>>>(ix.packed, n, len, K, b, kin, vin);
-        KERNEL_CHECK();
-        ix.timer.end(t);
-        for (int p = 0; p < P0; ++p) {
-            t = ix.timer.begin("radix_pass0", (double)len * 24.0);
-            S::pass(kin, vin, kout, vout, len, p * RB, RB, bases0 + (size_t)p * BINS, lookback, ticket, st);
-            ix.timer.end(t);
-            std::swap(kin, kout);
-            std::swap(vin, vout);
-        }
-        const u64 *keys0 = kin;  // vin == ix.sa.ptr
-        u32 *newgrp0 = (u32 *)kout;  // (the other key buffer is free: new ranks by sorted index)
-
-        t = ix.timer.begin("rank0", (double)len * 16.0);
-        CUDA_CHECK(cudaMemsetAsync(headbits, 0, hb_bytes, st));
-        CUDA_CHECK(cudaMemsetAsync(rank, 0xff, (size_t)len * 4, st));  // nothing materialised yet
-        ra.keys = keys0; ra.vals = sa; ra.m = len; ra.gs = 64; ra.keymask = keymask0; ra.K0 = K; ra.n = n;
-        ra.rank = rank; ra.newgrp = newgrp0; ra.scatter_all = 0; ra.sa_out = nullptr; ra.headbits = headbits;
-        ra.bwt = want_bwt ? ix.bwt.ptr : nullptr; ra.prev_shift = pshift; ra.packed = ix.packed; ra.bits = b;
-        ra.primary = d_primary.ptr;
-        rank_kernel<<<div_up_u(len, RK_TILE), RK_NT, 0, st>>>(ra);
-        KERNEL_CHECK();
-        ix.timer.end(t);
-
-        t = ix.timer.begin("compact0", (double)len * 0.125);
-        m = count_active<false>(headbits, len, tile_counts, d_total, st);
-        if (m) {
-            grp = ar.get<u32>(m);
-            scatter_active<false>(headbits, sa, newgrp0, len, tile_counts, act, grp, st);  // valsV is free once the sort is done
-            heads_to_actbits_kernel<<<div_up_u(act_words64 - 2, 256), 256, 0, st>>>(headbits, len, (u64 *)actbits, act_words64 - 2);
-            KERNEL_CHECK();
-        }
-        ix.timer.end(t);
-        lr.keys0 = keys0; lr.keymask = keymask0; lr.K = K; lr.kb = K * b;
-        rk_free[0] = kout;  // (keys0 stays: lazy ranks are looked up in it)
-    }
-
-    // ---- doubling rounds over the active set ----
-    u8 *bwt_rows = (want_bwt && bwt_in_sort) ? ix.bwt.ptr : nullptr;
-    bool need_bwt_fix = false;
-    // the list as round 0 left it: what rank[] has to hold for its suffixes (round0_msd.cu writes no ranks)
-    const u32 *act0 = act, *row0 = grp;
-    u32 m0 = m;
-    const u32 m_round0 = m;  // rows round 0 left active (their bits are set in `actbits`)
-    bool rank_marked = false;  // rank[] has been set to "not materialised" (and holds the ranks of decided suffixes)
-    const int pairs_mode = env_int("B200SA_PAIRS", 1);  // 0: off, 2: on lists of any size (tests)
-    // the tie-break below leaves its list permuted, with a "stays" byte per element, when the pair path follows it:
-    // one compaction serves both
-    bool deferred = false;
-    u32 *dl_act = nullptr, *dl_row = nullptr, dl_nres = 0;
-    u8 *dl_keep = nullptr;
+    RankSource rsrc{L.act, L.grp, L.m, false};
+    PendingList pend;
     // (a large active set that the pair path takes next: that path orders groups of two and three -- a chance collision
-    // next to a pair included -- by the text itself; the pass below would only add a trip over the list)
-    const bool pairs_first = done0 && rk_free[1] && pairs_mode == 1 && (u64)m * 64 >= (u64)len;
-    if (m && b <= 8 && !pairs_first && !env_int("B200SA_NO_EXT_TIEBREAK", 0)) {
-        // groups of two to four equal keys are ordered by the next 64 bits of text (pairs only while the active set
-        // is small: in a large one they are copies of repeats)
-        t = ix.timer.begin("resolve_small", (double)m * 40.0);
-        u32 *d_nres = ar.get<u32>(2);
-        CUDA_CHECK(cudaMemsetAsync(d_nres, 0, 8, st));
-        const int skip_pairs = (u64)m * 64 > (u64)len ? 1 : 0;
-        // (when most suffixes are active the groups are usually giant -- periodic texts: a cheap look first)
-        u32 nsmall = 1;
-        if ((u64)m * 2 > (u64)len) {
-            count_small_groups_kernel<<<div_up_u(m, 256), 256, 0, st>>>(grp, m, skip_pairs, d_nres + 1);
-            KERNEL_CHECK();
-            read_back(&nsmall, d_nres + 1, 4, st);
-            if ((u64)nsmall * 64 < (u64)m) nsmall = 0;  // (a trip over the whole list for a sprinkle of small groups: the rounds take them)
-        }
-        if (nsmall) {
-            // the permuted list goes into a buffer that is dead until the rounds write their keys (both m <= len words)
-            u8 *keep8 = ar.get<u8>((size_t)m + 64);
-            u32 *act_p = (u32 *)rk_free[0], *row_p = act_p + (((size_t)m + 3) & ~(size_t)3);  // (vector stores: 16-byte aligned)
-            u32 *act_old = act, *grp_old = grp;
-            resolve_small_groups_kernel<<<div_up_u(m, 256), 256, 0, st>>>(act, grp, m, ix.packed, b, K, n, skip_pairs, sa,
-                                                                          done0 ? nullptr : rank, act_p, row_p, bwt_rows,
-                                                                          d_primary.ptr, keep8, d_nres);
-            KERNEL_CHECK();
-            u32 nres = 0;
-            read_back(&nres, d_nres, 4, st);
-            ix.stats.resolved_small = nres;
-            // (the permuted list replaces the old one even when nothing was decided: sub-groups may have formed)
-            act0 = act_p;
-            row0 = row_p;
-            // the list the rounds start from goes back into the buffers of the old one (dead now); act0 / row0 stay
-            // where they are until the ranks have been scattered
-            if (nres && done0 && nres < m) {
-                // the suffixes decided here are final but their rows still count as "active after round 0": when rounds
-                // follow, their ranks are materialised now (the pair path below may replace the list the other ranks
-                // are scattered from)
-                CUDA_CHECK(cudaMemsetAsync(rank, 0xff, (size_t)len * 4, st));
-                scatter_ranks_left_kernel<<<div_up_u(m, 256), 256, 0, st>>>(act_p, row_p, keep8, m, rank);
-                KERNEL_CHECK();
-                rank_marked = true;
-            }
-            const bool pairs_next = done0 && rk_free[1] && pairs_mode && ((u64)m * 64 >= (u64)len || pairs_mode == 2);
-            if (nres && nres < m && pairs_next) {
-                deferred = true;
-                dl_act = act_p; dl_row = row_p; dl_keep = keep8; dl_nres = nres;
-            } else if (nres) {
-                const u64 kw = ((u64)m + 63) / 64;
-                CUDA_CHECK(cudaMemsetAsync(headbits, 0, (kw + 2) * 8, st));
-                bytes_to_bits_kernel<<<div_up_u(kw, 256), 256, 0, st>>>(keep8, m, (u64 *)headbits, kw);
-                KERNEL_CHECK();
-                const u32 m2 = count_active<true>(headbits, m, tile_counts, d_total, st);
-                if (m2) scatter_active<true>(headbits, act_p, row_p, m, tile_counts, act_old, grp_old, st);
-                m = m2;
-            } else {
-                CUDA_CHECK(cudaMemcpyAsync(act_old, act_p, (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
-                CUDA_CHECK(cudaMemcpyAsync(grp_old, row_p, (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
-            }
-        }
-        ix.timer.end(t);
-    }
-    // (the list the pair path reads: the permuted one when the tie-break left its compaction to this path)
-    const u32 *pl_act = deferred ? dl_act : act, *pl_grp = deferred ? dl_row : grp;
-    bool pairs_done = false;
-    if (m && done0 && rk_free[1] && b <= 8 && pairs_mode && ((u64)m * 64 >= (u64)len || pairs_mode == 2)) {
-        // pairs of a text with long exact repeats: decided by one comparison per copied segment (pair_runs_kernel)
-        t = ix.timer.begin("pair_partner", (double)m * 16.0 + (double)len * 4.0);
-        const size_t pt_entries = (size_t)len + PR_CAP + 2 * PR_TILE + 16;
-        const size_t pt_padded = (pt_entries + 127) & ~(size_t)127;
-        const size_t ord_bytes = (((size_t)len + PR_TILE) / PR_TILE + 1) * PR_TILE;
-        // (in the round-key buffer that is free now when the text is long enough for the padding to fit, else carved)
-        u32 *partner = pt_padded * 4 + ord_bytes <= ((size_t)len + 2) * 8 ? (u32 *)rk_free[1]
-                                                                        : (u32 *)ar.get<u8>(pt_padded * 4 + ord_bytes);
-        u8 *ord = (u8 *)(partner + pt_padded);
-        u32 *d_pr = ar.get<u32>(2);
-        CUDA_CHECK(cudaMemsetAsync(partner, 0xff, pt_entries * 4, st));
-        CUDA_CHECK(cudaMemsetAsync(d_pr, 0, 8, st));
-        pair_partner_kernel<<<div_up_u(m, 256 * PQ), 256, 0, st>>>(pl_act, pl_grp, m, partner, d_pr);
-        KERNEL_CHECK();
-        u32 npairs = 0;
-        read_back(&npairs, d_pr, 4, st);
-        ix.timer.end(t);
-        if (npairs && ((u64)npairs * 8 >= (u64)m || pairs_mode == 2)) {  // (two members each: at least a quarter of the list)
-            t = ix.timer.begin("pair_runs", (double)len * 5.0);
-            CUDA_CHECK(cudaMemsetAsync(ord, 0, ord_bytes, st));
-            pair_runs_kernel<<<div_up_u(len, PR_TILE), PR_NT, 0, st>>>(partner, n, ix.packed, b, K, ord);
-            KERNEL_CHECK();
-            ix.timer.end(t);
-            t = ix.timer.begin("pair_place", (double)m * 14.0);
-            u8 *keep8 = ar.get<u8>((size_t)m + 64);
-            pair_place_kernel<<<div_up_u(m, 256 * PQ), 256, 0, st>>>(pl_act, pl_grp, m, ord, sa, bwt_rows, actbits, d_primary.ptr,
-                                                                    deferred ? dl_keep : nullptr, keep8, d_pr + 1);
-            KERNEL_CHECK();
-            u32 nplaced = 0;
-            read_back(&nplaced, d_pr + 1, 4, st);
-            ix.stats.pair_placed = nplaced;
-            ix.timer.end(t);
-            t = ix.timer.begin("pair_compact", (double)m * 10.0);
-            if (nplaced) {
-                // the rest of the list (its ranks are the only ones that are needed: only suffixes that stay active get
-                // one).  From the tie-break's permuted list it goes straight into the list's own buffers; else through
-                // the buffer that held the list round 0 left
-                const u64 kw = ((u64)m + 63) / 64;
-                CUDA_CHECK(cudaMemsetAsync(headbits, 0, (kw + 2) * 8, st));
-                bytes_to_bits_kernel<<<div_up_u(kw, 256), 256, 0, st>>>(keep8, m, (u64 *)headbits, kw);
-                KERNEL_CHECK();
-                const u32 m2 = count_active<true>(headbits, m, tile_counts, d_total, st);
-                if (m2 != m - nplaced - (deferred ? dl_nres : 0u))
-                    throw std::runtime_error("pair path: list accounting is inconsistent (internal error)");
-                if (m2 && deferred) {
-                    scatter_active<true>(headbits, pl_act, pl_grp, m, tile_counts, const_cast<u32 *>(act), grp, st);
-                } else if (m2) {
-                    u32 *tmpA = (u32 *)rk_free[0], *tmpB = tmpA + m;
-                    scatter_active<true>(headbits, act, grp, m, tile_counts, tmpA, tmpB, st);
-                    CUDA_CHECK(cudaMemcpyAsync(const_cast<u32 *>(act), tmpA, (size_t)m2 * 4, cudaMemcpyDeviceToDevice, st));
-                    CUDA_CHECK(cudaMemcpyAsync(grp, tmpB, (size_t)m2 * 4, cudaMemcpyDeviceToDevice, st));
-                }
-                m = m2;
-                act0 = act;
-                row0 = grp;
-                m0 = m;
-                pairs_done = true;
-                if (env_int("B200SA_DEBUG_RESIDUAL", 0) && m) {  // (development aid: what the pair path left)
-                    u32 h[2] = {0, 0};
-                    CUDA_CHECK(cudaMemsetAsync(d_pr, 0, 8, st));
-                    count_small_groups_kernel<<<div_up_u(m, 256), 256, 0, st>>>(grp, m, 0, d_pr);
-                    count_small_groups_kernel<<<div_up_u(m, 256), 256, 0, st>>>(grp, m, 1, d_pr + 1);
-                    read_back(h, d_pr, 8, st);
-                    fprintf(stderr, "[b200sa] after the pair path: %u of %u placed, %u left: %u in groups of 2..4 (%u in 3..4)\n",
-                            nplaced, m + nplaced, m, h[0], h[1]);
-                }
-            }
-            ix.timer.end(t);
-        }
-    }
-    if (deferred && !pairs_done) {
-        // the pair path placed nothing: the tie-break's own compaction after all
-        t = ix.timer.begin("resolve_small", (double)m * 16.0);
-        const u64 kw = ((u64)m + 63) / 64;
-        CUDA_CHECK(cudaMemsetAsync(headbits, 0, (kw + 2) * 8, st));
-        bytes_to_bits_kernel<<<div_up_u(kw, 256), 256, 0, st>>>(dl_keep, m, (u64 *)headbits, kw);
-        KERNEL_CHECK();
-        const u32 m2 = count_active<true>(headbits, m, tile_counts, d_total, st);
-        if (m2) scatter_active<true>(headbits, dl_act, dl_row, m, tile_counts, const_cast<u32 *>(act), grp, st);
-        m = m2;
-        ix.timer.end(t);
-    }
-    if (m && done0) {
-        // bucketed round 0: ranks of the suffixes that were active after it (first row of their group, or their final
-        // row where the text decided); everything else is marked "not materialised" first.  A text without repeats
-        // never gets here: its few chance collisions are all decided above.  (LSD round 0: rank_kernel wrote the ranks,
-        // the kernel above kept them up to date.)
-        t = ix.timer.begin("rank_scatter", (double)m0 * 12.0 + (double)len * 4.0);
-        if (!rank_marked) CUDA_CHECK(cudaMemsetAsync(rank, 0xff, (size_t)len * 4, st));
-        scatter_ranks_kernel<<<div_up_u(m0, 256), 256, 0, st>>>(act0, row0, m0, short_rank, rank);
-        KERNEL_CHECK();
-        ix.timer.end(t);
-    }
-    if (m) {
-        // complete ranks ("dense") from the start when most suffixes are active; otherwise ranks of
-        // retired suffixes are recovered on demand, until a round needs many of them
-        auto go_dense = [&]() {
-            int tt = ix.timer.begin("rank0_fill", (double)len * 16.0);
-            fill_singleton_ranks(ix, actbits, rank);
-            ix.timer.end(tt);
-            lr.sparse = false;
-        };
-        if ((u64)m * 2 > (u64)len) {
-            go_dense();
-            if (!done0) rk_free[1] = const_cast<u64 *>(lr.keys0);  // the sorted round-0 keys are dead now
-        }
-        u64 *rkA = rk_free[0] ? rk_free[0] : ar.get<u64>(m);
-        u64 *rkB = rk_free[1] ? rk_free[1] : ar.get<u64>(m);
-        u32 *act2 = ar.get<u32>(m), *grp2 = ar.get<u32>(m);
-        const int lo_bits = std::max(1, log2len);
-        const int key_bits = std::min(64, 2 * lo_bits);
-        u64 h = depth0 ? (u64)depth0 : (u64)K;
-        u32 huniform[8];
-        const u32 bwt_small = std::max(1u, len / (u32)std::max(1, env_int("B200SA_BWT_ROUND_FRAC", 32)));
-        // One region serves the chain arrays (live from chain_flags to make_keys) and the outputs of the
-        // small-group path (live from there to the end of the round).
-        bool chain_on = env_int("B200SA_CHAIN", 1) != 0 &&
-                        (u64)m * (u64)std::max(1, env_int("B200SA_CHAIN_MIN_FRAC", 64)) >= (u64)len;
-        bool small_on = env_int("B200SA_SMALL_PATH", 1) != 0;
-        bool pivot_on = env_int("B200SA_PIVOT", 1) != 0;
-        int small_pause = 0, small_fails = 0;  // rounds the small-group path sits out after finding almost nothing
-        int pivot_pause = 0, pivot_fails = 0;  // the same for the pivot path
-        bool ids_are_heads = true;             // rank[] of an active suffix is the first row of its group (until the pivot path runs)
-        const size_t cont_bytes = ((size_t)len + 2 * (size_t)CHAIN_CAP + 8192 + 511) & ~(size_t)511;
-        const size_t m_init = m;
-        const size_t third = (m_init * 4 + 64 + 511) & ~(size_t)511;
-        size_t chain_bytes = chain_on ? cont_bytes + (size_t)len * 4 + ((m_init + 511) & ~(size_t)511) : 0;
-        size_t split_bytes = (small_on || pivot_on) ? 3 * third : 0;
-        // the optional paths are dropped, the larger first, rather than running the device out of memory
-        const size_t mem_margin = (size_t)2 << 30;
-        if (split_bytes > chain_bytes && !ar.can_fit(split_bytes, mem_margin)) {
-            split_bytes = 0;
-            small_on = pivot_on = false;
-        }
-        if (chain_bytes && !ar.can_fit(std::max(chain_bytes, split_bytes), mem_margin)) {
-            chain_bytes = 0;
-            chain_on = false;
-            if (split_bytes && !ar.can_fit(split_bytes, mem_margin)) {
-                split_bytes = 0;
-                small_on = pivot_on = false;
-            }
-        }
-        u8 *region = ar.get<u8>(std::max<size_t>(std::max(chain_bytes, split_bytes), 512));
-        u8 *cont8 = region, *cslot = region + cont_bytes + (size_t)len * 4;
-        u32 *chainkey = (u32 *)(region + cont_bytes);
-        // three list-sized buffers of the split paths; `r0` changes places with the list when the pivot path has
-        // assembled the next one there (every list buffer holds m_init words) -- from then on the region holds a
-        // list and the chain arrays, which share it, are not used any more
-        u32 *r0 = (u32 *)region, *newgrpT = (u32 *)(region + third), *bvals = (u32 *)(region + 2 * third);
-        u32 *d_ncont = ar.get<u32>(4), *d_handled = d_ncont + 1, *d_nheads = d_ncont + 2;
-        const size_t bm_bytes = ((m_init + 63) / 64 + 2) * 8;
-        u8 *notdone = ar.get<u8>(bm_bytes), *headB = ar.get<u8>(bm_bytes);
-        // pivot path: per-group tables by (head row) / 2, E bitmap, per-tile counts
-        const size_t pv_entries = (size_t)len / 2 + 2;
-        if (pivot_on && !ar.can_fit(pv_entries * 12 + 2 * bm_bytes, mem_margin)) pivot_on = false;
-        u8 *ebits8 = pivot_on ? ar.get<u8>(bm_bytes) : nullptr;
-        u32 *pv_tile_e = pivot_on ? ar.get<u32>((size_t)div_up_u(m_init, PV_TILE) + 2) : nullptr;
-        u8 *rbits8 = pivot_on ? ar.get<u8>(bm_bytes) : nullptr;
-        unsigned long long *d_pvtot = ar.get<unsigned long long>(2);
-        unsigned long long *pv_cnt = pivot_on ? ar.get<unsigned long long>(pv_entries) : nullptr;
-        u32 *pv_piv = pivot_on ? ar.get<u32>(pv_entries) : nullptr;
-        // large groups or small ones?  (decides which of the two split paths a round tries first)
-        const u32 pivot_min = (u32)std::max(2, env_int("B200SA_PIVOT_MIN", 1 << 16));
-        const bool pivot_force = env_int("B200SA_PIVOT_FORCE", 0) != 0;  // (tests: every round, whatever it finds)
-        const u32 pivot_sub_min = std::max(2u, pivot_min / 16u);  // lists of the pivot path that are split again
-        bool prefer_pivot = pivot_force;
-        if (pivot_on && !pivot_force && m >= pivot_min) {
-            CUDA_CHECK(cudaMemsetAsync(d_nheads, 0, 4, st));
-            count_heads_kernel<<<std::max(1u, std::min(div_up_u(m, 256 * 8), 148u * 8u)), 256, 0, st>>>(grp, m, d_nheads);
-            KERNEL_CHECK();
-            u32 nheads = 0;
-            read_back(&nheads, d_nheads, 4, st);
-            prefer_pivot = (u64)nheads * 64 <= (u64)m;
-        }
-        while (m > 0) {
-            ix.stats.rounds++;
-            ix.stats.sorted_total += m;
-            CUDA_CHECK(cudaMemsetAsync(d_lazy, 0, 4, st));
-            // ---- chain offsets (see chain_flags_kernel): tried while the active set is a noticeable part of the
-            // text, dropped for good once a round finds few groups that continue ----
-            bool use_chain = false;
-            if (chain_on && h <= (u64)CHAIN_CAP && (u64)m * (u64)std::max(1, env_int("B200SA_CHAIN_MIN_FRAC", 64)) >= (u64)len) {
-                t = ix.timer.begin("chain_flags", (double)m * 13.0 + (double)len);
-                CUDA_CHECK(cudaMemsetAsync(cont8, 0, cont_bytes, st));
-                CUDA_CHECK(cudaMemsetAsync(cslot, 0, m, st));
-                CUDA_CHECK(cudaMemsetAsync(d_ncont, 0, 4, st));
-                const u32 cf_tiles = div_up_u(m, CF_STEP);
-                u32 ncont = 0;
-                bool worth = true;
-                if (cf_tiles > 16384) {
-                    // a sample of 2 048 tiles first: a list whose groups do not continue (diverged copies, periodic
-                    // texts) is not worth the full pass (what the sample marks is what the full pass would mark)
-                    const u32 mul = cf_tiles / 2048;
-                    chain_flags_kernel<<<2048, CF_NT, 0, st>>>(act, grp, m, rank, cslot, cont8, d_ncont, mul);
-                    KERNEL_CHECK();
-                    read_back(&ncont, d_ncont, 4, st);
-                    worth = (u64)ncont * (u64)std::max(1, env_int("B200SA_CHAIN_USE_FRAC", 2)) * 2 >= (u64)2048 * CF_STEP;
-                    CUDA_CHECK(cudaMemsetAsync(d_ncont, 0, 4, st));
-                    ncont = 0;
-                }
-                if (worth) {
-                    chain_flags_kernel<<<cf_tiles, CF_NT, 0, st>>>(act, grp, m, rank, cslot, cont8, d_ncont, 1);
-                    KERNEL_CHECK();
-                    read_back(&ncont, d_ncont, 4, st);
-                }
-                ix.timer.end(t);
-                // worth it when most groups continue (copies of long segments); texts whose groups are large and
-                // shallow (many diverged copies) gain nothing from it
-                if ((u64)ncont * (u64)std::max(1, env_int("B200SA_CHAIN_USE_FRAC", 2)) >= (u64)m) {
-                    t = ix.timer.begin("chain_keys", (double)len + (double)ncont * 4.0);
-                    chain_keys_kernel<<<div_up_u(len, CK_TILE), CK_NT, 0, st>>>(cont8, len, lr, h, chainkey, d_lazy);
-                    KERNEL_CHECK();
-                    ix.timer.end(t);
-                    use_chain = true;
-                    ix.stats.chain_rounds++;
-                    ix.stats.chain_elems += ncont;
-                } else {
-                    chain_on = false;
-                }
-            }
-            t = ix.timer.begin("round_keys", (double)m * 16.0);
-            const bool try_pivot = pivot_on && prefer_pivot && pivot_pause == 0 && m >= pivot_min;
-            if (lr.sparse)
-                make_keys_round_kernel<<<std::max(1u, std::min(div_up_u(m, 256 * 4), 148u * 16u)), 256, 0, st>>>(
-                    act, grp, m, lr, h, lo_bits, use_chain ? cslot : nullptr, chainkey, rkA, d_lazy,
-                    try_pivot ? pv_piv : nullptr, pv_cnt);
-            else
-                make_keys_dense_kernel<<<std::max(1u, std::min(div_up_u(m, 256 * 4), 148u * 16u)), 256, 0, st>>>(
-                    act, grp, m, rank, h, len, lo_bits, use_chain ? cslot : nullptr, chainkey, rkA,
-                    try_pivot ? pv_piv : nullptr, pv_cnt);
-            KERNEL_CHECK();
-            ix.timer.end(t);
-
-            // ---- large groups that mostly stay together: split around a pivot key (pivot_classify_kernel).  The
-            // E part of every group goes straight into the next list; its L members and its R members, each
-            // compacted into a list of their own, are split again the same way (a group whose members carry two
-            // or three distinct second keys -- a Fibonacci string -- never reaches the radix sort); lists that are
-            // small, or whose groups scatter, are sorted ----
-            bool pivoted = false;
-            u32 m2 = 0;
-            if (try_pivot) {
-                const int key_bits_here = key_bits;
-                PivotArgs base{};
-                base.lo_bits = lo_bits; base.piv = pv_piv; base.cnt64 = pv_cnt; base.ebits8 = ebits8; base.lbits8 = notdone;
-                base.rbits8 = rbits8; base.tile_e = pv_tile_e; base.totals = d_pvtot; base.sa = sa; base.rank = rank;
-                base.primary = d_primary.ptr; base.singles = d_nheads;
-                u32 out_n = 0;           // entries of the next list (r0 / grp2) written so far
-                u64 pv_e = 0, pv_sorted = 0;
-                auto classify = [&](u64 *kx, const u32 *vx, u32 n, bool publish, u32 &ne, u32 &nl) {
-                    PivotArgs pv = base;
-                    pv.keys = kx; pv.act = vx; pv.m = n;
-                    const u32 ntl = div_up_u(n, PV_TILE);
-                    const u64 kw = ((u64)n + 63) / 64;
-                    CUDA_CHECK(cudaMemsetAsync(ebits8 + kw * 8, 0, 16, st));
-                    CUDA_CHECK(cudaMemsetAsync(notdone + kw * 8, 0, 16, st));
-                    CUDA_CHECK(cudaMemsetAsync(rbits8 + kw * 8, 0, 16, st));
-                    CUDA_CHECK(cudaMemsetAsync(d_pvtot, 0, 16, st));
-                    if (publish) {
-                        pivot_heads_kernel<<<div_up_u(n, PV_TILE), PV_NT, 0, st>>>(kx, n, lo_bits, pv_piv, pv_cnt);
-                        KERNEL_CHECK();
-                    }
-                    pivot_classify_kernel<<<ntl, PV_NT, 0, st>>>(pv);
-                    KERNEL_CHECK();
-                    scan_tiles_kernel<<<1, 1024, 0, st>>>(pv_tile_e, ntl, d_pvtot);
-                    KERNEL_CHECK();
-                    unsigned long long tot[2] = {0, 0};
-                    read_back(tot, d_pvtot, 16, st);
-                    ne = (u32)tot[0];
-                    nl = (u32)tot[1];
-                };
-                // radix sort of one list, new ranks, survivors appended to the next list
-                auto sort_list = [&](u64 *kx, u32 *vx, u32 n, u64 *ky, u32 *vy, u32 *ng) {
-                    int npass = (key_bits_here + RB - 1) / RB;
-                    int tt = ix.timer.begin("round_hist", (double)n * 8.0);
-                    S::histogram(kx, n, 0, key_bits_here, npass, hist, st);
-                    S::scan(hist, n, npass, uniform, st);
-                    read_back(huniform, uniform, (size_t)npass * 4, st);
-                    ix.timer.end(tt);
-                    u64 *rin = kx, *rout = ky;
-                    u32 *ain = vx, *aout = vy;
-                    for (int p = 0; p < npass; ++p) {
-                        if (huniform[p]) continue;
-                        int bits_here = std::min(RB, key_bits_here - p * RB);
-                        tt = ix.timer.begin("radix_pass", (double)n * 24.0);
-                        S::pass(rin, ain, rout, aout, n, p * RB, bits_here, hist + (size_t)p * BINS, lookback, ticket, st);
-                        ix.timer.end(tt);
-                        ix.stats.passes_elems += n;
-                        std::swap(rin, rout);
-                        std::swap(ain, aout);
-                    }
-                    tt = ix.timer.begin("round_rank", (double)n * 20.0);
-                    CUDA_CHECK(cudaMemsetAsync(headB, 0, (((size_t)n + 63) / 64 + 2) * 8, st));
-                    RankArgs rr{};
-                    rr.keys = rin; rr.vals = ain; rr.m = n; rr.gs = lo_bits; rr.keymask = ~0ull; rr.K0 = 0; rr.n = ix.n;
-                    rr.rank = rank; rr.newgrp = ng; rr.scatter_all = 0; rr.sa_out = sa; rr.headbits = headB;
-                    rr.bwt = nullptr; rr.prev_shift = 0; rr.packed = ix.packed; rr.bits = b;
-                    rr.primary = d_primary.ptr;
-                    rr.always_write = 1;
-                    rank_kernel<<<div_up_u(n, RK_TILE), RK_NT, 0, st>>>(rr);
-                    KERNEL_CHECK();
-                    ix.timer.end(tt);
-                    tt = ix.timer.begin("compact", (double)n * 4.0);
-                    const u32 mB = count_active<false>(headB, n, tile_counts, d_total, st);
-                    if (mB) scatter_active<false>(headB, ain, ng, n, tile_counts, r0 + out_n, grp2 + out_n, st);
-                    out_n += mB;
-                    pv_sorted += n;
-                    ix.timer.end(tt);
-                };
-                // one list: keys / values in (kx, vx); (ky, vy) = the other buffer pair over the same index range;
-                // ng = as many free words (new ranks by sorted index)
-                std::function<void(int, u64 *, u32 *, u32, u64 *, u32 *, u32 *, u32, u32)> process;
-                process = [&](int level, u64 *kx, u32 *vx, u32 n, u64 *ky, u32 *vy, u32 *ng, u32 ne, u32 nl) {
-                    // (level 0 arrives classified)
-                    bool go = level == 0;
-                    if (level > 0 && level < 8 && n >= pivot_sub_min) {
-                        int tt = ix.timer.begin("pivot_classify", (double)n * 16.0);
-                        classify(kx, vx, n, true, ne, nl);
-                        ix.timer.end(tt);
-                        go = (u64)ne * 3 >= (u64)n || pivot_force;
-                    }
-                    if (!go) {
-                        sort_list(kx, vx, n, ky, vy, ng);
-                        return;
-                    }
-                    int tt = ix.timer.begin("pivot_apply", (double)n * 24.0);
-                    PivotArgs pv = base;
-                    pv.keys = kx; pv.act = vx; pv.m = n;
-                    pv.out_act = r0 + out_n; pv.out_grp = grp2 + out_n; pv.out_base = out_n; pv.dropbits = (u32 *)headbits;
-                    pivot_apply_kernel<<<div_up_u(n, PV_TILE), PV_NT, 0, st>>>(pv);
-                    KERNEL_CHECK();
-                    ix.timer.end(tt);
-                    out_n += ne;
-                    pv_e += ne;
-                    const u32 nr = n - ne - nl;
-                    if (nl | nr) {
-                        tt = ix.timer.begin("compact_big", (double)n * 0.25 + (double)(nl + nr) * 24.0);
-                        const u32 sub = compaction_sub(n);
-                        if (nl) {
-                            const u32 cnt = count_active<true>(notdone, n, tile_counts, d_total, st);
-                            if (cnt != nl) throw std::runtime_error("pivot path: L members miscounted (internal error)");
-                            scatter_pairs_kernel<<<div_up_u(n, (u64)CP_TILE * sub), CP_NT, 0, st>>>(notdone, kx, vx, n, sub, tile_counts, ky, vy);
-                            KERNEL_CHECK();
-                        }
-                        if (nr) {
-                            const u32 cnt = count_active<true>(rbits8, n, tile_counts, d_total, st);
-                            if (cnt != nr) throw std::runtime_error("pivot path: R members miscounted (internal error)");
-                            scatter_pairs_kernel<<<div_up_u(n, (u64)CP_TILE * sub), CP_NT, 0, st>>>(rbits8, kx, vx, n, sub, tile_counts, ky + nl, vy + nl);
-                            KERNEL_CHECK();
-                        }
-                        ix.timer.end(tt);
-                        if (nl) process(level + 1, ky, vy, nl, kx, vx, ng, 0, 0);
-                        if (nr) process(level + 1, ky + nl, vy + nl, nr, kx + nl, vx + nl, ng + nl, 0, 0);
-                    }
-                };
-                t = ix.timer.begin("pivot_classify", (double)m * 16.0);
-                u32 n_e = 0, n_l = 0;
-                classify(rkA, act, m, false, n_e, n_l);
-                ix.timer.end(t);
-                if ((u64)n_e * 3 >= (u64)m || pivot_force) {
-                    pivoted = true;
-                    ids_are_heads = false;
-                    chain_on = false;
-                    pivot_fails = 0;
-                    CUDA_CHECK(cudaMemsetAsync(d_nheads, 0, 4, st));
-                    CUDA_CHECK(cudaMemsetAsync(headbits, 0, (((size_t)m + 63) / 64 + 2) * 8, st));  // (no entry of the next list is dropped)
-                    // (the old list is dead once its L and R members have been copied out: its value buffer is the
-                    // scratch of the deeper levels; the old group heads are dead already, the keys carry them)
-                    process(0, rkA, const_cast<u32 *>(act), m, rkB, bvals, grp, n_e, n_l);
-                    ix.stats.sorted_total -= (u64)m - pv_sorted;
-                    ix.stats.pivot_rounds++;
-                    ix.stats.pivot_elems += pv_e;
-                    if (bwt_rows) need_bwt_fix = true;  // (this path does not write BWT rows)
-                    // E groups of one member are final: out of the list (rare; through two buffers that are free now)
-                    u32 n_single = 0;
-                    read_back(&n_single, d_nheads, 4, st);
-                    m2 = out_n;
-                    if (n_single) {
-                        // the survivors are copied to the old list's buffers (free now), which stay the list
-                        t = ix.timer.begin("compact", (double)out_n * 16.0);
-                        const u64 kw = ((u64)out_n + 63) / 64;
-                        pivot_keep_kernel<<<div_up_u(kw, 256), 256, 0, st>>>((u64 *)headbits, out_n, kw);
-                        KERNEL_CHECK();
-                        m2 = count_active<true>(headbits, out_n, tile_counts, d_total, st);
-                        if (m2 != out_n - n_single) throw std::runtime_error("pivot path: single-member groups miscounted (internal error)");
-                        if (m2) scatter_active<true>(headbits, r0, grp2, out_n, tile_counts, const_cast<u32 *>(act), newgrpT, st);
-                        std::swap(grp2, newgrpT);
-                        ix.timer.end(t);
-                    } else {
-                        std::swap(act, r0);
-                    }
-                } else {  // the groups scatter: nothing was changed, the round goes on as usual; back off 2, 4, 8 ... rounds
-                    pivot_pause = 2 << std::min(pivot_fails, 4);
-                    ++pivot_fails;
-                }
-            } else if (pivot_pause > 0) {
-                --pivot_pause;
-            }
-
-            if (!pivoted) {
-            // ---- groups of up to RS_GMAX members are ordered where they stand (round_small_kernel) ----
-            u32 handled = 0;
-            if (small_on && small_pause == 0) {
-                t = ix.timer.begin("round_small", (double)m * 28.0);
-                const u64 kw = ((u64)m + 63) / 64;
-                CUDA_CHECK(cudaMemsetAsync(headbits + kw * 8, 0, 16, st));
-                CUDA_CHECK(cudaMemsetAsync(notdone + kw * 8, 0, 16, st));
-                CUDA_CHECK(cudaMemsetAsync(d_handled, 0, 4, st));
-                SmallArgs sm{};
-                sm.act = act; sm.grp = grp; sm.keys = rkA; sm.m = m; sm.lo_bits = lo_bits; sm.sa = sa; sm.rank = rank;
-                sm.vals_out = r0; sm.newgrp_out = newgrpT; sm.headbits64 = (u64 *)headbits; sm.notdone64 = (u64 *)notdone;
-                sm.primary = d_primary.ptr; sm.handled = d_handled; sm.always_write = ids_are_heads ? 0 : 1;
-                round_small_kernel<<<div_up_u(m, RS_STEP), RS_NT, 0, st>>>(sm);
-                KERNEL_CHECK();
-                read_back(&handled, d_handled, 4, st);
-                ix.timer.end(t);
-                ix.stats.small_path_elems += handled;
-                if ((u64)handled * 32 < (u64)m) {  // (periodic texts: a few giant groups) -- back off 3, 6, 12 ... rounds
-                    small_pause = 3 << std::min(small_fails, 4);
-                    ++small_fails;
-                    prefer_pivot = true;  // (large groups: the pivot path is the one to try)
-                }
-                if (handled && bwt_rows) need_bwt_fix = true;     // (this path does not write BWT rows)
-            } else if (small_pause > 0) {
-                --small_pause;
-            }
-            const bool split = handled != 0;  // part of the list has been placed without the sort
-
-            // ---- everything else: radix sort of (group, rank) keys, new ranks from the sorted list ----
-            const u32 mb = m - handled;
-            const u64 *bk = rkA;   // keys / values of the elements that go through the sort
-            const u32 *bv = act;
-            u64 *k_other = rkB;
-            u32 *v_other = act2;
-            if (split && mb) {
-                t = ix.timer.begin("compact_big", (double)m * 0.125 + (double)mb * 24.0);
-                const u32 cnt = count_active<true>(notdone, m, tile_counts, d_total, st);
-                if (cnt != mb) throw std::runtime_error("split paths: slot accounting is inconsistent (internal error)");
-                const u32 sub = compaction_sub(m);
-                scatter_pairs_kernel<<<div_up_u(m, (u64)CP_TILE * sub), CP_NT, 0, st>>>(notdone, rkA, act, m, sub, tile_counts,
-                                                                                       rkB, bvals);
-                KERNEL_CHECK();
-                ix.timer.end(t);
-                bk = rkB; bv = bvals; k_other = rkA; v_other = act2;
-            }
-            u8 *hb_big = split ? headB : headbits;
-            const u32 *sorted_vals = nullptr;
-            if (mb) {
-                int npass = (key_bits + RB - 1) / RB;
-                t = ix.timer.begin("round_hist", (double)mb * 8.0);
-                S::histogram(bk, mb, 0, key_bits, npass, hist, st);
-                S::scan(hist, mb, npass, uniform, st);
-                read_back(huniform, uniform, (size_t)npass * 4, st);
-                ix.timer.end(t);
-                u64 *rin = const_cast<u64 *>(bk), *rout = k_other;
-                u32 *ain = const_cast<u32 *>(bv), *aout = v_other;
-                for (int p = 0; p < npass; ++p) {
-                    if (huniform[p]) continue;
-                    int bits_here = std::min(RB, key_bits - p * RB);
-                    t = ix.timer.begin("radix_pass", (double)mb * 24.0);
-                    S::pass(rin, ain, rout, aout, mb, p * RB, bits_here, hist + (size_t)p * BINS, lookback, ticket, st);
-                    ix.timer.end(t);
-                    ix.stats.passes_elems += mb;
-                    std::swap(rin, rout);
-                    std::swap(ain, aout);
-                }
-                t = ix.timer.begin("round_rank", (double)mb * 20.0);
-                size_t hbm = (((size_t)mb + 63) / 64 + 2) * 8;
-                CUDA_CHECK(cudaMemsetAsync(hb_big, 0, hbm, st));
-                RankArgs rr{};
-                rr.keys = rin; rr.vals = ain; rr.m = mb; rr.gs = lo_bits; rr.keymask = ~0ull; rr.K0 = 0; rr.n = n;
-                rr.rank = rank; rr.newgrp = grp; rr.scatter_all = 0; rr.sa_out = sa; rr.headbits = hb_big;  // (newgrp: the old heads are dead, the keys carry them)
-                // BWT rows of moved suffixes: one gather per element and round -- kept in the rounds while the
-                // active set is small, otherwise one pass over the rows of round 0's active set at the end
-                rr.bwt = m <= bwt_small ? bwt_rows : nullptr;
-                if (bwt_rows && !rr.bwt) need_bwt_fix = true;
-                rr.prev_shift = 0; rr.packed = ix.packed; rr.bits = b;
-                rr.primary = d_primary.ptr;
-                rr.always_write = ids_are_heads ? 0 : 1;
-                rank_kernel<<<div_up_u(mb, RK_TILE), RK_NT, 0, st>>>(rr);
-                KERNEL_CHECK();
-                ix.timer.end(t);
-                sorted_vals = ain;
-            }
-            // ---- next active set: the survivors of both paths, one after the other (groups stay contiguous) ----
-            t = ix.timer.begin("compact", (double)m * 4.0);
-            if (!handled) {
-                // (the whole list went through the sort: its survivors go to the value buffer the sort left free)
-                u32 *dst = sorted_vals == act ? act2 : const_cast<u32 *>(act);
-                m2 = count_active<false>(hb_big, m, tile_counts, d_total, st);
-                if (m2) scatter_active<false>(hb_big, sorted_vals, grp, m, tile_counts, dst, grp2, st);
-                if (dst == act2) std::swap(act, act2);
-            } else {
-                // (`act` was read for the last time by the compaction of the sorted part)
-                u32 *dst = sorted_vals == act ? act2 : const_cast<u32 *>(act);
-                if (mb && sorted_vals == act) {
-                    // the sorted values sit in `act` itself: survivors go to act2
-                }
-                const u32 mA = count_active<false>(headbits, m, tile_counts, d_total, st);
-                if (mA) scatter_active<false>(headbits, r0, newgrpT, m, tile_counts, dst, grp2, st);
-                u32 mB = 0;
-                if (mb) {
-                    mB = count_active<false>(hb_big, mb, tile_counts, d_total, st);
-                    if (mB) scatter_active<false>(hb_big, sorted_vals, grp, mb, tile_counts, dst + mA, grp2 + mA, st);
-                }
-                m2 = mA + mB;
-                if (dst == act2) std::swap(act, act2);
-            }
-            ix.timer.end(t);
-            }  // !pivoted
-            u32 nlazy = 0;
-            read_back(&nlazy, d_lazy, 4, st);
-            ix.stats.lazy_lookups += nlazy;
-            std::swap(grp, grp2);
-            m = m2;
-            h *= 2;
-            if (h > (u64)len * 2 + 2 && m > 0)
-                throw std::runtime_error("prefix doubling failed to converge (internal error)");
-            // a lookup costs several random accesses, completing the ranks one random store per suffix
-            if (m > 0 && lr.sparse && (u64)nlazy * (u64)std::max(1, env_int("B200SA_DENSE_FACTOR", 12)) > (u64)len) {
-                go_dense();
-            }
-        }
-    }
-    if (need_bwt_fix) {
-        t = ix.timer.begin("bwt_fix", (double)len * 0.125);
-        // rows still marked: those round 0 left active minus the ones the pair path made final
-        const u64 marked = (u64)m_round0 - (u64)ix.stats.pair_placed;
-        if (marked * 8 > (u64)len)
-            bwt_fix_rows_kernel<<<div_up_u(len, 256), 256, 0, st>>>(actbits, sa, len, ix.packed, b, ix.bwt.ptr, d_primary.ptr);
-        else
-            bwt_fix_kernel<<<div_up_u(div_up_u(len, 32), 256), 256, 0, st>>>(actbits, sa, len, ix.packed, b, ix.bwt.ptr, d_primary.ptr);
-        KERNEL_CHECK();
-        ix.timer.end(t);
-    }
+    // next to a pair included -- by the text itself; the tie-break would only add a trip over the list)
+    const bool pairs_first = L.bucketed && kn.pairs == 1 && (u64)L.m * 64 >= (u64)len;
+    if (L.m && c.b <= 8 && !pairs_first && kn.ext_tiebreak) text_tiebreak(c, L, rsrc, pend);
+    if (L.m && c.b <= 8 && pair_path_applies(c, L)) pair_path(c, L, rsrc, pend);
+    if (L.m && L.bucketed) scatter_round0_ranks(c, L, rsrc);
+    if (L.m) doubling_rounds<RB>(c, L);
+    if (c.need_bwt_fix) bwt_fix(c, m_round0);
     read_back(&ix.primary, d_primary.ptr, 4, st);
-    if (want_bwt && !bwt_in_sort) gather_bwt(ix);  // the element had no room for the preceding symbol
+    if (want_bwt && !L.bwt_in_sort) gather_bwt(ix);  // the element had no room for the preceding symbol
 }
 
 void build_suffix_array(DeviceIndex &ix, bool want_bwt) {
-    int rb = env_int("B200SA_RADIX_BITS", 8);
+    const BuildKnobs kn = read_build_knobs();
     // the digit must hold a whole number of packed symbols
-    if (rb == 10 && (10 % ix.pk.bits) == 0) build_sa_impl<10>(ix, want_bwt);
-    else build_sa_impl<8>(ix, want_bwt);
+    if (kn.radix_bits == 10 && (10 % ix.pk.bits) == 0) build_sa_impl<10>(ix, kn, want_bwt);
+    else build_sa_impl<8>(ix, kn, want_bwt);
 }
 
 // inverse suffix array on request (stralg/suffix_array.c:55-62): isa[sa[r]] = r

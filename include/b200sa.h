@@ -243,10 +243,59 @@ int b200sa_sa_lookup(const b200sa_index *idx, const uint32_t *rows, uint64_t cou
  * format stores what is resident in HBM: a fixed header (magic "B200SAIX", version, byte-order
  * mark, n, sigma, primary, C table, O layout) followed by tagged sections {tag[8], element bytes,
  * count, raw array}: SA, ISA, LCP, BWT, OCC (sampled O blocks), TEXT (packed text), KTABLE,
- * SSAMARK / SSAVAL (sampled suffix array).  b200sa_load returns an index that answers search /
+ * SSAMARK / SSAVAL (sampled suffix array), RECOFF (record offsets of a records index).  b200sa_load returns an index that answers search /
  * locate / approximate search exactly like the one that was saved, without rebuilding. */
 int b200sa_save(const b200sa_index *idx, const char *path);
 b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200sa_error *err);
+
+/* ---- records index: many records in one build ------------------------------------------------
+ * A multi-record reference (chromosomes and contigs, transcript sets) in ONE index.  The records are
+ * codes 2..sigma-1; code 1 is the separator, which the library inserts after every record, the last
+ * one included:  r0 1 r1 1 ... r(k-1) 1 $.  Record r has len_r = rec_off[r+1] - rec_off[r] >= 0
+ * symbols and starts at text position start_r = rec_off[r] + r; its separator at start_r + len_r
+ * plays its own sentinel.  n = rec_off[nrec] + nrec <= 2^32 - 2; sigma (b200sa_stats) counts the
+ * separator.  The separator sorts below every letter, so the global suffix array restricted to one
+ * record's positions is that record's own suffix array, in the same order: one build serves every
+ * record, and an exact match never crosses a record (patterns never hold code 1).
+ *
+ * b200sa_build_records: `codes` holds the records back to back without separators, rec_off[nrec + 1]
+ * (host; rec_off[0] = 0) the record boundaries, so `codes` has rec_off[nrec] symbols (a host array, or a
+ * device array with B200SA_TEXT_ON_DEVICE).  The separators are inserted on the device; the text then
+ * takes the path of b200sa_build.  Flags: OCC, TEXTCMP, KTABLE, DROP_SA, PROFILE, TEXT_ON_DEVICE; ISA,
+ * LCP or BWT -> B200SA_ERR_BAD_ARGUMENT (per-record tables of that kind do not exist).  A code 0, 1 or
+ * >= sigma -> _BAD_SYMBOL; offsets that decrease or rec_off[0] != 0 -> _BAD_ARGUMENT; n > 2^32 - 2 ->
+ * _TOO_LARGE.
+ *
+ * On a records index every other entry point works on the whole text and returns global rows
+ * (search, locate, sample_sa, sa_lookup).  b200sa_search_batch and b200sa_approx_batch refuse a
+ * pattern holding code 1 (_BAD_SYMBOL); with b200sa_search_device keeping code 1 out is the caller's
+ * duty.  The packed-read entry points refuse a records index whatever its sigma (_NOT_BUILT): packed
+ * base 0 would be code 1, the separator (a DNA records index, ACGT and the separator, has the byte
+ * O-table layout anyway).  b200sa_extend -> _BAD_ARGUMENT.  The approximate
+ * search never consumes the separator: same report order per record as the record's own index.
+ * b200sa_replicate and b200sa_save / b200sa_load carry the record offsets (file section RECOFF;
+ * builds of the library from before records indices refuse such a file as an unknown section).
+ *
+ * b200sa_records: *nrec (0 for a plain index) and, when rec_off is not NULL, its nrec + 1 offsets.
+ * b200sa_copy_record_sas / _device: every record's own suffix array back to back -- record r's
+ * len_r + 1 entries, in local positions, at offset start_r; n entries in all (the global sentinel row
+ * belongs to no record).  Each equals b200sa_copy_sa of b200sa_build on that record alone.  Needs the
+ * full suffix array (_NOT_BUILT after DROP_SA).
+ * b200sa_locate_records / _device: like b200sa_locate_batch, a CSR pos_off[npat + 1] over entries that
+ * are (rec[k], pos[k]) pairs: the record and the local position.  Within a pattern, records ascend and
+ * the positions of one record come in that record's suffix-array order (the reference iterator's order
+ * on the record's own index).  Row 0 (the global sentinel) is skipped.  rec and pos are both NULL to
+ * size the output (*total).  A plain index -> _BAD_ARGUMENT. */
+b200sa_index *b200sa_build_records(const uint8_t *codes, const uint64_t *rec_off, uint32_t nrec, uint32_t sigma,
+                                   uint32_t flags, int device, void *stream, enum b200sa_error *err);
+int b200sa_records(const b200sa_index *idx, uint32_t *nrec, uint64_t *rec_off /* NULL or nrec + 1 entries */);
+int b200sa_copy_record_sas(const b200sa_index *idx, uint32_t *host /* n entries */);
+int b200sa_record_sas_device(const b200sa_index *idx, uint32_t *d_out, void *stream);
+int b200sa_locate_records(const b200sa_index *idx, const uint32_t *L, const uint32_t *R, uint64_t npat,
+                          uint64_t *pos_off, uint32_t *rec, uint32_t *pos, uint64_t capacity, uint64_t *total);
+int b200sa_locate_records_device(const b200sa_index *idx, const uint32_t *d_L, const uint32_t *d_R, uint64_t npat,
+                                 uint64_t *d_pos_off, uint32_t *d_rec, uint32_t *d_pos, uint64_t capacity,
+                                 uint64_t *total, void *stream);
 
 /* ---- batched approximate search (SURVEY 8f rank 4) -------------------------------------------
  * Replaces init_bwt_approx_iter / next_bwt_approx_match (bwt.h:246-333, bwt.c:226-409): all

@@ -216,6 +216,18 @@ uint64_t bwt_map_fastq_exact(FILE *fastq, FILE *samfile, uint32_t nrecords, cons
  * order, positions in suffix-array order) with the tool's CIGARs.  Byte-identical to the tool. */
 uint64_t bwt_map_fastq(FILE *fastq, FILE *samfile, uint32_t nrecords, const char *const *record_names,
                        struct bwt_table *const *tables, int edits, uint64_t batch_reads);
+/* The same mapping against ONE records index (include/b200sa.h: b200sa_build_records) over all the tables'
+ * strings, turned back into bytes with their remap tables and remapped with one union alphabet: per batch
+ * one search or approximate-search call and one b200sa_locate_records call, however many records there
+ * are, where bwt_map_fastq makes one call per record and remaps every read once per record on the host.
+ * Same contract, byte-identical SAM: a read with a letter missing from record r's own alphabet gives no
+ * line for r (the tool's remap() skip), lines in the tool's order.  With edits > 0 and reverse O tables in
+ * every table, the D table comes from an index of the reversed text (it prunes, the results are the same).
+ * A record's letters are those its remap table codes (as for bwt_map_fastq's remap of a read); the tables'
+ * codes must follow byte order, as init_remap_table / build_complete_table make them, so that the union
+ * alphabet takes a record's letters in the order its own table does (the approximate search's report order). */
+uint64_t bwt_map_fastq_records(FILE *fastq, FILE *samfile, uint32_t nrecords, const char *const *record_names,
+                               struct bwt_table *const *tables, int edits, uint64_t batch_reads);
 /* The multi-record index file of `bwt_readmapper -p` (bwt_readmapper.c:48-61): [u32 records], then per
  * record [u32 len][name incl. NUL] (string_utils.c:48-65) + write_complete_bwt_info.  The tool writes
  * the FASTA records in REVERSE file order (bioinf/fasta.c:131 prepends) and maps in the reverse of

@@ -5,6 +5,6 @@ The package holds only what the hot path needs: ``csrc/`` (sm_100a CUDA kernels 
 CPU fallback: everything calls into ``lib/libb200sa.so``.
 """
 from ._lib import B200saError, LIB_PATH, load  # noqa: F401
-from .index import (RemapTable, SuffixArrayIndex, build_complete_table, pack_reads, qsort_sa_construction,  # noqa: F401
+from .index import (RecordsRemap, RemapTable, SuffixArrayIndex, build_complete_table, pack_reads, qsort_sa_construction,  # noqa: F401
                     search_sharded_packed,
                     sa_is_construction, sa_is_mem_construction, skew_sa_construction)

@@ -119,6 +119,15 @@ SIGNATURES = {
     "b200sa_synth_reads": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64, C.c_uint32,
                                      C.c_uint32, C.c_uint64, C.c_int, C.c_void_p]),
     "b200sa_device_count": (C.c_int, []),
+    "b200sa_build_records": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int,
+                                          C.c_void_p, C.POINTER(C.c_int)]),
+    "b200sa_records": (C.c_int, [C.c_void_p, u32p, C.c_void_p]),
+    "b200sa_copy_record_sas": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "b200sa_record_sas_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200sa_locate_records": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_uint64, u64p]),
+    "b200sa_locate_records_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_uint64, u64p, C.c_void_p]),
 }
 
 

@@ -320,6 +320,36 @@ static void replicate_buf(const DevBuf<T> &src, int src_dev, DevBuf<T> &dst, int
     CUDA_CHECK(cudaMemcpyPeerAsync(dst.ptr, dst_dev, src.ptr, src_dev, src.count * sizeof(T), st));
 }
 
+// device bytes from cudaMalloc, freed with cudaFree (which waits for the device) when released or destroyed
+struct DeviceBytes {
+    u8 *ptr = nullptr;
+    void alloc(size_t bytes) { ptr = (u8 *)malloc_or_purge(bytes); }
+    void release() {
+        if (ptr) cudaFree(ptr);
+        ptr = nullptr;
+    }
+    ~DeviceBytes() { release(); }
+};
+
+// records index (records.cu): the host offsets and the device record starts start[r] = rec_off[r] + r
+static void set_records(DeviceIndex &ix, const std::vector<u64> &rec_off, cudaStream_t st) {
+    ix.nrec = (u32)(rec_off.size() - 1);
+    ix.rec_off = rec_off;
+    std::vector<u64> start(rec_off.size());
+    for (size_t r = 0; r < rec_off.size(); ++r) start[r] = rec_off[r] + r;
+    ix.rec_start.alloc(start.size(), st);
+    CUDA_CHECK(cudaMemcpyAsync(ix.rec_start.ptr, start.data(), start.size() * 8, cudaMemcpyHostToDevice, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));  // (`start` is pageable host memory)
+}
+
+// a pattern of a host batch that holds the separator (code 1) of a records index
+static bool holds_separator(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
+                            uint64_t npat) {
+    if (!idx->ix.nrec || !npat) return false;
+    const uint64_t b0 = offsets ? offsets[0] : 0, b1 = offsets ? offsets[npat] : (uint64_t)fixed_len * npat;
+    return b1 > b0 && memchr(patterns + b0, 1, (size_t)(b1 - b0)) != nullptr;
+}
+
 #pragma GCC visibility push(default)
 extern "C" {
 
@@ -430,12 +460,103 @@ b200sa_index *b200sa_build(const uint8_t *codes, uint64_t n, uint32_t sigma, uin
     return h;
 }
 
+b200sa_index *b200sa_build_records(const uint8_t *codes, const uint64_t *rec_off, uint32_t nrec, uint32_t sigma,
+                                   uint32_t flags, int device, void *stream, enum b200sa_error *err) {
+    const uint32_t accepted = B200SA_BUILD_OCC | B200SA_BUILD_TEXTCMP | B200SA_BUILD_KTABLE | B200SA_DROP_SA |
+                              B200SA_PROFILE | B200SA_TEXT_ON_DEVICE;
+    if (!rec_off || nrec == 0 || sigma < 3 || sigma > 256 || (flags & ~accepted)) {
+        fail(B200SA_ERR_BAD_ARGUMENT,
+             "b200sa_build_records: null offsets, no record, sigma outside 3..256, or a flag other than OCC, TEXTCMP, "
+             "KTABLE, DROP_SA, PROFILE, TEXT_ON_DEVICE (per-record ISA, LCP and BWT do not exist)", err);
+        return nullptr;
+    }
+    if (rec_off[0] != 0) {
+        fail(B200SA_ERR_BAD_ARGUMENT, "b200sa_build_records: rec_off[0] must be 0", err);
+        return nullptr;
+    }
+    for (uint32_t r = 0; r < nrec; ++r)
+        if (rec_off[r + 1] < rec_off[r]) {
+            fail(B200SA_ERR_BAD_ARGUMENT, "b200sa_build_records: record offsets decrease", err);
+            return nullptr;
+        }
+    const uint64_t ncodes = rec_off[nrec];
+    if (!codes && ncodes) {
+        fail(B200SA_ERR_BAD_ARGUMENT, "b200sa_build_records: null codes", err);
+        return nullptr;
+    }
+    if (ncodes > 0xFFFFFFFEull || ncodes + nrec > 0xFFFFFFFEull) {
+        fail(B200SA_ERR_TOO_LARGE, "records and separators exceed 2^32 - 2 symbols (uint32 suffix arrays)", err);
+        return nullptr;
+    }
+    const uint64_t n = ncodes + nrec;
+    b200sa_index *h = new (std::nothrow) b200sa_index();
+    if (!h) {
+        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
+        return nullptr;
+    }
+    int rc = 0;
+    try {
+        DeviceGuard guard(device);
+        cudaStream_t st = (cudaStream_t)stream;
+        const std::vector<u64> off(rec_off, rec_off + nrec + 1);
+        // The text with separators, assembled on the device; it then takes the path of any other text.  The two
+        // byte buffers are plain allocations given back to the driver as soon as they are dead (the staged records
+        // right after the assembly), not blocks of the library's pool, which keeps what it is given.
+        DeviceBytes text, staged;
+        text.alloc(n + 1);
+        DevBuf<u64> d_off(nrec + 1, st);
+        DevBuf<int> d_err(1, st);
+        const u8 *d_codes = codes;
+        if (!(flags & B200SA_TEXT_ON_DEVICE)) {
+            staged.alloc(ncodes ? ncodes : 1);
+            if (ncodes) CUDA_CHECK(cudaMemcpyAsync(staged.ptr, codes, ncodes, cudaMemcpyHostToDevice, st));
+            d_codes = staged.ptr;
+        }
+        CUDA_CHECK(cudaMemcpyAsync(d_off.ptr, off.data(), (nrec + 1) * 8, cudaMemcpyHostToDevice, st));
+        CUDA_CHECK(cudaMemsetAsync(d_err.ptr, 0, 4, st));
+        records_assemble(d_codes, ncodes, d_off.ptr, nrec, sigma, text.ptr, d_err.ptr, st);
+        int herr = 0;
+        read_back(&herr, d_err.ptr, 4, st);  // (synchronises the stream: the assembly is done)
+        staged.release();
+        d_off.release();
+        if (herr) {
+            rc = fail(B200SA_ERR_BAD_SYMBOL, "a record holds a code outside 2..sigma-1 (1 is the separator)", err);
+        } else {
+            rc = build_into(h, text.ptr, n, sigma, flags | B200SA_TEXT_ON_DEVICE, device, stream, err);
+            if (rc == 0) {
+                h->flags = flags & ~B200SA_TEXT_ON_DEVICE;
+                set_records(h->ix, off, st);
+            }
+        }
+    } catch (const CudaFailure &e) {
+        cudaGetLastError();
+        rc = fail(code_of(e.code), e.what(), err);
+    } catch (const std::bad_alloc &) {
+        rc = fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
+    } catch (const std::exception &e) {
+        rc = fail(B200SA_ERR_INTERNAL, e.what(), err);
+    }
+    if (rc != 0) {
+        b200sa_free(h);
+        return nullptr;
+    }
+    return h;
+}
+
+int b200sa_records(const b200sa_index *idx, uint32_t *nrec, uint64_t *rec_off) {
+    if (!idx || !nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
+    *nrec = idx->ix.nrec;
+    if (rec_off && idx->ix.nrec) memcpy(rec_off, idx->ix.rec_off.data(), idx->ix.rec_off.size() * 8);
+    return 0;
+}
+
 namespace {
 void mail_server_release(const b200sa_index *idx);  // (the resident one-pattern search holds pointers into the index)
 }
 int b200sa_extend(b200sa_index *idx, const uint8_t *codes, uint32_t flags) {
     if (!idx || (!codes && idx->ix.n)) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     DeviceIndex &ix = idx->ix;
+    if (ix.nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "b200sa_extend does not apply to a records index", nullptr);
     if (!ix.sa.ptr) return fail(B200SA_ERR_NOT_BUILT, "suffix array was dropped (B200SA_DROP_SA)", nullptr);
     const bool need_textcmp = (flags & B200SA_BUILD_TEXTCMP) && !ix.text_packed.ptr;
     const bool need_isa = ((flags & B200SA_BUILD_ISA) || need_textcmp) && !ix.isa.ptr;
@@ -870,6 +991,8 @@ int b200sa_search_batch(const b200sa_index *idx, const uint8_t *patterns, const 
     if (!idx || (npat && (!patterns || !L || !R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (idx->ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", nullptr);
     if (!npat) return 0;
+    if (holds_separator(idx, patterns, offsets, fixed_len, npat))
+        return fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", nullptr);
     API_GUARD_BEGIN
     const DeviceIndex &ix = idx->ix;
     DeviceGuard guard(ix.device);
@@ -945,6 +1068,9 @@ static int packed_args_ok(const b200sa_index *idx, uint32_t read_len, uint32_t &
     if (!idx) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (idx->ix.occ_layout != OCC_DNA32)
         return fail(B200SA_ERR_NOT_BUILT, "packed reads need a DNA index (sigma <= 5) with the O table", nullptr);
+    // (packed base 0 is code 1, the separator of a records index: a packed read could match across records)
+    if (idx->ix.nrec)
+        return fail(B200SA_ERR_NOT_BUILT, "packed reads do not apply to a records index (code 1 is its separator)", nullptr);
     if (read_len == 0) return fail(B200SA_ERR_BAD_ARGUMENT, "empty reads", nullptr);
     const uint32_t need = (read_len + 3u) / 4u;
     if (stride == 0) stride = need;
@@ -1112,6 +1238,7 @@ b200sa_index *b200sa_replicate(const b200sa_index *src, int device, void *stream
         replicate_buf(a.ssa_marks, sd, ix.ssa_marks, device, st, false);
         replicate_buf(a.ssa_vals, sd, ix.ssa_vals, device, st, false);
         replicate_buf(a.c_table, sd, ix.c_table, device, st, false);
+        if (a.nrec) set_records(ix, a.rec_off, st);
         CUDA_CHECK(cudaStreamSynchronize(st));
         ok(err);
         return h;
@@ -1130,6 +1257,8 @@ int b200sa_search_sharded_packed(const b200sa_index *const *replicas, int nrep, 
     if (!replicas || nrep < 1 || nrep > 64) return fail(B200SA_ERR_BAD_ARGUMENT, "bad replica list", nullptr);
     for (int g = 0; g < nrep; ++g) {
         if (!replicas[g]) return fail(B200SA_ERR_BAD_ARGUMENT, "null replica", nullptr);
+        if (replicas[g]->ix.nrec)
+            return fail(B200SA_ERR_NOT_BUILT, "packed reads do not apply to a records index (code 1 is its separator)", nullptr);
         if (replicas[g]->ix.len != replicas[0]->ix.len || replicas[g]->ix.primary != replicas[0]->ix.primary)
             return fail(B200SA_ERR_BAD_ARGUMENT, "replicas are not copies of one index", nullptr);
         for (int k = 0; k < g; ++k)
@@ -1282,6 +1411,112 @@ int b200sa_locate_batch_sorted(const b200sa_index *idx, const uint32_t *L, const
     return locate_batch_impl(idx, L, R, npat, pos_off, pos, pos_capacity, total, true);
 }
 
+// ---- records index (records.cu) ----
+int b200sa_record_sas_device(const b200sa_index *idx, uint32_t *d_out, void *stream) {
+    if (!idx || !d_out) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
+    if (!idx->ix.nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "not a records index (b200sa_build_records)", nullptr);
+    if (!idx->ix.sa.ptr) return fail(B200SA_ERR_NOT_BUILT, "the record suffix arrays need the full suffix array (dropped)", nullptr);
+    API_GUARD_BEGIN
+    DeviceGuard guard(idx->ix.device);
+    record_sas(idx->ix, d_out, (cudaStream_t)stream);
+    return 0;
+    API_GUARD_END(nullptr)
+}
+
+int b200sa_copy_record_sas(const b200sa_index *idx, uint32_t *host) {
+    if (!idx || !host) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
+    if (!idx->ix.nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "not a records index (b200sa_build_records)", nullptr);
+    if (!idx->ix.sa.ptr) return fail(B200SA_ERR_NOT_BUILT, "the record suffix arrays need the full suffix array (dropped)", nullptr);
+    API_GUARD_BEGIN
+    const DeviceIndex &ix = idx->ix;
+    DeviceGuard guard(ix.device);
+    cudaStream_t st = ix.stream;
+    DevBuf<u32> d(ix.n, st);
+    record_sas(ix, d.ptr, st);
+    if (ix.n) CUDA_CHECK(cudaMemcpyAsync(host, d.ptr, (size_t)ix.n * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));
+    return 0;
+    API_GUARD_END(nullptr)
+}
+
+// The rows [max(L, 1), R): row 0 is the global sentinel, which belongs to no record.  The count clamps L into d_L1
+// and fills d_pos_off; the fill locates the global positions and turns them into (record, local position) pairs.
+static u64 locate_records_count(const DeviceIndex &ix, const u32 *d_L, const u32 *d_R, u64 npat, u64 *d_pos_off,
+                                u32 *d_L1, cudaStream_t st) {
+    records_clamp_rows(d_L, npat, d_L1, st);
+    return fm_locate_count(ix, d_L1, d_R, npat, d_pos_off, st);
+}
+static void locate_records_fill(const DeviceIndex &ix, const u32 *d_L1, const u32 *d_R, u64 npat, const u64 *d_pos_off,
+                                u64 total, u32 *d_rec, u32 *d_pos, cudaStream_t st) {
+    if (!total) return;
+    DevBuf<u32> global(total, st);
+    locate_fill_any(ix, d_L1, d_R, npat, d_pos_off, total, global.ptr, st);
+    locate_records_group(ix, npat, d_pos_off, total, global.ptr, d_rec, d_pos, st);
+}
+
+static int locate_records_args_ok(const b200sa_index *idx, const void *L, const void *R, uint64_t npat, const void *pos_off,
+                                  const void *rec, const void *pos) {
+    if (!idx || !pos_off || (npat && (!L || !R)) || (!rec != !pos))
+        return fail(B200SA_ERR_BAD_ARGUMENT, "null argument (rec and pos are given together)", nullptr);
+    if (!idx->ix.nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "not a records index (b200sa_build_records)", nullptr);
+    if (!can_locate(idx)) return fail(B200SA_ERR_NOT_BUILT, "no suffix array to locate with (dropped and not sampled)", nullptr);
+    return 0;
+}
+
+static int locate_records_fits(u64 t, u64 npat, u64 capacity) {
+    if (t > capacity) return fail(B200SA_ERR_BAD_ARGUMENT, "position buffer too small", nullptr);
+    if (t > 0xFFFFFFFFull || npat > 0xFFFFFFFFull)
+        return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 positions or patterns in one batch", nullptr);
+    return 0;
+}
+
+int b200sa_locate_records_device(const b200sa_index *idx, const uint32_t *d_L, const uint32_t *d_R, uint64_t npat,
+                                 uint64_t *d_pos_off, uint32_t *d_rec, uint32_t *d_pos, uint64_t capacity,
+                                 uint64_t *total, void *stream) {
+    if (int rc = locate_records_args_ok(idx, d_L, d_R, npat, d_pos_off, d_rec, d_pos)) return rc;
+    API_GUARD_BEGIN
+    const DeviceIndex &ix = idx->ix;
+    DeviceGuard guard(ix.device);
+    cudaStream_t st = (cudaStream_t)stream;
+    DevBuf<u32> dL1(npat ? npat : 1, st);
+    const u64 t = locate_records_count(ix, d_L, d_R, npat, d_pos_off, dL1.ptr, st);
+    if (total) *total = t;
+    if (d_pos && t) {
+        if (int rc = locate_records_fits(t, npat, capacity)) return rc;
+        locate_records_fill(ix, dL1.ptr, d_R, npat, d_pos_off, t, d_rec, d_pos, st);
+    }
+    return 0;
+    API_GUARD_END(nullptr)
+}
+
+int b200sa_locate_records(const b200sa_index *idx, const uint32_t *L, const uint32_t *R, uint64_t npat,
+                          uint64_t *pos_off, uint32_t *rec, uint32_t *pos, uint64_t capacity, uint64_t *total) {
+    if (int rc = locate_records_args_ok(idx, L, R, npat, pos_off, rec, pos)) return rc;
+    API_GUARD_BEGIN
+    const DeviceIndex &ix = idx->ix;
+    DeviceGuard guard(ix.device);
+    cudaStream_t st = ix.stream;
+    DevBuf<u32> dL(npat ? npat : 1, st), dR(npat ? npat : 1, st), dL1(npat ? npat : 1, st);
+    DevBuf<u64> doff(npat + 1, st);
+    if (npat) {
+        CUDA_CHECK(cudaMemcpyAsync(dL.ptr, L, npat * 4, cudaMemcpyHostToDevice, st));
+        CUDA_CHECK(cudaMemcpyAsync(dR.ptr, R, npat * 4, cudaMemcpyHostToDevice, st));
+    }
+    const u64 t = locate_records_count(ix, dL.ptr, dR.ptr, npat, doff.ptr, dL1.ptr, st);
+    if (total) *total = t;
+    CUDA_CHECK(cudaMemcpyAsync(pos_off, doff.ptr, (npat + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (pos && t) {
+        if (int rc = locate_records_fits(t, npat, capacity)) return rc;
+        DevBuf<u32> drec(t, st), dpos(t, st);
+        locate_records_fill(ix, dL1.ptr, dR.ptr, npat, doff.ptr, t, drec.ptr, dpos.ptr, st);
+        CUDA_CHECK(cudaMemcpyAsync(rec, drec.ptr, t * 4, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaMemcpyAsync(pos, dpos.ptr, t * 4, cudaMemcpyDeviceToHost, st));
+    }
+    CUDA_CHECK(cudaStreamSynchronize(st));
+    return 0;
+    API_GUARD_END(nullptr)
+}
+
 int b200sa_sample_sa(b200sa_index *idx, uint32_t rate, int drop_sa) {
     if (!idx || rate < 1) return fail(B200SA_ERR_BAD_ARGUMENT, "null index or sampling rate 0", nullptr);
     mail_server_release(idx);
@@ -1339,6 +1574,12 @@ int b200sa_save(const b200sa_index *idx, const char *path) {
         if (ix.ssa_rate) {
             secs.push_back({"SSAMARK", ix.ssa_marks.ptr, 16, ix.ssa_marks.count});
             secs.push_back({"SSAVAL", ix.ssa_vals.ptr, 4, ix.ssa_vals.count});
+        }
+        DevBuf<u64> d_recoff;  // (sections are written from device memory)
+        if (ix.nrec) {
+            d_recoff.alloc(ix.rec_off.size(), st);
+            CUDA_CHECK(cudaMemcpyAsync(d_recoff.ptr, ix.rec_off.data(), ix.rec_off.size() * 8, cudaMemcpyHostToDevice, st));
+            secs.push_back({"RECOFF", d_recoff.ptr, 8, ix.rec_off.size()});
         }
         IndexFileHeader h{};
         memcpy(h.magic, "B200SAIX", 8);
@@ -1469,6 +1710,15 @@ b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200s
                 if (!fh.ssa_rate) throw std::invalid_argument("index file header is inconsistent");
                 read_section(f, sh, ix.ssa_vals, (size_t)ix.n / fh.ssa_rate + 1, buf, st);
                 have_vals = true;
+            } else if (tag == "RECOFF") {
+                if (sh.elem_bytes != 8 || sh.count < 2 || sh.count - 1 > fh.n)
+                    throw std::invalid_argument("index file: section RECOFF has an unexpected shape");
+                std::vector<u64> off(sh.count);
+                if (fread(off.data(), 8, sh.count, f) != sh.count) throw std::invalid_argument("index file: truncated section");
+                bool good = off[0] == 0 && off.back() + (sh.count - 1) == fh.n;
+                for (size_t r = 1; r < off.size() && good; ++r) good = off[r] >= off[r - 1];
+                if (!good) throw std::invalid_argument("index file: record offsets are inconsistent");
+                set_records(ix, off, st);
             } else
                 throw std::invalid_argument("index file: unknown section " + tag);
         }
@@ -1536,6 +1786,10 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
     }
     if (max_m > 65000u) {
         fail(B200SA_ERR_TOO_LARGE, "approximate search takes patterns of up to 65000 symbols", err);
+        return nullptr;
+    }
+    if (holds_separator(idx, patterns, offsets, fixed_len, npat)) {
+        fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", err);
         return nullptr;
     }
     b200sa_approx_result *res = new (std::nothrow) b200sa_approx_result();

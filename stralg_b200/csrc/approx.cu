@@ -18,6 +18,10 @@
 // (hits and CIGAR bytes per pattern), an exclusive scan, and an emitting pass that
 // writes every hit at its final offset -- no atomics, deterministic output.
 //
+// Records index (records.cu): letter 1 is the separator between records.  Its match / substitution
+// and deletion children are not viable, so no walk crosses a record boundary; child numbering, and
+// so the report order, is that of the plain walk.  The flag is off for a plain index.
+//
 // D table (bwt.c:319-337): forward over the pattern with the O table of the REVERSED text (a
 // second index), restarting the interval whenever it empties; D[i] = restarts so far.
 #include "engine.h"
@@ -37,6 +41,7 @@ struct ApproxArgs {
     u64 first, count;      // patterns [first, first + count) of the batch run in this launch
     const u8 *dtab;        // D value per pattern symbol (same offsets as `pat`), or null
     int max_edits;
+    bool no_sep;           // records index: letter 1 is the record separator and is never consumed
     uint4 *stack;          // count * max_depth frames
     u32 max_depth;
     // counting pass
@@ -146,7 +151,8 @@ __global__ void __launch_bounds__(128, 8) approx_walk_kernel(ApproxArgs A) {
             ci = i;
             cleft = left - 1;
         }
-        bool viable = cidx >= cursor && cidx < nchildren && cleft >= 0;
+        // (on a records index a match / substitution or deletion of the separator would run into the next record)
+        bool viable = cidx >= cursor && cidx < nchildren && cleft >= 0 && !(A.no_sep && a == 1);
         if (viable) {
             const int need = (ci >= 0 && dt) ? (int)dt[ci] : 0;
             viable = cleft >= need;
@@ -394,6 +400,7 @@ void approx_count(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 
     A.pat = d_pat; A.off = d_off; A.fixed_len = fixed_len;
     A.dtab = d_dtab;
     A.max_edits = max_edits;
+    A.no_sep = ix.nrec > 0;
     A.max_depth = max_m + (u32)max_edits + 2;
     A.hit_count = hit_count.ptr;
     A.ops_count = ops_count.ptr;
@@ -420,6 +427,7 @@ void approx_emit(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 f
     A.pat = d_pat; A.off = d_off; A.fixed_len = fixed_len;
     A.dtab = d_dtab;
     A.max_edits = max_edits;
+    A.no_sep = ix.nrec > 0;
     A.max_depth = max_m + (u32)max_edits + 2;
     A.hit_off = d_hit_off;
     A.ops_off = d_ops_off;

@@ -16,6 +16,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -843,6 +844,188 @@ uint64_t bwt_map_fastq(FILE *fastq, FILE *samfile, uint32_t nrecords, const char
             results[r] = nullptr;
         }
     }
+    return lines;
+}
+
+// The same mapping against ONE records index (include/b200sa.h: b200sa_build_records) built from all the tables'
+// strings: one search or approximate-search call and one b200sa_locate_records call per batch, whatever the number
+// of records.  A read is remapped once, with the union alphabet; the tool's rule that a read with a letter missing
+// from record r's own alphabet produces no line for r is applied per (read, record) through letter masks -- with
+// edits, a substitution could otherwise align such a read to r.
+uint64_t bwt_map_fastq_records(FILE *fastq, FILE *samfile, uint32_t nrecords, const char *const *record_names,
+                               struct bwt_table *const *tables, int edits, uint64_t batch_reads) {
+    if (batch_reads == 0) batch_reads = edits > 0 ? 1u << 16 : 1u << 20;
+    // The records as bytes (rev_table of each table).  A record's letters are the letters its remap table codes, as
+    // bwt_map_fastq remaps a read with that table: mask[r] is that set (it may hold letters the string lacks, when the
+    // table was made for a wider alphabet), and the union table gives codes 2..sigma-1 to the letters of all tables.
+    std::vector<std::vector<uint8_t>> raw(nrecords);
+    std::vector<std::vector<bool>> mask(nrecords, std::vector<bool>(256, false));
+    bool present[256] = {false};
+    bool all_ro = true;
+    for (uint32_t r = 0; r < nrecords; ++r) {
+        const struct suffix_array *sa = tables[r]->sa;
+        const struct remap_table *rt = tables[r]->remap_table;
+        all_ro = all_ro && tables[r]->ro_table != nullptr;
+        for (int b = 1; b < 256; ++b)
+            if (rt->table[b] > 0) mask[r][b] = present[b] = true;
+        raw[r].resize(sa->length - 1);
+        for (uint32_t i = 0; i + 1 < sa->length; ++i) {
+            const uint8_t c = sa->string[i];
+            const int b = c < 128 ? rt->rev_table[c] : -1;
+            if (b <= 0 || !mask[r][b]) {
+                fprintf(stderr, "stralg_b200: bwt_map_fastq_records: record %u holds a code without a letter\n", r);
+                abort();
+            }
+            raw[r][i] = (uint8_t)b;
+        }
+    }
+    int16_t code[256];
+    uint32_t sigma = 2;
+    for (int b = 0; b < 256; ++b) code[b] = b > 0 && present[b] ? (int16_t)sigma++ : (int16_t)-1;
+    if (sigma == 2) {  // no record has a letter (or there is no record): no read maps, as with bwt_map_fastq
+        std::vector<char> line(kFastqLine + 1);
+        while (fgets(line.data(), kFastqLine, fastq)) {
+        }
+        return 0;
+    }
+    if (sigma > 256) {
+        fprintf(stderr, "stralg_b200: bwt_map_fastq_records: more than 254 letters\n");
+        abort();
+    }
+    std::vector<uint64_t> rec_off(nrecords + 1, 0);
+    for (uint32_t r = 0; r < nrecords; ++r) rec_off[r + 1] = rec_off[r] + raw[r].size();
+    std::vector<uint8_t> codes(rec_off[nrecords]);
+    for (uint32_t r = 0; r < nrecords; ++r)
+        for (size_t i = 0; i < raw[r].size(); ++i) codes[rec_off[r] + i] = (uint8_t)code[raw[r][i]];
+    raw.clear();
+    enum b200sa_error err;
+    const uint32_t flags = edits > 0 ? B200SA_BUILD_OCC : B200SA_BUILD_OCC | B200SA_BUILD_TEXTCMP | B200SA_BUILD_KTABLE;
+    b200sa_index *idx = b200sa_build_records(codes.data(), rec_off.data(), nrecords, sigma, flags, device_id(), nullptr, &err);
+    if (!idx) die("bwt_map_fastq_records");
+    // the tool's D table comes from the tables' reverse O rows; here from an index of the reversed text, separators
+    // included: it bounds every record's D table from below, so it prunes less and changes no result
+    b200sa_index *rev = nullptr;
+    if (edits > 0 && all_ro) {
+        const uint64_t n = rec_off[nrecords] + nrecords;
+        std::vector<uint8_t> text(n);
+        for (uint32_t r = 0; r < nrecords; ++r) {
+            std::copy(codes.begin() + rec_off[r], codes.begin() + rec_off[r + 1], text.begin() + rec_off[r] + r);
+            text[rec_off[r + 1] + r] = 1;
+        }
+        std::reverse(text.begin(), text.end());
+        rev = b200sa_build(text.data(), n, sigma, B200SA_BUILD_OCC, device_id(), nullptr, &err);
+        if (!rev) die("bwt_map_fastq_records");
+    }
+    codes.clear();
+    codes.shrink_to_fit();
+
+    std::vector<char> line(kFastqLine + 1);
+    std::vector<std::string> names, seqs, quals;
+    std::vector<uint8_t> pat;
+    std::vector<uint64_t> off, hit_off, pos_off;
+    std::vector<uint32_t> which, L, R, rec, pos;
+    std::vector<std::string> cigars;
+    std::vector<uint64_t> order;
+    uint64_t lines = 0;
+    bool more = true;
+    while (more) {
+        names.clear(); seqs.clear(); quals.clear();
+        while (names.size() < batch_reads) {
+            std::string name, seq, plus, qual;
+            if (!fastq_line(fastq, line.data(), &name, 1)) {
+                more = false;
+                break;
+            }
+            fastq_line(fastq, line.data(), &seq, 0);
+            fastq_line(fastq, line.data(), &plus, 0);
+            fastq_line(fastq, line.data(), &qual, 0);
+            names.push_back(name); seqs.push_back(seq); quals.push_back(qual);
+        }
+        const size_t nreads = names.size();
+        if (!nreads) break;
+        // every read once through the union table; a letter that no record holds skips the read for all of them
+        pat.clear(); off.assign(1, 0); which.clear();
+        for (size_t q = 0; q < nreads; ++q) {
+            const std::string &sq = seqs[q];
+            if (sq.empty()) continue;
+            const size_t at = pat.size();
+            pat.resize(at + sq.size());
+            bool ok = true;
+            for (size_t k = 0; k < sq.size() && ok; ++k) {
+                const int16_t c = code[(unsigned char)sq[k]];
+                ok = c > 0;
+                pat[at + k] = (uint8_t)c;
+            }
+            if (!ok) {
+                pat.resize(at);
+                continue;
+            }
+            off.push_back(pat.size());
+            which.push_back((uint32_t)q);
+        }
+        const size_t nvalid = which.size();
+        // hits of read which[k]: [hit_off[k], hit_off[k + 1]), each an interval with its CIGAR
+        L.clear(); R.clear(); cigars.clear();
+        hit_off.assign(nvalid + 1, 0);
+        if (nvalid && edits > 0) {
+            b200sa_approx_result *res = b200sa_approx_batch(idx, rev, nullptr, pat.data(), off.data(), 0, nvalid, edits, &err);
+            if (!res) die("bwt_map_fastq_records");
+            const uint64_t nh = b200sa_approx_hits(res);
+            const uint64_t *ho = b200sa_approx_hit_offsets(res), *coff = b200sa_approx_cigar_offsets(res);
+            const char *cig = b200sa_approx_cigars(res);
+            L.assign(b200sa_approx_L(res), b200sa_approx_L(res) + nh);
+            R.assign(b200sa_approx_R(res), b200sa_approx_R(res) + nh);
+            hit_off.assign(ho, ho + nvalid + 1);
+            cigars.resize(nh);
+            for (uint64_t h = 0; h < nh; ++h) cigars[h] = cig + coff[h];
+            b200sa_approx_free(res);
+        } else if (nvalid) {
+            L.resize(nvalid);
+            R.resize(nvalid);
+            if (b200sa_search_batch(idx, pat.data(), off.data(), 0, nvalid, L.data(), R.data())) die("bwt_map_fastq_records");
+            for (size_t k = 0; k <= nvalid; ++k) hit_off[k] = k;
+        }
+        // (record, local position) of every interval: records ascending, each record's suffix-array order
+        const uint64_t nh = L.size();
+        pos_off.assign(nh + 1, 0);
+        uint64_t total = 0;
+        if (b200sa_locate_records(idx, L.data(), R.data(), nh, pos_off.data(), nullptr, nullptr, 0, &total))
+            die("bwt_map_fastq_records");
+        rec.resize(total);
+        pos.resize(total);
+        if (total && b200sa_locate_records(idx, L.data(), R.data(), nh, pos_off.data(), rec.data(), pos.data(), total, &total))
+            die("bwt_map_fastq_records");
+        // SAM lines in the tool's order: reads, records, intervals in report order, positions in suffix-array order
+        for (size_t k = 0; k < nvalid; ++k) {
+            const size_t q = which[k];
+            const std::string &sq = seqs[q];
+            order.clear();
+            for (uint64_t h = hit_off[k]; h < hit_off[k + 1]; ++h)
+                for (uint64_t e = pos_off[h]; e < pos_off[h + 1]; ++e) order.push_back(e);
+            std::stable_sort(order.begin(), order.end(), [&](uint64_t a, uint64_t b) { return rec[a] < rec[b]; });
+            char exact_cigar[32];
+            snprintf(exact_cigar, sizeof exact_cigar, "%zuM", sq.size());
+            for (size_t j = 0; j < order.size();) {
+                const uint32_t r = rec[order[j]];
+                size_t j1 = j;
+                while (j1 < order.size() && rec[order[j1]] == r) ++j1;
+                bool in_r = true;
+                for (size_t c = 0; c < sq.size() && in_r; ++c) in_r = mask[r][(unsigned char)sq[c]];
+                for (; in_r && j < j1; ++j) {
+                    const uint64_t e = order[j];
+                    // the interval of entry e: the last hit of this read whose entries start at or before e
+                    const uint64_t h = std::upper_bound(pos_off.begin() + hit_off[k], pos_off.begin() + hit_off[k + 1],
+                                                        e) - pos_off.begin() - 1;
+                    fprintf(samfile, "%s\t0\t%s\t%u\t0\t%s\t*\t0\t0\t%s\t%s\n", names[q].c_str(), record_names[r],
+                            pos[e] + 1, edits > 0 ? cigars[h].c_str() : exact_cigar, sq.c_str(), quals[q].c_str());
+                    ++lines;
+                }
+                j = j1;
+            }
+        }
+    }
+    b200sa_free(rev);
+    b200sa_free(idx);
     return lines;
 }
 

@@ -2,6 +2,8 @@
 #pragma once
 #include "common.cuh"
 
+#include <vector>
+
 namespace b200sa {
 
 // Text packing parameters derived from the alphabet size (sentinel included in sigma).
@@ -70,6 +72,10 @@ struct DeviceIndex {
     u32 occ_block_bytes = 0;
     BuildStats stats{};
     StageTimer timer;
+    // records index (records.cu): nrec records, record r at text positions start[r] .. start[r] + len_r (its separator)
+    u32 nrec = 0;                 // 0: a plain index
+    std::vector<u64> rec_off;     // nrec + 1 offsets into the records without separators
+    DevBuf<u64> rec_start;        // nrec + 1 entries: start[r] = rec_off[r] + r, start[nrec] = n
 };
 
 // sa_build.cu
@@ -114,6 +120,13 @@ void approx_count(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 
 void approx_emit(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fixed_len, u64 npat, u32 max_m,
                  const u8 *d_dtab, int max_edits, const u64 *d_hit_off, const u64 *d_ops_off, u32 *d_L, u32 *d_R,
                  u32 *d_mlen, u64 *d_hit_ops_off, char *d_ops, cudaStream_t st);
+// records.cu
+void records_assemble(const u8 *d_codes, u64 ncodes, const u64 *d_rec_off, u32 nrec, u32 sigma, u8 *d_text,
+                      int *d_err, cudaStream_t st);  // d_text: ncodes + nrec + 1 bytes
+void record_sas(const DeviceIndex &ix, u32 *d_out, cudaStream_t st);  // needs ix.sa; n entries
+void records_clamp_rows(const u32 *d_L, u64 npat, u32 *d_out, cudaStream_t st);  // max(L, 1)
+void locate_records_group(const DeviceIndex &ix, u64 npat, const u64 *d_pos_off, u64 total, const u32 *d_pos,
+                          u32 *d_rec, u32 *d_local, cudaStream_t st);
 // synth.cu
 void synth_codes(u8 *d_text, u64 n, u32 nsym, u64 seed, cudaStream_t st);
 void synth_reads(const u8 *d_text, u64 n, u32 nsym, u8 *d_reads, u64 nreads, u32 m, u32 miss_per_1024,

@@ -55,6 +55,40 @@ class RemapTable:
         return self.rev_table[np.asarray(codes, dtype=np.uint8)].astype(np.uint8).tobytes()
 
 
+class RecordsRemap:
+    """Alphabet of a records index (include/b200sa.h, b200sa_build_records): the bytes present in any
+    record get codes 2..sigma-1 in byte order, code 1 is the separator the library inserts after every
+    record, 0 the sentinel.  ``masks[r]`` is the 256-entry set of bytes record r holds: a read with a
+    byte outside it has no code in record r's own ``RemapTable`` (the reference skips such a read for
+    that record, remap.c:80-84)."""
+
+    def __init__(self, records: Sequence[bytes]):
+        self.masks = np.zeros((len(records), 256), dtype=bool)
+        for r, rec in enumerate(records):
+            self.masks[r, np.frombuffer(bytes(rec), dtype=np.uint8)] = True
+        self.masks[:, 0] = False
+        seen = self.masks.any(axis=0)
+        letters = np.nonzero(seen)[0]
+        self.table = np.full(256, -1, dtype=np.int16)
+        self.rev_table = np.full(256, -1, dtype=np.int16)
+        self.table[0] = 0
+        self.rev_table[0] = 0
+        self.table[letters] = np.arange(2, len(letters) + 2, dtype=np.int16)
+        self.rev_table[2:len(letters) + 2] = letters
+        self.alphabet_size = len(letters) + 2  # sentinel + separator + letters
+
+    def remap(self, text: bytes) -> Optional[np.ndarray]:
+        """Codes 2..sigma-1 for ``text``; None if a byte is in no record."""
+        codes = self.table[np.frombuffer(bytes(text), dtype=np.uint8)]
+        if (codes <= 0).any():
+            return None
+        return codes.astype(np.uint8)
+
+    def in_record(self, text: bytes, r: int) -> bool:
+        """Whether every byte of ``text`` occurs in record r (its own RemapTable can remap it)."""
+        return bool(self.masks[r, np.frombuffer(bytes(text), dtype=np.uint8)].all())
+
+
 class SuffixArrayIndex:
     """Device-resident suffix array + optional ISA / LCP / BWT / C / O tables for one text.
 
@@ -94,6 +128,26 @@ class SuffixArrayIndex:
             ptr, n = _np_ptr(keep), keep.size
         err = C.c_int(0)
         h = lib.b200sa_build(ptr, n, sigma, flags, device, C.c_void_p(stream), C.byref(err))
+        if not h:
+            raise B200saError(err.value, lib.b200sa_last_error().decode())
+        return cls(h, device)
+
+    @classmethod
+    def build_records(cls, records, sigma: int, *, occ=True, textcmp=False, ktable=False, drop_sa=False,
+                      profile=False, device: int = 0, stream: int = 0) -> "SuffixArrayIndex":
+        """One index over many records (b200sa_build_records): ``records`` is a sequence of code arrays /
+        bytes over 2..sigma-1 (code 1 is the separator the library inserts after every record)."""
+        lib = _lib.load()
+        flags = (BUILD_OCC if occ else 0) | (BUILD_TEXTCMP if textcmp else 0) | (BUILD_KTABLE if ktable else 0) | \
+                (DROP_SA if drop_sa else 0) | (PROFILE if profile else 0)
+        parts = [np.frombuffer(r, dtype=np.uint8) if isinstance(r, (bytes, bytearray)) else np.asarray(r, dtype=np.uint8)
+                 for r in records]
+        off = np.zeros(len(parts) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum([p.size for p in parts], dtype=np.uint64)
+        codes = np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros(0, np.uint8), dtype=np.uint8)
+        err = C.c_int(0)
+        h = lib.b200sa_build_records(_np_ptr(codes), _np_ptr(off), len(parts), sigma, flags, device,
+                                     C.c_void_p(stream), C.byref(err))
         if not h:
             raise B200saError(err.value, lib.b200sa_last_error().decode())
         return cls(h, device)
@@ -326,6 +380,58 @@ class SuffixArrayIndex:
             self._h, C.c_void_p(d_L.data_ptr()), C.c_void_p(d_R.data_ptr()), npat, C.c_void_p(d_pos_off.data_ptr()),
             C.c_void_p(d_pos.data_ptr()) if d_pos is not None else None, capacity, C.byref(total), C.c_void_p(stream)))
         return int(total.value)
+
+    # ---- records index (b200sa_build_records) ----------------------------------------------------
+    def record_offsets(self) -> np.ndarray:
+        """rec_off[nrec + 1] of a records index (b200sa_records); an empty array for a plain index."""
+        lib = _lib.load()
+        nrec = C.c_uint32(0)
+        check(lib.b200sa_records(self._h, C.byref(nrec), None))
+        if not nrec.value:
+            return np.zeros(0, dtype=np.uint64)
+        off = np.empty(nrec.value + 1, dtype=np.uint64)
+        check(lib.b200sa_records(self._h, C.byref(nrec), _np_ptr(off)))
+        return off
+
+    def record_sas(self) -> list:
+        """Every record's own suffix array (b200sa_copy_record_sas), one array per record in local positions."""
+        off = self.record_offsets()
+        flat = self._copy(_lib.load().b200sa_copy_record_sas, np.uint32, self.length - 1)
+        start = off + np.arange(len(off), dtype=np.uint64)
+        return [flat[int(start[r]):int(start[r + 1])] for r in range(len(off) - 1)]
+
+    def record_sas_device(self, d_out, stream: int = 0) -> None:
+        """b200sa_record_sas_device: every record's own suffix array into ``d_out`` (a CUDA uint32 tensor of
+        length - 1 entries, record r at rec_off[r] + r); asynchronous on ``stream``."""
+        check(_lib.load().b200sa_record_sas_device(self._h, C.c_void_p(d_out.data_ptr()), C.c_void_p(stream)))
+
+    def locate_records_device(self, d_L, d_R, npat: int, d_pos_off, d_rec=None, d_pos=None, capacity: int = 0,
+                              stream: int = 0) -> int:
+        """b200sa_locate_records_device (torch CUDA tensors): fills d_pos_off[npat + 1] and, when given, d_rec and
+        d_pos; returns the number of entries."""
+        total = C.c_uint64(0)
+        check(_lib.load().b200sa_locate_records_device(
+            self._h, C.c_void_p(d_L.data_ptr()), C.c_void_p(d_R.data_ptr()), npat, C.c_void_p(d_pos_off.data_ptr()),
+            C.c_void_p(d_rec.data_ptr()) if d_rec is not None else None,
+            C.c_void_p(d_pos.data_ptr()) if d_pos is not None else None, capacity, C.byref(total), C.c_void_p(stream)))
+        return int(total.value)
+
+    def locate_records(self, L, R) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """(offsets[npat + 1], rec, pos) (b200sa_locate_records): per pattern, records ascending, the
+        local positions of one record in that record's suffix-array order."""
+        L = np.ascontiguousarray(L, dtype=np.uint32)
+        R = np.ascontiguousarray(R, dtype=np.uint32)
+        npat = len(L)
+        off = np.empty(npat + 1, dtype=np.uint64)
+        total = C.c_uint64(0)
+        fn = _lib.load().b200sa_locate_records
+        check(fn(self._h, _np_ptr(L), _np_ptr(R), npat, _np_ptr(off), None, None, 0, C.byref(total)))
+        rec = np.empty(total.value, dtype=np.uint32)
+        pos = np.empty(total.value, dtype=np.uint32)
+        if total.value:
+            check(fn(self._h, _np_ptr(L), _np_ptr(R), npat, _np_ptr(off), _np_ptr(rec), _np_ptr(pos), total.value,
+                     C.byref(total)))
+        return off, rec, pos
 
     def exact_matches(self, pattern_codes) -> np.ndarray:
         """All match positions of one pattern in SA order (the iterator loop of match_test.c:599-603)."""

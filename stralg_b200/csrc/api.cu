@@ -9,6 +9,7 @@
 #include <new>
 #include <string.h>
 #include <algorithm>
+#include <type_traits>
 #include <atomic>
 #include <chrono>
 #include <vector>
@@ -42,52 +43,83 @@ static enum b200sa_error code_of(cudaError_t e) {
     return e == cudaErrorMemoryAllocation ? B200SA_ERR_OUT_OF_MEMORY : B200SA_ERR_CUDA;
 }
 
-#define API_GUARD_BEGIN try {
-#define API_GUARD_END(errptr)                                                    \
-    }                                                                            \
-    catch (const CudaFailure &e) {                                               \
-        cudaGetLastError();                                                      \
-        return fail(code_of(e.code), e.what(), errptr);                          \
-    }                                                                            \
-    catch (const std::bad_alloc &) {                                             \
-        return fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", errptr); \
-    }                                                                            \
-    catch (const std::exception &e) {                                            \
-        return fail(B200SA_ERR_INTERNAL, e.what(), errptr);                      \
+// Runs `body`, which returns 0 or a code it has reported through fail(), and turns what it throws into the
+// entry point's error code.  (A template, not std::function: the one-pattern search is a microsecond path.)
+template <class F>
+static int guarded(enum b200sa_error *err, F &&body) {
+    try {
+        return body();
+    } catch (const CudaFailure &e) {
+        cudaGetLastError();
+        return fail(code_of(e.code), e.what(), err);
+    } catch (const std::bad_alloc &) {
+        return fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
+    } catch (const std::invalid_argument &e) {  // (a malformed index file)
+        return fail(B200SA_ERR_BAD_ARGUMENT, e.what(), err);
+    } catch (const std::exception &e) {
+        return fail(B200SA_ERR_INTERNAL, e.what(), err);
     }
+}
+
+// The pointer-returning entry points: a new T filled by `fill(T *)` under guarded().  On any error the object
+// is freed and the result is nullptr; on success `err` is written with B200SA_OK.
+template <class T, class F>
+static T *new_handle(enum b200sa_error *err, F &&fill) {
+    T *h = new (std::nothrow) T();
+    if (!h) {
+        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
+        return nullptr;
+    }
+    if (guarded(err, [&] { return fill(h); }) != 0) {
+        if constexpr (std::is_same<T, b200sa_index>::value) b200sa_free(h);  // (frees its tables on its device)
+        else delete h;
+        return nullptr;
+    }
+    ok(err);
+    return h;
+}
 
 namespace b200sa {
 __global__ void read_back_kernel(const u32 *__restrict__ src, u32 *__restrict__ dst, u32 words) {
     for (u32 i = threadIdx.x; i < words; i += blockDim.x) dst[i] = src[i];
 }
 namespace {
-struct Mailbox {  // one per host thread and device: 4 KB of mapped pinned memory
-    u32 *host[64] = {};
-    u32 *dev[64] = {};
-    ~Mailbox() {
+// One buffer of mapped pinned memory per host thread and device (0 <= device < 64), allocated on first use:
+// read_back uses its first 4 KB, the small-batch search (b200sa_search_batch) all 8 KB.
+const size_t kStagingBytes = 8192;
+struct MappedStaging {
+    u8 *host[64] = {};
+    u8 *dev[64] = {};
+    ~MappedStaging() {
         for (auto p : host)
             if (p) cudaFreeHost(p);
     }
 };
-thread_local Mailbox t_mailbox;
+thread_local MappedStaging t_staging;
 }  // namespace
+static void mapped_staging(int device, u8 *&host, u8 *&dev) {
+    MappedStaging &ms = t_staging;
+    if (!ms.host[device]) {
+        CUDA_CHECK(cudaHostAlloc((void **)&ms.host[device], kStagingBytes, cudaHostAllocMapped));
+        CUDA_CHECK(cudaHostGetDevicePointer((void **)&ms.dev[device], ms.host[device], 0));
+    }
+    host = ms.host[device];
+    dev = ms.dev[device];
+}
 void read_back(void *dst, const void *dev_src, size_t bytes, cudaStream_t st) {
     int device = 0;
     CUDA_CHECK(cudaGetDevice(&device));
-    Mailbox &mb = t_mailbox;
     if (bytes > 4096 || (bytes & 3) || device < 0 || device >= 64) {  // not a mailbox case: plain copy
         CUDA_CHECK(cudaMemcpyAsync(dst, dev_src, bytes, cudaMemcpyDeviceToHost, st));
         CUDA_CHECK(cudaStreamSynchronize(st));
         return;
     }
-    if (!mb.host[device]) {
-        CUDA_CHECK(cudaHostAlloc((void **)&mb.host[device], 4096, cudaHostAllocMapped));
-        CUDA_CHECK(cudaHostGetDevicePointer((void **)&mb.dev[device], mb.host[device], 0));
-    }
-    read_back_kernel<<<1, 64, 0, st>>>((const u32 *)dev_src, mb.dev[device], (u32)(bytes / 4));
+    u8 *host, *dev;
+    mapped_staging(device, host, dev);
+    read_back_kernel<<<1, 64, 0, st>>>((const u32 *)dev_src, (u32 *)dev, (u32)(bytes / 4));
     KERNEL_CHECK();
     CUDA_CHECK(cudaStreamSynchronize(st));
-    memcpy(dst, mb.host[device], bytes);
+    memcpy(dst, host, bytes);
 }
 }  // namespace b200sa
 
@@ -234,6 +266,52 @@ struct SearchLanes {
 static SearchLanes g_lanes[64];
 static SearchLanes &search_lanes(int device) { return g_lanes[device & 63]; }
 
+// Runs `search(d_counters)`.  With `counts`, the kernel counts its traffic into four zeroed device counters,
+// which are read back into `counts`; without, d_counters is null.
+template <class Search>
+static void count_traffic(uint64_t *counts, cudaStream_t st, Search &&search) {
+    if (!counts) return search(nullptr);
+    DevBuf<unsigned long long> d(4, st);
+    CUDA_CHECK(cudaMemsetAsync(d.ptr, 0, 4 * sizeof(unsigned long long), st));
+    search(d.ptr);
+    unsigned long long h[4];
+    CUDA_CHECK(cudaMemcpyAsync(h, d.ptr, sizeof h, cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(cudaStreamSynchronize(st));
+    for (int i = 0; i < 4; ++i) counts[i] = h[i];
+}
+
+// The pipeline of the host-buffer searches: the batch is cut into pieces that alternate between the device's
+// two lanes, so that while the kernel of one piece runs the next piece's patterns cross PCIe and the previous
+// piece's (L, R) return (pinned host memory makes the copies truly asynchronous; pageable memory still works,
+// staged by the driver).  Pieces hold about `piece_bytes` of patterns and start at multiples of 8 patterns.
+// `piece(q0, q1, lane, d_patterns, d_L, d_R)` copies the patterns of [q0, q1) in on `lane` and searches them
+// into d_L / d_R (the piece's slices); the lanes first wait for the work `st` holds.
+template <class Piece>
+static void search_pieces(int device, cudaStream_t st, uint64_t npat, uint64_t total, uint64_t piece_bytes, uint32_t *L,
+                          uint32_t *R, Piece &&piece) {
+    SearchLanes &ln = search_lanes(device);
+    std::lock_guard<std::mutex> lock(ln.mu);
+    ln.reserve(total + 16, npat);
+    uint64_t per = npat;
+    if (total > 2 * piece_bytes) {
+        const uint64_t avg = std::max<uint64_t>(1, total / npat);
+        per = std::max<uint64_t>(1024, (piece_bytes / avg) & ~(uint64_t)7);
+    }
+    CUDA_CHECK(cudaEventRecord(ln.ready, st));
+    CUDA_CHECK(cudaStreamWaitEvent(ln.s[0], ln.ready, 0));
+    CUDA_CHECK(cudaStreamWaitEvent(ln.s[1], ln.ready, 0));
+    uint64_t k = 0;
+    for (uint64_t q0 = 0; q0 < npat; q0 += per, ++k) {
+        const uint64_t q1 = std::min(npat, q0 + per);
+        cudaStream_t ls = ln.s[k & 1];
+        piece(q0, q1, ls, ln.patterns, ln.L + q0, ln.R + q0);
+        CUDA_CHECK(cudaMemcpyAsync(L + q0, ln.L + q0, (q1 - q0) * 4, cudaMemcpyDeviceToHost, ls));
+        CUDA_CHECK(cudaMemcpyAsync(R + q0, ln.R + q0, (q1 - q0) * 4, cudaMemcpyDeviceToHost, ls));
+    }
+    CUDA_CHECK(cudaStreamSynchronize(ln.s[0]));
+    CUDA_CHECK(cudaStreamSynchronize(ln.s[1]));
+}
+
 // ---- native index file ---------------------------------------------------------------------------
 // [header][section]*: the header carries the scalars, every section is {tag, element size, count}
 // + the raw device array, padded to 8 bytes.  Host-endian like the reference's own dumps
@@ -259,6 +337,11 @@ struct SectionHeader {
     uint64_t elem_bytes, count;
 };
 const size_t kIoChunk = (size_t)64 << 20;
+
+struct CloseFile {
+    void operator()(FILE *f) const { fclose(f); }
+};
+using File = std::unique_ptr<FILE, CloseFile>;
 
 struct Section {
     const char *tag;
@@ -300,6 +383,11 @@ void read_section(FILE *f, const SectionHeader &sh, DevBuf<T> &dst, size_t expec
     if (bytes % 8 && fseek(f, (long)(8 - bytes % 8), SEEK_CUR) != 0) throw std::runtime_error("index file: truncated section");
 }
 }  // namespace
+
+static int needs_o_table(const DeviceIndex &ix, enum b200sa_error *err = nullptr) {
+    if (ix.occ_layout != OCC_NONE) return 0;
+    return fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", err);
+}
 
 static bool can_locate(const b200sa_index *idx) {
     return idx->ix.sa.ptr || (idx->ix.ssa_rate && idx->ix.occ_layout != OCC_NONE);
@@ -350,6 +438,37 @@ static bool holds_separator(const b200sa_index *idx, const uint8_t *patterns, co
     return b1 > b0 && memchr(patterns + b0, 1, (size_t)(b1 - b0)) != nullptr;
 }
 
+// ---- the text of a build or an extension: staged, packed with its bad-symbol check, kept for TEXTCMP ----
+static size_t packed_words(const DeviceIndex &ix) { return ((size_t)ix.len + ix.pk.cpw - 1) / ix.pk.cpw + 4; }
+
+// the caller's device text as given, or the host text copied into the arena's side buffer (text[n] = 0)
+static void stage_text(DeviceIndex &ix, Arena &arena, const uint8_t *codes, uint32_t flags) {
+    if (flags & B200SA_TEXT_ON_DEVICE) {
+        ix.text_ptr = codes;
+        return;
+    }
+    u8 *stage = (u8 *)arena.side_alloc((size_t)ix.n + 1);
+    if (ix.n) CUDA_CHECK(cudaMemcpyAsync(stage, codes, ix.n, cudaMemcpyHostToDevice, ix.stream));
+    CUDA_CHECK(cudaMemsetAsync(stage + ix.n, 0, 1, ix.stream));
+    ix.text_ptr = stage;
+}
+
+// pack_text; false when the text holds a code outside 1..sigma-1
+static bool pack_text_checked(DeviceIndex &ix) {
+    DevBuf<int> d_err(1, ix.stream);
+    CUDA_CHECK(cudaMemsetAsync(d_err.ptr, 0, 4, ix.stream));
+    pack_text(ix, d_err.ptr);
+    int herr = 0;
+    read_back(&herr, d_err.ptr, 4, ix.stream);
+    return herr == 0;
+}
+
+static void keep_packed_text(DeviceIndex &ix) {
+    const size_t words = packed_words(ix);
+    ix.text_packed.alloc_output(words, ix.stream);
+    CUDA_CHECK(cudaMemcpyAsync(ix.text_packed.ptr, ix.packed, words * 8, cudaMemcpyDeviceToDevice, ix.stream));
+}
+
 #pragma GCC visibility push(default)
 extern "C" {
 
@@ -364,9 +483,9 @@ int b200sa_device_count(void) {
     return n;
 }
 
+// (called under guarded(): throws on a CUDA failure)
 static int build_into(b200sa_index *h, const uint8_t *codes, uint64_t n, uint32_t sigma, uint32_t flags, int device,
                       void *stream, enum b200sa_error *err) {
-    API_GUARD_BEGIN
     DeviceGuard guard(device);
     DeviceIndex &ix = h->ix;
     ix.stream = (cudaStream_t)stream;
@@ -382,24 +501,12 @@ static int build_into(b200sa_index *h, const uint8_t *codes, uint64_t n, uint32_
     // one build at a time per device: the workspace arena is shared and persistent
     std::lock_guard<std::mutex> arena_lock(g_arena_mu[device & 63]);
     Arena &arena = g_arena[device & 63];
-    if (flags & B200SA_TEXT_ON_DEVICE) {
-        ix.text_ptr = codes;
-    } else {
-        u8 *stage = (u8 *)arena.side_alloc((size_t)n + 1);
-        if (n) CUDA_CHECK(cudaMemcpyAsync(stage, codes, n, cudaMemcpyHostToDevice, st));
-        CUDA_CHECK(cudaMemsetAsync(stage + n, 0, 1, st));
-        ix.text_ptr = stage;
-    }
+    stage_text(ix, arena, codes, flags);
     arena.reset();
     arena.reserve_first(build_workspace_estimate(ix.len, ix.pk.bits));
     ix.arena = &arena;
 
-    DevBuf<int> d_err(1, st);
-    CUDA_CHECK(cudaMemsetAsync(d_err.ptr, 0, 4, st));
-    pack_text(ix, d_err.ptr);
-    int herr = 0;
-    read_back(&herr, d_err.ptr, 4, st);
-    if (herr) {
+    if (!pack_text_checked(ix)) {
         ix.arena = nullptr;
         return fail(B200SA_ERR_BAD_SYMBOL, "text holds a code outside 1..sigma-1", err);
     }
@@ -413,11 +520,7 @@ static int build_into(b200sa_index *h, const uint8_t *codes, uint64_t n, uint32_
     if (flags & (B200SA_BUILD_ISA | B200SA_BUILD_TEXTCMP)) build_inverse(ix);
     if (flags & B200SA_BUILD_LCP) build_lcp(ix);
     if (flags & B200SA_BUILD_OCC) build_bwt_tables(ix, flags & B200SA_BUILD_BWT);
-    if (flags & B200SA_BUILD_TEXTCMP) {
-        size_t words = ((size_t)ix.len + ix.pk.cpw - 1) / ix.pk.cpw + 4;
-        ix.text_packed.alloc_output(words, st);
-        CUDA_CHECK(cudaMemcpyAsync(ix.text_packed.ptr, ix.packed, words * 8, cudaMemcpyDeviceToDevice, st));
-    }
+    if (flags & B200SA_BUILD_TEXTCMP) keep_packed_text(ix);
     ix.packed = nullptr;
     ix.arena = nullptr;
     if ((flags & B200SA_BUILD_KTABLE) && (flags & B200SA_BUILD_OCC)) build_ktable(ix);
@@ -434,8 +537,7 @@ static int build_into(b200sa_index *h, const uint8_t *codes, uint64_t n, uint32_
         }
         ix.timer.clear();
     }
-    return ok(err);
-    API_GUARD_END(err)
+    return 0;
 }
 
 b200sa_index *b200sa_build(const uint8_t *codes, uint64_t n, uint32_t sigma, uint32_t flags, int device,
@@ -448,16 +550,8 @@ b200sa_index *b200sa_build(const uint8_t *codes, uint64_t n, uint32_t sigma, uin
         fail(B200SA_ERR_TOO_LARGE, "n exceeds 2^32 - 2 (uint32 suffix arrays, suffix_array.h:10-20)", err);
         return nullptr;
     }
-    b200sa_index *h = new (std::nothrow) b200sa_index();
-    if (!h) {
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-        return nullptr;
-    }
-    if (build_into(h, codes, n, sigma, flags, device, stream, err) != 0) {
-        b200sa_free(h);
-        return nullptr;
-    }
-    return h;
+    return new_handle<b200sa_index>(
+        err, [&](b200sa_index *h) { return build_into(h, codes, n, sigma, flags, device, stream, err); });
 }
 
 b200sa_index *b200sa_build_records(const uint8_t *codes, const uint64_t *rec_off, uint32_t nrec, uint32_t sigma,
@@ -489,13 +583,7 @@ b200sa_index *b200sa_build_records(const uint8_t *codes, const uint64_t *rec_off
         return nullptr;
     }
     const uint64_t n = ncodes + nrec;
-    b200sa_index *h = new (std::nothrow) b200sa_index();
-    if (!h) {
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-        return nullptr;
-    }
-    int rc = 0;
-    try {
+    return new_handle<b200sa_index>(err, [&](b200sa_index *h) {
         DeviceGuard guard(device);
         cudaStream_t st = (cudaStream_t)stream;
         const std::vector<u64> off(rec_off, rec_off + nrec + 1);
@@ -519,28 +607,12 @@ b200sa_index *b200sa_build_records(const uint8_t *codes, const uint64_t *rec_off
         read_back(&herr, d_err.ptr, 4, st);  // (synchronises the stream: the assembly is done)
         staged.release();
         d_off.release();
-        if (herr) {
-            rc = fail(B200SA_ERR_BAD_SYMBOL, "a record holds a code outside 2..sigma-1 (1 is the separator)", err);
-        } else {
-            rc = build_into(h, text.ptr, n, sigma, flags | B200SA_TEXT_ON_DEVICE, device, stream, err);
-            if (rc == 0) {
-                h->flags = flags & ~B200SA_TEXT_ON_DEVICE;
-                set_records(h->ix, off, st);
-            }
-        }
-    } catch (const CudaFailure &e) {
-        cudaGetLastError();
-        rc = fail(code_of(e.code), e.what(), err);
-    } catch (const std::bad_alloc &) {
-        rc = fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-    } catch (const std::exception &e) {
-        rc = fail(B200SA_ERR_INTERNAL, e.what(), err);
-    }
-    if (rc != 0) {
-        b200sa_free(h);
-        return nullptr;
-    }
-    return h;
+        if (herr) return fail(B200SA_ERR_BAD_SYMBOL, "a record holds a code outside 2..sigma-1 (1 is the separator)", err);
+        if (int rc = build_into(h, text.ptr, n, sigma, flags | B200SA_TEXT_ON_DEVICE, device, stream, err)) return rc;
+        h->flags = flags & ~B200SA_TEXT_ON_DEVICE;
+        set_records(h->ix, off, st);
+        return 0;
+    });
 }
 
 int b200sa_records(const b200sa_index *idx, uint32_t *nrec, uint64_t *rec_off) {
@@ -566,67 +638,53 @@ int b200sa_extend(b200sa_index *idx, const uint8_t *codes, uint32_t flags) {
     const bool need_ktable = (flags & B200SA_BUILD_KTABLE) && !ix.ktable.ptr && (need_occ || ix.occ_layout != OCC_NONE);
     if (!need_isa && !need_lcp && !need_bwt && !need_textcmp && !need_ktable) return 0;
     mail_server_release(idx);  // (the resident one-pattern search was launched with the tables as they were)
-    API_GUARD_BEGIN
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    std::lock_guard<std::mutex> arena_lock(g_arena_mu[ix.device & 63]);
-    Arena &arena = g_arena[ix.device & 63];
-    arena.reset();
-    arena.reserve_first((size_t)ix.len * ix.pk.bits / 8 + (need_lcp ? (size_t)ix.len * 13 : 0) + ((size_t)64 << 20));
-    ix.arena = &arena;
-    if (flags & B200SA_TEXT_ON_DEVICE) {
-        ix.text_ptr = codes;
-    } else {
-        u8 *stage = (u8 *)arena.side_alloc((size_t)ix.n + 1);
-        if (ix.n) CUDA_CHECK(cudaMemcpyAsync(stage, codes, ix.n, cudaMemcpyHostToDevice, st));
-        ix.text_ptr = stage;
-    }
-    DevBuf<int> d_err(1, st);
-    CUDA_CHECK(cudaMemsetAsync(d_err.ptr, 0, 4, st));
-    // the text must be the one the suffix array was built from: same symbol counts, no bad code
-    // (pack_text recomputes the C table; the index keeps its own until the text has been accepted)
-    u32 c_saved[256];
-    u64 counts_saved[256];
-    memcpy(c_saved, ix.c_host, sizeof c_saved);
-    memcpy(counts_saved, ix.sym_counts_host, sizeof counts_saved);
-    DevBuf<u32> c_table_saved = std::move(ix.c_table);
-    pack_text(ix, d_err.ptr);
-    int herr = 0;
-    read_back(&herr, d_err.ptr, 4, st);
-    const bool same_text = memcmp(counts_saved, ix.sym_counts_host, sizeof counts_saved) == 0;
-    if (herr || !same_text) {
-        memcpy(ix.c_host, c_saved, sizeof c_saved);
-        memcpy(ix.sym_counts_host, counts_saved, sizeof counts_saved);
-        ix.c_table = std::move(c_table_saved);
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        std::lock_guard<std::mutex> arena_lock(g_arena_mu[ix.device & 63]);
+        Arena &arena = g_arena[ix.device & 63];
+        arena.reset();
+        arena.reserve_first((size_t)ix.len * ix.pk.bits / 8 + (need_lcp ? (size_t)ix.len * 13 : 0) + ((size_t)64 << 20));
+        ix.arena = &arena;
+        stage_text(ix, arena, codes, flags);
+        // the text must be the one the suffix array was built from: same symbol counts, no bad code
+        // (pack_text recomputes the C table; the index keeps its own until the text has been accepted)
+        u32 c_saved[256];
+        u64 counts_saved[256];
+        memcpy(c_saved, ix.c_host, sizeof c_saved);
+        memcpy(counts_saved, ix.sym_counts_host, sizeof counts_saved);
+        DevBuf<u32> c_table_saved = std::move(ix.c_table);
+        const bool good_symbols = pack_text_checked(ix);
+        const bool same_text = memcmp(counts_saved, ix.sym_counts_host, sizeof counts_saved) == 0;
+        if (!good_symbols || !same_text) {
+            memcpy(ix.c_host, c_saved, sizeof c_saved);
+            memcpy(ix.sym_counts_host, counts_saved, sizeof counts_saved);
+            ix.c_table = std::move(c_table_saved);
+            ix.text_ptr = nullptr;
+            ix.packed = nullptr;
+            ix.arena = nullptr;
+            if (!good_symbols) return fail(B200SA_ERR_BAD_SYMBOL, "text holds a code outside 1..sigma-1", nullptr);
+            return fail(B200SA_ERR_BAD_ARGUMENT, "b200sa_extend: not the text this index was built from (symbol counts differ)", nullptr);
+        }
+        ix.text.release();
         ix.text_ptr = nullptr;
+        if (need_isa) build_inverse(ix);
+        if (need_lcp) build_lcp(ix);
+        if (need_bwt) {
+            const bool had_bwt = ix.bwt.ptr != nullptr;
+            if (!had_bwt) gather_bwt(ix);
+            if (need_occ) build_bwt_tables(ix, had_bwt || (flags & B200SA_BUILD_BWT));
+        }
+        if (need_textcmp) keep_packed_text(ix);
         ix.packed = nullptr;
         ix.arena = nullptr;
-        if (herr) return fail(B200SA_ERR_BAD_SYMBOL, "text holds a code outside 1..sigma-1", nullptr);
-        return fail(B200SA_ERR_BAD_ARGUMENT, "b200sa_extend: not the text this index was built from (symbol counts differ)", nullptr);
-    }
-    ix.text.release();
-    ix.text_ptr = nullptr;
-    if (need_isa) build_inverse(ix);
-    if (need_lcp) build_lcp(ix);
-    if (need_bwt) {
-        const bool had_bwt = ix.bwt.ptr != nullptr;
-        if (!had_bwt) gather_bwt(ix);
-        if (need_occ) build_bwt_tables(ix, had_bwt || (flags & B200SA_BUILD_BWT));
-    }
-    if (need_textcmp) {
-        size_t words = ((size_t)ix.len + ix.pk.cpw - 1) / ix.pk.cpw + 4;
-        ix.text_packed.alloc_output(words, st);
-        CUDA_CHECK(cudaMemcpyAsync(ix.text_packed.ptr, ix.packed, words * 8, cudaMemcpyDeviceToDevice, st));
-    }
-    ix.packed = nullptr;
-    ix.arena = nullptr;
-    if (need_ktable) build_ktable(ix);
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    idx->flags |= flags & (B200SA_BUILD_ISA | B200SA_BUILD_LCP | B200SA_BUILD_BWT | B200SA_BUILD_OCC);
-    if (ix.text_packed.ptr) idx->flags |= B200SA_BUILD_TEXTCMP;
-    if (ix.ktable.ptr) idx->flags |= B200SA_BUILD_KTABLE;
-    return 0;
-    API_GUARD_END(nullptr)
+        if (need_ktable) build_ktable(ix);
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        idx->flags |= flags & (B200SA_BUILD_ISA | B200SA_BUILD_LCP | B200SA_BUILD_BWT | B200SA_BUILD_OCC);
+        if (ix.text_packed.ptr) idx->flags |= B200SA_BUILD_TEXTCMP;
+        if (ix.ktable.ptr) idx->flags |= B200SA_BUILD_KTABLE;
+        return 0;
+    });
 }
 
 // ---- resident one-pattern search (fm_search.cu: fm_mailbox_server_kernel) --------------------------------
@@ -807,60 +865,49 @@ const uint32_t *b200sa_device_lcp(const b200sa_index *idx) { return idx ? idx->i
 const uint8_t *b200sa_device_bwt(const b200sa_index *idx) { return idx ? idx->ix.bwt.ptr : nullptr; }
 const uint8_t *b200sa_device_occ(const b200sa_index *idx) { return idx ? idx->ix.occ.ptr : nullptr; }
 
-static int copy_out(const b200sa_index *idx, const void *dptr, void *host, size_t bytes, const char *what) {
-    if (!idx || !host) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    if (!dptr) return fail(B200SA_ERR_NOT_BUILT, std::string(what) + " was not requested at build time", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    const size_t piece = (size_t)32 << 20;  // (pieces measured faster than one multi-gigabyte copy: 57 vs 52 GB/s)
-    for (size_t at = 0; at < bytes; at += piece)
-        CUDA_CHECK(cudaMemcpyAsync((char *)host + at, (const char *)dptr + at, std::min(piece, bytes - at),
-                                   cudaMemcpyDeviceToHost, idx->ix.stream));
-    CUDA_CHECK(cudaStreamSynchronize(idx->ix.stream));
-    return 0;
-    API_GUARD_END(nullptr)
+// (device pointer, bytes, name) of a table; false for an unknown table id
+static bool table_of(const DeviceIndex &ix, int what, const void *&dptr, size_t &bytes, const char *&name) {
+    switch (what) {
+        case B200SA_TABLE_SA: dptr = ix.sa.ptr; bytes = (size_t)ix.len * 4; name = "SA"; return true;
+        case B200SA_TABLE_ISA: dptr = ix.isa.ptr; bytes = (size_t)ix.len * 4; name = "ISA"; return true;
+        case B200SA_TABLE_LCP: dptr = ix.lcp.ptr; bytes = (size_t)ix.len * 4; name = "LCP"; return true;
+        case B200SA_TABLE_BWT: dptr = ix.bwt.ptr; bytes = (size_t)ix.len; name = "BWT"; return true;
+        case B200SA_TABLE_OCC: dptr = ix.occ.ptr; bytes = ix.occ.bytes(); name = "O table"; return true;
+        default: return false;
+    }
 }
 
-int b200sa_copy_sa(const b200sa_index *idx, uint32_t *host) {
-    return copy_out(idx, idx ? idx->ix.sa.ptr : nullptr, host, idx ? (size_t)idx->ix.len * 4 : 0, "SA");
-}
-int b200sa_copy_isa(const b200sa_index *idx, uint32_t *host) {
-    return copy_out(idx, idx ? idx->ix.isa.ptr : nullptr, host, idx ? (size_t)idx->ix.len * 4 : 0, "ISA");
-}
-int b200sa_copy_lcp(const b200sa_index *idx, uint32_t *host) {
-    return copy_out(idx, idx ? idx->ix.lcp.ptr : nullptr, host, idx ? (size_t)idx->ix.len * 4 : 0, "LCP");
-}
-int b200sa_copy_bwt(const b200sa_index *idx, uint8_t *host) {
-    return copy_out(idx, idx ? idx->ix.bwt.ptr : nullptr, host, idx ? (size_t)idx->ix.len : 0, "BWT");
-}
-int b200sa_copy_occ(const b200sa_index *idx, uint8_t *host) {
-    return copy_out(idx, idx ? idx->ix.occ.ptr : nullptr, host, idx ? idx->ix.occ.bytes() : 0, "O table");
-}
-// Asynchronous copy of one table into caller-owned (pinned) host memory, ordered on `stream`.
-int b200sa_copy_async(const b200sa_index *idx, int what, void *host, void *stream) {
+// One table into host memory: ordered on `stream`, or on the index's stream and waited for (`wait`).
+static int copy_table(const b200sa_index *idx, int what, void *host, void *stream, bool wait) {
     if (!idx || !host) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    const DeviceIndex &ix = idx->ix;
     const void *src = nullptr;
     size_t bytes = 0;
-    switch (what) {
-        case B200SA_TABLE_SA: src = ix.sa.ptr; bytes = (size_t)ix.len * 4; break;
-        case B200SA_TABLE_ISA: src = ix.isa.ptr; bytes = (size_t)ix.len * 4; break;
-        case B200SA_TABLE_LCP: src = ix.lcp.ptr; bytes = (size_t)ix.len * 4; break;
-        case B200SA_TABLE_BWT: src = ix.bwt.ptr; bytes = (size_t)ix.len; break;
-        case B200SA_TABLE_OCC: src = ix.occ.ptr; bytes = ix.occ.bytes(); break;
-        default: return fail(B200SA_ERR_BAD_ARGUMENT, "unknown table", nullptr);
-    }
-    if (!src) return fail(B200SA_ERR_NOT_BUILT, "table was not requested at build time (or was dropped)", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(ix.device);
-    // in pieces: the device-to-host copy engine serves one copy at a time, and a build running next to
-    // this transfer reads a few words back per stage -- those must not queue behind gigabytes
-    const size_t piece = (size_t)32 << 20;
-    for (size_t at = 0; at < bytes; at += piece)
-        CUDA_CHECK(cudaMemcpyAsync((char *)host + at, (const char *)src + at, std::min(piece, bytes - at),
-                                   cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    return 0;
-    API_GUARD_END(nullptr)
+    const char *name = nullptr;
+    if (!table_of(idx->ix, what, src, bytes, name)) return fail(B200SA_ERR_BAD_ARGUMENT, "unknown table", nullptr);
+    if (!src) return fail(B200SA_ERR_NOT_BUILT, std::string(name) + " was not requested at build time (or was dropped)", nullptr);
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(idx->ix.device);
+        const cudaStream_t st = wait ? idx->ix.stream : (cudaStream_t)stream;
+        // in pieces: they measured faster than one multi-gigabyte copy (57 vs 52 GB/s), and the device-to-host
+        // copy engine serves one copy at a time -- a build running next to this transfer reads a few words back
+        // per stage, and those must not queue behind gigabytes
+        const size_t piece = (size_t)32 << 20;
+        for (size_t at = 0; at < bytes; at += piece)
+            CUDA_CHECK(cudaMemcpyAsync((char *)host + at, (const char *)src + at, std::min(piece, bytes - at),
+                                       cudaMemcpyDeviceToHost, st));
+        if (wait) CUDA_CHECK(cudaStreamSynchronize(st));
+        return 0;
+    });
+}
+
+int b200sa_copy_sa(const b200sa_index *idx, uint32_t *host) { return copy_table(idx, B200SA_TABLE_SA, host, nullptr, true); }
+int b200sa_copy_isa(const b200sa_index *idx, uint32_t *host) { return copy_table(idx, B200SA_TABLE_ISA, host, nullptr, true); }
+int b200sa_copy_lcp(const b200sa_index *idx, uint32_t *host) { return copy_table(idx, B200SA_TABLE_LCP, host, nullptr, true); }
+int b200sa_copy_bwt(const b200sa_index *idx, uint8_t *host) { return copy_table(idx, B200SA_TABLE_BWT, host, nullptr, true); }
+int b200sa_copy_occ(const b200sa_index *idx, uint8_t *host) { return copy_table(idx, B200SA_TABLE_OCC, host, nullptr, true); }
+// Asynchronous copy of one table into caller-owned (pinned) host memory, ordered on `stream`.
+int b200sa_copy_async(const b200sa_index *idx, int what, void *host, void *stream) {
+    return copy_table(idx, what, host, stream, false);
 }
 uint64_t b200sa_launch_count(void) { return b200sa::g_kernel_launches; }
 int b200sa_plan_round0(uint32_t len, uint32_t sigma, const uint64_t *sym_counts, uint64_t out[16]) {
@@ -875,20 +922,20 @@ int b200sa_plan_round0(uint32_t len, uint32_t sigma, const uint64_t *sym_counts,
 }
 uint64_t b200sa_workspace_bytes(int device) { return g_arena[device & 63].reserved(); }
 int b200sa_release_workspace(int device) {
-    API_GUARD_BEGIN
-    DeviceGuard guard(device);
-    std::lock_guard<std::mutex> lock(g_arena_mu[device & 63]);
-    g_arena[device & 63].release_all();
-    output_cache_purge(device);
-    cudaDeviceSynchronize();
-    cudaMemPoolTrimTo(library_pool(), 0);
-    {
-        SearchLanes &ln = search_lanes(device);
-        std::lock_guard<std::mutex> l2(ln.mu);
-        ln.release();
-    }
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(device);
+        std::lock_guard<std::mutex> lock(g_arena_mu[device & 63]);
+        g_arena[device & 63].release_all();
+        output_cache_purge(device);
+        cudaDeviceSynchronize();
+        cudaMemPoolTrimTo(library_pool(), 0);
+        {
+            SearchLanes &ln = search_lanes(device);
+            std::lock_guard<std::mutex> l2(ln.mu);
+            ln.release();
+        }
+        return 0;
+    });
 }
 int b200sa_copy_c_table(const b200sa_index *idx, uint32_t *host) {
     if (!idx || !host) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
@@ -899,171 +946,143 @@ int b200sa_copy_c_table(const b200sa_index *idx, uint32_t *host) {
 int b200sa_copy_o_dense(const b200sa_index *idx, uint32_t *host) {
     if (!idx || !host) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     const DeviceIndex &ix = idx->ix;
-    if (ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", nullptr);
+    if (int rc = needs_o_table(ix)) return rc;
     uint64_t entries = ((uint64_t)ix.len + 1) * ix.sigma;
     if (entries * 4 > 0xFFFFFFFFull)
         return fail(B200SA_ERR_TOO_LARGE, "dense O table exceeds the reference's u32 byte size (bwt.c:50)", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(ix.device);
-    DevBuf<u32> d(entries, ix.stream);
-    occ_dense(ix, d.ptr);
-    CUDA_CHECK(cudaMemcpyAsync(host, d.ptr, entries * 4, cudaMemcpyDeviceToHost, ix.stream));
-    CUDA_CHECK(cudaStreamSynchronize(ix.stream));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(ix.device);
+        DevBuf<u32> d(entries, ix.stream);
+        occ_dense(ix, d.ptr);
+        CUDA_CHECK(cudaMemcpyAsync(host, d.ptr, entries * 4, cudaMemcpyDeviceToHost, ix.stream));
+        CUDA_CHECK(cudaStreamSynchronize(ix.stream));
+        return 0;
+    });
 }
 
 int b200sa_occ(const b200sa_index *idx, const uint8_t *a, const uint32_t *i, uint64_t count, uint32_t *out) {
     if (!idx || (count && (!a || !i || !out))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     const DeviceIndex &ix = idx->ix;
-    if (ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", nullptr);
+    if (int rc = needs_o_table(ix)) return rc;
     for (uint64_t q = 0; q < count; ++q)
         if (a[q] >= ix.sigma || i[q] > ix.len) return fail(B200SA_ERR_BAD_ARGUMENT, "O(a,i) query out of range", nullptr);
     if (!count) return 0;
-    API_GUARD_BEGIN
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    DevBuf<u8> da(count, st);
-    DevBuf<u32> di(count, st), dout(count, st);
-    CUDA_CHECK(cudaMemcpyAsync(da.ptr, a, count, cudaMemcpyHostToDevice, st));
-    CUDA_CHECK(cudaMemcpyAsync(di.ptr, i, count * 4, cudaMemcpyHostToDevice, st));
-    occ_probe(ix, da.ptr, di.ptr, count, dout.ptr);
-    CUDA_CHECK(cudaMemcpyAsync(out, dout.ptr, count * 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        DevBuf<u8> da(count, st);
+        DevBuf<u32> di(count, st), dout(count, st);
+        CUDA_CHECK(cudaMemcpyAsync(da.ptr, a, count, cudaMemcpyHostToDevice, st));
+        CUDA_CHECK(cudaMemcpyAsync(di.ptr, i, count * 4, cudaMemcpyHostToDevice, st));
+        occ_probe(ix, da.ptr, di.ptr, count, dout.ptr);
+        CUDA_CHECK(cudaMemcpyAsync(out, dout.ptr, count * 4, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        return 0;
+    });
+}
+
+// b200sa_search_device and, with `traffic`, b200sa_search_traffic
+static int search_device(const b200sa_index *idx, const uint8_t *d_patterns, const uint64_t *d_offsets, uint32_t fixed_len,
+                         uint64_t npat, uint32_t *d_L, uint32_t *d_R, bool traffic, uint64_t *counts, void *stream) {
+    if (!idx || (traffic && !counts) || (npat && (!d_patterns || !d_L || !d_R)))
+        return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
+    if (int rc = needs_o_table(idx->ix)) return rc;
+    if (traffic && (idx->ix.occ_layout != OCC_DNA32 || (((uintptr_t)d_patterns) & 7)))
+        return fail(B200SA_ERR_NOT_BUILT, "traffic counters exist for the DNA search kernel (8-byte aligned patterns) only", nullptr);
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(idx->ix.device);
+        const cudaStream_t st = (cudaStream_t)stream;
+        count_traffic(counts, st, [&](unsigned long long *d_counts) {
+            fm_search(idx->ix, d_patterns, d_offsets, fixed_len, npat, d_L, d_R, st, d_counts);
+        });
+        return 0;
+    });
 }
 
 int b200sa_search_device(const b200sa_index *idx, const uint8_t *d_patterns, const uint64_t *d_offsets,
                          uint32_t fixed_len, uint64_t npat, uint32_t *d_L, uint32_t *d_R, void *stream) {
-    if (!idx || (npat && (!d_patterns || !d_L || !d_R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    if (idx->ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    fm_search(idx->ix, d_patterns, d_offsets, fixed_len, npat, d_L, d_R, (cudaStream_t)stream);
-    return 0;
-    API_GUARD_END(nullptr)
+    return search_device(idx, d_patterns, d_offsets, fixed_len, npat, d_L, d_R, false, nullptr, stream);
 }
 
 int b200sa_search_traffic(const b200sa_index *idx, const uint8_t *d_patterns, const uint64_t *d_offsets,
                           uint32_t fixed_len, uint64_t npat, uint32_t *d_L, uint32_t *d_R, uint64_t counts[4],
                           void *stream) {
-    if (!idx || !counts || (npat && (!d_patterns || !d_L || !d_R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    if (idx->ix.occ_layout != OCC_DNA32 || (((uintptr_t)d_patterns) & 7))
-        return fail(B200SA_ERR_NOT_BUILT, "traffic counters exist for the DNA search kernel (8-byte aligned patterns) only", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    cudaStream_t st = (cudaStream_t)stream;
-    DevBuf<unsigned long long> d(4, st);
-    CUDA_CHECK(cudaMemsetAsync(d.ptr, 0, 4 * sizeof(unsigned long long), st));
-    fm_search(idx->ix, d_patterns, d_offsets, fixed_len, npat, d_L, d_R, st, d.ptr);
-    unsigned long long h[4];
-    CUDA_CHECK(cudaMemcpyAsync(h, d.ptr, sizeof h, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    for (int i = 0; i < 4; ++i) counts[i] = h[i];
-    return 0;
-    API_GUARD_END(nullptr)
+    return search_device(idx, d_patterns, d_offsets, fixed_len, npat, d_L, d_R, true, counts, stream);
 }
 
 // Host buffers in, host (L, R) out.
 //  * A handful of short patterns (the reference's one-pattern iterator, bwt.c:164-199, through the
 //    drop-in): the patterns are written into mapped pinned memory, one kernel reads them there and
 //    stores (L, R) next to them -- one launch and one stream synchronisation, no cudaMemcpy.
-//  * Otherwise the batch is cut into pieces that alternate between two internal streams: while the
-//    kernel of one piece runs, the patterns of the next cross PCIe and the results of the previous
-//    one return (pinned host memory makes the copies truly asynchronous; pageable memory still
-//    works, staged by the driver).  Streams and device staging persist per device (SearchLanes).
+//  * Otherwise the batch goes through search_pieces (two internal streams per device, SearchLanes).
 namespace {
-struct SearchMailbox {  // per host thread and device: 8 KB of mapped pinned memory
-    u8 *host[64] = {};
-    u8 *dev[64] = {};
-    ~SearchMailbox() {
-        for (auto p : host)
-            if (p) cudaFreeHost(p);
-    }
-};
-thread_local SearchMailbox t_search_mailbox;
-const size_t kMailPat = 4096, kMailOff = 4096, kMailL = 4096 + 65 * 8, kMailR = kMailL + 64 * 4, kMailBytes = 8192;
+const size_t kMailPat = 4096, kMailOff = 4096, kMailL = 4096 + 65 * 8, kMailR = kMailL + 64 * 4;
+static_assert(kMailR + 64 * 4 <= kStagingBytes, "the small-batch layout fits the mapped staging buffer");
 }  // namespace
 
 int b200sa_search_batch(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets,
                         uint32_t fixed_len, uint64_t npat, uint32_t *L, uint32_t *R) {
     if (!idx || (npat && (!patterns || !L || !R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    if (idx->ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", nullptr);
+    if (int rc = needs_o_table(idx->ix)) return rc;
     if (!npat) return 0;
     if (holds_separator(idx, patterns, offsets, fixed_len, npat))
         return fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", nullptr);
-    API_GUARD_BEGIN
-    const DeviceIndex &ix = idx->ix;
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    const uint64_t total = offsets ? offsets[npat] : (uint64_t)fixed_len * npat;
-    if (npat == 1) {  // one pattern: the resident kernel, when there is one to be had
-        const uint64_t b0 = offsets ? offsets[0] : 0;
-        if (total - b0 <= kMailMaxPat && mail_server_search(idx, patterns + b0, (uint32_t)(total - b0), L, R)) return 0;
-    }
-    if (npat <= 64 && total + 16 <= kMailPat && ix.device >= 0 && ix.device < 64) {
-        SearchMailbox &mb = t_search_mailbox;
-        if (!mb.host[ix.device]) {
-            CUDA_CHECK(cudaHostAlloc((void **)&mb.host[ix.device], kMailBytes, cudaHostAllocMapped));
-            CUDA_CHECK(cudaHostGetDevicePointer((void **)&mb.dev[ix.device], mb.host[ix.device], 0));
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        const uint64_t total = offsets ? offsets[npat] : (uint64_t)fixed_len * npat;
+        if (npat == 1) {  // one pattern: the resident kernel, when there is one to be had
+            const uint64_t b0 = offsets ? offsets[0] : 0;
+            if (total - b0 <= kMailMaxPat && mail_server_search(idx, patterns + b0, (uint32_t)(total - b0), L, R)) return 0;
         }
-        u8 *h = mb.host[ix.device], *d = mb.dev[ix.device];
-        const uint64_t base = offsets ? offsets[0] : 0;
-        memcpy(h, patterns + base, (size_t)(total - base));
-        memset(h + (total - base), 0, 16);
-        uint64_t *ho = (uint64_t *)(h + kMailOff);
-        if (offsets)
-            for (uint64_t q = 0; q <= npat; ++q) ho[q] = offsets[q] - base;
-        fm_search(ix, d, offsets ? (const u64 *)(d + kMailOff) : nullptr, fixed_len, npat, (u32 *)(d + kMailL),
-                  (u32 *)(d + kMailR), st);
-        CUDA_CHECK(cudaStreamSynchronize(st));
-        memcpy(L, h + kMailL, npat * 4);
-        memcpy(R, h + kMailR, npat * 4);
+        if (npat <= 64 && total + 16 <= kMailPat && ix.device >= 0 && ix.device < 64) {
+            u8 *h, *d;
+            mapped_staging(ix.device, h, d);
+            const uint64_t base = offsets ? offsets[0] : 0;
+            memcpy(h, patterns + base, (size_t)(total - base));
+            memset(h + (total - base), 0, 16);
+            uint64_t *ho = (uint64_t *)(h + kMailOff);
+            if (offsets)
+                for (uint64_t q = 0; q <= npat; ++q) ho[q] = offsets[q] - base;
+            fm_search(ix, d, offsets ? (const u64 *)(d + kMailOff) : nullptr, fixed_len, npat, (u32 *)(d + kMailL),
+                      (u32 *)(d + kMailR), st);
+            CUDA_CHECK(cudaStreamSynchronize(st));
+            memcpy(L, h + kMailL, npat * 4);
+            memcpy(R, h + kMailR, npat * 4);
+            return 0;
+        }
+        DevBuf<u64> doff;
+        if (offsets) {  // (copied in `st`, which the lanes wait for)
+            doff.alloc(npat + 1, st);
+            CUDA_CHECK(cudaMemcpyAsync(doff.ptr, offsets, (npat + 1) * 8, cudaMemcpyHostToDevice, st));
+        }
+        // pieces of ~64 MB of pattern bytes; with a fixed length, multiples of 8 patterns keep every piece's first
+        // byte 8-byte aligned (variable-length patterns share one base pointer)
+        search_pieces(ix.device, st, npat, total, (uint64_t)64 << 20, L, R,
+                      [&](uint64_t q0, uint64_t q1, cudaStream_t ls, u8 *dp, u32 *dL, u32 *dR) {
+                          const uint64_t b0 = offsets ? offsets[q0] : q0 * fixed_len;
+                          const uint64_t b1 = offsets ? offsets[q1] : q1 * fixed_len;
+                          if (b1 > b0) CUDA_CHECK(cudaMemcpyAsync(dp + b0, patterns + b0, b1 - b0, cudaMemcpyHostToDevice, ls));
+                          if (offsets)  // absolute offsets: same pattern base, the piece's slice of the offset array
+                              fm_search(ix, dp, doff.ptr + q0, 0, q1 - q0, dL, dR, ls);
+                          else
+                              fm_search(ix, dp + b0, nullptr, fixed_len, q1 - q0, dL, dR, ls);
+                      });
+        CUDA_CHECK(cudaStreamSynchronize(st));  // (the offsets' buffer is freed on return)
         return 0;
-    }
-    SearchLanes &ln = search_lanes(ix.device);
-    std::lock_guard<std::mutex> lock(ln.mu);
-    ln.reserve(total + 16, npat);
-    u8 *dp = ln.patterns;
-    u32 *dL = ln.L, *dR = ln.R;
-    DevBuf<u64> doff;
-    if (offsets) {
-        doff.alloc(npat + 1, st);
-        CUDA_CHECK(cudaMemcpyAsync(doff.ptr, offsets, (npat + 1) * 8, cudaMemcpyHostToDevice, st));
-    }
-    // pieces of ~64 MB of pattern bytes, cut at multiples of 8 patterns of a fixed length that keep
-    // every piece's first byte 8-byte aligned (variable-length patterns share one base pointer)
-    const uint64_t piece_bytes = (uint64_t)64 << 20;
-    uint64_t per = npat;
-    if (total > 2 * piece_bytes) {
-        const uint64_t avg = std::max<uint64_t>(1, total / npat);
-        per = std::max<uint64_t>(1024, (piece_bytes / avg) & ~(uint64_t)7);
-    }
-    CUDA_CHECK(cudaEventRecord(ln.ready, st));  // (the offsets are copied in `st`)
-    CUDA_CHECK(cudaStreamWaitEvent(ln.s[0], ln.ready, 0));
-    CUDA_CHECK(cudaStreamWaitEvent(ln.s[1], ln.ready, 0));
-    uint64_t k = 0;
-    for (uint64_t q0 = 0; q0 < npat; q0 += per, ++k) {
-        const uint64_t q1 = std::min(npat, q0 + per);
-        cudaStream_t ls = ln.s[k & 1];
-        const uint64_t b0 = offsets ? offsets[q0] : q0 * fixed_len, b1 = offsets ? offsets[q1] : q1 * fixed_len;
-        if (b1 > b0) CUDA_CHECK(cudaMemcpyAsync(dp + b0, patterns + b0, b1 - b0, cudaMemcpyHostToDevice, ls));
-        if (offsets)  // absolute offsets: same pattern base, the piece's slice of the offset array
-            fm_search(ix, dp, doff.ptr + q0, 0, q1 - q0, dL + q0, dR + q0, ls);
-        else
-            fm_search(ix, dp + b0, nullptr, fixed_len, q1 - q0, dL + q0, dR + q0, ls);
-        CUDA_CHECK(cudaMemcpyAsync(L + q0, dL + q0, (q1 - q0) * 4, cudaMemcpyDeviceToHost, ls));
-        CUDA_CHECK(cudaMemcpyAsync(R + q0, dR + q0, (q1 - q0) * 4, cudaMemcpyDeviceToHost, ls));
-    }
-    CUDA_CHECK(cudaStreamSynchronize(ln.s[0]));
-    CUDA_CHECK(cudaStreamSynchronize(ln.s[1]));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return 0;
-    API_GUARD_END(nullptr)
+    });
 }
 
 // ---- packed reads ---------------------------------------------------------------------------------
+// stride 0 stands for ceil(read_len / 4), the least a read of read_len bases takes
+static int packed_stride_ok(uint32_t read_len, uint32_t &stride) {
+    const uint32_t need = (read_len + 3u) / 4u;
+    if (stride == 0) stride = need;
+    if (stride < need) return fail(B200SA_ERR_BAD_ARGUMENT, "stride_bytes smaller than ceil(read_len / 4)", nullptr);
+    return 0;
+}
+
 static int packed_args_ok(const b200sa_index *idx, uint32_t read_len, uint32_t &stride) {
     if (!idx) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (idx->ix.occ_layout != OCC_DNA32)
@@ -1072,48 +1091,39 @@ static int packed_args_ok(const b200sa_index *idx, uint32_t read_len, uint32_t &
     if (idx->ix.nrec)
         return fail(B200SA_ERR_NOT_BUILT, "packed reads do not apply to a records index (code 1 is its separator)", nullptr);
     if (read_len == 0) return fail(B200SA_ERR_BAD_ARGUMENT, "empty reads", nullptr);
-    const uint32_t need = (read_len + 3u) / 4u;
-    if (stride == 0) stride = need;
-    if (stride < need) return fail(B200SA_ERR_BAD_ARGUMENT, "stride_bytes smaller than ceil(read_len / 4)", nullptr);
-    return 0;
+    return packed_stride_ok(read_len, stride);
+}
+
+// b200sa_search_device_packed and, with `traffic`, b200sa_search_traffic_packed
+static int search_device_packed(const b200sa_index *idx, const uint8_t *d_packed, uint32_t read_len, uint32_t stride,
+                                uint64_t npat, uint32_t *d_L, uint32_t *d_R, bool traffic, uint64_t *counts, void *stream) {
+    if (int rc = packed_args_ok(idx, read_len, stride)) return rc;
+    if ((traffic && !counts) || (npat && (!d_packed || !d_L || !d_R)))
+        return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
+    if (((uintptr_t)d_packed) & 7) return fail(B200SA_ERR_BAD_ARGUMENT, "packed reads must be 8-byte aligned", nullptr);
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(idx->ix.device);
+        const cudaStream_t st = (cudaStream_t)stream;
+        count_traffic(counts, st, [&](unsigned long long *d_counts) {
+            fm_search_packed(idx->ix, d_packed, read_len, stride, npat, d_L, d_R, st, d_counts);
+        });
+        return 0;
+    });
 }
 
 int b200sa_search_device_packed(const b200sa_index *idx, const uint8_t *d_packed, uint32_t read_len, uint32_t stride,
                                 uint64_t npat, uint32_t *d_L, uint32_t *d_R, void *stream) {
-    if (int rc = packed_args_ok(idx, read_len, stride)) return rc;
-    if (npat && (!d_packed || !d_L || !d_R)) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    if (((uintptr_t)d_packed) & 7) return fail(B200SA_ERR_BAD_ARGUMENT, "packed reads must be 8-byte aligned", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    fm_search_packed(idx->ix, d_packed, read_len, stride, npat, d_L, d_R, (cudaStream_t)stream);
-    return 0;
-    API_GUARD_END(nullptr)
+    return search_device_packed(idx, d_packed, read_len, stride, npat, d_L, d_R, false, nullptr, stream);
 }
 
 int b200sa_search_traffic_packed(const b200sa_index *idx, const uint8_t *d_packed, uint32_t read_len, uint32_t stride,
                                  uint64_t npat, uint32_t *d_L, uint32_t *d_R, uint64_t counts[4], void *stream) {
-    if (int rc = packed_args_ok(idx, read_len, stride)) return rc;
-    if (!counts || (npat && (!d_packed || !d_L || !d_R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    if (((uintptr_t)d_packed) & 7) return fail(B200SA_ERR_BAD_ARGUMENT, "packed reads must be 8-byte aligned", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    cudaStream_t st = (cudaStream_t)stream;
-    DevBuf<unsigned long long> d(4, st);
-    CUDA_CHECK(cudaMemsetAsync(d.ptr, 0, 4 * sizeof(unsigned long long), st));
-    fm_search_packed(idx->ix, d_packed, read_len, stride, npat, d_L, d_R, st, d.ptr);
-    unsigned long long h[4];
-    CUDA_CHECK(cudaMemcpyAsync(h, d.ptr, sizeof h, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    for (int i = 0; i < 4; ++i) counts[i] = h[i];
-    return 0;
-    API_GUARD_END(nullptr)
+    return search_device_packed(idx, d_packed, read_len, stride, npat, d_L, d_R, true, counts, stream);
 }
 
 int b200sa_pack_reads(const uint8_t *codes, uint32_t read_len, uint32_t stride, uint64_t npat, uint8_t *packed) {
     if ((npat && (!codes || !packed)) || read_len == 0) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    const uint32_t need = (read_len + 3u) / 4u;
-    if (stride == 0) stride = need;
-    if (stride < need) return fail(B200SA_ERR_BAD_ARGUMENT, "stride_bytes smaller than ceil(read_len / 4)", nullptr);
+    if (int rc = packed_stride_ok(read_len, stride)) return rc;
     bool bad = false;
     for (uint64_t q = 0; q < npat; ++q) {
         const uint8_t *r = codes + q * (uint64_t)read_len;
@@ -1140,61 +1150,38 @@ int b200sa_pack_reads(const uint8_t *codes, uint32_t read_len, uint32_t stride, 
 int b200sa_pack_reads_device(const uint8_t *d_codes, uint32_t read_len, uint32_t stride, uint64_t npat,
                              uint8_t *d_packed, int device, void *stream) {
     if ((npat && (!d_codes || !d_packed)) || read_len == 0) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
-    const uint32_t need = (read_len + 3u) / 4u;
-    if (stride == 0) stride = need;
-    if (stride < need) return fail(B200SA_ERR_BAD_ARGUMENT, "stride_bytes smaller than ceil(read_len / 4)", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(device);
-    cudaStream_t st = (cudaStream_t)stream;
-    DevBuf<int> d_err(1, st);
-    CUDA_CHECK(cudaMemsetAsync(d_err.ptr, 0, 4, st));
-    pack_reads(d_codes, read_len, stride, npat, d_packed, d_err.ptr, st);
-    int herr = 0;
-    read_back(&herr, d_err.ptr, 4, st);
-    if (herr) return fail(B200SA_ERR_BAD_SYMBOL, "a read holds a code outside 1..4", nullptr);
-    return 0;
-    API_GUARD_END(nullptr)
+    if (int rc = packed_stride_ok(read_len, stride)) return rc;
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(device);
+        cudaStream_t st = (cudaStream_t)stream;
+        DevBuf<int> d_err(1, st);
+        CUDA_CHECK(cudaMemsetAsync(d_err.ptr, 0, 4, st));
+        pack_reads(d_codes, read_len, stride, npat, d_packed, d_err.ptr, st);
+        int herr = 0;
+        read_back(&herr, d_err.ptr, 4, st);
+        if (herr) return fail(B200SA_ERR_BAD_SYMBOL, "a read holds a code outside 1..4", nullptr);
+        return 0;
+    });
 }
 
-// Host packed reads in, host (L, R) out: pieces of ~16 MB of packed reads alternate between two
-// internal streams, so that while the kernel of one piece runs the next piece crosses PCIe and the
-// results of the previous one return (pinned host memory makes the copies truly asynchronous).
+// Host packed reads in, host (L, R) out, through search_pieces in pieces of ~16 MB of packed reads.
 int b200sa_search_batch_packed(const b200sa_index *idx, const uint8_t *packed, uint32_t read_len, uint32_t stride,
                                uint64_t npat, uint32_t *L, uint32_t *R) {
     if (int rc = packed_args_ok(idx, read_len, stride)) return rc;
     if (npat && (!packed || !L || !R)) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (!npat) return 0;
-    API_GUARD_BEGIN
-    const DeviceIndex &ix = idx->ix;
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    const uint64_t total = (uint64_t)stride * npat;
-    // a piece starts at a multiple of 8 reads, hence (any stride) at a multiple of 8 bytes
-    uint64_t per = npat;
-    const uint64_t piece_bytes = (uint64_t)16 << 20;
-    if (total > 2 * piece_bytes) per = std::max<uint64_t>(1024, (piece_bytes / stride) & ~(uint64_t)7);
-    SearchLanes &ln = search_lanes(ix.device);
-    std::lock_guard<std::mutex> lock(ln.mu);
-    ln.reserve(total + 16, npat);
-    u8 *dp = ln.patterns;
-    u32 *dL = ln.L, *dR = ln.R;
-    CUDA_CHECK(cudaEventRecord(ln.ready, st));
-    CUDA_CHECK(cudaStreamWaitEvent(ln.s[0], ln.ready, 0));
-    CUDA_CHECK(cudaStreamWaitEvent(ln.s[1], ln.ready, 0));
-    uint64_t k = 0;
-    for (uint64_t q0 = 0; q0 < npat; q0 += per, ++k) {
-        const uint64_t q1 = std::min(npat, q0 + per);
-        cudaStream_t ls = ln.s[k & 1];
-        const uint64_t b0 = q0 * stride, b1 = q1 * stride;
-        CUDA_CHECK(cudaMemcpyAsync(dp + b0, packed + b0, b1 - b0, cudaMemcpyHostToDevice, ls));
-        fm_search_packed(ix, dp + b0, read_len, stride, q1 - q0, dL + q0, dR + q0, ls);
-        CUDA_CHECK(cudaMemcpyAsync(L + q0, dL + q0, (q1 - q0) * 4, cudaMemcpyDeviceToHost, ls));
-        CUDA_CHECK(cudaMemcpyAsync(R + q0, dR + q0, (q1 - q0) * 4, cudaMemcpyDeviceToHost, ls));
-    }
-    CUDA_CHECK(cudaStreamSynchronize(ln.s[0]));
-    CUDA_CHECK(cudaStreamSynchronize(ln.s[1]));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        // a piece starts at a multiple of 8 reads, hence (any stride) at a multiple of 8 bytes
+        search_pieces(ix.device, ix.stream, npat, (uint64_t)stride * npat, (uint64_t)16 << 20, L, R,
+                      [&](uint64_t q0, uint64_t q1, cudaStream_t ls, u8 *dp, u32 *dL, u32 *dR) {
+                          const uint64_t b0 = q0 * stride, b1 = q1 * stride;
+                          CUDA_CHECK(cudaMemcpyAsync(dp + b0, packed + b0, b1 - b0, cudaMemcpyHostToDevice, ls));
+                          fm_search_packed(ix, dp + b0, read_len, stride, q1 - q0, dL, dR, ls);
+                      });
+        return 0;
+    });
 }
 
 // ---- several devices in one process ------------------------------------------------------------------
@@ -1203,12 +1190,7 @@ b200sa_index *b200sa_replicate(const b200sa_index *src, int device, void *stream
         fail(B200SA_ERR_BAD_ARGUMENT, "null argument", err);
         return nullptr;
     }
-    b200sa_index *h = new (std::nothrow) b200sa_index();
-    if (!h) {
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-        return nullptr;
-    }
-    try {
+    return new_handle<b200sa_index>(err, [&](b200sa_index *h) {
         {
             DeviceGuard gs(src->ix.device);
             CUDA_CHECK(cudaStreamSynchronize(src->ix.stream));  // the source tables are complete
@@ -1240,16 +1222,8 @@ b200sa_index *b200sa_replicate(const b200sa_index *src, int device, void *stream
         replicate_buf(a.c_table, sd, ix.c_table, device, st, false);
         if (a.nrec) set_records(ix, a.rec_off, st);
         CUDA_CHECK(cudaStreamSynchronize(st));
-        ok(err);
-        return h;
-    } catch (const CudaFailure &e) {
-        cudaGetLastError();
-        fail(code_of(e.code), e.what(), err);
-    } catch (const std::exception &e) {
-        fail(B200SA_ERR_INTERNAL, e.what(), err);
-    }
-    b200sa_free(h);
-    return nullptr;
+        return 0;
+    });
 }
 
 int b200sa_search_sharded_packed(const b200sa_index *const *replicas, int nrep, const uint8_t *packed,
@@ -1269,93 +1243,93 @@ int b200sa_search_sharded_packed(const b200sa_index *const *replicas, int nrep, 
     if (npat && (!packed || !L || !R)) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (!npat) return 0;
     if (nrep == 1) return b200sa_search_batch_packed(replicas[0], packed, read_len, stride, npat, L, R);
-    API_GUARD_BEGIN
-    int prev = -1;
-    cudaGetDevice(&prev);
-    struct Restore {
-        int d;
-        ~Restore() { if (d >= 0) cudaSetDevice(d); }
-    } restore{prev};
-    const int dev0 = replicas[0]->ix.device;
-    // shards: contiguous, boundaries at multiples of 8 reads (every shard's first byte 8-byte aligned)
-    std::vector<uint64_t> lo(nrep + 1);
-    const uint64_t per = ((npat + nrep - 1) / nrep + 7) & ~(uint64_t)7;
-    for (int g = 0; g <= nrep; ++g) lo[g] = std::min(npat, per * (uint64_t)g);
-    // result array in the first replica's HBM
-    std::vector<std::unique_lock<std::mutex>> locks;
-    for (int g = 0; g < nrep; ++g) locks.emplace_back(search_lanes(replicas[g]->ix.device).mu);
-    CUDA_CHECK(cudaSetDevice(dev0));
-    SearchLanes &l0 = search_lanes(dev0);
-    l0.reserve((lo[1] - lo[0]) * stride + 16, npat);
-    std::vector<cudaEvent_t> done(nrep, nullptr);
-    std::vector<char> direct(nrep, 0);
-    for (int g = 0; g < nrep; ++g) {
-        const int dev = replicas[g]->ix.device;
-        CUDA_CHECK(cudaSetDevice(dev));
-        SearchLanes &ln = search_lanes(dev);
-        const uint64_t cnt = lo[g + 1] - lo[g];
-        if (g) ln.reserve(cnt * stride + 16, cnt);
-        else ln.reserve(cnt * stride + 16, npat);
-        u32 *outL = ln.L, *outR = ln.R;
-        if (g) {
-            int can = 0;
-            CUDA_CHECK(cudaDeviceCanAccessPeer(&can, dev, dev0));
-            if (can) {
-                cudaError_t e = cudaDeviceEnablePeerAccess(dev0, 0);
-                if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
-                else if (e != cudaSuccess) can = 0, cudaGetLastError();
+    return guarded(nullptr, [&] {
+        int prev = -1;
+        cudaGetDevice(&prev);
+        struct Restore {
+            int d;
+            ~Restore() { if (d >= 0) cudaSetDevice(d); }
+        } restore{prev};
+        const int dev0 = replicas[0]->ix.device;
+        // shards: contiguous, boundaries at multiples of 8 reads (every shard's first byte 8-byte aligned)
+        std::vector<uint64_t> lo(nrep + 1);
+        const uint64_t per = ((npat + nrep - 1) / nrep + 7) & ~(uint64_t)7;
+        for (int g = 0; g <= nrep; ++g) lo[g] = std::min(npat, per * (uint64_t)g);
+        // result array in the first replica's HBM
+        std::vector<std::unique_lock<std::mutex>> locks;
+        for (int g = 0; g < nrep; ++g) locks.emplace_back(search_lanes(replicas[g]->ix.device).mu);
+        CUDA_CHECK(cudaSetDevice(dev0));
+        SearchLanes &l0 = search_lanes(dev0);
+        l0.reserve((lo[1] - lo[0]) * stride + 16, npat);
+        std::vector<cudaEvent_t> done(nrep, nullptr);
+        std::vector<char> direct(nrep, 0);
+        for (int g = 0; g < nrep; ++g) {
+            const int dev = replicas[g]->ix.device;
+            CUDA_CHECK(cudaSetDevice(dev));
+            SearchLanes &ln = search_lanes(dev);
+            const uint64_t cnt = lo[g + 1] - lo[g];
+            if (g) ln.reserve(cnt * stride + 16, cnt);
+            else ln.reserve(cnt * stride + 16, npat);
+            u32 *outL = ln.L, *outR = ln.R;
+            if (g) {
+                int can = 0;
+                CUDA_CHECK(cudaDeviceCanAccessPeer(&can, dev, dev0));
+                if (can) {
+                    cudaError_t e = cudaDeviceEnablePeerAccess(dev0, 0);
+                    if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+                    else if (e != cudaSuccess) can = 0, cudaGetLastError();
+                }
+                if (can) {  // the kernel stores this shard's (L, R) straight into the first replica's HBM
+                    outL = l0.L + lo[g];
+                    outR = l0.R + lo[g];
+                    direct[g] = 1;
+                }
             }
-            if (can) {  // the kernel stores this shard's (L, R) straight into the first replica's HBM
-                outL = l0.L + lo[g];
-                outR = l0.R + lo[g];
-                direct[g] = 1;
+            cudaStream_t ls = ln.s[0];
+            if (cnt) {
+                CUDA_CHECK(cudaMemcpyAsync(ln.patterns, packed + lo[g] * stride, cnt * stride, cudaMemcpyHostToDevice, ls));
+                fm_search_packed(replicas[g]->ix, ln.patterns, read_len, stride, cnt, outL, outR, ls);
+                if (g && !direct[g]) {
+                    CUDA_CHECK(cudaMemcpyAsync(L + lo[g], outL, cnt * 4, cudaMemcpyDeviceToHost, ls));
+                    CUDA_CHECK(cudaMemcpyAsync(R + lo[g], outR, cnt * 4, cudaMemcpyDeviceToHost, ls));
+                }
             }
+            CUDA_CHECK(cudaEventCreateWithFlags(&done[g], cudaEventDisableTiming));
+            CUDA_CHECK(cudaEventRecord(done[g], ls));
         }
-        cudaStream_t ls = ln.s[0];
-        if (cnt) {
-            CUDA_CHECK(cudaMemcpyAsync(ln.patterns, packed + lo[g] * stride, cnt * stride, cudaMemcpyHostToDevice, ls));
-            fm_search_packed(replicas[g]->ix, ln.patterns, read_len, stride, cnt, outL, outR, ls);
-            if (g && !direct[g]) {
-                CUDA_CHECK(cudaMemcpyAsync(L + lo[g], outL, cnt * 4, cudaMemcpyDeviceToHost, ls));
-                CUDA_CHECK(cudaMemcpyAsync(R + lo[g], outR, cnt * 4, cudaMemcpyDeviceToHost, ls));
-            }
+        // the first replica's stream waits for every peer's kernel, then the result goes home in one piece per range
+        CUDA_CHECK(cudaSetDevice(dev0));
+        for (int g = 1; g < nrep; ++g) CUDA_CHECK(cudaStreamWaitEvent(l0.s[0], done[g], 0));
+        for (int g = 0; g < nrep; ++g) {
+            const uint64_t cnt = lo[g + 1] - lo[g];
+            if (!cnt || (g && !direct[g])) continue;
+            CUDA_CHECK(cudaMemcpyAsync(L + lo[g], l0.L + lo[g], cnt * 4, cudaMemcpyDeviceToHost, l0.s[0]));
+            CUDA_CHECK(cudaMemcpyAsync(R + lo[g], l0.R + lo[g], cnt * 4, cudaMemcpyDeviceToHost, l0.s[0]));
         }
-        CUDA_CHECK(cudaEventCreateWithFlags(&done[g], cudaEventDisableTiming));
-        CUDA_CHECK(cudaEventRecord(done[g], ls));
-    }
-    // the first replica's stream waits for every peer's kernel, then the result goes home in one piece per range
-    CUDA_CHECK(cudaSetDevice(dev0));
-    for (int g = 1; g < nrep; ++g) CUDA_CHECK(cudaStreamWaitEvent(l0.s[0], done[g], 0));
-    for (int g = 0; g < nrep; ++g) {
-        const uint64_t cnt = lo[g + 1] - lo[g];
-        if (!cnt || (g && !direct[g])) continue;
-        CUDA_CHECK(cudaMemcpyAsync(L + lo[g], l0.L + lo[g], cnt * 4, cudaMemcpyDeviceToHost, l0.s[0]));
-        CUDA_CHECK(cudaMemcpyAsync(R + lo[g], l0.R + lo[g], cnt * 4, cudaMemcpyDeviceToHost, l0.s[0]));
-    }
-    for (int g = 0; g < nrep; ++g) {
-        CUDA_CHECK(cudaSetDevice(replicas[g]->ix.device));
-        CUDA_CHECK(cudaStreamSynchronize(search_lanes(replicas[g]->ix.device).s[0]));
-        cudaEventDestroy(done[g]);
-    }
-    return 0;
-    API_GUARD_END(nullptr)
+        for (int g = 0; g < nrep; ++g) {
+            CUDA_CHECK(cudaSetDevice(replicas[g]->ix.device));
+            CUDA_CHECK(cudaStreamSynchronize(search_lanes(replicas[g]->ix.device).s[0]));
+            cudaEventDestroy(done[g]);
+        }
+        return 0;
+    });
 }
 
 int b200sa_locate_device(const b200sa_index *idx, const uint32_t *d_L, const uint32_t *d_R, uint64_t npat,
                          uint64_t *d_pos_off, uint32_t *d_pos, uint64_t pos_capacity, uint64_t *total, void *stream) {
     if (!idx || !d_pos_off || (npat && (!d_L || !d_R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (!can_locate(idx)) return fail(B200SA_ERR_NOT_BUILT, "no suffix array to locate with (dropped and not sampled)", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    cudaStream_t st = (cudaStream_t)stream;
-    u64 t = fm_locate_count(idx->ix, d_L, d_R, npat, d_pos_off, st);
-    if (total) *total = t;
-    if (d_pos) {
-        if (t > pos_capacity) return fail(B200SA_ERR_BAD_ARGUMENT, "position buffer too small", nullptr);
-        locate_fill_any(idx->ix, d_L, d_R, npat, d_pos_off, t, d_pos, st);
-    }
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(idx->ix.device);
+        cudaStream_t st = (cudaStream_t)stream;
+        u64 t = fm_locate_count(idx->ix, d_L, d_R, npat, d_pos_off, st);
+        if (total) *total = t;
+        if (d_pos) {
+            if (t > pos_capacity) return fail(B200SA_ERR_BAD_ARGUMENT, "position buffer too small", nullptr);
+            locate_fill_any(idx->ix, d_L, d_R, npat, d_pos_off, t, d_pos, st);
+        }
+        return 0;
+    });
 }
 
 int b200sa_sort_positions_device(const b200sa_index *idx, uint64_t npat, const uint64_t *d_pos_off, uint64_t total,
@@ -1363,43 +1337,43 @@ int b200sa_sort_positions_device(const b200sa_index *idx, uint64_t npat, const u
     if (!idx || !d_pos_off || (total && !d_pos)) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (total > 0xFFFFFFFFull || npat > 0xFFFFFFFFull)
         return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 positions or patterns in one batch", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    sort_positions(idx->ix, npat, d_pos_off, total, d_pos, (cudaStream_t)stream);
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(idx->ix.device);
+        sort_positions(idx->ix, npat, d_pos_off, total, d_pos, (cudaStream_t)stream);
+        return 0;
+    });
 }
 
 static int locate_batch_impl(const b200sa_index *idx, const uint32_t *L, const uint32_t *R, uint64_t npat,
                         uint64_t *pos_off, uint32_t *pos, uint64_t pos_capacity, uint64_t *total, bool sorted) {
     if (!idx || !pos_off || (npat && (!L || !R))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (!can_locate(idx)) return fail(B200SA_ERR_NOT_BUILT, "no suffix array to locate with (dropped and not sampled)", nullptr);
-    API_GUARD_BEGIN
-    const DeviceIndex &ix = idx->ix;
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    DevBuf<u32> dL(npat ? npat : 1, st), dR(npat ? npat : 1, st);
-    DevBuf<u64> doff(npat + 1, st);
-    if (npat) {
-        CUDA_CHECK(cudaMemcpyAsync(dL.ptr, L, npat * 4, cudaMemcpyHostToDevice, st));
-        CUDA_CHECK(cudaMemcpyAsync(dR.ptr, R, npat * 4, cudaMemcpyHostToDevice, st));
-    }
-    u64 t = fm_locate_count(ix, dL.ptr, dR.ptr, npat, doff.ptr, st);
-    if (total) *total = t;
-    CUDA_CHECK(cudaMemcpyAsync(pos_off, doff.ptr, (npat + 1) * 8, cudaMemcpyDeviceToHost, st));
-    if (pos && t) {
-        if (t > pos_capacity) return fail(B200SA_ERR_BAD_ARGUMENT, "position buffer too small", nullptr);
-        DevBuf<u32> dpos(t, st);
-        locate_fill_any(ix, dL.ptr, dR.ptr, npat, doff.ptr, t, dpos.ptr, st);
-        if (sorted) {
-            if (t > 0xFFFFFFFFull) return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 positions in one batch", nullptr);
-            sort_positions(ix, npat, doff.ptr, t, dpos.ptr, st);
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        DevBuf<u32> dL(npat ? npat : 1, st), dR(npat ? npat : 1, st);
+        DevBuf<u64> doff(npat + 1, st);
+        if (npat) {
+            CUDA_CHECK(cudaMemcpyAsync(dL.ptr, L, npat * 4, cudaMemcpyHostToDevice, st));
+            CUDA_CHECK(cudaMemcpyAsync(dR.ptr, R, npat * 4, cudaMemcpyHostToDevice, st));
         }
-        CUDA_CHECK(cudaMemcpyAsync(pos, dpos.ptr, t * 4, cudaMemcpyDeviceToHost, st));
-    }
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return 0;
-    API_GUARD_END(nullptr)
+        u64 t = fm_locate_count(ix, dL.ptr, dR.ptr, npat, doff.ptr, st);
+        if (total) *total = t;
+        CUDA_CHECK(cudaMemcpyAsync(pos_off, doff.ptr, (npat + 1) * 8, cudaMemcpyDeviceToHost, st));
+        if (pos && t) {
+            if (t > pos_capacity) return fail(B200SA_ERR_BAD_ARGUMENT, "position buffer too small", nullptr);
+            DevBuf<u32> dpos(t, st);
+            locate_fill_any(ix, dL.ptr, dR.ptr, npat, doff.ptr, t, dpos.ptr, st);
+            if (sorted) {
+                if (t > 0xFFFFFFFFull) return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 positions in one batch", nullptr);
+                sort_positions(ix, npat, doff.ptr, t, dpos.ptr, st);
+            }
+            CUDA_CHECK(cudaMemcpyAsync(pos, dpos.ptr, t * 4, cudaMemcpyDeviceToHost, st));
+        }
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        return 0;
+    });
 }
 
 int b200sa_locate_batch(const b200sa_index *idx, const uint32_t *L, const uint32_t *R, uint64_t npat,
@@ -1416,27 +1390,27 @@ int b200sa_record_sas_device(const b200sa_index *idx, uint32_t *d_out, void *str
     if (!idx || !d_out) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (!idx->ix.nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "not a records index (b200sa_build_records)", nullptr);
     if (!idx->ix.sa.ptr) return fail(B200SA_ERR_NOT_BUILT, "the record suffix arrays need the full suffix array (dropped)", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(idx->ix.device);
-    record_sas(idx->ix, d_out, (cudaStream_t)stream);
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(idx->ix.device);
+        record_sas(idx->ix, d_out, (cudaStream_t)stream);
+        return 0;
+    });
 }
 
 int b200sa_copy_record_sas(const b200sa_index *idx, uint32_t *host) {
     if (!idx || !host) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     if (!idx->ix.nrec) return fail(B200SA_ERR_BAD_ARGUMENT, "not a records index (b200sa_build_records)", nullptr);
     if (!idx->ix.sa.ptr) return fail(B200SA_ERR_NOT_BUILT, "the record suffix arrays need the full suffix array (dropped)", nullptr);
-    API_GUARD_BEGIN
-    const DeviceIndex &ix = idx->ix;
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    DevBuf<u32> d(ix.n, st);
-    record_sas(ix, d.ptr, st);
-    if (ix.n) CUDA_CHECK(cudaMemcpyAsync(host, d.ptr, (size_t)ix.n * 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        DevBuf<u32> d(ix.n, st);
+        record_sas(ix, d.ptr, st);
+        if (ix.n) CUDA_CHECK(cudaMemcpyAsync(host, d.ptr, (size_t)ix.n * 4, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        return 0;
+    });
 }
 
 // The rows [max(L, 1), R): row 0 is the global sentinel, which belongs to no record.  The count clamps L into d_L1
@@ -1474,47 +1448,47 @@ int b200sa_locate_records_device(const b200sa_index *idx, const uint32_t *d_L, c
                                  uint64_t *d_pos_off, uint32_t *d_rec, uint32_t *d_pos, uint64_t capacity,
                                  uint64_t *total, void *stream) {
     if (int rc = locate_records_args_ok(idx, d_L, d_R, npat, d_pos_off, d_rec, d_pos)) return rc;
-    API_GUARD_BEGIN
-    const DeviceIndex &ix = idx->ix;
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = (cudaStream_t)stream;
-    DevBuf<u32> dL1(npat ? npat : 1, st);
-    const u64 t = locate_records_count(ix, d_L, d_R, npat, d_pos_off, dL1.ptr, st);
-    if (total) *total = t;
-    if (d_pos && t) {
-        if (int rc = locate_records_fits(t, npat, capacity)) return rc;
-        locate_records_fill(ix, dL1.ptr, d_R, npat, d_pos_off, t, d_rec, d_pos, st);
-    }
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = (cudaStream_t)stream;
+        DevBuf<u32> dL1(npat ? npat : 1, st);
+        const u64 t = locate_records_count(ix, d_L, d_R, npat, d_pos_off, dL1.ptr, st);
+        if (total) *total = t;
+        if (d_pos && t) {
+            if (int rc = locate_records_fits(t, npat, capacity)) return rc;
+            locate_records_fill(ix, dL1.ptr, d_R, npat, d_pos_off, t, d_rec, d_pos, st);
+        }
+        return 0;
+    });
 }
 
 int b200sa_locate_records(const b200sa_index *idx, const uint32_t *L, const uint32_t *R, uint64_t npat,
                           uint64_t *pos_off, uint32_t *rec, uint32_t *pos, uint64_t capacity, uint64_t *total) {
     if (int rc = locate_records_args_ok(idx, L, R, npat, pos_off, rec, pos)) return rc;
-    API_GUARD_BEGIN
-    const DeviceIndex &ix = idx->ix;
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    DevBuf<u32> dL(npat ? npat : 1, st), dR(npat ? npat : 1, st), dL1(npat ? npat : 1, st);
-    DevBuf<u64> doff(npat + 1, st);
-    if (npat) {
-        CUDA_CHECK(cudaMemcpyAsync(dL.ptr, L, npat * 4, cudaMemcpyHostToDevice, st));
-        CUDA_CHECK(cudaMemcpyAsync(dR.ptr, R, npat * 4, cudaMemcpyHostToDevice, st));
-    }
-    const u64 t = locate_records_count(ix, dL.ptr, dR.ptr, npat, doff.ptr, dL1.ptr, st);
-    if (total) *total = t;
-    CUDA_CHECK(cudaMemcpyAsync(pos_off, doff.ptr, (npat + 1) * 8, cudaMemcpyDeviceToHost, st));
-    if (pos && t) {
-        if (int rc = locate_records_fits(t, npat, capacity)) return rc;
-        DevBuf<u32> drec(t, st), dpos(t, st);
-        locate_records_fill(ix, dL1.ptr, dR.ptr, npat, doff.ptr, t, drec.ptr, dpos.ptr, st);
-        CUDA_CHECK(cudaMemcpyAsync(rec, drec.ptr, t * 4, cudaMemcpyDeviceToHost, st));
-        CUDA_CHECK(cudaMemcpyAsync(pos, dpos.ptr, t * 4, cudaMemcpyDeviceToHost, st));
-    }
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        DevBuf<u32> dL(npat ? npat : 1, st), dR(npat ? npat : 1, st), dL1(npat ? npat : 1, st);
+        DevBuf<u64> doff(npat + 1, st);
+        if (npat) {
+            CUDA_CHECK(cudaMemcpyAsync(dL.ptr, L, npat * 4, cudaMemcpyHostToDevice, st));
+            CUDA_CHECK(cudaMemcpyAsync(dR.ptr, R, npat * 4, cudaMemcpyHostToDevice, st));
+        }
+        const u64 t = locate_records_count(ix, dL.ptr, dR.ptr, npat, doff.ptr, dL1.ptr, st);
+        if (total) *total = t;
+        CUDA_CHECK(cudaMemcpyAsync(pos_off, doff.ptr, (npat + 1) * 8, cudaMemcpyDeviceToHost, st));
+        if (pos && t) {
+            if (int rc = locate_records_fits(t, npat, capacity)) return rc;
+            DevBuf<u32> drec(t, st), dpos(t, st);
+            locate_records_fill(ix, dL1.ptr, dR.ptr, npat, doff.ptr, t, drec.ptr, dpos.ptr, st);
+            CUDA_CHECK(cudaMemcpyAsync(rec, drec.ptr, t * 4, cudaMemcpyDeviceToHost, st));
+            CUDA_CHECK(cudaMemcpyAsync(pos, dpos.ptr, t * 4, cudaMemcpyDeviceToHost, st));
+        }
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        return 0;
+    });
 }
 
 int b200sa_sample_sa(b200sa_index *idx, uint32_t rate, int drop_sa) {
@@ -1523,13 +1497,13 @@ int b200sa_sample_sa(b200sa_index *idx, uint32_t rate, int drop_sa) {
     DeviceIndex &ix = idx->ix;
     if (!ix.sa.ptr) return fail(B200SA_ERR_NOT_BUILT, "suffix array was dropped (B200SA_DROP_SA)", nullptr);
     if (ix.occ_layout == OCC_NONE) return fail(B200SA_ERR_NOT_BUILT, "the sampled suffix array needs the O table (B200SA_BUILD_OCC)", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(ix.device);
-    build_sampled_sa(ix, rate);
-    if (drop_sa && !(idx->flags & B200SA_BUILD_TEXTCMP)) ix.sa.release();
-    CUDA_CHECK(cudaStreamSynchronize(ix.stream));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(ix.device);
+        build_sampled_sa(ix, rate);
+        if (drop_sa && !(idx->flags & B200SA_BUILD_TEXTCMP)) ix.sa.release();
+        CUDA_CHECK(cudaStreamSynchronize(ix.stream));
+        return 0;
+    });
 }
 
 int b200sa_sa_lookup(const b200sa_index *idx, const uint32_t *rows, uint64_t count, uint32_t *out, int force_sampled) {
@@ -1540,16 +1514,16 @@ int b200sa_sa_lookup(const b200sa_index *idx, const uint32_t *rows, uint64_t cou
     for (uint64_t q = 0; q < count; ++q)
         if (rows[q] >= ix.len) return fail(B200SA_ERR_BAD_ARGUMENT, "row out of range", nullptr);
     if (!count) return 0;
-    API_GUARD_BEGIN
-    DeviceGuard guard(ix.device);
-    cudaStream_t st = ix.stream;
-    DevBuf<u32> dr(count, st), dout(count, st);
-    CUDA_CHECK(cudaMemcpyAsync(dr.ptr, rows, count * 4, cudaMemcpyHostToDevice, st));
-    sa_lookup_rows(ix, dr.ptr, count, dout.ptr, force_sampled != 0, st);
-    CUDA_CHECK(cudaMemcpyAsync(out, dout.ptr, count * 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(ix.device);
+        cudaStream_t st = ix.stream;
+        DevBuf<u32> dr(count, st), dout(count, st);
+        CUDA_CHECK(cudaMemcpyAsync(dr.ptr, rows, count * 4, cudaMemcpyHostToDevice, st));
+        sa_lookup_rows(ix, dr.ptr, count, dout.ptr, force_sampled != 0, st);
+        CUDA_CHECK(cudaMemcpyAsync(out, dout.ptr, count * 4, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        return 0;
+    });
 }
 
 // ---- native index file: b200sa_save / b200sa_load (layout above, next to the helpers) ----
@@ -1557,12 +1531,13 @@ int b200sa_sa_lookup(const b200sa_index *idx, const uint32_t *rows, uint64_t cou
 int b200sa_save(const b200sa_index *idx, const char *path) {
     if (!idx || !path) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
     const DeviceIndex &ix = idx->ix;
-    FILE *f = fopen(path, "wb");
-    if (!f) return fail(B200SA_ERR_BAD_ARGUMENT, std::string("cannot open ") + path + " for writing", nullptr);
-    try {
+    File file(fopen(path, "wb"));
+    if (!file) return fail(B200SA_ERR_BAD_ARGUMENT, std::string("cannot open ") + path + " for writing", nullptr);
+    return guarded(nullptr, [&] {
+        FILE *f = file.get();
         DeviceGuard guard(ix.device);
         cudaStream_t st = ix.stream;
-        const size_t words = ((size_t)ix.len + ix.pk.cpw - 1) / ix.pk.cpw + 4;
+        const size_t words = packed_words(ix);
         std::vector<Section> secs;
         if (ix.sa.ptr) secs.push_back({"SA", ix.sa.ptr, 4, ix.len});
         if (ix.isa.ptr) secs.push_back({"ISA", ix.isa.ptr, 4, ix.len});
@@ -1603,22 +1578,9 @@ int b200sa_save(const b200sa_index *idx, const char *path) {
         if (fwrite(&h, sizeof h, 1, f) != 1) throw std::runtime_error("index file: short write");
         std::vector<char> buf(kIoChunk);
         for (const Section &sc : secs) write_section(f, sc, buf, st);
-        if (fclose(f) != 0) {
-            f = nullptr;
-            throw std::runtime_error("index file: close failed");
-        }
+        if (fclose(file.release()) != 0) throw std::runtime_error("index file: close failed");  // (buffered data not written)
         return 0;
-    } catch (const CudaFailure &e) {
-        if (f) fclose(f);
-        cudaGetLastError();
-        return fail(code_of(e.code), e.what(), nullptr);
-    } catch (const std::bad_alloc &) {
-        if (f) fclose(f);
-        return fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", nullptr);
-    } catch (const std::exception &e) {
-        if (f) fclose(f);
-        return fail(B200SA_ERR_INTERNAL, e.what(), nullptr);
-    }
+    });
 }
 
 b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200sa_error *err) {
@@ -1626,18 +1588,13 @@ b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200s
         fail(B200SA_ERR_BAD_ARGUMENT, "null path", err);
         return nullptr;
     }
-    FILE *f = fopen(path, "rb");
-    if (!f) {
+    File file(fopen(path, "rb"));
+    if (!file) {
         fail(B200SA_ERR_BAD_ARGUMENT, std::string("cannot open ") + path, err);
         return nullptr;
     }
-    b200sa_index *h = new (std::nothrow) b200sa_index();
-    if (!h) {
-        fclose(f);
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-        return nullptr;
-    }
-    try {
+    return new_handle<b200sa_index>(err, [&](b200sa_index *h) {
+        FILE *f = file.get();
         DeviceGuard guard(device);
         IndexFileHeader fh;
         if (fread(&fh, sizeof fh, 1, f) != 1 || memcmp(fh.magic, "B200SAIX", 8) != 0)
@@ -1678,7 +1635,7 @@ b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200s
         memcpy(ix.sym_counts_host, fh.sym_counts, sizeof fh.sym_counts);
         ix.c_table.alloc(ix.sigma, st);
         CUDA_CHECK(cudaMemcpyAsync(ix.c_table.ptr, ix.c_host, (size_t)ix.sigma * 4, cudaMemcpyHostToDevice, st));
-        const size_t words = ((size_t)ix.len + ix.pk.cpw - 1) / ix.pk.cpw + 4;
+        const size_t words = packed_words(ix);
         const size_t bwt_bytes = (((size_t)ix.len + 63) / 64 + 1) * 64;
         std::vector<char> buf(kIoChunk);
         bool have_occ = false, have_marks = false, have_vals = false;
@@ -1726,24 +1683,9 @@ b200sa_index *b200sa_load(const char *path, int device, void *stream, enum b200s
             (fh.ktable_k != 0) != (ix.ktable.ptr != nullptr))
             throw std::invalid_argument("index file: sections do not match the header");
         ix.ssa_rate = fh.ssa_rate;
-        fclose(f);
-        f = nullptr;
         CUDA_CHECK(cudaStreamSynchronize(st));
-        ok(err);
-        return h;
-    } catch (const CudaFailure &e) {
-        cudaGetLastError();
-        fail(code_of(e.code), e.what(), err);
-    } catch (const std::bad_alloc &) {
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-    } catch (const std::invalid_argument &e) {
-        fail(B200SA_ERR_BAD_ARGUMENT, e.what(), err);
-    } catch (const std::exception &e) {
-        fail(B200SA_ERR_INTERNAL, e.what(), err);
-    }
-    if (f) fclose(f);
-    b200sa_free(h);
-    return nullptr;
+        return 0;
+    });
 }
 
 // ---- approximate search ------------------------------------------------------------------------
@@ -1762,10 +1704,7 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
         return nullptr;
     }
     const DeviceIndex &ix = idx->ix;
-    if (ix.occ_layout == OCC_NONE) {
-        fail(B200SA_ERR_NOT_BUILT, "O table was not requested at build time", err);
-        return nullptr;
-    }
+    if (needs_o_table(ix, err)) return nullptr;
     if (rev_idx && (rev_idx->ix.occ_layout == OCC_NONE || rev_idx->ix.len != ix.len || rev_idx->ix.sigma != ix.sigma ||
                     rev_idx->ix.device != ix.device)) {
         fail(B200SA_ERR_BAD_ARGUMENT, "the reverse index must be an O-table index of the reversed text on the same device", err);
@@ -1792,12 +1731,7 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
         fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", err);
         return nullptr;
     }
-    b200sa_approx_result *res = new (std::nothrow) b200sa_approx_result();
-    if (!res) {
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-        return nullptr;
-    }
-    try {
+    return new_handle<b200sa_approx_result>(err, [&](b200sa_approx_result *res) {
         DeviceGuard guard(ix.device);
         cudaStream_t st = ix.stream;
         res->hit_off.assign(npat + 1, 0);
@@ -1859,18 +1793,8 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
                         ms(t_c, t_d));
             }
         }
-        ok(err);
-        return res;
-    } catch (const CudaFailure &e) {
-        cudaGetLastError();
-        fail(code_of(e.code), e.what(), err);
-    } catch (const std::bad_alloc &) {
-        fail(B200SA_ERR_OUT_OF_MEMORY, "host allocation failed", err);
-    } catch (const std::exception &e) {
-        fail(B200SA_ERR_INTERNAL, e.what(), err);
-    }
-    delete res;
-    return nullptr;
+        return 0;
+    });
 }
 
 uint64_t b200sa_approx_hits(const b200sa_approx_result *r) { return r ? r->L.size() : 0; }
@@ -1884,21 +1808,21 @@ void b200sa_approx_free(b200sa_approx_result *r) { delete r; }
 
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device, void *stream) {
     if (!d_text || nsym < 1 || nsym > 255) return fail(B200SA_ERR_BAD_ARGUMENT, "bad argument", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(device);
-    synth_codes(d_text, n, nsym, seed, (cudaStream_t)stream);
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(device);
+        synth_codes(d_text, n, nsym, seed, (cudaStream_t)stream);
+        return 0;
+    });
 }
 
 int b200sa_synth_reads(const uint8_t *d_text, uint64_t n, uint32_t nsym, uint8_t *d_reads, uint64_t nreads,
                        uint32_t m, uint32_t miss_per_1024, uint64_t seed, int device, void *stream) {
     if (!d_text || !d_reads || nsym < 1 || nsym > 255) return fail(B200SA_ERR_BAD_ARGUMENT, "bad argument", nullptr);
-    API_GUARD_BEGIN
-    DeviceGuard guard(device);
-    synth_reads(d_text, n, nsym, d_reads, nreads, m, miss_per_1024, seed, (cudaStream_t)stream);
-    return 0;
-    API_GUARD_END(nullptr)
+    return guarded(nullptr, [&] {
+        DeviceGuard guard(device);
+        synth_reads(d_text, n, nsym, d_reads, nreads, m, miss_per_1024, seed, (cudaStream_t)stream);
+        return 0;
+    });
 }
 
 }  // extern "C"

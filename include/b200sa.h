@@ -322,6 +322,40 @@ const uint64_t *b200sa_approx_cigar_offsets(const b200sa_approx_result *r); /* h
 const char *b200sa_approx_cigars(const b200sa_approx_result *r);  /* NUL-terminated, back to back */
 void b200sa_approx_free(b200sa_approx_result *r);
 
+/* ---- matching statistics and super-maximal exact matches (SMEMs) ----------------------------
+ * Seeds for reads that do not occur whole (sequencing errors, SNPs, long reads), as BWA-MEM seeds.
+ * Patterns take the form of b200sa_search_batch (patterns / offsets / fixed_len, host buffers).
+ * For a pattern P[0..m) in remapped codes and every end j (0 <= j < m):
+ *   s_j   = the smallest s such that P[s..j] occurs in the text; j + 1 when no suffix of P[0..j] does;
+ *   ms[j] = j + 1 - s_j, the length of the longest substring of P that ends at j and occurs in the text;
+ *   [L[j], R[j]) = the SA interval of P[s_j..j], what b200sa_search_batch returns for that substring;
+ *                  (1, 0), the search's no-match pair, when ms[j] = 0.
+ * An SMEM is (start = s_j, length = ms[j], L[j], R[j]) for every j with ms[j] >= min_len and
+ * (j = m - 1 or ms[j+1] <= ms[j]), i.e. s_{j+1} > s_j: since s never decreases, exactly the occurring
+ * pieces of P that no other occurring piece contains.  Per pattern, SMEMs come in ascending start.
+ * A code 0 or >= sigma in a pattern occurs nowhere: it gets ms = 0 and breaks every match across it
+ * (not an error, as the search answers (1, 0) for it).  On a records index a pattern holding code 1,
+ * the separator, is refused with B200SA_ERR_BAD_SYMBOL, so an SMEM never crosses a record; its
+ * positions come from b200sa_locate_records over (L, R).  An empty pattern has no entries and no
+ * SMEMs.  min_len = 0 -> B200SA_ERR_BAD_ARGUMENT; an index without OCC -> B200SA_ERR_NOT_BUILT.
+ * TEXTCMP and KTABLE make the computation faster; results are identical with and without them.
+ * b200sa_matching_stats: ms, L and R are laid out like `patterns` (entry offsets[p] + j); L and R may
+ * be NULL.  b200sa_smem_batch: accessors return host arrays owned by the result (valid until
+ * b200sa_smem_free).  Both stage long batches in pieces of about 64 MB of pattern symbols. */
+int b200sa_matching_stats(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets,
+                          uint32_t fixed_len, uint64_t npat, uint32_t *ms, uint32_t *L, uint32_t *R);
+typedef struct b200sa_smem_result b200sa_smem_result;
+b200sa_smem_result *b200sa_smem_batch(const b200sa_index *idx, const uint8_t *patterns,
+                                      const uint64_t *offsets, uint32_t fixed_len, uint64_t npat,
+                                      uint32_t min_len, enum b200sa_error *err);
+uint64_t b200sa_smem_count(const b200sa_smem_result *r);             /* SMEMs in total        */
+const uint64_t *b200sa_smem_offsets(const b200sa_smem_result *r);    /* npat + 1 (CSR)        */
+const uint32_t *b200sa_smem_start(const b200sa_smem_result *r);
+const uint32_t *b200sa_smem_length(const b200sa_smem_result *r);
+const uint32_t *b200sa_smem_L(const b200sa_smem_result *r);
+const uint32_t *b200sa_smem_R(const b200sa_smem_result *r);
+void b200sa_smem_free(b200sa_smem_result *r);
+
 /* ---- synthetic inputs on the device (bench / tests; mirrors performance/suffix_array_search.c:13-32)
  * d_text must hold n + 1 bytes; symbols are 1 + hash(seed + i) % nsym, d_text[n] = 0. */
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device,

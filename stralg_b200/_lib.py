@@ -115,6 +115,17 @@ SIGNATURES = {
     "b200sa_approx_cigar_offsets": (u64p, [C.c_void_p]),
     "b200sa_approx_cigars": (C.POINTER(C.c_char), [C.c_void_p]),
     "b200sa_approx_free": (None, [C.c_void_p]),
+    "b200sa_matching_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p,
+                                        C.c_void_p, C.c_void_p]),
+    "b200sa_smem_batch": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint32,
+                                       C.POINTER(C.c_int)]),
+    "b200sa_smem_count": (C.c_uint64, [C.c_void_p]),
+    "b200sa_smem_offsets": (u64p, [C.c_void_p]),
+    "b200sa_smem_start": (u32p, [C.c_void_p]),
+    "b200sa_smem_length": (u32p, [C.c_void_p]),
+    "b200sa_smem_L": (u32p, [C.c_void_p]),
+    "b200sa_smem_R": (u32p, [C.c_void_p]),
+    "b200sa_smem_free": (None, [C.c_void_p]),
     "b200sa_synth_codes": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, C.c_int, C.c_void_p]),
     "b200sa_synth_reads": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64, C.c_uint32,
                                      C.c_uint32, C.c_uint64, C.c_int, C.c_void_p]),

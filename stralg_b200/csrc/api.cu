@@ -1806,6 +1806,139 @@ const uint64_t *b200sa_approx_cigar_offsets(const b200sa_approx_result *r) { ret
 const char *b200sa_approx_cigars(const b200sa_approx_result *r) { return r ? r->cigars.data() : nullptr; }
 void b200sa_approx_free(b200sa_approx_result *r) { delete r; }
 
+}  // extern "C"
+#pragma GCC visibility pop
+
+// ---- matching statistics and SMEMs ---------------------------------------------------------------
+// the refusals of b200sa_matching_stats and b200sa_smem_batch that come before any CUDA call
+static int mems_args_ok(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
+                        uint64_t npat, enum b200sa_error *err) {
+    if (int rc = needs_o_table(idx->ix, err)) return rc;
+    if (offsets)
+        for (uint64_t q = 0; q < npat; ++q) {
+            if (offsets[q + 1] < offsets[q]) return fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
+            if (offsets[q + 1] - offsets[q] > 0xFFFFFFFFull)
+                return fail(B200SA_ERR_TOO_LARGE, "a pattern longer than 2^32 - 1 symbols", err);
+        }
+    if (holds_separator(idx, patterns, offsets, fixed_len, npat))
+        return fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", err);
+    return 0;
+}
+
+// The first pass over a host batch, in pieces of about 64 MB of pattern bytes (whole patterns; a longer pattern is a
+// piece of its own), so that device memory stays bounded whatever the batch: a piece's patterns are copied in
+// (8-byte aligned and padded, as the kernels read whole words), its offsets rebased to the piece, and mems_stats
+// stores ms / L / R per symbol and, with `count`, the SMEMs of each pattern.  Then `piece(q0, q1, b0, d_off, d_ms,
+// d_L, d_R, d_count)` takes over the results of patterns [q0, q1), whose symbols start at b0 in the batch, on the
+// index's stream; it returns when it no longer needs them.
+template <class Piece>
+static void mems_pieces(const DeviceIndex &ix, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
+                        uint64_t npat, uint32_t min_len, bool count, Piece &&piece) {
+    const uint64_t kPieceBytes = (uint64_t)64 << 20;
+    const cudaStream_t st = ix.stream;
+    auto at = [&](uint64_t q) { return offsets ? offsets[q] : q * (uint64_t)fixed_len; };
+    std::vector<uint64_t> hoff;
+    for (uint64_t q0 = 0, q1; q0 < npat; q0 = q1) {
+        q1 = q0 + 1;
+        if (offsets)
+            while (q1 < npat && offsets[q1 + 1] - offsets[q0] <= kPieceBytes) ++q1;
+        else
+            q1 = std::min(npat, q0 + std::max<uint64_t>(1, kPieceBytes / std::max<uint32_t>(1, fixed_len)));
+        const uint64_t b0 = at(q0), bytes = at(q1) - b0;
+        DevBuf<u8> dp(bytes + 16, st);
+        DevBuf<u32> dms(bytes, st), dL(bytes, st), dR(bytes, st);
+        DevBuf<u64> doff, dcnt;
+        if (bytes) CUDA_CHECK(cudaMemcpyAsync(dp.ptr, patterns + b0, bytes, cudaMemcpyHostToDevice, st));
+        CUDA_CHECK(cudaMemsetAsync(dp.ptr + bytes, 0, 16, st));
+        if (offsets) {
+            hoff.resize(q1 - q0 + 1);
+            for (uint64_t q = q0; q <= q1; ++q) hoff[q - q0] = offsets[q] - b0;
+            doff.alloc(hoff.size(), st);
+            CUDA_CHECK(cudaMemcpyAsync(doff.ptr, hoff.data(), hoff.size() * 8, cudaMemcpyHostToDevice, st));
+        }
+        if (count) dcnt.alloc(q1 - q0 + 1, st);  // (+1: the scan's total)
+        mems_stats(ix, dp.ptr, doff.ptr, fixed_len, q1 - q0, min_len, dms.ptr, dL.ptr, dR.ptr, dcnt.ptr, st);
+        piece(q0, q1, b0, doff.ptr, dms.ptr, dL.ptr, dR.ptr, dcnt.ptr);
+        CUDA_CHECK(cudaStreamSynchronize(st));  // (`hoff` and the piece's buffers are reused or freed next)
+    }
+}
+
+struct b200sa_smem_result {
+    std::vector<uint64_t> off;  // npat + 1
+    std::vector<uint32_t> start, length, L, R;
+};
+
+#pragma GCC visibility push(default)
+extern "C" {
+
+int b200sa_matching_stats(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
+                          uint64_t npat, uint32_t *ms, uint32_t *L, uint32_t *R) {
+    if (!idx || (npat && (!patterns || !ms))) return fail(B200SA_ERR_BAD_ARGUMENT, "null argument", nullptr);
+    if (int rc = mems_args_ok(idx, patterns, offsets, fixed_len, npat, nullptr)) return rc;
+    if (!npat) return 0;
+    return guarded(nullptr, [&] {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        const cudaStream_t st = ix.stream;
+        mems_pieces(ix, patterns, offsets, fixed_len, npat, 1, false,
+                    [&](uint64_t q0, uint64_t q1, uint64_t b0, const u64 *, const u32 *dms, const u32 *dL, const u32 *dR,
+                        u64 *) {
+                        const size_t bytes = (size_t)((offsets ? offsets[q1] : q1 * (uint64_t)fixed_len) - b0) * 4;
+                        if (!bytes) return;
+                        CUDA_CHECK(cudaMemcpyAsync(ms + b0, dms, bytes, cudaMemcpyDeviceToHost, st));
+                        if (L) CUDA_CHECK(cudaMemcpyAsync(L + b0, dL, bytes, cudaMemcpyDeviceToHost, st));
+                        if (R) CUDA_CHECK(cudaMemcpyAsync(R + b0, dR, bytes, cudaMemcpyDeviceToHost, st));
+                    });
+        return 0;
+    });
+}
+
+b200sa_smem_result *b200sa_smem_batch(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets,
+                                      uint32_t fixed_len, uint64_t npat, uint32_t min_len, enum b200sa_error *err) {
+    if (!idx || (npat && !patterns) || min_len == 0) {
+        fail(B200SA_ERR_BAD_ARGUMENT, "null argument or min_len 0", err);
+        return nullptr;
+    }
+    if (mems_args_ok(idx, patterns, offsets, fixed_len, npat, err)) return nullptr;
+    return new_handle<b200sa_smem_result>(err, [&](b200sa_smem_result *res) {
+        const DeviceIndex &ix = idx->ix;
+        DeviceGuard guard(ix.device);
+        const cudaStream_t st = ix.stream;
+        res->off.assign(npat + 1, 0);
+        mems_pieces(ix, patterns, offsets, fixed_len, npat, min_len, true,
+                    [&](uint64_t q0, uint64_t q1, uint64_t, const u64 *doff, const u32 *dms, const u32 *dL, const u32 *dR,
+                        u64 *dcnt) {
+                        const uint64_t np = q1 - q0, base = res->start.size();
+                        scan_u64(dcnt, np, st);
+                        CUDA_CHECK(cudaMemcpyAsync(res->off.data() + q0, dcnt, (np + 1) * 8, cudaMemcpyDeviceToHost, st));
+                        CUDA_CHECK(cudaStreamSynchronize(st));
+                        for (uint64_t q = q0; q <= q1; ++q) res->off[q] += base;
+                        const uint64_t total = res->off[q1] - base;
+                        if (!total) return;
+                        res->start.resize(base + total);
+                        res->length.resize(base + total);
+                        res->L.resize(base + total);
+                        res->R.resize(base + total);
+                        DevBuf<u32> ds(total, st), dn(total, st), dsL(total, st), dsR(total, st);
+                        mems_emit(ix, doff, fixed_len, np, min_len, dms, dL, dR, dcnt, ds.ptr, dn.ptr, dsL.ptr, dsR.ptr, st);
+                        CUDA_CHECK(cudaMemcpyAsync(res->start.data() + base, ds.ptr, total * 4, cudaMemcpyDeviceToHost, st));
+                        CUDA_CHECK(cudaMemcpyAsync(res->length.data() + base, dn.ptr, total * 4, cudaMemcpyDeviceToHost, st));
+                        CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dsL.ptr, total * 4, cudaMemcpyDeviceToHost, st));
+                        CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dsR.ptr, total * 4, cudaMemcpyDeviceToHost, st));
+                        CUDA_CHECK(cudaStreamSynchronize(st));  // (the output buffers are freed on return)
+                    });
+        return 0;
+    });
+}
+
+uint64_t b200sa_smem_count(const b200sa_smem_result *r) { return r ? r->start.size() : 0; }
+const uint64_t *b200sa_smem_offsets(const b200sa_smem_result *r) { return r ? r->off.data() : nullptr; }
+const uint32_t *b200sa_smem_start(const b200sa_smem_result *r) { return r ? r->start.data() : nullptr; }
+const uint32_t *b200sa_smem_length(const b200sa_smem_result *r) { return r ? r->length.data() : nullptr; }
+const uint32_t *b200sa_smem_L(const b200sa_smem_result *r) { return r ? r->L.data() : nullptr; }
+const uint32_t *b200sa_smem_R(const b200sa_smem_result *r) { return r ? r->R.data() : nullptr; }
+void b200sa_smem_free(b200sa_smem_result *r) { delete r; }
+
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device, void *stream) {
     if (!d_text || nsym < 1 || nsym > 255) return fail(B200SA_ERR_BAD_ARGUMENT, "bad argument", nullptr);
     return guarded(nullptr, [&] {

@@ -104,6 +104,7 @@ u64 fm_locate_count(const DeviceIndex &ix, const u32 *d_L, const u32 *d_R, u64 n
                     cudaStream_t st);
 void fm_locate_fill(const DeviceIndex &ix, const u32 *d_L, const u32 *d_R, u64 npat, const u64 *d_pos_off,
                     u64 total, u32 *d_pos, cudaStream_t st);
+void scan_u64(u64 *d_vals, u64 count, cudaStream_t st);  // exclusive scan in place; d_vals[count] = the total
 // locate.cu
 void build_sampled_sa(DeviceIndex &ix, u32 rate);  // fills ix.ssa_* from ix.sa
 void fm_locate_fill_ssa(const DeviceIndex &ix, const u32 *d_L, u64 npat, const u64 *d_pos_off, u64 total,
@@ -120,6 +121,13 @@ void approx_count(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 
 void approx_emit(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fixed_len, u64 npat, u32 max_m,
                  const u8 *d_dtab, int max_edits, const u64 *d_hit_off, const u64 *d_ops_off, u32 *d_L, u32 *d_R,
                  u32 *d_mlen, u64 *d_hit_ops_off, char *d_ops, cudaStream_t st);
+// mems.cu: matching statistics (ms / L / R per pattern symbol, laid out like d_pat) and, with d_count, the SMEMs of
+// each pattern counted; mems_emit writes them at d_smem_off (exclusive scan of the counts)
+void mems_stats(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fixed_len, u64 npat, u32 min_len,
+                u32 *d_ms, u32 *d_L, u32 *d_R, u64 *d_count, cudaStream_t st);
+void mems_emit(const DeviceIndex &ix, const u64 *d_off, u32 fixed_len, u64 npat, u32 min_len, const u32 *d_ms,
+               const u32 *d_L, const u32 *d_R, const u64 *d_smem_off, u32 *d_start, u32 *d_len, u32 *d_sL, u32 *d_sR,
+               cudaStream_t st);
 // records.cu
 void records_assemble(const u8 *d_codes, u64 ncodes, const u64 *d_rec_off, u32 nrec, u32 sigma, u8 *d_text,
                       int *d_err, cudaStream_t st);  // d_text: ncodes + nrec + 1 bytes

@@ -9,28 +9,12 @@
 // A pattern symbol outside 1..sigma-1 (the reference asserts, bwt.c:189-190) yields the empty
 // interval (1, 0).  An empty pattern yields (0, len) (the reference underflows, bwt.c:185).
 #include "engine.h"
-#include "occ.cuh"
+#include "fm_step.cuh"
 
 #include <algorithm>
 #include <cstdlib>
 
 namespace b200sa {
-
-struct CTable5 {
-    u32 c[8];
-};
-
-struct TextCmp {
-    const u32 *sa;
-    const u32 *isa;
-    const u64 *packed;  // 2-bit symbols, big-endian inside each word (sa_build.cu pack_kernel<2>)
-};
-
-struct KTable {
-    const uint2 *tab;
-    int k;
-    u32 nsym;  // 0: 2-bit symbols (entry index = the k symbols as a 2k-bit number); else the index is their base-nsym number
-};
 
 // Any alphabet (byte-wide O blocks).  SC: once a single candidate row is left, the remaining symbols are compared
 // with the packed text at SA[L] instead of one O lookup each (the recurrence would walk ISA[s-1], ISA[s-2], ... as
@@ -76,14 +60,8 @@ __global__ void __launch_bounds__(256) fm_search_kernel(OccView ov, CTable5 c5, 
     if (LAYOUT == 2 && kt.tab && m >= (u64)kt.k && L < R) {
         // the last k symbols select the interval the first k steps would reach (an entry with L >= R is the pair at
         // the step that emptied the interval); a byte outside 1..nsym takes the stepwise path
-        u32 x = 0;
-        bool valid = true;
-        for (int j = 0; j < kt.k; ++j) {
-            const u32 a = P(i - j);
-            valid = valid && (a - 1u < kt.nsym);
-            x = x * kt.nsym + (a - 1u);
-        }
-        if (valid) {
+        u32 x;
+        if (seed_key(P, i, kt, x)) {
             const uint2 lr = kt.tab[x];
             L = lr.x;
             R = lr.y;
@@ -113,22 +91,8 @@ __global__ void __launch_bounds__(256) fm_search_kernel(OccView ov, CTable5 c5, 
     if (SC && LAYOUT == 2 && i >= 0 && R - L == 1) {
         const u32 s = tc.sa[L];
         const u64 rem = (u64)i + 1;
-        const u32 mask = (1u << bits) - 1u;
-        const u32 lg = bits == 8 ? 3u : bits == 4 ? 4u : bits == 2 ? 5u : 6u;  // log2 of the symbols per word
-        u64 k = 0, tw = 0, tw_idx = ~0ull;
-        u32 a = 0;
-        while (k < rem) {
-            a = P(i - (int64_t)k);
-            if (k >= (u64)s) break;  // suffix 0 is preceded by the sentinel only
-            const u64 t = (u64)s - 1 - k;
-            if ((t >> lg) != tw_idx) {
-                tw_idx = t >> lg;
-                tw = tc.packed[tw_idx];
-            }
-            const u32 sym = (u32)(tw >> (64u - (u32)bits - (u32)(t & ((1u << lg) - 1u)) * (u32)bits)) & mask;
-            if (a - 1u != sym) break;
-            ++k;
-        }
+        u32 a;
+        const u64 k = text_agree(P, i, s, tc.packed, bits, a);
         if (k == rem) {
             L = tc.isa[s - (u32)rem];
             R = L + 1;
@@ -147,46 +111,11 @@ __global__ void __launch_bounds__(256) fm_search_kernel(OccView ov, CTable5 c5, 
 }
 
 // ---------------------------------------------------------------------------------------------
-// DNA32 fast path.  Per backward step a lane issues ONE 256-bit load per distinct block (the L and
-// R rows share a block once the interval is narrower than 64 rows, i.e. after ~log4(len) steps on
-// random DNA), and pattern symbols come from an aligned 8-byte word fetched once per 8 steps.
+// DNA32 fast path.  Per backward step a lane issues ONE 256-bit load per distinct block (dna_step),
+// and pattern symbols come from an aligned 8-byte word fetched once per 8 steps.
 // Requires the pattern buffer to be 8-byte aligned and readable up to the next 8-byte boundary
 // (true for cudaMalloc / torch allocations; the host entry point pads its staging buffer).
 // ---------------------------------------------------------------------------------------------
-struct BlockRegs {
-    u32 c0, c1, c2, c3;
-    u64 w0, w1;
-};
-
-__device__ __forceinline__ BlockRegs load_dna_block(const u8 *blocks, u32 b) {
-    u64 a, bb, c, d;
-    const u8 *p = blocks + (size_t)b * 32;
-    asm volatile("ld.global.nc.L1::no_allocate.L2::64B.v4.u64 {%0,%1,%2,%3}, [%4];"
-                 : "=l"(a), "=l"(bb), "=l"(c), "=l"(d) : "l"(p));
-    BlockRegs r;
-    r.c0 = (u32)a; r.c1 = (u32)(a >> 32); r.c2 = (u32)bb; r.c3 = (u32)(bb >> 32);
-    r.w0 = c; r.w1 = d;
-    return r;
-}
-
-__device__ __forceinline__ u32 rank_in_block(const BlockRegs &blk, u32 a, u32 i, u32 primary) {
-    u32 base = a == 1 ? blk.c0 : a == 2 ? blk.c1 : a == 3 ? blk.c2 : blk.c3;
-    u32 c = base + dna_match_count(blk.w0, blk.w1, a - 1, i & 63u);
-    if (a == 1) {
-        u32 start = i & ~63u;
-        if (primary >= start && primary < i) c -= 1;  // the sentinel row is stored as value 0
-    }
-    return c;
-}
-
-// Pointers for the unique-interval shortcut (B200SA_BUILD_TEXTCMP); all null when it is off.
-
-// STATS: count the memory operations of the batch (b200sa_search_traffic, a measurement aid):
-// stats[0] 32-byte O-block loads, [1] 8-byte pattern words, [2] 8-byte text words, [3] 4-byte SA/ISA loads.
-// k-mer seed table (B200SA_BUILD_KTABLE): tab[x] = the (L, R) the recurrence reaches on the k-mer
-// whose symbols, in the order the recurrence consumes them (last pattern symbol first), are the
-// base-4 digits of x, most significant first; an entry with L >= R is the interval at the step
-// that emptied it, i.e. the final answer of every pattern ending in that k-mer.
 
 __global__ void __launch_bounds__(256) ktable_build_kernel(OccView ov, CTable5 c5, u32 len, int k, u64 entries,
                                                            uint2 *__restrict__ tab) {
@@ -208,6 +137,8 @@ __global__ void __launch_bounds__(256) ktable_build_kernel(OccView ov, CTable5 c
     tab[x] = make_uint2(L, R);
 }
 
+// STATS: count the memory operations of the batch (b200sa_search_traffic, a measurement aid):
+// stats[0] 32-byte O-block loads, [1] 8-byte pattern words, [2] 8-byte text words, [3] 4-byte SA/ISA loads.
 // one pattern: pat[begin .. begin + m), readable in aligned 8-byte words; (L, R) = the interval of bwt.c:171-198
 template <bool SC, bool STATS>
 __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTable5 &c5, const TextCmp &tc, const KTable &kt,
@@ -223,20 +154,9 @@ __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTabl
     int64_t i = (int64_t)m - 1;
     if (kt.tab && m >= (u64)kt.k && L < R) {
         // the last k symbols select the interval the first k steps would reach
-        u32 x = 0;
-        bool valid = true;
-        for (int j = 0; j < kt.k; ++j) {
-            u64 addr = begin + (u64)i - (u64)j;
-            if ((addr & ~7ull) != word_addr) {
-                word_addr = addr & ~7ull;
-                word = *(const u64 *)(pat + word_addr);
-                if (STATS) ++n_pw;
-            }
-            const u32 a = (u32)(word >> (8 * (addr & 7))) & 0xffu;
-            valid = valid && (a - 1u <= 3u);
-            x = (x << 2) | ((a - 1u) & 3u);
-        }
-        if (valid) {  // a byte outside 1..4 takes the stepwise path (it answers (1, 0) where it is reached)
+        u32 x;
+        if (dna_seed_key<STATS>(pat, begin, i, kt.k, word, word_addr, n_pw, x)) {
+            // (a byte outside 1..4 takes the stepwise path: it answers (1, 0) where it is reached)
             const uint2 lr = kt.tab[x];
             if (STATS) n_sa += 2;  // one 8-byte table entry
             L = lr.x;
@@ -248,118 +168,22 @@ __device__ __forceinline__ void fm_search_dna_one(const OccView &ov, const CTabl
     // the lanes of a warp reach that point after different numbers of steps, and run the comparison
     // below together, once
     for (; i >= 0 && L < R && !(SC && R - L == 1); --i) {
-        u64 addr = begin + (u64)i;
-        if ((addr & ~7ull) != word_addr) {
-            word_addr = addr & ~7ull;
-            word = *(const u64 *)(pat + word_addr);
-            if (STATS) ++n_pw;
-        }
-        u32 a = (u32)(word >> (8 * (addr & 7))) & 0xffu;
+        const u32 a = pattern_byte<STATS>(pat, begin + (u64)i, word, word_addr, n_pw);
         if (a - 1u > 3u || a >= ov.sigma) {
             L = 1;
             R = 0;
             break;
         }
-        const u32 bL = L >> 6, bR = R >> 6;
-        BlockRegs kL = load_dna_block(ov.blocks, bL);
-        BlockRegs kR = kL;
-        if (bR != bL) kR = load_dna_block(ov.blocks, bR);
-        if (STATS) n_blk += bR != bL ? 2u : 1u;
-        const u32 ca = c5.c[a];
-        L = ca + rank_in_block(kL, a, L, ov.primary);
-        R = ca + rank_in_block(kR, a, R, ov.primary);
+        const uint2 lr = dna_step<STATS>(ov, c5, a, L, R, n_blk);
+        L = lr.x;
+        R = lr.y;
     }
     if (SC && i >= 0 && R - L == 1) {
-        // One candidate suffix s = SA[L] is left.  The recurrence would now consume the remaining
-        // symbols pattern[i], pattern[i-1], ... one O lookup each, moving to ISA[s-1], ISA[s-2], ...
-        // as long as they equal text[s-1], text[s-2], ...; compare them against the text instead.
         const u32 s = tc.sa[L];
         if (STATS) ++n_sa;
         const u64 rem = (u64)i + 1;
-        u64 k = 0;
-        u64 tw = 0, tw_idx = ~0ull;
-        u32 a = 0;
-        // Eight symbols per step while at least eight are left on both sides: the pattern bytes
-        // pattern[i-k-7 .. i-k] (an unaligned 8-byte window, byte-swapped so that pattern[i-k]
-        // comes first) are packed to 16 bits and compared with the 16 bits of packed text that
-        // hold text[s-1-k-7 .. s-1-k]; the first difference, in the order the recurrence would
-        // meet the symbols, ends the run.  The scalar loop below takes over from there (it finds
-        // the failing symbol at once, or finishes a tail shorter than eight).
-        {
-            const u64 ones = 0x0101010101010101ull;
-            u64 plo = 0, phi = 0, pbase = ~0ull;  // aligned pattern words at pbase and pbase + 8
-            while (rem - k >= 8 && (u64)s - k >= 8) {
-                const u64 first = begin + (u64)i - k - 7;  // address of pattern[i-k-7]
-                const u64 base8 = first & ~7ull;
-                const u32 sh = (u32)(first & 7u) * 8u;
-                if (base8 != pbase) {
-                    phi = (pbase != ~0ull && base8 + 8 == pbase) ? plo : (sh ? *(const u64 *)(pat + base8 + 8) : 0ull);
-                    plo = *(const u64 *)(pat + base8);
-                    if (STATS) n_pw += (pbase != ~0ull && base8 + 8 == pbase) ? 1u : (sh ? 2u : 1u);
-                    pbase = base8;
-                }
-                const u64 P = sh ? (plo >> sh) | (phi << (64u - sh)) : plo;  // byte j = pattern[i-k-7+j]
-                const u64 v = P - ones;
-                if (v & 0xFCFCFCFCFCFCFCFCull) break;  // a byte outside 1..4: the scalar loop decides
-                // byte-swap (pattern[i-k] to the low end), then squeeze the 2-bit symbols together
-                u64 y = ((u64)__byte_perm((u32)v, 0, 0x0123) << 32) | (u64)__byte_perm((u32)(v >> 32), 0, 0x0123);
-                y &= 0x0303030303030303ull;
-                y = (y | (y >> 6)) & 0x000F000F000F000Full;
-                y = (y | (y >> 12)) & 0x000000FF000000FFull;
-                y = (y | (y >> 24)) & 0xFFFFull;  // bits 2j..2j+1 = pattern[i-k-j] - 1
-                // text[s-1-k-j] for j = 0..7 in the same order: position t = s-1-k sits lowest
-                const u64 t = (u64)s - 1 - k;
-                const u64 w = t >> 5;
-                const u32 tsh = 62u - 2u * (u32)(t & 31u);
-                if (w != tw_idx) {
-                    tw_idx = w;
-                    tw = tc.packed[w];
-                    if (STATS) ++n_tw;
-                }
-                u64 T = tw >> tsh;
-                if ((t & 31u) < 7u) {  // the field runs into the previous word
-                    const u64 prev = tc.packed[w - 1];
-                    if (STATS) ++n_tw;
-                    T |= prev << (64u - tsh);
-                    // going on downwards, the previous word is the next current one
-                    tw_idx = w - 1;
-                    tw = prev;
-                }
-                const u32 d = (u32)((T ^ y) & 0xFFFFull);
-                if (d) {
-                    k += (u64)((__ffs((int)d) - 1) >> 1);
-                    break;
-                }
-                k += 8;
-            }
-            // hand the pattern word the scalar loop will ask for first over to its one-word cache
-            if (pbase != ~0ull && k < rem) {
-                const u64 need = (begin + (u64)i - k) & ~7ull;
-                if (need == pbase) {
-                    word_addr = need;
-                    word = plo;
-                }
-            }
-        }
-        while (k < rem) {
-            u64 addr = begin + (u64)i - k;
-            if ((addr & ~7ull) != word_addr) {
-                word_addr = addr & ~7ull;
-                word = *(const u64 *)(pat + word_addr);
-                if (STATS) ++n_pw;
-            }
-            a = (u32)(word >> (8 * (addr & 7))) & 0xffu;
-            if (k >= (u64)s) break;  // suffix 0 is preceded by the sentinel only
-            u64 t = (u64)s - 1 - k;
-            if ((t >> 5) != tw_idx) {
-                tw_idx = t >> 5;
-                tw = tc.packed[tw_idx];
-                if (STATS) ++n_tw;
-            }
-            u32 sym = (u32)(tw >> (62 - 2 * (t & 31))) & 3u;
-            if (a - 1u != sym) break;
-            ++k;
-        }
+        u32 a;
+        const u64 k = dna_text_agree<STATS>(pat, begin, i, s, tc.packed, word, word_addr, a, n_pw, n_tw);
         if (k == rem) {
             L = tc.isa[s - (u32)rem];
             R = L + 1;
@@ -855,6 +679,11 @@ __global__ void __launch_bounds__(1024) scan_u64_kernel(u64 *__restrict__ vals, 
         __syncthreads();
     }
     if (threadIdx.x == 0) *total = carry;
+}
+
+void scan_u64(u64 *d_vals, u64 count, cudaStream_t st) {
+    scan_u64_kernel<<<1, 1024, 0, st>>>(d_vals, count, d_vals + count);
+    KERNEL_CHECK();
 }
 
 __global__ void __launch_bounds__(LC_NT) locate_add_kernel(u64 *__restrict__ pos_off, u64 npat,

@@ -359,6 +359,49 @@ class SuffixArrayIndex:
             lib.b200sa_approx_free(r)
         return {"offsets": hoff, "L": L, "R": R, "match_length": ml, "cigars": cig}
 
+    # ---- matching statistics and super-maximal exact matches (include/b200sa.h) ----------------------
+    @staticmethod
+    def _batch(patterns, offsets, fixed_len):
+        pat = np.ascontiguousarray(patterns, dtype=np.uint8)
+        if offsets is not None:
+            off = np.ascontiguousarray(offsets, dtype=np.uint64)
+            return pat, off, len(off) - 1, _np_ptr(off)
+        assert fixed_len > 0
+        return pat, None, pat.size // fixed_len, None
+
+    def matching_stats(self, patterns, offsets=None, fixed_len: int = 0) -> dict:
+        """Per pattern symbol, laid out like ``patterns``: ms (the length of the longest substring of the pattern that
+        ends there and occurs in the text) and the SA interval [L, R) of that substring ((1, 0) where ms = 0).
+        Returns dict(ms, L, R)."""
+        pat, _, npat, offp = self._batch(patterns, offsets, fixed_len)
+        ms = np.zeros(pat.size, dtype=np.uint32)
+        L = np.zeros(pat.size, dtype=np.uint32)
+        R = np.zeros(pat.size, dtype=np.uint32)
+        check(_lib.load().b200sa_matching_stats(self._h, _np_ptr(pat), offp, fixed_len, npat, _np_ptr(ms), _np_ptr(L),
+                                                _np_ptr(R)))
+        return {"ms": ms, "L": L, "R": R}
+
+    def smems(self, patterns, offsets=None, fixed_len: int = 0, min_len: int = 1) -> dict:
+        """Super-maximal exact matches of at least ``min_len`` symbols, per pattern in ascending start.
+        Returns dict(offsets[npat+1], start, length, L, R)."""
+        lib = _lib.load()
+        pat, _, npat, offp = self._batch(patterns, offsets, fixed_len)
+        err = C.c_int(0)
+        r = lib.b200sa_smem_batch(self._h, _np_ptr(pat), offp, fixed_len, npat, min_len, C.byref(err))
+        if not r:
+            raise B200saError(err.value, lib.b200sa_last_error().decode())
+        r = C.c_void_p(r)
+        try:
+            n = int(lib.b200sa_smem_count(r))
+            soff = np.ctypeslib.as_array(lib.b200sa_smem_offsets(r), shape=(npat + 1,)).copy()
+            cols = {}
+            for k, fn in (("start", lib.b200sa_smem_start), ("length", lib.b200sa_smem_length),
+                          ("L", lib.b200sa_smem_L), ("R", lib.b200sa_smem_R)):
+                cols[k] = np.ctypeslib.as_array(fn(r), shape=(n,)).copy() if n else np.zeros(0, np.uint32)
+        finally:
+            lib.b200sa_smem_free(r)
+        return {"offsets": soff, **cols}
+
     # ---- sampled suffix array (SURVEY 8f rank 3) -----------------------------------------------
     def sample_sa(self, rate: int = 32, drop_sa: bool = False) -> None:
         """Keep SA only at text positions that are multiples of ``rate``; with ``drop_sa`` the full

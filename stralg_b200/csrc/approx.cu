@@ -26,6 +26,7 @@
 // second index), restarting the interval whenever it empties; D[i] = restarts so far.
 #include "engine.h"
 #include "occ.cuh"
+#include "scan.cuh"
 
 #include <algorithm>
 
@@ -320,15 +321,7 @@ __global__ void __launch_bounds__(1024) approx_scan_kernel(const u32 *__restrict
     for (u64 base = 0; base < npat; base += 1024) {
         const u64 k = base + threadIdx.x;
         const u64 v0 = k < npat ? (u64)hit_count[k] : 0, v1 = k < npat ? ops_count[k] : 0;
-        u64 i0 = v0, i1 = v1;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const u64 t0 = __shfl_up_sync(0xffffffffu, i0, o), t1 = __shfl_up_sync(0xffffffffu, i1, o);
-            if (lane_id() >= (unsigned)o) {
-                i0 += t0;
-                i1 += t1;
-            }
-        }
+        const u64 i0 = warp_inclusive(v0, SumOp()), i1 = warp_inclusive(v1, SumOp());
         if (lane_id() == 31) {
             wsum[threadIdx.x >> 5][0] = i0;
             wsum[threadIdx.x >> 5][1] = i1;

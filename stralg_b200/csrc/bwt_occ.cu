@@ -9,6 +9,7 @@
 // popcounts.  occ_dense() re-creates the reference layout for small inputs (compat shims, tests).
 #include "engine.h"
 #include "occ.cuh"
+#include "scan.cuh"
 
 namespace b200sa {
 
@@ -120,30 +121,10 @@ __global__ void __launch_bounds__(OD_NT) occ_dna_count_kernel(const u8 *__restri
 
 // grid = nsym blocks; block x scans tile_counts[tile * nsym + x] over tiles (exclusive, in place)
 __global__ void __launch_bounds__(1024) occ_scan_tiles_kernel(u32 *__restrict__ tile_counts, u32 ntiles, u32 nsym) {
-    __shared__ u32 wsum[32];
-    __shared__ u32 carry;
-    const u32 x = blockIdx.x;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (u32 base = 0; base < ntiles; base += 1024) {
-        u32 i = base + threadIdx.x;
-        u32 v = i < ntiles ? tile_counts[(size_t)i * nsym + x] : 0;
-        u32 incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane_id() >= (unsigned)o) incl += t;
-        }
-        if (lane_id() == 31) wsum[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        u32 wb = 0;
-        for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) wb += wsum[w];
-        u32 excl = carry + wb + incl - v;
-        if (i < ntiles) tile_counts[(size_t)i * nsym + x] = excl;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = excl + v;
-        __syncthreads();
-    }
+    u32 *col = tile_counts + blockIdx.x;
+    cta_exclusive_scan(
+        ntiles, [=](u32 i) { return col[(size_t)i * nsym]; }, [=](u32 i, u32 e) { col[(size_t)i * nsym] = e; }, SumOp(),
+        0u);
 }
 
 __global__ void __launch_bounds__(OD_NT) occ_dna_finalize_kernel(DnaBlock *__restrict__ blocks, u64 nblocks,
@@ -157,14 +138,7 @@ __global__ void __launch_bounds__(OD_NT) occ_dna_finalize_kernel(DnaBlock *__res
     }
     u32 incl[4];
 #pragma unroll
-    for (int x = 0; x < 4; ++x) {
-        incl[x] = v[x];
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl[x], o);
-            if (lane_id() >= (unsigned)o) incl[x] += t;
-        }
-    }
+    for (int x = 0; x < 4; ++x) incl[x] = warp_inclusive(v[x], SumOp());
     if (lane_id() == 31)
         for (int x = 0; x < 4; ++x) wsum[threadIdx.x >> 5][x] = incl[x];
     __syncthreads();

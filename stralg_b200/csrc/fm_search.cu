@@ -10,6 +10,7 @@
 // interval (1, 0).  An empty pattern yields (0, len) (the reference underflows, bwt.c:185).
 #include "engine.h"
 #include "fm_step.cuh"
+#include "scan.cuh"
 
 #include <algorithm>
 #include <cstdlib>
@@ -640,51 +641,13 @@ __global__ void __launch_bounds__(LC_NT) locate_count_kernel(const u32 *__restri
         u32 l = L[q], r = R[q];
         v = r > l ? (u64)(r - l) : 0;
     }
-    u64 incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u64 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane_id() >= (unsigned)o) incl += t;
-    }
-    if (lane_id() == 31) wsum[threadIdx.x >> 5] = incl;
-    __syncthreads();
-    u64 wb = 0;
-    for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) wb += wsum[w];
-    if (q < npat) pos_off[q] = wb + incl - v;
-    if (threadIdx.x == LC_NT - 1) tile_tot[blockIdx.x] = wb + incl;
+    u64 total;
+    const u64 excl = block_exclusive<LC_NT>(v, wsum, &total);
+    if (q < npat) pos_off[q] = excl;
+    if (threadIdx.x == 0) tile_tot[blockIdx.x] = total;
 }
 
-__global__ void __launch_bounds__(1024) scan_u64_kernel(u64 *__restrict__ vals, u64 count, u64 *__restrict__ total) {
-    __shared__ u64 wsum[32];
-    __shared__ u64 carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (u64 base = 0; base < count; base += 1024) {
-        u64 i = base + threadIdx.x;
-        u64 v = i < count ? vals[i] : 0;
-        u64 incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u64 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane_id() >= (unsigned)o) incl += t;
-        }
-        if (lane_id() == 31) wsum[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        u64 wb = 0;
-        for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) wb += wsum[w];
-        u64 excl = carry + wb + incl - v;
-        if (i < count) vals[i] = excl;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = excl + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *total = carry;
-}
-
-void scan_u64(u64 *d_vals, u64 count, cudaStream_t st) {
-    scan_u64_kernel<<<1, 1024, 0, st>>>(d_vals, count, d_vals + count);
-    KERNEL_CHECK();
-}
+void scan_u64(u64 *d_vals, u64 count, cudaStream_t st) { scan_sum(d_vals, count, st, d_vals + count); }
 
 __global__ void __launch_bounds__(LC_NT) locate_add_kernel(u64 *__restrict__ pos_off, u64 npat,
                                                            const u64 *__restrict__ tile_prefix,
@@ -704,8 +667,7 @@ u64 fm_locate_count(const DeviceIndex &ix, const u32 *d_L, const u32 *d_R, u64 n
     DevBuf<u64> tile_tot(tiles, st), total(1, st);
     locate_count_kernel<<<tiles, LC_NT, 0, st>>>(d_L, d_R, npat, d_pos_off, tile_tot.ptr);
     KERNEL_CHECK();
-    scan_u64_kernel<<<1, 1024, 0, st>>>(tile_tot.ptr, tiles, total.ptr);
-    KERNEL_CHECK();
+    scan_sum(tile_tot.ptr, (u64)tiles, st, total.ptr);
     locate_add_kernel<<<tiles, LC_NT, 0, st>>>(d_pos_off, npat, tile_tot.ptr, total.ptr);
     KERNEL_CHECK();
     u64 h = 0;

@@ -15,6 +15,7 @@
 //   lcp_gather            lcp[r] = v[sa[r]] - sa[r]
 #include "engine.h"
 #include "round0_msd.cuh"  // window_at
+#include "scan.cuh"
 
 namespace b200sa {
 
@@ -149,6 +150,9 @@ __global__ void __launch_bounds__(256) plcp_long_kernel(const u64 *__restrict__ 
 static constexpr int FL_NT = 256, FL_IPT = 8, FL_TILE = FL_NT * FL_IPT;
 
 __device__ __forceinline__ u32 pick(u32 left, u32 right) { return right != UNDEF ? right : left; }
+struct PickOp {
+    __device__ __forceinline__ u32 operator()(u32 left, u32 right) const { return pick(left, right); }
+};
 
 __global__ void __launch_bounds__(FL_NT) plcp_tile_last_kernel(const u32 *__restrict__ v, u64 count,
                                                                u32 *__restrict__ tile_last) {
@@ -158,11 +162,7 @@ __global__ void __launch_bounds__(FL_NT) plcp_tile_last_kernel(const u32 *__rest
 #pragma unroll
     for (int q = 0; q < FL_IPT; ++q)
         if (base + q < count) last = pick(last, v[base + q]);
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, last, o);
-        if (lane_id() >= (unsigned)o) last = pick(t, last);
-    }
+    last = warp_inclusive(last, PickOp());
     if (lane_id() == 31) wl[threadIdx.x >> 5] = last;
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -174,31 +174,8 @@ __global__ void __launch_bounds__(FL_NT) plcp_tile_last_kernel(const u32 *__rest
 
 // exclusive "last defined" scan over the tile aggregates, in place (single block)
 __global__ void __launch_bounds__(1024) plcp_scan_tiles_kernel(u32 *__restrict__ tile_last, u32 ntiles) {
-    __shared__ u32 wl[32];
-    __shared__ u32 carry;
-    if (threadIdx.x == 0) carry = UNDEF;
-    __syncthreads();
-    for (u32 base = 0; base < ntiles; base += 1024) {
-        u32 i = base + threadIdx.x;
-        u32 mine = i < ntiles ? tile_last[i] : UNDEF;
-        u32 incl = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane_id() >= (unsigned)o) incl = pick(t, incl);
-        }
-        if (lane_id() == 31) wl[threadIdx.x >> 5] = incl;
-        u32 excl = __shfl_up_sync(0xffffffffu, incl, 1);
-        if (lane_id() == 0) excl = UNDEF;
-        __syncthreads();
-        u32 pre = carry;
-        for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) pre = pick(pre, wl[w]);
-        excl = pick(pre, excl);
-        if (i < ntiles) tile_last[i] = excl;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = pick(excl, mine);
-        __syncthreads();
-    }
+    cta_exclusive_scan(
+        ntiles, [=](u32 i) { return tile_last[i]; }, [=](u32 i, u32 e) { tile_last[i] = e; }, PickOp(), UNDEF);
 }
 
 __global__ void __launch_bounds__(FL_NT) plcp_fill_kernel(u32 *__restrict__ v, u64 count,
@@ -212,15 +189,9 @@ __global__ void __launch_bounds__(FL_NT) plcp_fill_kernel(u32 *__restrict__ v, u
         x[q] = base + q < count ? v[base + q] : UNDEF;
         last = pick(last, x[q]);
     }
-    u32 incl = last;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane_id() >= (unsigned)o) incl = pick(t, incl);
-    }
+    const u32 incl = warp_inclusive(last, PickOp());
     if (lane_id() == 31) wl[threadIdx.x >> 5] = incl;
-    u32 excl = __shfl_up_sync(0xffffffffu, incl, 1);
-    if (lane_id() == 0) excl = UNDEF;
+    const u32 excl = warp_exclusive(incl, last, PickOp(), UNDEF);
     __syncthreads();
     u32 pre = tile_carry[blockIdx.x];
     for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) pre = pick(pre, wl[w]);

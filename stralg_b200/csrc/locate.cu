@@ -46,33 +46,6 @@ __global__ void __launch_bounds__(256) ssa_mark_kernel(const u32 *__restrict__ s
     }
 }
 
-// exclusive scan of `count` u32 values by one CTA (in place)
-__global__ void __launch_bounds__(1024) scan_u32_kernel(u32 *__restrict__ vals, u32 count) {
-    __shared__ u32 wsum[32];
-    __shared__ u32 carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (u32 base = 0; base < count; base += 1024) {
-        const u32 i = base + threadIdx.x;
-        const u32 v = i < count ? vals[i] : 0;
-        u32 incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane_id() >= (unsigned)o) incl += t;
-        }
-        if (lane_id() == 31) wsum[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        u32 wb = 0;
-        for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) wb += wsum[w];
-        const u32 excl = carry + wb + incl - v;
-        if (i < count) vals[i] = excl;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = excl + v;
-        __syncthreads();
-    }
-}
-
 // one CTA per tile of mark words: counts -> ranks, then the sampled values are stored
 __global__ void __launch_bounds__(SS_TILE_WORDS) ssa_fill_kernel(const u32 *__restrict__ sa, u64 nwords,
                                                                  const u32 *__restrict__ tile_prefix,
@@ -81,19 +54,9 @@ __global__ void __launch_bounds__(SS_TILE_WORDS) ssa_fill_kernel(const u32 *__re
     const u64 w = (u64)blockIdx.x * SS_TILE_WORDS + threadIdx.x;
     uint4 mk = make_uint4(0, 0, 0, 0);
     if (w < nwords) mk = marks[w];
-    const u32 c = mk.z;
-    u32 incl = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane_id() >= (unsigned)o) incl += t;
-    }
-    if (lane_id() == 31) wsum[threadIdx.x >> 5] = incl;
-    __syncthreads();
-    u32 wb = 0;
-    for (unsigned q = 0; q < (threadIdx.x >> 5); ++q) wb += wsum[q];
+    const u32 excl = block_exclusive<SS_TILE_WORDS>(mk.z, wsum);
     if (w >= nwords) return;
-    const u32 rank = tile_prefix[blockIdx.x] + wb + incl - c;
+    const u32 rank = tile_prefix[blockIdx.x] + excl;
     mk.z = rank;
     marks[w] = mk;
     u64 bits = ((u64)mk.y << 32) | mk.x;
@@ -117,8 +80,7 @@ void build_sampled_sa(DeviceIndex &ix, u32 rate) {
     unsigned blocks = std::max(1u, std::min(div_up_u(nwords, 8), 148u * 16u));
     ssa_mark_kernel<<<blocks, 256, 0, st>>>(ix.sa.ptr, ix.len, rate, nwords, ix.ssa_marks.ptr, tile_tot.ptr);
     KERNEL_CHECK();
-    scan_u32_kernel<<<1, 1024, 0, st>>>(tile_tot.ptr, ntiles);
-    KERNEL_CHECK();
+    scan_sum(tile_tot.ptr, ntiles, st);
     ssa_fill_kernel<<<ntiles, SS_TILE_WORDS, 0, st>>>(ix.sa.ptr, nwords, tile_tot.ptr, ix.ssa_marks.ptr, ix.ssa_vals.ptr);
     KERNEL_CHECK();
     ix.ssa_rate = rate;  // (tile_tot is released in stream order)
@@ -255,34 +217,17 @@ void sort_positions(const DeviceIndex &ix, u64 npat, const u64 *d_pos_off, u64 t
     if (total < 2) return;
     if (total > 0xFFFFFFFFull || npat > 0xFFFFFFFFull)
         throw std::runtime_error("sort_positions: more than 2^32 - 1 positions or patterns in one batch");
-    constexpr int RB = 8;
-    typedef rs::Sorter<RB> S;
-    constexpr int BINS = 1 << RB;
-    const u32 m = (u32)total;
     int qbits = 0;
     while ((1ull << qbits) < npat) ++qbits;
-    const int key_bits = 32 + qbits;
-    const int npass = (key_bits + RB - 1) / RB;
-    DevBuf<u64> kA(total, st), kB(total, st), lookback(S::lookback_words(m), st);
-    DevBuf<u32> vA(total, st), vB(total, st), hist((size_t)8 * BINS, st), uniform(8, st), ticket(1, st);
+    DevBuf<u64> kA(total, st), kB(total, st);
+    DevBuf<u32> vA(total, st), vB(total, st);
     CUDA_CHECK(cudaMemsetAsync(vA.ptr, 0, total * 4, st));
     sort_keys_make_kernel<<<div_up_u(total, 256), 256, 0, st>>>(d_pos, d_pos_off, npat, total, kA.ptr);
     KERNEL_CHECK();
-    S::histogram(kA.ptr, m, 0, key_bits, npass, hist.ptr, st);
-    S::scan(hist.ptr, m, npass, uniform.ptr, st);
-    u32 huniform[8];
-    CUDA_CHECK(cudaMemcpyAsync(huniform, uniform.ptr, (size_t)npass * 4, cudaMemcpyDeviceToHost, st));
-    CUDA_CHECK(cudaStreamSynchronize(st));
-    u64 *kin = kA.ptr, *kout = kB.ptr;
-    u32 *vin = vA.ptr, *vout = vB.ptr;
-    for (int p = 0; p < npass; ++p) {
-        if (huniform[p]) continue;
-        const int bits_here = std::min(RB, key_bits - p * RB);
-        S::pass(kin, vin, kout, vout, m, p * RB, bits_here, hist.ptr + (size_t)p * BINS, lookback.ptr, ticket.ptr, st);
-        std::swap(kin, kout);
-        std::swap(vin, vout);
-    }
-    sort_keys_take_kernel<<<div_up_u(total, 256), 256, 0, st>>>(kin, total, d_pos);
+    u64 *kb[2] = {kA.ptr, kB.ptr};
+    u32 *vb[2] = {vA.ptr, vB.ptr};
+    const auto sorted = rs::Sorter<8>::sort(kb, vb, (u32)total, 32 + qbits, st);
+    sort_keys_take_kernel<<<div_up_u(total, 256), 256, 0, st>>>(sorted.keys, total, d_pos);
     KERNEL_CHECK();
     (void)ix;  // (the work buffers are released in stream order)
 }

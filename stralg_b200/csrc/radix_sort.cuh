@@ -8,7 +8,7 @@
 // for round 0).  Replaces the byte-wise CPU radix passes of stralg/skew.c:53-99 and the bucket
 // scatters of stralg/sa_is.c:203-263; none of that code is reused.
 #pragma once
-#include "common.cuh"
+#include "scan.cuh"
 
 namespace b200sa {
 namespace rs {
@@ -80,17 +80,7 @@ __global__ void __launch_bounds__(256) scan_hist_kernel(u32 *__restrict__ hist, 
         sum += v[q];
     }
     if (full) any_full = 1;
-    u32 incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane_id() >= (unsigned)o) incl += t;
-    }
-    if (lane_id() == 31) warp_tot[threadIdx.x >> 5] = incl;
-    __syncthreads();
-    u32 base = 0;
-    for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) base += warp_tot[w];
-    u32 run = base + incl - sum;
+    u32 run = block_exclusive<NT>(sum, warp_tot);
 #pragma unroll
     for (int q = 0; q < DPT; ++q) {
         int d = threadIdx.x * DPT + q;
@@ -212,17 +202,7 @@ __global__ void __launch_bounds__(NT, (NT <= 256 ? 4 : (NT <= 384 ? 2 : 2))) one
     }
     // block exclusive scan of the tile's digit counts -> tile_start[]
     {
-        u32 incl = tsum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= (unsigned)o) incl += t;
-        }
-        if (lane == 31) misc[warp] = incl;
-        __syncthreads();
-        u32 wb = 0;
-        for (unsigned w = 0; w < warp; ++w) wb += misc[w];
-        u32 run = wb + incl - tsum;
+        u32 run = block_exclusive<NT>(tsum, misc);
 #pragma unroll
         for (int q = 0; q < DPT; ++q) {
             int d = tid * DPT + q;
@@ -339,6 +319,47 @@ struct Sorter {
         onesweep_pass_kernel<RB, PASS_NT, PASS_IPT><<<tiles, PASS_NT, Cfg::SMEM, st>>>(kin, vin, kout, vout, n, shift, mask,
                                                                                      digit_base, lookback, ticket);
         KERNEL_CHECK();
+    }
+
+    struct Sorted {
+        u64 *keys;   // the buffer pair that holds the sorted pairs
+        u32 *vals;
+        int passes;  // passes run (the others had one digit for every key)
+    };
+
+    // Stable sort of (keys[0], vals[0]) on the low key_bits (<= 64) bits of the keys; (keys[1], vals[1]) is the
+    // other buffer pair.  One histogram of every digit, then one pass per digit that is not the same for every
+    // key.  Work buffers: hist 8 * BINS words, uniform 8 words, lookback lookback_words(n), ticket 1 word.
+    // With a timer: stages "round_hist" (histogram, scan and the read-back of the uniform flags) and "radix_pass".
+    static Sorted sort(u64 *keys[2], u32 *vals[2], u32 n, int key_bits, u32 *hist, u32 *uniform, u64 *lookback,
+                       u32 *ticket, cudaStream_t st, StageTimer *timer = nullptr) {
+        if (key_bits <= 0 || n < 2) return Sorted{keys[0], vals[0], 0};
+        const int npass = (key_bits + RB - 1) / RB;
+        u32 huniform[8];
+        int t = timer ? timer->begin("round_hist", (double)n * 8.0) : -1;
+        histogram(keys[0], n, 0, key_bits, npass, hist, st);
+        scan(hist, n, npass, uniform, st);
+        read_back(huniform, uniform, (size_t)npass * 4, st);
+        if (timer) timer->end(t);
+        int in = 0, passes = 0;
+        for (int p = 0; p < npass; ++p) {
+            if (huniform[p]) continue;
+            const int bits_here = key_bits - p * RB < RB ? key_bits - p * RB : RB;
+            t = timer ? timer->begin("radix_pass", (double)n * 24.0) : -1;
+            pass(keys[in], vals[in], keys[in ^ 1], vals[in ^ 1], n, p * RB, bits_here, hist + (size_t)p * BINS,
+                 lookback, ticket, st);
+            if (timer) timer->end(t);
+            in ^= 1;
+            ++passes;
+        }
+        return Sorted{keys[in], vals[in], passes};
+    }
+
+    // the same with work buffers of its own, from the library's pool
+    static Sorted sort(u64 *keys[2], u32 *vals[2], u32 n, int key_bits, cudaStream_t st) {
+        DevBuf<u64> lookback(lookback_words(n), st);
+        DevBuf<u32> hist((size_t)8 * BINS, st), uniform(8, st), ticket(1, st);
+        return sort(keys, vals, n, key_bits, hist.ptr, uniform.ptr, lookback.ptr, ticket.ptr, st);
     }
 };
 

@@ -15,8 +15,6 @@
 #include "engine.h"
 #include "radix_sort.cuh"
 
-#include <algorithm>
-
 namespace b200sa {
 
 // the largest r < nrec with bound[r] <= p, for bound[0] <= p < bound[nrec] (bound: rec_off or start)
@@ -106,36 +104,6 @@ static int bits_for(u64 count) {  // bits of the largest value below `count`
     return b;
 }
 
-// Stable LSD radix sort of (keys, vals) on the low key_bits bits (radix_sort.cuh, as sort_positions in locate.cu);
-// returns the buffers that hold the result (A or B).
-static void sort_pairs(DevBuf<u64> &kA, DevBuf<u32> &vA, DevBuf<u64> &kB, DevBuf<u32> &vB, u32 m, int key_bits,
-                       u64 **kout_res, u32 **vout_res, cudaStream_t st) {
-    u64 *kin = kA.ptr, *kout = kB.ptr;
-    u32 *vin = vA.ptr, *vout = vB.ptr;
-    if (key_bits > 0 && m > 1) {
-        constexpr int RB = 8;
-        typedef rs::Sorter<RB> S;
-        constexpr int BINS = 1 << RB;
-        const int npass = (key_bits + RB - 1) / RB;
-        DevBuf<u64> lookback(S::lookback_words(m), st);
-        DevBuf<u32> hist((size_t)8 * BINS, st), uniform(8, st), ticket(1, st);
-        S::histogram(kA.ptr, m, 0, key_bits, npass, hist.ptr, st);
-        S::scan(hist.ptr, m, npass, uniform.ptr, st);
-        u32 huniform[8];
-        read_back(huniform, uniform.ptr, (size_t)npass * 4, st);
-        for (int p = 0; p < npass; ++p) {
-            if (huniform[p]) continue;
-            const int bits_here = std::min(RB, key_bits - p * RB);
-            S::pass(kin, vin, kout, vout, m, p * RB, bits_here, hist.ptr + (size_t)p * BINS, lookback.ptr, ticket.ptr,
-                    st);
-            std::swap(kin, kout);
-            std::swap(vin, vout);
-        }
-    }
-    *kout_res = kin;
-    *vout_res = vin;
-}
-
 void record_sas(const DeviceIndex &ix, u32 *d_out, cudaStream_t st) {
     const u64 rows = (u64)ix.len - 1;  // = n, the entries of all records' arrays together
     if (!rows) return;
@@ -143,11 +111,11 @@ void record_sas(const DeviceIndex &ix, u32 *d_out, cudaStream_t st) {
     DevBuf<u32> vA(rows, st), vB(rows, st);
     record_rows_kernel<<<div_up_u(rows, 256), 256, 0, st>>>(ix.sa.ptr, rows, ix.rec_start.ptr, ix.nrec, kA.ptr, vA.ptr);
     KERNEL_CHECK();
-    u64 *k = nullptr;
-    u32 *v = nullptr;
-    sort_pairs(kA, vA, kB, vB, (u32)rows, bits_for(ix.nrec), &k, &v, st);
+    u64 *kb[2] = {kA.ptr, kB.ptr};
+    u32 *vb[2] = {vA.ptr, vB.ptr};
+    const auto sorted = rs::Sorter<8>::sort(kb, vb, (u32)rows, bits_for(ix.nrec), st);
     // record r's rows, in the global order, are entries start[r] .. start[r + 1] - 1 of the partition
-    CUDA_CHECK(cudaMemcpyAsync(d_out, v, rows * 4, cudaMemcpyDeviceToDevice, st));
+    CUDA_CHECK(cudaMemcpyAsync(d_out, sorted.vals, rows * 4, cudaMemcpyDeviceToDevice, st));
 }
 
 void records_clamp_rows(const u32 *d_L, u64 npat, u32 *d_out, cudaStream_t st) {
@@ -167,10 +135,11 @@ void locate_records_group(const DeviceIndex &ix, u64 npat, const u64 *d_pos_off,
     record_keys_kernel<<<div_up_u(total, 256), 256, 0, st>>>(d_pos, d_pos_off, npat, total, ix.rec_start.ptr, ix.nrec,
                                                              rbits, kA.ptr, vA.ptr);
     KERNEL_CHECK();
-    u64 *k = nullptr;
-    u32 *v = nullptr;
-    sort_pairs(kA, vA, kB, vB, (u32)total, qbits + rbits, &k, &v, st);
-    record_take_kernel<<<div_up_u(total, 256), 256, 0, st>>>(k, v, total, (1ull << rbits) - 1ull, d_rec, d_local);
+    u64 *kb[2] = {kA.ptr, kB.ptr};
+    u32 *vb[2] = {vA.ptr, vB.ptr};
+    const auto sorted = rs::Sorter<8>::sort(kb, vb, (u32)total, qbits + rbits, st);
+    record_take_kernel<<<div_up_u(total, 256), 256, 0, st>>>(sorted.keys, sorted.vals, total, (1ull << rbits) - 1ull,
+                                                             d_rec, d_local);
     KERNEL_CHECK();
 }
 

@@ -23,6 +23,7 @@
 // round0_msd.cuh): any monotone, injective map of K-symbol prefixes serves, and only the level-1
 // kernels that read the text know which one is in use.
 #include "round0_msd.cuh"
+#include "scan.cuh"
 
 #include <vector>
 
@@ -269,23 +270,15 @@ __global__ void __launch_bounds__(1024) msd_scan_children_kernel(u32 *__restrict
     const size_t at = (size_t)p * B + d0;
     u32 c0 = d0 < B ? hist[at] : 0u;
     u32 c1 = (per > 1 && d0 + 1 < B) ? hist[at + 1] : 0u;
-    const u32 c = c0 + c1;
-    u32 incl = c;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (unsigned)o) incl += t;
-    }
     u32 mx = max(c0, c1);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-    if (lane == 31) wsum[warp] = incl;
     if (lane == 0) wmax[warp] = mx;
-    __syncthreads();
-    u32 base = parent_start ? parent_start[p] : 0u;
-    for (unsigned w = 0; w < warp; ++w) base += wsum[w];
+    // (a block of fewer than 1024 threads leaves the last words of wsum unwritten: they only reach the
+    // prefixes of warps that do not exist)
+    const u32 excl = block_exclusive<1024>(c0 + c1, wsum);
     if (d0 < B) {
-        u32 st = base + incl - c;
+        u32 st = (parent_start ? parent_start[p] : 0u) + excl;
         child_start[at] = st;
         hist[at] = st;
         if (per > 1 && d0 + 1 < B) {
@@ -308,34 +301,12 @@ __global__ void __launch_bounds__(1024) msd_scan_children_kernel(u32 *__restrict
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(1024) msd_tile_offsets_kernel(const u32 *__restrict__ pstart, u32 nparents,
                                                                 u32 *__restrict__ tile_off, u32 *__restrict__ d_ntiles) {
-    __shared__ u32 wsum[32];
-    __shared__ u32 carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-    for (u32 base = 0; base < nparents; base += 1024) {
-        u32 p = base + threadIdx.x;
-        u32 nt = 0;
-        if (p < nparents) nt = (pstart[p + 1] - pstart[p] + (P_TILE - 1)) / P_TILE;
-        u32 incl = nt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= (unsigned)o) incl += t;
-        }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        u32 wb = 0;
-        for (unsigned w = 0; w < warp; ++w) wb += wsum[w];
-        u32 excl = carry + wb + incl - nt;
-        if (p < nparents) tile_off[p] = excl;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = excl + nt;
-        __syncthreads();
-    }
+    const u32 ntiles = cta_exclusive_scan(
+        nparents, [=](u32 p) { return (pstart[p + 1] - pstart[p] + (P_TILE - 1)) / P_TILE; },
+        [=](u32 p, u32 e) { tile_off[p] = e; }, SumOp(), 0u);
     if (threadIdx.x == 0) {
-        tile_off[nparents] = carry;
-        *d_ntiles = carry;
+        tile_off[nparents] = ntiles;
+        *d_ntiles = ntiles;
     }
 }
 
@@ -397,30 +368,6 @@ __global__ void __launch_bounds__(P_NT) msd_hist_elems_kernel(const u64 *__restr
     u32 *h = hist + (size_t)parent * B;
     for (u32 i = threadIdx.x; i < B; i += P_NT)
         if (sh[i]) atomicAdd(&h[i], sh[i]);
-}
-
-// exclusive prefix of `v` over an NT-thread block (wsum: NT / 32 words of shared memory)
-template <int NT>
-__device__ __forceinline__ u32 block_exclusive(u32 v, u32 *wsum) {
-    constexpr int NW = NT / 32;
-    const u32 lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-    u32 incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (unsigned)o) incl += t;
-    }
-    if (lane == 31) wsum[warp] = incl;
-    __syncthreads();
-    u32 ws = lane < (u32)NW ? wsum[lane] : 0u;
-    u32 wi = ws;
-#pragma unroll
-    for (int o = 1; o < NW; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, wi, o);
-        if (lane >= (unsigned)o) wi += t;
-    }
-    const u32 wbase = __shfl_sync(0xffffffffu, wi - ws, warp);
-    return wbase + incl - v;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -804,13 +751,7 @@ __device__ __forceinline__ void l3_segments(const u32 *__restrict__ bstart, u32 
             loc[q] = (u32)__popc(segmask[tid * WPL + q]);
             sum += loc[q];
         }
-        u32 incl = sum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (tid >= (unsigned)o) incl += t;
-        }
-        u32 run = incl - sum;
+        u32 run = warp_inclusive(sum, SumOp()) - sum;
 #pragma unroll
         for (int q = 0; q < WPL; ++q) {
             segpre[tid * WPL + q] = run;
@@ -1078,22 +1019,7 @@ __global__ void __launch_bounds__(L3_NT, L3_CTAS) msd_local_sort_kernel(L3Args a
                     v[q] = mine ? bytesum(cnt[base + q]) : 0u;
                     sum += v[q];
                 }
-                u32 incl = sum;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    u32 x = __shfl_up_sync(0xffffffffu, incl, o);
-                    if (lane >= (unsigned)o) incl += x;
-                }
-                if (lane == 31) misc[warp] = incl;
-                __syncthreads();
-                u32 ws = lane < (u32)(L3_NT / 32) ? misc[lane] : 0u;
-                u32 wi = ws;
-#pragma unroll
-                for (int o = 1; o < L3_NT / 32; o <<= 1) {
-                    u32 x = __shfl_up_sync(0xffffffffu, wi, o);
-                    if (lane >= (unsigned)o) wi += x;
-                }
-                u32 run = __shfl_sync(0xffffffffu, wi - ws, warp) + incl - sum;
+                u32 run = block_exclusive<L3_NT>(sum, misc);
                 if (mine) {
 #pragma unroll
                     for (int q = 0; q < L3_IPT; ++q) {

@@ -197,17 +197,7 @@ __global__ void __launch_bounds__(256) round0_bases_kernel(const u32 *__restrict
         v[q] = d < BINS ? h[d] : 0;
         sum += v[q];
     }
-    u32 incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane_id() >= (unsigned)o) incl += t;
-    }
-    if (lane_id() == 31) warp_tot[threadIdx.x >> 5] = incl;
-    __syncthreads();
-    u32 base = 0;
-    for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) base += warp_tot[w];
-    u32 run = base + incl - sum;
+    u32 run = block_exclusive<NT>(sum, warp_tot);
 #pragma unroll
     for (int q = 0; q < DPT; ++q) {
         int d = threadIdx.x * DPT + q;
@@ -540,15 +530,9 @@ __global__ void __launch_bounds__(CF_NT) chain_flags_kernel(const u32 *__restric
             pg = g[q];
         }
     }
-    u32 ex = run;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const u32 t = __shfl_up_sync(0xffffffffu, ex, o);
-        if (lane >= (u32)o) ex = max(ex, t);
-    }
+    const u32 ex = warp_inclusive(run, MaxOp());
     if (lane == 31) wmax[warp] = ex;
-    u32 pre = __shfl_up_sync(0xffffffffu, ex, 1);
-    if (lane == 0) pre = 0;
+    u32 pre = warp_exclusive(ex, run, MaxOp(), 0u);
     __syncthreads();
     for (u32 w = 0; w < warp; ++w) pre = max(pre, wmax[w]);
 #pragma unroll
@@ -894,23 +878,12 @@ __global__ void __launch_bounds__(RK_NT) rank_kernel(RankArgs a) {
     }
 
     // ---- block-wide "last head so far" (max-scan; indices grow with position) ----
-    u32 ex_s = run_s, ex_b = run_b;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        u32 ts = __shfl_up_sync(0xffffffffu, ex_s, o);
-        u32 tb = __shfl_up_sync(0xffffffffu, ex_b, o);
-        if (lane >= (unsigned)o) {
-            ex_s = max(ex_s, ts);
-            ex_b = max(ex_b, tb);
-        }
-    }
+    const u32 ex_s = warp_inclusive(run_s, MaxOp()), ex_b = warp_inclusive(run_b, MaxOp());
     if (lane == 31) {
         warp_s[warp] = ex_s;
         warp_b[warp] = ex_b;
     }
-    u32 pre_s = __shfl_up_sync(0xffffffffu, ex_s, 1);
-    u32 pre_b = __shfl_up_sync(0xffffffffu, ex_b, 1);
-    if (lane == 0) pre_s = pre_b = 0;
+    u32 pre_s = warp_exclusive(ex_s, run_s, MaxOp(), 0u), pre_b = warp_exclusive(ex_b, run_b, MaxOp(), 0u);
     __syncthreads();
     for (unsigned w = 0; w < warp; ++w) {
         pre_s = max(pre_s, warp_s[w]);
@@ -1021,35 +994,6 @@ __global__ void __launch_bounds__(CP_NT) count_active_kernel(const u8 *__restric
     }
 }
 
-// single-block exclusive scan of u32 counts; total (u64) written to *total
-__global__ void __launch_bounds__(1024) scan_tiles_kernel(u32 *__restrict__ counts, u32 ntiles,
-                                                          unsigned long long *__restrict__ total) {
-    __shared__ u64 wsum[32];
-    __shared__ u64 carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (u32 base = 0; base < ntiles; base += 1024) {
-        u32 i = base + threadIdx.x;
-        u64 v = i < ntiles ? counts[i] : 0;
-        u64 incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u64 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane_id() >= (unsigned)o) incl += t;
-        }
-        if (lane_id() == 31) wsum[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        u64 wb = 0;
-        for (unsigned w = 0; w < (threadIdx.x >> 5); ++w) wb += wsum[w];
-        u64 excl = carry + wb + incl - v;
-        if (i < ntiles) counts[i] = (u32)excl;  // active counts fit u32 (<= m < 2^32)
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = excl + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *total = carry;
-}
-
 // RAW: `headbits` is the bitmap of the elements to keep (bit per element), not a head bitmap
 template <bool RAW>
 __global__ void __launch_bounds__(CP_NT) scatter_active_kernel(const u8 *__restrict__ headbits,
@@ -1065,20 +1009,8 @@ __global__ void __launch_bounds__(CP_NT) scatter_active_kernel(const u8 *__restr
         const u64 word = ((u64)blockIdx.x * sub + q) * CP_NT + threadIdx.x;
         const u64 mask = RAW ? raw_mask(headbits, word, m) : active_mask(headbits, word, m);
         const u32 c = __popcll(mask);
-        u32 incl = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= (unsigned)o) incl += t;
-        }
-        if (lane == 31) wsum[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        u32 wb = 0, total = 0;
-        for (unsigned w = 0; w < CP_NT / 32; ++w) {
-            if (w < (threadIdx.x >> 5)) wb += wsum[w];
-            total += wsum[w];
-        }
-        const u32 o = base + wb + incl - c;
+        u32 total;
+        const u32 o = base + block_exclusive<CP_NT>(c, wsum, &total);
         base += total;
         __syncthreads();  // wsum is rewritten by the next sub-tile
         if (!__any_sync(0xffffffffu, mask != 0)) continue;  // (most warps of a sparse bitmap)
@@ -1181,15 +1113,9 @@ __global__ void __launch_bounds__(RS_NT) round_small_kernel(SmallArgs a) {
             pg = g[q];
         }
     }
-    u32 ex = run;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const u32 t = __shfl_up_sync(0xffffffffu, ex, o);
-        if (lane >= (u32)o) ex = max(ex, t);
-    }
+    const u32 ex = warp_inclusive(run, MaxOp());
     if (lane == 31) wmax[warp] = ex;
-    u32 pre = __shfl_up_sync(0xffffffffu, ex, 1);
-    if (lane == 0) pre = 0;
+    u32 pre = warp_exclusive(ex, run, MaxOp(), 0u);
     __syncthreads();
     for (u32 w = 0; w < warp; ++w) pre = max(pre, wmax[w]);
 #pragma unroll
@@ -1265,20 +1191,8 @@ __global__ void __launch_bounds__(CP_NT) scatter_pairs_kernel(const u8 *__restri
         const u64 word = ((u64)blockIdx.x * sub + q) * CP_NT + threadIdx.x;
         const u64 mask = raw_mask(bits, word, m);
         const u32 c = __popcll(mask);
-        u32 incl = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= (unsigned)o) incl += t;
-        }
-        if (lane == 31) wsum[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        u32 wb = 0, total = 0;
-        for (unsigned w = 0; w < CP_NT / 32; ++w) {
-            if (w < (threadIdx.x >> 5)) wb += wsum[w];
-            total += wsum[w];
-        }
-        const u32 o = base + wb + incl - c;
+        u32 total;
+        const u32 o = base + block_exclusive<CP_NT>(c, wsum, &total);
         base += total;
         __syncthreads();
         if (!__any_sync(0xffffffffu, mask != 0)) continue;
@@ -1332,24 +1246,6 @@ __global__ void __launch_bounds__(CP_NT) scatter_pairs_kernel(const u8 *__restri
 // ---------------------------------------------------------------------------------------------
 static constexpr int PV_NT = 256, PV_IPT = 8, PV_TILE = PV_NT * PV_IPT;
 
-// exclusive prefix of `v` over an NT-thread block (wsum: NT / 32 words of shared memory; one barrier inside)
-template <int NT>
-__device__ __forceinline__ u32 block_exclusive_u32(u32 v, u32 *wsum) {
-    constexpr int NW = NT / 32;
-    const u32 lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-    u32 incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const u32 t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (u32)o) incl += t;
-    }
-    if (lane == 31) wsum[warp] = incl;
-    __syncthreads();
-    u32 wb = 0;
-    for (u32 w = 0; w < warp && w < (u32)NW; ++w) wb += wsum[w];
-    return wb + incl - v;
-}
-
 struct PivotArgs {
     const u32 *act;               // values (suffixes) of the list
     u64 *keys;                    // its round keys: [first row of the group : lo_bits | second key : lo_bits]; R members
@@ -1360,7 +1256,7 @@ struct PivotArgs {
     unsigned long long *cnt64;    // by head row >> 1: |E| << 32 | |L|
     u8 *ebits8, *lbits8, *rbits8; // bit per list element: its class
     u32 *tile_e;                  // [tiles + 1] E members per tile (exclusive offsets after the scan)
-    unsigned long long *totals;   // [0] E members (written by the scan), [1] L members (accumulated here)
+    u32 *totals;                  // [0] E members (written by the scan), [1] L members (accumulated here)
     u32 *sa, *rank, *primary;
     u32 *out_act, *out_grp;       // where the E part goes in the next list
     u32 *singles;                 // [1] E groups of one member (final; they are taken out of the next list afterwards)
@@ -1503,7 +1399,7 @@ __global__ void __launch_bounds__(PV_NT) pivot_classify_kernel(PivotArgs a) {
         for (int w = 0; w < PV_NT / 32; ++w) t += wsum[w];
         a.tile_e[blockIdx.x] = t;
         if (blkL | blkE) atomicAdd(&a.cnt64[g0 >> 1], ((unsigned long long)blkE << 32) | (unsigned long long)blkL);
-        if (allL) atomicAdd(&a.totals[1], (unsigned long long)allL);
+        if (allL) atomicAdd(&a.totals[1], allL);
     }
 }
 
@@ -1539,15 +1435,9 @@ __global__ void __launch_bounds__(PV_NT, 4) pivot_apply_kernel(PivotArgs a) {
             hidx[q] = run;
             pg = g[q];
         }
-        u32 ex = run;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const u32 t = __shfl_up_sync(0xffffffffu, ex, o);
-            if (lane >= (u32)o) ex = max(ex, t);
-        }
+        const u32 ex = warp_inclusive(run, MaxOp());
         if (lane == 31) wmax[warp] = ex;
-        u32 pre = __shfl_up_sync(0xffffffffu, ex, 1);
-        if (lane == 0) pre = 0;
+        u32 pre = warp_exclusive(ex, run, MaxOp(), 0u);
         __syncthreads();
         for (u32 w = 0; w < warp; ++w) pre = max(pre, wmax[w]);
 #pragma unroll
@@ -1555,7 +1445,8 @@ __global__ void __launch_bounds__(PV_NT, 4) pivot_apply_kernel(PivotArgs a) {
             if (hidx[q] == 0) hidx[q] = pre;
     }
     // E members of the tile before this thread's elements
-    const u32 excl = block_exclusive_u32<PV_NT>((u32)__popc(ebyte), wsum);
+    u32 ne;  // E members of the tile
+    const u32 excl = block_exclusive<PV_NT>((u32)__popc(ebyte), wsum, &ne);
     const u32 tile_off = a.tile_e[blockIdx.x];
     // identifier of an E group: the old one while it lies inside the new range, else the middle of the range (a
     // group that loses members at one end, or at both, keeps it for many rounds)
@@ -1615,8 +1506,6 @@ __global__ void __launch_bounds__(PV_NT, 4) pivot_apply_kernel(PivotArgs a) {
     }
     __syncthreads();
     // consecutive threads write consecutive entries of the next list
-    u32 ne = 0;  // E members of the tile (the warp totals of the prefix sum above)
-    for (int w = 0; w < PV_NT / 32; ++w) ne += wsum[w];
     for (u32 k = tid; k < ne; k += PV_NT) {
         const u32 sv = sh_s[PV_PAD(k)], rk = sh_rk[PV_PAD(k)];
         a.out_act[tile_off + k] = sv;
@@ -2074,16 +1963,15 @@ static void launch_cmer_hist(const DeviceIndex &ix, u64 nwords_data, u32 *hist, 
 // element is kept unless it is a singleton.
 static u32 compaction_sub(u32 m) { return m > (1u << 26) ? 8u : 1u; }
 template <bool RAW>
-static u32 count_active(const u8 *bits, u32 m, u32 *tile_counts, unsigned long long *d_total, cudaStream_t st) {
+static u32 count_active(const u8 *bits, u32 m, u32 *tile_counts, u32 *d_total, cudaStream_t st) {
     const u32 sub = compaction_sub(m);
     u32 ntiles = div_up_u(m, (u64)CP_TILE * sub);
     count_active_kernel<RAW><<<ntiles, CP_NT, 0, st>>>(bits, m, sub, tile_counts);
     KERNEL_CHECK();
-    scan_tiles_kernel<<<1, 1024, 0, st>>>(tile_counts, ntiles, d_total);
-    KERNEL_CHECK();
-    unsigned long long total = 0;
-    read_back(&total, d_total, 8, st);
-    return (u32)total;
+    scan_sum(tile_counts, ntiles, st, d_total);  // (the count is at most m < 2^32)
+    u32 total = 0;
+    read_back(&total, d_total, 4, st);
+    return total;
 }
 template <bool RAW>
 static void scatter_active(const u8 *bits, const u32 *vals, const u32 *grp_in, u32 m, const u32 *tile_offsets, u32 *out,
@@ -2322,7 +2210,7 @@ struct BuildCtx {
     u64 *keysA, *keysB, *lookback;
     u32 *valsV, *rank, *actbits, *hist, *uniform, *ticket, *tile_counts, *d_lazy;
     u8 *headbits;
-    unsigned long long *d_total;
+    u32 *d_total;
     u8 *bwt_rows = nullptr;     // BWT output while the sort writes its rows as it goes
     bool need_bwt_fix = false;  // a path moved rows without writing their BWT rows
 
@@ -2384,31 +2272,18 @@ static RankArgs rank_args(const BuildCtx &c, const u64 *keys, const u32 *vals, u
 template <int RB>
 static u32 *sort_and_rank(BuildCtx &c, u64 *keys, u32 *vals, u64 *keys_other, u32 *vals_other, u32 m, u32 *newgrp,
                           u8 *headbits, u8 *bwt, int always_write) {
-    typedef rs::Sorter<RB> S;
-    const int npass = (c.key_bits + RB - 1) / RB;
-    u32 huniform[8];
-    int t = c.ix.timer.begin("round_hist", (double)m * 8.0);
-    S::histogram(keys, m, 0, c.key_bits, npass, c.hist, c.st);
-    S::scan(c.hist, m, npass, c.uniform, c.st);
-    read_back(huniform, c.uniform, (size_t)npass * 4, c.st);
-    c.ix.timer.end(t);
-    for (int p = 0; p < npass; ++p) {
-        if (huniform[p]) continue;
-        const int bits_here = std::min(RB, c.key_bits - p * RB);
-        t = c.ix.timer.begin("radix_pass", (double)m * 24.0);
-        S::pass(keys, vals, keys_other, vals_other, m, p * RB, bits_here, c.hist + (size_t)p * (1 << RB), c.lookback,
-                c.ticket, c.st);
-        c.ix.timer.end(t);
-        c.ix.stats.passes_elems += m;
-        std::swap(keys, keys_other);
-        std::swap(vals, vals_other);
-    }
-    t = c.ix.timer.begin("round_rank", (double)m * 20.0);
+    u64 *kb[2] = {keys, keys_other};
+    u32 *vb[2] = {vals, vals_other};
+    const auto sorted = rs::Sorter<RB>::sort(kb, vb, m, c.key_bits, c.hist, c.uniform, c.lookback, c.ticket, c.st,
+                                             &c.ix.timer);
+    c.ix.stats.passes_elems += (u64)m * sorted.passes;
+    int t = c.ix.timer.begin("round_rank", (double)m * 20.0);
     CUDA_CHECK(cudaMemsetAsync(headbits, 0, (((size_t)m + 63) / 64 + 2) * 8, c.st));
-    rank_kernel<<<div_up_u(m, RK_TILE), RK_NT, 0, c.st>>>(rank_args(c, keys, vals, m, newgrp, headbits, bwt, always_write));
+    rank_kernel<<<div_up_u(m, RK_TILE), RK_NT, 0, c.st>>>(
+        rank_args(c, sorted.keys, sorted.vals, m, newgrp, headbits, bwt, always_write));
     KERNEL_CHECK();
     c.ix.timer.end(t);
-    return vals;
+    return sorted.vals;
 }
 
 // the list elements whose keep byte is set, (act, row) -> (act_out, row_out) in list order; returns their number
@@ -2702,7 +2577,8 @@ struct RoundState {
     // pivot path: per-group tables by (head row) / 2, E bitmap, per-tile counts
     u8 *ebits8, *rbits8;
     u32 *pv_tile_e, *pv_piv;
-    unsigned long long *d_pvtot, *pv_cnt;
+    u32 *d_pvtot;
+    unsigned long long *pv_cnt;
     bool chain_on, small_on, pivot_on;
     bool prefer_pivot;            // large groups or small ones?  (decides which of the two split paths a round tries first)
     bool ids_are_heads = true;    // rank[] of an active suffix is the first row of its group (until the pivot path runs)
@@ -2780,19 +2656,18 @@ static bool pivot_round(BuildCtx &c, RoundState &R, u32 &m2) {
         CUDA_CHECK(cudaMemsetAsync(R.ebits8 + kw * 8, 0, 16, st));
         CUDA_CHECK(cudaMemsetAsync(R.notdone + kw * 8, 0, 16, st));
         CUDA_CHECK(cudaMemsetAsync(R.rbits8 + kw * 8, 0, 16, st));
-        CUDA_CHECK(cudaMemsetAsync(R.d_pvtot, 0, 16, st));
+        CUDA_CHECK(cudaMemsetAsync(R.d_pvtot, 0, 8, st));
         if (publish) {
             pivot_heads_kernel<<<div_up_u(n, PV_TILE), PV_NT, 0, st>>>(kx, n, c.lo_bits, R.pv_piv, R.pv_cnt);
             KERNEL_CHECK();
         }
         pivot_classify_kernel<<<ntl, PV_NT, 0, st>>>(pv);
         KERNEL_CHECK();
-        scan_tiles_kernel<<<1, 1024, 0, st>>>(R.pv_tile_e, ntl, R.d_pvtot);
-        KERNEL_CHECK();
-        unsigned long long tot[2] = {0, 0};
-        read_back(tot, R.d_pvtot, 16, st);
-        ne = (u32)tot[0];
-        nl = (u32)tot[1];
+        scan_sum(R.pv_tile_e, ntl, st, R.d_pvtot);
+        u32 tot[2] = {0, 0};
+        read_back(tot, R.d_pvtot, 8, st);
+        ne = tot[0];
+        nl = tot[1];
     };
     // radix sort of one list, new ranks, survivors appended to the next list
     auto sort_list = [&](u64 *kx, u32 *vx, u32 n, u64 *ky, u32 *vy, u32 *ng) {
@@ -3023,7 +2898,7 @@ static void doubling_rounds(BuildCtx &c, ActiveList &L) {
     R.ebits8 = R.pivot_on ? ar.get<u8>(bm_bytes) : nullptr;
     R.pv_tile_e = R.pivot_on ? ar.get<u32>((size_t)div_up_u(m_init, PV_TILE) + 2) : nullptr;
     R.rbits8 = R.pivot_on ? ar.get<u8>(bm_bytes) : nullptr;
-    R.d_pvtot = ar.get<unsigned long long>(2);
+    R.d_pvtot = ar.get<u32>(2);
     R.pv_cnt = R.pivot_on ? ar.get<unsigned long long>(pv_entries) : nullptr;
     R.pv_piv = R.pivot_on ? ar.get<u32>(pv_entries) : nullptr;
     R.prefer_pivot = c.kn.pivot_force;
@@ -3117,7 +2992,7 @@ static void build_sa_impl(DeviceIndex &ix, const BuildKnobs &kn, bool want_bwt) 
     c.hist = ar.get<u32>((size_t)8 * BINS); c.uniform = ar.get<u32>(8); c.ticket = ar.get<u32>(1);
     c.headbits = ar.get<u8>((((size_t)len + 63) / 64 + 2) * 8);
     c.tile_counts = ar.get<u32>(div_up_u(len, CP_TILE) + 1);
-    c.d_total = ar.get<unsigned long long>(1);
+    c.d_total = ar.get<u32>(1);
     c.d_lazy = ar.get<u32>(1);
 
     ActiveList L;

@@ -356,6 +356,43 @@ const uint32_t *b200sa_smem_L(const b200sa_smem_result *r);
 const uint32_t *b200sa_smem_R(const b200sa_smem_result *r);
 void b200sa_smem_free(b200sa_smem_result *r);
 
+/* ---- batched k-mismatch search on a bidirectional FM index -----------------------------------
+ * Every distinct text string within Hamming distance k of a read, each reported once: for short
+ * reads, barcodes, primers and off-target scans that need substitutions only.  (b200sa_approx_batch
+ * is the edit-distance search of the reference: it reports every edit path, so the same interval
+ * many times, in the reference's order.)
+ * Patterns take the form of b200sa_search_batch: remapped codes, concatenated, in host buffers, with
+ * `offsets` or `fixed_len`.  For a pattern P of length m >= 1 and k = max_mismatches, the hits are
+ * every distinct string Q with
+ *   |Q| = m,  Q over the letters 1..sigma-1,  Q occurs in the text,  Hamming(P, Q) <= k;
+ * each hit is one triple (L, R, d): [L, R) is Q's SA interval in `idx` (what b200sa_search_batch
+ * returns for Q) and d = Hamming(P, Q).  Hits of one pattern come in ascending L: the intervals of
+ * distinct strings of one length are disjoint, so the order is total and does not depend on how the
+ * search runs.  A pattern symbol 0 or >= sigma is not an error: it differs from every letter and costs
+ * one mismatch there.  An empty pattern has no hits; k = 0 gives exactly the non-empty results of
+ * b200sa_search_batch, each with d = 0.  Positions: b200sa_locate_batch / _sorted over (L, R).
+ * `rev_idx` is required: an index (B200SA_BUILD_OCC) of the reversed text (codes n-1 .. 0) on the same
+ * device, as for b200sa_approx_batch's D table; it may drop its suffix array.  Only the checks below
+ * are made: beyond them the caller guarantees that it really is the reversed text.
+ * Refusals, all before any CUDA call: NULL idx or rev_idx, NULL patterns with npat > 0, decreasing
+ * offsets, max_mismatches > 8 -> B200SA_ERR_BAD_ARGUMENT; a pattern longer than 65000 symbols ->
+ * B200SA_ERR_TOO_LARGE; either index without OCC -> B200SA_ERR_NOT_BUILT; rev_idx of another length,
+ * sigma, device or C table, or either index a records index -> B200SA_ERR_BAD_ARGUMENT.
+ * TEXTCMP and KTABLE do not change the results.  Long batches are staged in pieces of about 64 MB of
+ * pattern symbols; a piece with more than 2^32 - 1 hits -> B200SA_ERR_TOO_LARGE.  Accessors return
+ * host arrays owned by the result (valid until b200sa_hamming_free). */
+typedef struct b200sa_hamming_result b200sa_hamming_result;
+b200sa_hamming_result *b200sa_hamming_batch(const b200sa_index *idx, const b200sa_index *rev_idx,
+                                            const uint8_t *patterns, const uint64_t *offsets,
+                                            uint32_t fixed_len, uint64_t npat, uint32_t max_mismatches,
+                                            enum b200sa_error *err);
+uint64_t b200sa_hamming_hits(const b200sa_hamming_result *r);          /* hits in total         */
+const uint64_t *b200sa_hamming_offsets(const b200sa_hamming_result *r);/* npat + 1 (CSR)        */
+const uint32_t *b200sa_hamming_L(const b200sa_hamming_result *r);
+const uint32_t *b200sa_hamming_R(const b200sa_hamming_result *r);
+const uint32_t *b200sa_hamming_mismatches(const b200sa_hamming_result *r);
+void b200sa_hamming_free(b200sa_hamming_result *r);
+
 /* ---- synthetic inputs on the device (bench / tests; mirrors performance/suffix_array_search.c:13-32)
  * d_text must hold n + 1 bytes; symbols are 1 + hash(seed + i) % nsym, d_text[n] = 0. */
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device,

@@ -1825,25 +1825,31 @@ static int mems_args_ok(const b200sa_index *idx, const uint8_t *patterns, const 
     return 0;
 }
 
-// The first pass over a host batch, in pieces of about 64 MB of pattern bytes (whole patterns; a longer pattern is a
-// piece of its own), so that device memory stays bounded whatever the batch: a piece's patterns are copied in
-// (8-byte aligned and padded, as the kernels read whole words), its offsets rebased to the piece, and mems_stats
-// stores ms / L / R per symbol and, with `count`, the SMEMs of each pattern.  Then `piece(q0, q1, b0, d_off, d_ms,
-// d_L, d_R, d_count)` takes over the results of patterns [q0, q1), whose symbols start at b0 in the batch, on the
-// index's stream; it returns when it no longer needs them.
+// The end of the piece of a host batch that starts at pattern q0: whole patterns of about 64 MB of symbols in all (a
+// longer pattern is a piece of its own), so that device memory stays bounded whatever the batch.
+static uint64_t piece_end(const uint64_t *offsets, uint32_t fixed_len, uint64_t npat, uint64_t q0) {
+    const uint64_t kPieceBytes = (uint64_t)64 << 20;
+    uint64_t q1 = q0 + 1;
+    if (offsets)
+        while (q1 < npat && offsets[q1 + 1] - offsets[q0] <= kPieceBytes) ++q1;
+    else
+        q1 = std::min(npat, q0 + std::max<uint64_t>(1, kPieceBytes / std::max<uint32_t>(1, fixed_len)));
+    return q1;
+}
+
+// The first pass over a host batch, in pieces (piece_end): a piece's patterns are copied in (8-byte aligned and
+// padded, as the kernels read whole words), its offsets rebased to the piece, and mems_stats stores ms / L / R per
+// symbol and, with `count`, the SMEMs of each pattern.  Then `piece(q0, q1, b0, d_off, d_ms, d_L, d_R, d_count)`
+// takes over the results of patterns [q0, q1), whose symbols start at b0 in the batch, on the index's stream; it
+// returns when it no longer needs them.
 template <class Piece>
 static void mems_pieces(const DeviceIndex &ix, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
                         uint64_t npat, uint32_t min_len, bool count, Piece &&piece) {
-    const uint64_t kPieceBytes = (uint64_t)64 << 20;
     const cudaStream_t st = ix.stream;
     auto at = [&](uint64_t q) { return offsets ? offsets[q] : q * (uint64_t)fixed_len; };
     std::vector<uint64_t> hoff;
     for (uint64_t q0 = 0, q1; q0 < npat; q0 = q1) {
-        q1 = q0 + 1;
-        if (offsets)
-            while (q1 < npat && offsets[q1 + 1] - offsets[q0] <= kPieceBytes) ++q1;
-        else
-            q1 = std::min(npat, q0 + std::max<uint64_t>(1, kPieceBytes / std::max<uint32_t>(1, fixed_len)));
+        q1 = piece_end(offsets, fixed_len, npat, q0);
         const uint64_t b0 = at(q0), bytes = at(q1) - b0;
         DevBuf<u8> dp(bytes + 16, st);
         DevBuf<u32> dms(bytes, st), dL(bytes, st), dR(bytes, st);
@@ -1938,6 +1944,99 @@ const uint32_t *b200sa_smem_length(const b200sa_smem_result *r) { return r ? r->
 const uint32_t *b200sa_smem_L(const b200sa_smem_result *r) { return r ? r->L.data() : nullptr; }
 const uint32_t *b200sa_smem_R(const b200sa_smem_result *r) { return r ? r->R.data() : nullptr; }
 void b200sa_smem_free(b200sa_smem_result *r) { delete r; }
+
+}  // extern "C"
+#pragma GCC visibility pop
+
+// ---- k-mismatch search ------------------------------------------------------------------------------
+struct b200sa_hamming_result {
+    std::vector<uint64_t> off;  // npat + 1
+    std::vector<uint32_t> L, R, d;
+};
+
+#pragma GCC visibility push(default)
+extern "C" {
+
+b200sa_hamming_result *b200sa_hamming_batch(const b200sa_index *idx, const b200sa_index *rev_idx,
+                                            const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
+                                            uint64_t npat, uint32_t max_mismatches, enum b200sa_error *err) {
+    if (!idx || !rev_idx || (npat && !patterns) || max_mismatches > 8) {
+        fail(B200SA_ERR_BAD_ARGUMENT, "null argument or max_mismatches above 8", err);
+        return nullptr;
+    }
+    uint32_t max_m = fixed_len;
+    if (offsets) {
+        max_m = 0;
+        for (uint64_t q = 0; q < npat; ++q) {
+            if (offsets[q + 1] < offsets[q]) {
+                fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
+                return nullptr;
+            }
+            max_m = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(max_m, offsets[q + 1] - offsets[q]), 0xFFFFFFFFull);
+        }
+    }
+    if (max_m > 65000u) {
+        fail(B200SA_ERR_TOO_LARGE, "k-mismatch search takes patterns of up to 65000 symbols", err);
+        return nullptr;
+    }
+    const DeviceIndex &ix = idx->ix, &rv = rev_idx->ix;
+    if (needs_o_table(ix, err) || needs_o_table(rv, err)) return nullptr;
+    if (rv.len != ix.len || rv.sigma != ix.sigma || rv.device != ix.device ||
+        memcmp(rv.c_host, ix.c_host, (size_t)ix.sigma * 4) != 0) {
+        fail(B200SA_ERR_BAD_ARGUMENT, "the reverse index must be an O-table index of the reversed text on the same device",
+             err);
+        return nullptr;
+    }
+    if (ix.nrec || rv.nrec) {
+        fail(B200SA_ERR_BAD_ARGUMENT, "k-mismatch search does not take a records index", err);
+        return nullptr;
+    }
+    const uint32_t k = max_mismatches;
+    return new_handle<b200sa_hamming_result>(err, [&](b200sa_hamming_result *res) {
+        DeviceGuard guard(ix.device);
+        const cudaStream_t st = ix.stream;
+        res->off.assign(npat + 1, 0);
+        auto at = [&](uint64_t q) { return offsets ? offsets[q] : q * (uint64_t)fixed_len; };
+        std::vector<uint64_t> hoff;
+        for (uint64_t q0 = 0, q1; q0 < npat; q0 = q1) {
+            q1 = piece_end(offsets, fixed_len, npat, q0);
+            const uint64_t np = q1 - q0, b0 = at(q0), bytes = at(q1) - b0, base = res->L.size();
+            DevBuf<u8> dp(bytes + 16, st);
+            DevBuf<u64> doff, duo(np * (k + 1) + 1, st), dpo(np + 1, st);
+            if (bytes) CUDA_CHECK(cudaMemcpyAsync(dp.ptr, patterns + b0, bytes, cudaMemcpyHostToDevice, st));
+            if (offsets) {
+                hoff.resize(np + 1);
+                for (uint64_t q = q0; q <= q1; ++q) hoff[q - q0] = offsets[q] - b0;
+                doff.alloc(np + 1, st);
+                CUDA_CHECK(cudaMemcpyAsync(doff.ptr, hoff.data(), (np + 1) * 8, cudaMemcpyHostToDevice, st));
+            }
+            const u64 hits = hamming_count(ix, rv, dp.ptr, doff.ptr, fixed_len, np, max_m, k, duo.ptr, st);
+            if (hits > 0xFFFFFFFFull || np > 0xFFFFFFFFull)
+                return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 hits or patterns in one piece of the batch", err);
+            res->L.resize(base + hits);
+            res->R.resize(base + hits);
+            res->d.resize(base + hits);
+            DevBuf<u32> dL(hits ? hits : 1, st), dR(hits ? hits : 1, st), dd(hits ? hits : 1, st);
+            hamming_emit(ix, rv, dp.ptr, doff.ptr, fixed_len, np, max_m, k, duo.ptr, hits, dpo.ptr, dL.ptr, dR.ptr, dd.ptr, st);
+            CUDA_CHECK(cudaMemcpyAsync(res->off.data() + q0, dpo.ptr, (np + 1) * 8, cudaMemcpyDeviceToHost, st));
+            if (hits) {
+                CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dL.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dR.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaMemcpyAsync(res->d.data() + base, dd.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+            }
+            CUDA_CHECK(cudaStreamSynchronize(st));  // (`hoff` and the piece's buffers are reused or freed next)
+            for (uint64_t q = q0; q <= q1; ++q) res->off[q] += base;
+        }
+        return 0;
+    });
+}
+
+uint64_t b200sa_hamming_hits(const b200sa_hamming_result *r) { return r ? r->L.size() : 0; }
+const uint64_t *b200sa_hamming_offsets(const b200sa_hamming_result *r) { return r ? r->off.data() : nullptr; }
+const uint32_t *b200sa_hamming_L(const b200sa_hamming_result *r) { return r ? r->L.data() : nullptr; }
+const uint32_t *b200sa_hamming_R(const b200sa_hamming_result *r) { return r ? r->R.data() : nullptr; }
+const uint32_t *b200sa_hamming_mismatches(const b200sa_hamming_result *r) { return r ? r->d.data() : nullptr; }
+void b200sa_hamming_free(b200sa_hamming_result *r) { delete r; }
 
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device, void *stream) {
     if (!d_text || nsym < 1 || nsym > 255) return fail(B200SA_ERR_BAD_ARGUMENT, "bad argument", nullptr);

@@ -112,6 +112,9 @@ void fm_locate_fill_ssa(const DeviceIndex &ix, const u32 *d_L, u64 npat, const u
 void sa_lookup_rows(const DeviceIndex &ix, const u32 *d_rows, u64 count, u32 *d_out, bool force_sampled,
                     cudaStream_t st);
 void sort_positions(const DeviceIndex &ix, u64 npat, const u64 *d_pos_off, u64 total, u32 *d_pos, cudaStream_t st);
+// the stable radix sort of sort_positions on (keys[0], vals[0]), low key_bits bits; (keys[1], vals[1]) is the other
+// buffer pair, and the sorted pairs are left in the pair *_out points to
+void sort_pairs(u64 *keys[2], u32 *vals[2], u32 n, int key_bits, u64 *&keys_out, u32 *&vals_out, cudaStream_t st);
 // approx.cu
 void approx_dtable(const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len, u64 npat, u8 *d_dtab,
                    cudaStream_t st);
@@ -128,6 +131,14 @@ void mems_stats(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fi
 void mems_emit(const DeviceIndex &ix, const u64 *d_off, u32 fixed_len, u64 npat, u32 min_len, const u32 *d_ms,
                const u32 *d_L, const u32 *d_R, const u64 *d_smem_off, u32 *d_start, u32 *d_len, u32 *d_sL, u32 *d_sR,
                cudaStream_t st);
+// hamming.cu: k-mismatch search on ix (the text) and rev (the reversed text).  hamming_count: hits per (pattern,
+// search) unit, scanned in place into d_unit_off (npat * (k + 1) + 1 entries); returns the hits.  hamming_emit: the
+// CSR d_pat_off (npat + 1 entries) and the hits (L, R, d), every pattern's in ascending L.
+u64 hamming_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
+                  u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st);
+void hamming_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
+                  u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 hits, u64 *d_pat_off, u32 *d_L, u32 *d_R,
+                  u32 *d_d, cudaStream_t st);
 // records.cu
 void records_assemble(const u8 *d_codes, u64 ncodes, const u64 *d_rec_off, u32 nrec, u32 sigma, u8 *d_text,
                       int *d_err, cudaStream_t st);  // d_text: ncodes + nrec + 1 bytes

@@ -1,6 +1,7 @@
 // fm_step.cuh -- device pieces of the backward search recurrence that the exact search (fm_search.cu) and the
 // matching statistics (mems.cu) both run: the k-mer seed key, one O step of the DNA layout, and the comparison of
-// pattern symbols with the packed text that finishes a unique interval.
+// pattern symbols with the packed text that finishes a unique interval; and the bidirectional steps of the
+// k-mismatch search (hamming.cu).
 #pragma once
 #include "occ.cuh"
 
@@ -220,6 +221,50 @@ __device__ __forceinline__ u64 text_agree(Pat &&P, int64_t i, u32 s, const u64 *
         ++k;
     }
     return k;
+}
+
+// ---- bidirectional steps (hamming.cu) ------------------------------------------------------------------
+// A string X is held on two indices, F over the text T and B over reverse(T): [x, x + w) on the index a step runs
+// on, [y, y + w) on the other.  Extending X to the left (aX) is a step on F, extending it to the right (Xa) a step
+// on B; for both
+//   x_a = C[a] + O(a, x),   w_a = O(a, x + w) - O(a, x),   y_a = y + [x <= primary < x + w] + sum_{b < a} w_b
+// since on the other index the one-letter extensions of X sit side by side in letter order, after the one row that
+// ends in the sentinel when X starts the text (its row on the stepped index is `primary`).  Both indices have the
+// same C table.
+__device__ __forceinline__ u32 bidi_sentinel(const OccView &ov, u32 x, u32 w) { return ov.primary - x < w ? 1u : 0u; }
+
+struct BiChildren {
+    u32 x[4], w[4], y[4];  // the child of letter a at [a - 1]
+};
+
+// DNA layout: the children of all four letters from the one or two blocks that dna_step loads
+__device__ __forceinline__ BiChildren dna_bidi_children(const OccView &ov, const CTable5 &c5, u32 x, u32 w, u32 y) {
+    const u32 e = x + w;
+    const BlockRegs kL = load_dna_block(ov.blocks, x >> 6);
+    BlockRegs kR = kL;
+    if ((e >> 6) != (x >> 6)) kR = load_dna_block(ov.blocks, e >> 6);
+    BiChildren ch;
+    u32 run = y + bidi_sentinel(ov, x, w);
+#pragma unroll
+    for (u32 a = 1; a <= 4; ++a) {
+        const u32 lo = rank_in_block(kL, a, x, ov.primary), hi = rank_in_block(kR, a, e, ov.primary);
+        ch.x[a - 1] = c5.c[a] + lo;
+        ch.w[a - 1] = hi - lo;
+        ch.y[a - 1] = run;
+        run += hi - lo;
+    }
+    return ch;
+}
+
+// Byte layout, one letter at a time in ascending order: the child of letter a.  `run` is y_a on entry (start it at
+// y + bidi_sentinel) and y_{a+1} on return, so a walk over the letters costs two O lookups per letter.
+__device__ __forceinline__ void byte_bidi_child(const OccView &ov, const u32 *c, u32 a, u32 x, u32 w, u32 &run,
+                                                u32 &cx, u32 &cw, u32 &cy) {
+    const u32 lo = occ_byte(ov, a, x), hi = occ_byte(ov, a, x + w);
+    cx = c[a] + lo;
+    cw = hi - lo;
+    cy = run;
+    run += cw;
 }
 
 }  // namespace b200sa

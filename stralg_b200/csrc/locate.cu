@@ -232,4 +232,10 @@ void sort_positions(const DeviceIndex &ix, u64 npat, const u64 *d_pos_off, u64 t
     (void)ix;  // (the work buffers are released in stream order)
 }
 
+void sort_pairs(u64 *keys[2], u32 *vals[2], u32 n, int key_bits, u64 *&keys_out, u32 *&vals_out, cudaStream_t st) {
+    const auto sorted = rs::Sorter<8>::sort(keys, vals, n, key_bits, st);
+    keys_out = sorted.keys;
+    vals_out = sorted.vals;
+}
+
 }  // namespace b200sa

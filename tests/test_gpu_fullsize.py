@@ -55,6 +55,17 @@ def record(name, payload):
         pass
 
 
+def view(ptr, count, dtype):
+    """Zero-copy torch view of a device array owned by an index."""
+    import torch
+    itemsize = torch.empty(0, dtype=dtype).element_size()
+    iface = {"shape": (count,), "typestr": {1: "|u1", 4: "<i4"}[itemsize], "data": (ptr, False), "version": 2}
+
+    class Holder:
+        __cuda_array_interface__ = iface
+    return torch.as_tensor(Holder(), device=torch.device("cuda", 0))
+
+
 def test_fullsize_properties(engine):
     import torch
     lib = engine.load()
@@ -74,16 +85,6 @@ def test_fullsize_properties(engine):
         assert n == 3_000_000_000, n
     checks = []
     print(f"[fullsize] n = {n}, stats = {st}")
-
-    def view(ptr, count, dtype):
-        # zero-copy torch view of a device array owned by the index
-        itemsize = torch.empty(0, dtype=dtype).element_size()
-        iface = {"shape": (count,), "typestr": {1: "|u1", 4: "<i4"}[itemsize], "data": (ptr, False), "version": 2}
-
-        class Holder:
-            __cuda_array_interface__ = iface
-        return torch.as_tensor(Holder(), device=dev)
-
     sa = view(idx.device_ptr("sa"), length, torch.int32)
     bwt = view(idx.device_ptr("bwt"), length, torch.uint8)
 
@@ -341,3 +342,174 @@ def test_config2_sa_and_lcp_256M(engine):
         rec["checks"].append(f"SA and LCP memcmp-equal to the reference's sa_is_construction + compute_lcp ({dt:.0f} s on one host core)")
     record("test_config2_sa_and_lcp_256M", rec)
     idx.close()
+
+
+def test_fullsize_hamming_and_smems(engine):
+    """k-mismatch search and SMEMs on the 3 Gbp text, where SA intervals and positions pass 2^31.
+
+    The index pair of tools/hamming_probe.py: F with OCC (its suffix array kept), B of the flipped text with OCC and
+    DROP_SA.  The oracle of the k-mismatch hits is the exact search kernel, which test_fullsize_properties checks at
+    this size: every string at distance <= k from a read is enumerated on the device and searched, and the non-empty
+    intervals, sorted by L, are the read's complete hit list.  Independently of the exact search, the suffix array
+    shows that every hit's rows L and R - 1 hold a window at the hit's distance and that rows L - 1 and R hold
+    another string.  SMEMs: ms / L / R of every end of 2 000 reads with edits, by their characterisation through the
+    exact search, on plain OCC and on the search build of bench.py (TEXTCMP + KTABLE); the SMEM list is the one the
+    rule derives from ms."""
+    import itertools
+
+    import torch
+    from test_gpu_mems_scale import smems_from_ms, substrings
+    lib = engine.load()
+    n = pick_n(torch)
+    dev = torch.device("cuda", 0)
+    strm = torch.cuda.current_stream().cuda_stream
+    text = torch.empty(n + 1, dtype=torch.uint8, device=dev)
+    assert lib.b200sa_synth_codes(C.c_void_p(text.data_ptr()), n, 4, 424242, 0, None) == 0
+    torch.cuda.synchronize()
+    fwd = engine.SuffixArrayIndex.build(text[:n], 5)
+    rtext = torch.flip(text[:n], dims=[0]).contiguous()
+    rev = engine.SuffixArrayIndex.build(rtext, 5, drop_sa=True)
+    del rtext
+    lib.b200sa_release_workspace(0)
+    length = n + 1
+    sa = view(fwd.device_ptr("sa"), length, torch.int32)
+    checks = []
+
+    def search(idx, flat, offsets, m, count):
+        """(L, R) as int64 of `count` patterns through the exact search kernel."""
+        dL = torch.empty(count, dtype=torch.int32, device=dev)
+        dR = torch.empty(count, dtype=torch.int32, device=dev)
+        idx.search_device(flat, offsets, m, count, dL, dR, strm)
+        torch.cuda.synchronize()
+        return dL.long() & 0xFFFFFFFF, dR.long() & 0xFFFFFFFF
+
+    def window(rows, m):
+        pos = sa[rows].long() & 0xFFFFFFFF
+        return text[torch.clamp(pos[:, None] + torch.arange(m, device=dev)[None, :], max=n)], pos
+
+    def draw(nreads, m, seed):
+        """Reads of the text (10 % random), one substitution in every third."""
+        reads = torch.empty(nreads * m + 16, dtype=torch.uint8, device=dev)
+        assert lib.b200sa_synth_reads(C.c_void_p(text.data_ptr()), n, 4, C.c_void_p(reads.data_ptr()), nreads, m,
+                                      102, seed, 0, None) == 0
+        rd = reads[:nreads * m].view(nreads, m)
+        g = torch.Generator(device=dev).manual_seed(seed)
+        rows = torch.arange(0, nreads, 3, device=dev)
+        cols = torch.randint(0, m, (len(rows),), device=dev, generator=g)
+        shift = torch.randint(1, 4, (len(rows),), device=dev, generator=g).to(torch.uint8)
+        rd[rows, cols] = (rd[rows, cols] - 1 + shift) % 4 + 1
+        torch.cuda.synchronize()
+        return rd
+
+    def neighbours_hits(rd, k):
+        """(read, L, R, d) of every string at distance <= k from each read that occurs, sorted by (read, L)."""
+        nreads, m = rd.shape
+        out = []
+        for d in range(k + 1):
+            at = list(itertools.combinations(range(m), d))
+            to = list(itertools.product((1, 2, 3), repeat=d))
+            cols = torch.tensor(at, dtype=torch.long, device=dev).reshape(len(at), d)
+            shifts = torch.tensor(to, dtype=torch.uint8, device=dev).reshape(len(to), d)
+            cols = cols.repeat_interleave(len(shifts), 0)
+            shifts = shifts.repeat(len(cols) // len(shifts), 1)
+            nv = len(cols)
+            ar = torch.arange(nv, device=dev)
+            per = max(1, (1 << 26) // (nv * m))
+            for r0 in range(0, nreads, per):
+                blk = rd[r0:r0 + per]
+                var = blk[:, None, :].repeat(1, nv, 1)
+                for i in range(d):
+                    var[:, ar, cols[:, i]] = (var[:, ar, cols[:, i]] - 1 + shifts[:, i]) % 4 + 1
+                flat = torch.cat([var.reshape(-1), torch.zeros(16, dtype=torch.uint8, device=dev)])
+                L, R = search(fwd, flat, None, m, len(blk) * nv)
+                found = (R > L).nonzero()[:, 0]
+                read = found // nv + r0
+                out.append(torch.stack([read, L[found], R[found], torch.full_like(read, d)], 1))
+        hits = torch.cat(out)
+        order = torch.argsort(hits[:, 0] * (1 << 33) + hits[:, 1])
+        return hits[order]
+
+    hi_L = hi_pos = 0
+    for nreads, m, k, seed in ((5000, 100, 1, 31), (200, 100, 2, 32), (200, 12, 3, 33)):
+        rd = draw(nreads, m, seed)
+        res = fwd.hamming_search(rd.cpu().numpy().reshape(-1), fixed_len=m, max_mismatches=k, rev=rev)
+        want = neighbours_hits(rd, k)
+        counts = torch.bincount(want[:, 0], minlength=nreads).cpu().numpy()
+        assert res["offsets"].tolist() == [0] + np.cumsum(counts).tolist(), (m, k)
+        for col, name in ((1, "L"), (2, "R"), (3, "mismatches")):
+            assert np.array_equal(res[name].astype(np.int64), want[:, col].cpu().numpy()), (m, k, name)
+        # the suffix array alone: both border rows hold a window at distance d, the rows outside hold another string
+        L, R, d, q = want[:, 1], want[:, 2], want[:, 3], want[:, 0]
+        wl, pl = window(L, m)
+        wr, _ = window(R - 1, m)
+        assert bool(((wl != rd[q]).sum(1) == d).all()) and bool(((wr != rd[q]).sum(1) == d).all())
+        inner = L > 0
+        assert bool((window(L[inner] - 1, m)[0] != wl[inner]).any(1).all())
+        inner = R < length
+        assert bool((window(R[inner], m)[0] != wr[inner]).any(1).all())
+        hi_L += int((L >= 1 << 31).sum())
+        hi_pos += int((pl >= 1 << 31).sum())
+        checks.append(f"k = {k}, {nreads} reads of {m}: {len(want)} hits (widest interval {int((R - L).max())}) equal "
+                      f"the exact search of every string within distance {k}; border rows checked through SA")
+        del want, wl, wr, L, R, d, q
+    if n >= 3_000_000_000:
+        assert hi_L > 0 and hi_pos > 0, (hi_L, hi_pos)
+    checks.append(f"{hi_L} hits with L >= 2^31, {hi_pos} with a position >= 2^31")
+    rev.close()
+
+    # ---- SMEMs: 2 000 reads of 150 bp with substitutions, insertions and deletions ----
+    rng = np.random.default_rng(34)
+    nreads = 2000
+    starts = torch.from_numpy(rng.integers(0, n - 160, nreads)).to(dev)
+    win = text[starts[:, None] + torch.arange(160, device=dev)[None, :]].cpu().numpy()
+    pats = []
+    for q in range(nreads):
+        p = win[q, :150].tolist() if q % 10 else rng.integers(1, 5, 150).tolist()
+        for _ in range(int(rng.integers(0, 4))):
+            op, at, x = int(rng.integers(0, 3)), int(rng.integers(0, len(p))), int(rng.integers(1, 5))
+            if op == 0:
+                p[at] = x
+            elif op == 1:
+                p.insert(at, x)
+            else:
+                del p[at]
+        pats.append(p)
+    off = np.concatenate([[0], np.cumsum([len(p) for p in pats])]).astype(np.uint64)
+    pat = np.array([x for p in pats for x in p], np.uint8)
+    g = np.arange(int(off[-1]))
+    j = g - np.repeat(off[:-1].astype(np.int64), np.diff(off).astype(np.int64))
+
+    def characterised(idx, st):
+        """Every end: P[j - ms + 1 .. j] has exactly (L, R) and occurs, P[j - ms .. j] does not occur."""
+        ms, L, R = (st[x].astype(np.int64) for x in ("ms", "L", "R"))
+        zero = ms == 0
+        assert (L[zero] == 1).all() and (R[zero] == 0).all()
+        for sel, extra in ((~zero, 0), (ms <= j, 1)):
+            cat, so = substrings(pat, g[sel] - ms[sel] + 1 - extra, ms[sel] + extra)
+            flat = torch.from_numpy(np.concatenate([cat, np.zeros(16, np.uint8)])).to(dev)
+            Ls, Rs = search(idx, flat, torch.from_numpy(so.astype(np.int64)).to(dev), 0, len(so) - 1)
+            Ls, Rs = Ls.cpu().numpy(), Rs.cpu().numpy()
+            if extra:
+                assert (Ls >= Rs).all()
+            else:
+                assert np.array_equal(Ls, L[sel]) and np.array_equal(Rs, R[sel]) and (Ls < Rs).all()
+
+    results = []
+    for name in ("occ", "textcmp_ktable"):
+        if name == "textcmp_ktable":
+            fwd.close()
+            fwd = engine.SuffixArrayIndex.build(text[:n], 5, isa=False, bwt=True, occ=True, textcmp=True, ktable=True)
+            lib.b200sa_release_workspace(0)
+        st = fwd.matching_stats(pat, off)
+        characterised(fwd, st)
+        for min_len in (1, 19):
+            res = fwd.smems(pat, off, min_len=min_len)
+            want = smems_from_ms(off, st["ms"], st["L"], st["R"], min_len)
+            for col, w in zip(("offsets", "start", "length", "L", "R"), want):
+                assert np.array_equal(res[col].astype(np.int64), w), (name, min_len, col)
+        results.append(st)
+        checks.append(f"SMEMs ({name}): ms / L / R of all {len(pat)} ends of {nreads} reads with edits by their "
+                      f"characterisation; SMEM lists (min_len 1, 19) as derived from ms")
+    assert all(np.array_equal(results[0][x], results[1][x]) for x in ("ms", "L", "R"))
+    record("test_fullsize_hamming_and_smems", {"n": n, "checks": checks})
+    fwd.close()

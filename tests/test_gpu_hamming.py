@@ -7,28 +7,12 @@ import ctypes as C
 
 import numpy as np
 import pytest
-from numpy.lib.stride_tricks import sliding_window_view
+
+from _hamming_oracle import oracle_hits
 
 pytestmark = pytest.mark.gpu
 
 BAD_ARGUMENT, NOT_BUILT = 2, 5
-
-
-def oracle_hits(codes, isa, p, k):
-    """[(L, R, d)] of pattern p with at most k mismatches; codes holds the text and its trailing 0."""
-    n, m = len(codes) - 1, len(p)
-    if m == 0 or m > n:
-        return []
-    win = sliding_window_view(codes[:n], m)
-    dist = (win != np.asarray(p, np.uint8)).sum(axis=1)
-    sel = np.nonzero(dist <= k)[0]
-    if not len(sel):
-        return []
-    _, first, inv, cnt = np.unique(win[sel], axis=0, return_index=True, return_inverse=True, return_counts=True)
-    L = np.full(len(cnt), np.iinfo(np.int64).max, np.int64)
-    np.minimum.at(L, inv.reshape(-1), isa[sel].astype(np.int64))
-    d = dist[sel][first]
-    return sorted(zip(L.tolist(), (L + cnt).tolist(), d.tolist()))
 
 
 def _offsets(pats):

@@ -393,6 +393,43 @@ const uint32_t *b200sa_hamming_R(const b200sa_hamming_result *r);
 const uint32_t *b200sa_hamming_mismatches(const b200sa_hamming_result *r);
 void b200sa_hamming_free(b200sa_hamming_result *r);
 
+/* ---- batched edit-distance search on a bidirectional FM index -------------------------------
+ * Every distinct text string within Levenshtein distance k of a read, each reported once: for primers
+ * and guides with bulges, barcodes with synthesis indels and short reads from indel-prone platforms.
+ * (b200sa_approx_batch reports every edit path in the reference's order; b200sa_hamming_batch takes
+ * substitutions only.)  Patterns take the form of b200sa_search_batch.  For a pattern P of length
+ * m >= 1 and k = max_edits, the hits are every distinct string Q with
+ *   Q non-empty,  Q over the letters 1..sigma-1,  Q occurs in the text,  ED(P, Q) <= k,
+ * where ED is the Levenshtein distance with unit cost for substitution, insertion and deletion; so
+ * m - k <= |Q| <= m + k.  Each hit is (L, R, length, d): [L, R) is Q's SA interval in `idx` (what
+ * b200sa_search_batch returns for Q), length = |Q| and d = ED(P, Q).  Hits of one pattern come in
+ * ascending L, then ascending length: distinct strings of one length have disjoint intervals, so
+ * (L, length) identifies Q and the order does not depend on how the search runs.  A pattern symbol 0
+ * or >= sigma matches no letter (substituting or deleting it costs 1); it is not an error.  An empty
+ * pattern has no hits; k = 0 gives exactly the non-empty results of b200sa_search_batch, with
+ * length = m and d = 0.
+ * The set holds near-duplicates of every occurrence by design: an exact occurrence of P at position p
+ * also yields T[p+a .. p+m+b) for |a| + |b| <= k, up to 2k^2 + 2k + 1 hits (13 at k = 2).  Callers
+ * locate the hits (b200sa_locate_batch / _sorted over (L, R)) and choose among them.
+ * `rev_idx` and the refusals are those of b200sa_hamming_batch, all before any CUDA call, with
+ * max_edits > 4 -> B200SA_ERR_BAD_ARGUMENT.  TEXTCMP and KTABLE do not change the results.  Long
+ * batches are staged in pieces of about 64 MB of pattern symbols and at most 2^28 patterns; a piece
+ * with more than 2^32 - 1 raw hits (before the near-identical hits of several searches are merged)
+ * -> B200SA_ERR_TOO_LARGE.  Accessors return host arrays owned by the result (valid until
+ * b200sa_levenshtein_free). */
+typedef struct b200sa_levenshtein_result b200sa_levenshtein_result;
+b200sa_levenshtein_result *b200sa_levenshtein_batch(const b200sa_index *idx, const b200sa_index *rev_idx,
+                                                    const uint8_t *patterns, const uint64_t *offsets,
+                                                    uint32_t fixed_len, uint64_t npat, uint32_t max_edits,
+                                                    enum b200sa_error *err);
+uint64_t b200sa_levenshtein_hits(const b200sa_levenshtein_result *r);           /* hits in total  */
+const uint64_t *b200sa_levenshtein_offsets(const b200sa_levenshtein_result *r); /* npat + 1 (CSR) */
+const uint32_t *b200sa_levenshtein_L(const b200sa_levenshtein_result *r);
+const uint32_t *b200sa_levenshtein_R(const b200sa_levenshtein_result *r);
+const uint32_t *b200sa_levenshtein_length(const b200sa_levenshtein_result *r);
+const uint32_t *b200sa_levenshtein_distance(const b200sa_levenshtein_result *r);
+void b200sa_levenshtein_free(b200sa_levenshtein_result *r);
+
 /* ---- synthetic inputs on the device (bench / tests; mirrors performance/suffix_array_search.c:13-32)
  * d_text must hold n + 1 bytes; symbols are 1 + hash(seed + i) % nsym, d_text[n] = 0. */
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device,

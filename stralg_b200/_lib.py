@@ -134,6 +134,15 @@ SIGNATURES = {
     "b200sa_hamming_R": (u32p, [C.c_void_p]),
     "b200sa_hamming_mismatches": (u32p, [C.c_void_p]),
     "b200sa_hamming_free": (None, [C.c_void_p]),
+    "b200sa_levenshtein_batch": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                              C.c_uint64, C.c_uint32, C.POINTER(C.c_int)]),
+    "b200sa_levenshtein_hits": (C.c_uint64, [C.c_void_p]),
+    "b200sa_levenshtein_offsets": (u64p, [C.c_void_p]),
+    "b200sa_levenshtein_L": (u32p, [C.c_void_p]),
+    "b200sa_levenshtein_R": (u32p, [C.c_void_p]),
+    "b200sa_levenshtein_length": (u32p, [C.c_void_p]),
+    "b200sa_levenshtein_distance": (u32p, [C.c_void_p]),
+    "b200sa_levenshtein_free": (None, [C.c_void_p]),
     "b200sa_synth_codes":(C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, C.c_int, C.c_void_p]),
     "b200sa_synth_reads": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64, C.c_uint32,
                                      C.c_uint32, C.c_uint64, C.c_int, C.c_void_p]),

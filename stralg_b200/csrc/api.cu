@@ -1948,10 +1948,76 @@ void b200sa_smem_free(b200sa_smem_result *r) { delete r; }
 }  // extern "C"
 #pragma GCC visibility pop
 
-// ---- k-mismatch search ------------------------------------------------------------------------------
+// ---- k-mismatch and edit-distance search on an index pair --------------------------------------------
+// the refusals of b200sa_hamming_batch and b200sa_levenshtein_batch that come before any CUDA call; max_m gets the
+// longest pattern
+static int pair_args_ok(const b200sa_index *idx, const b200sa_index *rev_idx, const uint8_t *patterns,
+                        const uint64_t *offsets, uint32_t fixed_len, uint64_t npat, uint32_t k, uint32_t max_k,
+                        const char *what, const char *k_name, uint32_t &max_m, enum b200sa_error *err) {
+    if (!idx || !rev_idx || (npat && !patterns) || k > max_k)
+        return fail(B200SA_ERR_BAD_ARGUMENT,
+                    std::string("null argument or ") + k_name + " above " + std::to_string(max_k), err);
+    max_m = fixed_len;
+    if (offsets) {
+        max_m = 0;
+        for (uint64_t q = 0; q < npat; ++q) {
+            if (offsets[q + 1] < offsets[q]) return fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
+            max_m = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(max_m, offsets[q + 1] - offsets[q]), 0xFFFFFFFFull);
+        }
+    }
+    if (max_m > 65000u) return fail(B200SA_ERR_TOO_LARGE, std::string(what) + " search takes patterns of up to 65000 symbols", err);
+    const DeviceIndex &ix = idx->ix, &rv = rev_idx->ix;
+    if (int rc = needs_o_table(ix, err)) return rc;
+    if (int rc = needs_o_table(rv, err)) return rc;
+    if (rv.len != ix.len || rv.sigma != ix.sigma || rv.device != ix.device ||
+        memcmp(rv.c_host, ix.c_host, (size_t)ix.sigma * 4) != 0)
+        return fail(B200SA_ERR_BAD_ARGUMENT,
+                    "the reverse index must be an O-table index of the reversed text on the same device", err);
+    if (ix.nrec || rv.nrec)
+        return fail(B200SA_ERR_BAD_ARGUMENT, std::string(what) + " search does not take a records index", err);
+    return 0;
+}
+
+// A host batch searched on an index pair, in pieces (piece_end, and at most max_np patterns each): a piece's
+// patterns are copied in and its offsets rebased to the piece; `piece(np, d_pat, d_off, d_pat_off, base)` runs the
+// search of its np patterns, copies its hits back after the `base` hits of the earlier pieces and leaves the CSR of
+// its hits in d_pat_off (np + 1 entries), or returns an error code; res_off (npat + 1) gets the CSR of the batch.
+template <class Piece>
+static int pair_pieces(const DeviceIndex &ix, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
+                       uint64_t npat, uint64_t max_np, std::vector<uint64_t> &res_off, Piece &&piece) {
+    const cudaStream_t st = ix.stream;
+    res_off.assign(npat + 1, 0);
+    auto at = [&](uint64_t q) { return offsets ? offsets[q] : q * (uint64_t)fixed_len; };
+    std::vector<uint64_t> hoff;
+    for (uint64_t q0 = 0, q1; q0 < npat; q0 = q1) {
+        q1 = std::min(piece_end(offsets, fixed_len, npat, q0), q0 + max_np);
+        const uint64_t np = q1 - q0, b0 = at(q0), bytes = at(q1) - b0;
+        DevBuf<u8> dp(bytes + 16, st);
+        DevBuf<u64> doff, dpo(np + 1, st);
+        if (bytes) CUDA_CHECK(cudaMemcpyAsync(dp.ptr, patterns + b0, bytes, cudaMemcpyHostToDevice, st));
+        if (offsets) {
+            hoff.resize(np + 1);
+            for (uint64_t q = q0; q <= q1; ++q) hoff[q - q0] = offsets[q] - b0;
+            doff.alloc(np + 1, st);
+            CUDA_CHECK(cudaMemcpyAsync(doff.ptr, hoff.data(), (np + 1) * 8, cudaMemcpyHostToDevice, st));
+        }
+        uint64_t base = 0;
+        if (int rc = piece(np, dp.ptr, doff.ptr, dpo.ptr, base)) return rc;
+        CUDA_CHECK(cudaMemcpyAsync(res_off.data() + q0, dpo.ptr, (np + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));  // (`hoff` and the piece's buffers are reused or freed next)
+        for (uint64_t q = q0; q <= q1; ++q) res_off[q] += base;
+    }
+    return 0;
+}
+
 struct b200sa_hamming_result {
     std::vector<uint64_t> off;  // npat + 1
     std::vector<uint32_t> L, R, d;
+};
+
+struct b200sa_levenshtein_result {
+    std::vector<uint64_t> off;  // npat + 1
+    std::vector<uint32_t> L, R, length, d;
 };
 
 #pragma GCC visibility push(default)
@@ -1960,74 +2026,34 @@ extern "C" {
 b200sa_hamming_result *b200sa_hamming_batch(const b200sa_index *idx, const b200sa_index *rev_idx,
                                             const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
                                             uint64_t npat, uint32_t max_mismatches, enum b200sa_error *err) {
-    if (!idx || !rev_idx || (npat && !patterns) || max_mismatches > 8) {
-        fail(B200SA_ERR_BAD_ARGUMENT, "null argument or max_mismatches above 8", err);
+    uint32_t max_m = 0;
+    if (pair_args_ok(idx, rev_idx, patterns, offsets, fixed_len, npat, max_mismatches, 8, "k-mismatch", "max_mismatches",
+                     max_m, err))
         return nullptr;
-    }
-    uint32_t max_m = fixed_len;
-    if (offsets) {
-        max_m = 0;
-        for (uint64_t q = 0; q < npat; ++q) {
-            if (offsets[q + 1] < offsets[q]) {
-                fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
-                return nullptr;
-            }
-            max_m = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(max_m, offsets[q + 1] - offsets[q]), 0xFFFFFFFFull);
-        }
-    }
-    if (max_m > 65000u) {
-        fail(B200SA_ERR_TOO_LARGE, "k-mismatch search takes patterns of up to 65000 symbols", err);
-        return nullptr;
-    }
     const DeviceIndex &ix = idx->ix, &rv = rev_idx->ix;
-    if (needs_o_table(ix, err) || needs_o_table(rv, err)) return nullptr;
-    if (rv.len != ix.len || rv.sigma != ix.sigma || rv.device != ix.device ||
-        memcmp(rv.c_host, ix.c_host, (size_t)ix.sigma * 4) != 0) {
-        fail(B200SA_ERR_BAD_ARGUMENT, "the reverse index must be an O-table index of the reversed text on the same device",
-             err);
-        return nullptr;
-    }
-    if (ix.nrec || rv.nrec) {
-        fail(B200SA_ERR_BAD_ARGUMENT, "k-mismatch search does not take a records index", err);
-        return nullptr;
-    }
     const uint32_t k = max_mismatches;
     return new_handle<b200sa_hamming_result>(err, [&](b200sa_hamming_result *res) {
         DeviceGuard guard(ix.device);
         const cudaStream_t st = ix.stream;
-        res->off.assign(npat + 1, 0);
-        auto at = [&](uint64_t q) { return offsets ? offsets[q] : q * (uint64_t)fixed_len; };
-        std::vector<uint64_t> hoff;
-        for (uint64_t q0 = 0, q1; q0 < npat; q0 = q1) {
-            q1 = piece_end(offsets, fixed_len, npat, q0);
-            const uint64_t np = q1 - q0, b0 = at(q0), bytes = at(q1) - b0, base = res->L.size();
-            DevBuf<u8> dp(bytes + 16, st);
-            DevBuf<u64> doff, duo(np * (k + 1) + 1, st), dpo(np + 1, st);
-            if (bytes) CUDA_CHECK(cudaMemcpyAsync(dp.ptr, patterns + b0, bytes, cudaMemcpyHostToDevice, st));
-            if (offsets) {
-                hoff.resize(np + 1);
-                for (uint64_t q = q0; q <= q1; ++q) hoff[q - q0] = offsets[q] - b0;
-                doff.alloc(np + 1, st);
-                CUDA_CHECK(cudaMemcpyAsync(doff.ptr, hoff.data(), (np + 1) * 8, cudaMemcpyHostToDevice, st));
-            }
-            const u64 hits = hamming_count(ix, rv, dp.ptr, doff.ptr, fixed_len, np, max_m, k, duo.ptr, st);
+        return pair_pieces(ix, patterns, offsets, fixed_len, npat, npat, res->off,
+                           [&](uint64_t np, const u8 *dp, const u64 *doff, u64 *dpo, uint64_t &base) {
+            base = res->L.size();
+            DevBuf<u64> duo(np * (k + 1) + 1, st);
+            const u64 hits = hamming_count(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, st);
             if (hits > 0xFFFFFFFFull || np > 0xFFFFFFFFull)
                 return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 hits or patterns in one piece of the batch", err);
             res->L.resize(base + hits);
             res->R.resize(base + hits);
             res->d.resize(base + hits);
             DevBuf<u32> dL(hits ? hits : 1, st), dR(hits ? hits : 1, st), dd(hits ? hits : 1, st);
-            hamming_emit(ix, rv, dp.ptr, doff.ptr, fixed_len, np, max_m, k, duo.ptr, hits, dpo.ptr, dL.ptr, dR.ptr, dd.ptr, st);
-            CUDA_CHECK(cudaMemcpyAsync(res->off.data() + q0, dpo.ptr, (np + 1) * 8, cudaMemcpyDeviceToHost, st));
+            hamming_emit(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, hits, dpo, dL.ptr, dR.ptr, dd.ptr, st);
             if (hits) {
                 CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dL.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
                 CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dR.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
                 CUDA_CHECK(cudaMemcpyAsync(res->d.data() + base, dd.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
             }
-            CUDA_CHECK(cudaStreamSynchronize(st));  // (`hoff` and the piece's buffers are reused or freed next)
-            for (uint64_t q = q0; q <= q1; ++q) res->off[q] += base;
-        }
-        return 0;
+            return 0;
+        });
     });
 }
 
@@ -2037,6 +2063,54 @@ const uint32_t *b200sa_hamming_L(const b200sa_hamming_result *r) { return r ? r-
 const uint32_t *b200sa_hamming_R(const b200sa_hamming_result *r) { return r ? r->R.data() : nullptr; }
 const uint32_t *b200sa_hamming_mismatches(const b200sa_hamming_result *r) { return r ? r->d.data() : nullptr; }
 void b200sa_hamming_free(b200sa_hamming_result *r) { delete r; }
+
+b200sa_levenshtein_result *b200sa_levenshtein_batch(const b200sa_index *idx, const b200sa_index *rev_idx,
+                                                    const uint8_t *patterns, const uint64_t *offsets,
+                                                    uint32_t fixed_len, uint64_t npat, uint32_t max_edits,
+                                                    enum b200sa_error *err) {
+    uint32_t max_m = 0;
+    if (pair_args_ok(idx, rev_idx, patterns, offsets, fixed_len, npat, max_edits, 4, "edit-distance", "max_edits", max_m,
+                     err))
+        return nullptr;
+    const DeviceIndex &ix = idx->ix, &rv = rev_idx->ix;
+    const uint32_t k = max_edits;
+    return new_handle<b200sa_levenshtein_result>(err, [&](b200sa_levenshtein_result *res) {
+        DeviceGuard guard(ix.device);
+        const cudaStream_t st = ix.stream;
+        // a raw hit's sort key is [pattern | L | length - (m - k)]: 64 - 32 - 4 bits for the pattern
+        return pair_pieces(ix, patterns, offsets, fixed_len, npat, (uint64_t)1 << 28, res->off,
+                           [&](uint64_t np, const u8 *dp, const u64 *doff, u64 *dpo, uint64_t &base) {
+            base = res->L.size();
+            DevBuf<u64> duo(np * (k + 1) + 1, st);
+            const u64 raw = levenshtein_count(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, st);
+            if (raw > 0xFFFFFFFFull)
+                return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 raw hits in one piece of the batch", err);
+            DevBuf<u32> dL(raw ? raw : 1, st), dR(raw ? raw : 1, st), dn(raw ? raw : 1, st), dd(raw ? raw : 1, st);
+            const u64 hits =
+                levenshtein_emit(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, raw, dpo, dL.ptr, dR.ptr, dn.ptr,
+                                 dd.ptr, st);
+            res->L.resize(base + hits);
+            res->R.resize(base + hits);
+            res->length.resize(base + hits);
+            res->d.resize(base + hits);
+            if (hits) {
+                CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dL.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dR.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaMemcpyAsync(res->length.data() + base, dn.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+                CUDA_CHECK(cudaMemcpyAsync(res->d.data() + base, dd.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
+            }
+            return 0;
+        });
+    });
+}
+
+uint64_t b200sa_levenshtein_hits(const b200sa_levenshtein_result *r) { return r ? r->L.size() : 0; }
+const uint64_t *b200sa_levenshtein_offsets(const b200sa_levenshtein_result *r) { return r ? r->off.data() : nullptr; }
+const uint32_t *b200sa_levenshtein_L(const b200sa_levenshtein_result *r) { return r ? r->L.data() : nullptr; }
+const uint32_t *b200sa_levenshtein_R(const b200sa_levenshtein_result *r) { return r ? r->R.data() : nullptr; }
+const uint32_t *b200sa_levenshtein_length(const b200sa_levenshtein_result *r) { return r ? r->length.data() : nullptr; }
+const uint32_t *b200sa_levenshtein_distance(const b200sa_levenshtein_result *r) { return r ? r->d.data() : nullptr; }
+void b200sa_levenshtein_free(b200sa_levenshtein_result *r) { delete r; }
 
 int b200sa_synth_codes(uint8_t *d_text, uint64_t n, uint32_t nsym, uint64_t seed, int device, void *stream) {
     if (!d_text || nsym < 1 || nsym > 255) return fail(B200SA_ERR_BAD_ARGUMENT, "bad argument", nullptr);

@@ -139,6 +139,15 @@ u64 hamming_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat
 void hamming_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
                   u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 hits, u64 *d_pat_off, u32 *d_L, u32 *d_R,
                   u32 *d_d, cudaStream_t st);
+// levenshtein.cu: edit-distance search on ix (the text) and rev (the reversed text).  levenshtein_count: raw hits per
+// (pattern, search) unit, scanned in place into d_unit_off (npat * (k + 1) + 1 entries); returns the raw hits.
+// levenshtein_emit: the CSR d_pat_off (npat + 1 entries) and the merged hits (L, R, length, d), every pattern's in
+// ascending (L, length), into buffers of raw_hits entries; returns the merged hits.
+u64 levenshtein_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
+                      u32 fixed_len, u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st);
+u64 levenshtein_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
+                     u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 raw_hits, u64 *d_pat_off, u32 *d_L,
+                     u32 *d_R, u32 *d_len, u32 *d_d, cudaStream_t st);
 // records.cu
 void records_assemble(const u8 *d_codes, u64 ncodes, const u64 *d_rec_off, u32 nrec, u32 sigma, u8 *d_text,
                       int *d_err, cudaStream_t st);  // d_text: ncodes + nrec + 1 bytes

@@ -1,7 +1,7 @@
 // fm_step.cuh -- device pieces of the backward search recurrence that the exact search (fm_search.cu) and the
 // matching statistics (mems.cu) both run: the k-mer seed key, one O step of the DNA layout, and the comparison of
-// pattern symbols with the packed text that finishes a unique interval; and the bidirectional steps of the
-// k-mismatch search (hamming.cu).
+// pattern symbols with the packed text that finishes a unique interval; and the bidirectional steps and the pattern
+// split of the k-mismatch and edit-distance searches (hamming.cu, levenshtein.cu).
 #pragma once
 #include "occ.cuh"
 
@@ -223,7 +223,7 @@ __device__ __forceinline__ u64 text_agree(Pat &&P, int64_t i, u32 s, const u64 *
     return k;
 }
 
-// ---- bidirectional steps (hamming.cu) ------------------------------------------------------------------
+// ---- bidirectional steps (hamming.cu, levenshtein.cu) -------------------------------------------------
 // A string X is held on two indices, F over the text T and B over reverse(T): [x, x + w) on the index a step runs
 // on, [y, y + w) on the other.  Extending X to the left (aX) is a step on F, extending it to the right (Xa) a step
 // on B; for both
@@ -265,6 +265,30 @@ __device__ __forceinline__ void byte_bidi_child(const OccView &ov, const u32 *c,
     cw = hi - lo;
     cy = run;
     run += cw;
+}
+
+// The index a step runs on: B (the reversed text) for a right extension, F (the text) for a left one.  The two
+// indices share everything but their blocks and sentinel row.
+__device__ __forceinline__ OccView step_index(const OccView &fv, const OccView &bv, bool right) {
+    OccView ov = fv;
+    if (right) {
+        ov.blocks = bv.blocks;
+        ov.primary = bv.primary;
+    }
+    return ov;
+}
+
+// The k + 1 parts of a search scheme: a pattern of m = (k + 1) qs + r symbols splits into parts of qs + 1 symbols
+// (the r first) and of qs; part_start is the first position of part j, part_of the part of position pos.
+__device__ __forceinline__ u32 part_start(u32 j, u32 qs, u32 r) { return j * qs + min(j, r); }
+__device__ __forceinline__ u32 part_of(u32 pos, u32 qs, u32 r) {
+    const u32 big = r * (qs + 1);
+    return pos < big ? pos / (qs + 1) : r + (pos - big) / qs;
+}
+
+// v[a - 1] for a letter a in 1..4
+__device__ __forceinline__ u32 pick4(const u32 (&v)[4], u32 a) {
+    return a == 1 ? v[0] : a == 2 ? v[1] : a == 3 ? v[2] : v[3];
 }
 
 }  // namespace b200sa

@@ -50,17 +50,6 @@ struct HammingArgs {
     u32 *val, *R, *d;      // per hit: its index, R and its distance
 };
 
-// first position of part j of a pattern of m = (k + 1) qs + r symbols (the r longer parts first), and the part of pos
-__device__ __forceinline__ u32 part_start(u32 j, u32 qs, u32 r) { return j * qs + min(j, r); }
-__device__ __forceinline__ u32 part_of(u32 pos, u32 qs, u32 r) {
-    const u32 big = r * (qs + 1);
-    return pos < big ? pos / (qs + 1) : r + (pos - big) / qs;
-}
-
-__device__ __forceinline__ u32 pick4(const u32 (&v)[4], u32 a) {
-    return a == 1 ? v[0] : a == 2 ? v[1] : a == 3 ? v[2] : v[3];
-}
-
 // frame: x = x, y = y, z = w, w = step | mismatches << 16 | part flag << 20 | next letter << 21
 template <int LAYOUT, bool EMIT>
 __global__ void __launch_bounds__(256) hamming_walk_kernel(HammingArgs A) {
@@ -91,14 +80,7 @@ __global__ void __launch_bounds__(256) hamming_walk_kernel(HammingArgs A) {
         }
         ++nh;
     };
-    auto index_of = [&](bool right) {
-        OccView ov = A.fv;
-        if (right) {
-            ov.blocks = A.bv.blocks;
-            ov.primary = A.bv.primary;
-        }
-        return ov;
-    };
+    auto index_of = [&](bool right) { return step_index(A.fv, A.bv, right); };
     if (m && i <= m && nsym) {
         const u32 qs = m / (k + 1), r = m % (k + 1);
         const u32 st = part_start(i, qs, r), size_i = part_start(i + 1, qs, r) - st;

@@ -429,6 +429,33 @@ class SuffixArrayIndex:
             lib.b200sa_hamming_free(r)
         return {"offsets": hoff, **cols}
 
+    # ---- edit-distance search (include/b200sa.h: b200sa_levenshtein_batch) -------------------------
+    def levenshtein_search(self, patterns, offsets=None, fixed_len: int = 0, max_edits: int = 1,
+                           rev: "Optional[SuffixArrayIndex]" = None) -> dict:
+        """Every distinct non-empty text string within Levenshtein distance ``max_edits`` (<= 4) of each pattern,
+        once, per pattern in ascending (L, length).  ``rev``: the index of the reversed text (required).
+        Returns dict(offsets[npat+1], L, R, length, edits)."""
+        if rev is None:
+            raise ValueError("levenshtein_search needs rev, an O-table index of the reversed text")
+        lib = _lib.load()
+        pat, _, npat, offp = self._batch(patterns, offsets, fixed_len)
+        err = C.c_int(0)
+        r = lib.b200sa_levenshtein_batch(self._h, rev._h, _np_ptr(pat), offp, fixed_len, npat, max_edits,
+                                         C.byref(err))
+        if not r:
+            raise B200saError(err.value, lib.b200sa_last_error().decode())
+        r = C.c_void_p(r)
+        try:
+            n = int(lib.b200sa_levenshtein_hits(r))
+            hoff = np.ctypeslib.as_array(lib.b200sa_levenshtein_offsets(r), shape=(npat + 1,)).copy()
+            cols = {}
+            for k, fn in (("L", lib.b200sa_levenshtein_L), ("R", lib.b200sa_levenshtein_R),
+                          ("length", lib.b200sa_levenshtein_length), ("edits", lib.b200sa_levenshtein_distance)):
+                cols[k] = np.ctypeslib.as_array(fn(r), shape=(n,)).copy() if n else np.zeros(0, np.uint32)
+        finally:
+            lib.b200sa_levenshtein_free(r)
+        return {"offsets": hoff, **cols}
+
     # ---- sampled suffix array (SURVEY 8f rank 3) -----------------------------------------------
     def sample_sa(self, rate: int = 32, drop_sa: bool = False) -> None:
         """Keep SA only at text positions that are multiples of ``rate``; with ``drop_sa`` the full

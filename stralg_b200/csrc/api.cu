@@ -438,6 +438,34 @@ static bool holds_separator(const b200sa_index *idx, const uint8_t *patterns, co
     return b1 > b0 && memchr(patterns + b0, 1, (size_t)(b1 - b0)) != nullptr;
 }
 
+// The refusals of a host batch's pattern lengths: offsets that decrease, then a pattern longer than `limit` symbols
+// (B200SA_ERR_TOO_LARGE with `msg`); max_m gets the longest pattern.
+static int pattern_lengths_ok(const uint64_t *offsets, uint32_t fixed_len, uint64_t npat, uint64_t limit,
+                              const std::string &msg, uint32_t &max_m, enum b200sa_error *err) {
+    uint64_t longest = offsets ? 0 : fixed_len;
+    if (offsets)
+        for (uint64_t q = 0; q < npat; ++q) {
+            if (offsets[q + 1] < offsets[q]) return fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
+            longest = std::max(longest, offsets[q + 1] - offsets[q]);
+        }
+    if (longest > limit) return fail(B200SA_ERR_TOO_LARGE, msg, err);
+    max_m = (uint32_t)longest;
+    return 0;
+}
+
+// A piece's n results, one device column per host vector, appended after the `base` results of the earlier pieces
+// (asynchronous on st)
+struct Column {
+    std::vector<uint32_t> &host;
+    const u32 *dev;
+};
+static void append_columns(uint64_t base, uint64_t n, std::initializer_list<Column> cols, cudaStream_t st) {
+    for (const Column &c : cols) {
+        c.host.resize(base + n);
+        if (n) CUDA_CHECK(cudaMemcpyAsync(c.host.data() + base, c.dev, n * 4, cudaMemcpyDeviceToHost, st));
+    }
+}
+
 // ---- the text of a build or an extension: staged, packed with its bad-symbol check, kept for TEXTCMP ----
 static size_t packed_words(const DeviceIndex &ix) { return ((size_t)ix.len + ix.pk.cpw - 1) / ix.pk.cpw + 4; }
 
@@ -1711,22 +1739,10 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
         return nullptr;
     }
     uint64_t total = offsets ? offsets[npat] : (uint64_t)fixed_len * npat;
-    uint32_t max_m = fixed_len;
-    if (offsets) {
-        max_m = 0;
-        for (uint64_t q = 0; q < npat; ++q) {
-            if (offsets[q + 1] < offsets[q]) {
-                fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
-                return nullptr;
-            }
-            uint64_t m = offsets[q + 1] - offsets[q];
-            if (m > max_m) max_m = (uint32_t)std::min<uint64_t>(m, 0xFFFFFFFFull);
-        }
-    }
-    if (max_m > 65000u) {
-        fail(B200SA_ERR_TOO_LARGE, "approximate search takes patterns of up to 65000 symbols", err);
+    uint32_t max_m = 0;
+    if (pattern_lengths_ok(offsets, fixed_len, npat, 65000, "approximate search takes patterns of up to 65000 symbols",
+                           max_m, err))
         return nullptr;
-    }
     if (holds_separator(idx, patterns, offsets, fixed_len, npat)) {
         fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", err);
         return nullptr;
@@ -1751,17 +1767,10 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
                 ddt.alloc(total + 16, st);
                 approx_dtable(rev_idx->ix, dp.ptr, doff.ptr, fixed_len, npat, ddt.ptr, st);
             }
-            const bool dbg = getenv("B200SA_APPROX_DEBUG") != nullptr;
-            auto now = [&]() {
-                if (dbg) cudaStreamSynchronize(st);
-                return std::chrono::steady_clock::now();
-            };
-            auto t_a = now();
             u64 hits = 0, ops = 0;
             approx_count(ix, dp.ptr, doff.ptr, fixed_len, npat, max_m, ddt.ptr, max_edits, d_hit_off.ptr, d_ops_off.ptr,
                          &hits, &ops, st);
             CUDA_CHECK(cudaMemcpyAsync(res->hit_off.data(), d_hit_off.ptr, (npat + 1) * 8, cudaMemcpyDeviceToHost, st));
-            auto t_b = now();
             res->L.resize(hits);
             res->R.resize(hits);
             res->mlen.resize(hits);
@@ -1781,17 +1790,7 @@ b200sa_approx_result *b200sa_approx_batch(const b200sa_index *idx, const b200sa_
                 CUDA_CHECK(cudaMemcpyAsync(res->cigars.data(), dops.ptr, ops, cudaMemcpyDeviceToHost, st));
             }
             CUDA_CHECK(cudaStreamSynchronize(st));
-            auto t_c = now();
             res->cig_off[hits] = ops;
-            if (dbg) {
-                auto t_d = now();
-                auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-                    return std::chrono::duration<double, std::milli>(b - a).count();
-                };
-                fprintf(stderr, "b200sa_approx_batch: %llu patterns, %llu hits: count pass %.2f ms, emit pass + copies %.2f ms, "
-                        "host tail %.2f ms\n", (unsigned long long)npat, (unsigned long long)hits, ms(t_a, t_b), ms(t_b, t_c),
-                        ms(t_c, t_d));
-            }
         }
         return 0;
     });
@@ -1814,12 +1813,10 @@ void b200sa_approx_free(b200sa_approx_result *r) { delete r; }
 static int mems_args_ok(const b200sa_index *idx, const uint8_t *patterns, const uint64_t *offsets, uint32_t fixed_len,
                         uint64_t npat, enum b200sa_error *err) {
     if (int rc = needs_o_table(idx->ix, err)) return rc;
-    if (offsets)
-        for (uint64_t q = 0; q < npat; ++q) {
-            if (offsets[q + 1] < offsets[q]) return fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
-            if (offsets[q + 1] - offsets[q] > 0xFFFFFFFFull)
-                return fail(B200SA_ERR_TOO_LARGE, "a pattern longer than 2^32 - 1 symbols", err);
-        }
+    uint32_t max_m = 0;
+    if (int rc = pattern_lengths_ok(offsets, fixed_len, npat, 0xFFFFFFFFull, "a pattern longer than 2^32 - 1 symbols",
+                                    max_m, err))
+        return rc;
     if (holds_separator(idx, patterns, offsets, fixed_len, npat))
         return fail(B200SA_ERR_BAD_SYMBOL, "a pattern holds code 1, the record separator of this records index", err);
     return 0;
@@ -1921,16 +1918,10 @@ b200sa_smem_result *b200sa_smem_batch(const b200sa_index *idx, const uint8_t *pa
                         for (uint64_t q = q0; q <= q1; ++q) res->off[q] += base;
                         const uint64_t total = res->off[q1] - base;
                         if (!total) return;
-                        res->start.resize(base + total);
-                        res->length.resize(base + total);
-                        res->L.resize(base + total);
-                        res->R.resize(base + total);
                         DevBuf<u32> ds(total, st), dn(total, st), dsL(total, st), dsR(total, st);
                         mems_emit(ix, doff, fixed_len, np, min_len, dms, dL, dR, dcnt, ds.ptr, dn.ptr, dsL.ptr, dsR.ptr, st);
-                        CUDA_CHECK(cudaMemcpyAsync(res->start.data() + base, ds.ptr, total * 4, cudaMemcpyDeviceToHost, st));
-                        CUDA_CHECK(cudaMemcpyAsync(res->length.data() + base, dn.ptr, total * 4, cudaMemcpyDeviceToHost, st));
-                        CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dsL.ptr, total * 4, cudaMemcpyDeviceToHost, st));
-                        CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dsR.ptr, total * 4, cudaMemcpyDeviceToHost, st));
+                        append_columns(base, total, {{res->start, ds.ptr}, {res->length, dn.ptr}, {res->L, dsL.ptr},
+                                                     {res->R, dsR.ptr}}, st);
                         CUDA_CHECK(cudaStreamSynchronize(st));  // (the output buffers are freed on return)
                     });
         return 0;
@@ -1957,15 +1948,9 @@ static int pair_args_ok(const b200sa_index *idx, const b200sa_index *rev_idx, co
     if (!idx || !rev_idx || (npat && !patterns) || k > max_k)
         return fail(B200SA_ERR_BAD_ARGUMENT,
                     std::string("null argument or ") + k_name + " above " + std::to_string(max_k), err);
-    max_m = fixed_len;
-    if (offsets) {
-        max_m = 0;
-        for (uint64_t q = 0; q < npat; ++q) {
-            if (offsets[q + 1] < offsets[q]) return fail(B200SA_ERR_BAD_ARGUMENT, "pattern offsets must not decrease", err);
-            max_m = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(max_m, offsets[q + 1] - offsets[q]), 0xFFFFFFFFull);
-        }
-    }
-    if (max_m > 65000u) return fail(B200SA_ERR_TOO_LARGE, std::string(what) + " search takes patterns of up to 65000 symbols", err);
+    if (int rc = pattern_lengths_ok(offsets, fixed_len, npat, 65000,
+                                    std::string(what) + " search takes patterns of up to 65000 symbols", max_m, err))
+        return rc;
     const DeviceIndex &ix = idx->ix, &rv = rev_idx->ix;
     if (int rc = needs_o_table(ix, err)) return rc;
     if (int rc = needs_o_table(rv, err)) return rc;
@@ -2039,19 +2024,12 @@ b200sa_hamming_result *b200sa_hamming_batch(const b200sa_index *idx, const b200s
                            [&](uint64_t np, const u8 *dp, const u64 *doff, u64 *dpo, uint64_t &base) {
             base = res->L.size();
             DevBuf<u64> duo(np * (k + 1) + 1, st);
-            const u64 hits = hamming_count(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, st);
+            const u64 hits = pair_count(PairSearch::HAMMING, ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, st);
             if (hits > 0xFFFFFFFFull || np > 0xFFFFFFFFull)
                 return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 hits or patterns in one piece of the batch", err);
-            res->L.resize(base + hits);
-            res->R.resize(base + hits);
-            res->d.resize(base + hits);
             DevBuf<u32> dL(hits ? hits : 1, st), dR(hits ? hits : 1, st), dd(hits ? hits : 1, st);
             hamming_emit(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, hits, dpo, dL.ptr, dR.ptr, dd.ptr, st);
-            if (hits) {
-                CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dL.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-                CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dR.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-                CUDA_CHECK(cudaMemcpyAsync(res->d.data() + base, dd.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-            }
+            append_columns(base, hits, {{res->L, dL.ptr}, {res->R, dR.ptr}, {res->d, dd.ptr}}, st);
             return 0;
         });
     });
@@ -2082,23 +2060,14 @@ b200sa_levenshtein_result *b200sa_levenshtein_batch(const b200sa_index *idx, con
                            [&](uint64_t np, const u8 *dp, const u64 *doff, u64 *dpo, uint64_t &base) {
             base = res->L.size();
             DevBuf<u64> duo(np * (k + 1) + 1, st);
-            const u64 raw = levenshtein_count(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, st);
+            const u64 raw = pair_count(PairSearch::LEVENSHTEIN, ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, st);
             if (raw > 0xFFFFFFFFull)
                 return fail(B200SA_ERR_TOO_LARGE, "more than 2^32 - 1 raw hits in one piece of the batch", err);
             DevBuf<u32> dL(raw ? raw : 1, st), dR(raw ? raw : 1, st), dn(raw ? raw : 1, st), dd(raw ? raw : 1, st);
             const u64 hits =
                 levenshtein_emit(ix, rv, dp, doff, fixed_len, np, max_m, k, duo.ptr, raw, dpo, dL.ptr, dR.ptr, dn.ptr,
                                  dd.ptr, st);
-            res->L.resize(base + hits);
-            res->R.resize(base + hits);
-            res->length.resize(base + hits);
-            res->d.resize(base + hits);
-            if (hits) {
-                CUDA_CHECK(cudaMemcpyAsync(res->L.data() + base, dL.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-                CUDA_CHECK(cudaMemcpyAsync(res->R.data() + base, dR.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-                CUDA_CHECK(cudaMemcpyAsync(res->length.data() + base, dn.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-                CUDA_CHECK(cudaMemcpyAsync(res->d.data() + base, dd.ptr, hits * 4, cudaMemcpyDeviceToHost, st));
-            }
+            append_columns(base, hits, {{res->L, dL.ptr}, {res->R, dR.ptr}, {res->length, dn.ptr}, {res->d, dd.ptr}}, st);
             return 0;
         });
     });

@@ -24,11 +24,9 @@
 //
 // D table (bwt.c:319-337): forward over the pattern with the O table of the REVERSED text (a
 // second index), restarting the interval whenever it empties; D[i] = restarts so far.
-#include "engine.h"
 #include "occ.cuh"
 #include "scan.cuh"
-
-#include <algorithm>
+#include "walk.cuh"
 
 namespace b200sa {
 
@@ -44,7 +42,7 @@ struct ApproxArgs {
     int max_edits;
     bool no_sep;           // records index: letter 1 is the record separator and is never consumed
     uint4 *stack;          // count * max_depth frames
-    u32 max_depth;
+    u32 max_depth;         // max_m + max_edits + 2
     // counting pass
     u32 *hit_count;        // per pattern
     u64 *ops_count;        // per pattern: bytes of CIGAR text (NULs included)
@@ -350,27 +348,29 @@ __global__ void __launch_bounds__(1024) approx_scan_kernel(const u32 *__restrict
     }
 }
 
-static void launch_walk(const DeviceIndex &ix, ApproxArgs &A, bool emit, u64 npat, u32 max_m, cudaStream_t st) {
-    // lanes per launch: the frame stacks of one launch stay under ~1 GiB
-    const u64 frame_bytes = (u64)A.max_depth * 16;
-    u64 chunk = std::max<u64>(1024, ((u64)1 << 30) / frame_bytes);
-    chunk = std::min(chunk, npat);
+static WalkKernels<ApproxArgs> approx_walk_kernels = {{approx_walk_kernel<1, false>, approx_walk_kernel<1, true>},
+                                                      {approx_walk_kernel<2, false>, approx_walk_kernel<2, true>}};
+
+static ApproxArgs approx_args(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fixed_len, u32 max_m,
+                              const u8 *d_dtab, int max_edits) {
+    ApproxArgs A{};
+    A.ov = occ_view(ix);
+    A.c_dev = ix.c_table.ptr;
+    A.len = ix.len;
+    A.sigma = ix.sigma;
+    A.pat = d_pat; A.off = d_off; A.fixed_len = fixed_len;
+    A.dtab = d_dtab;
+    A.max_edits = max_edits;
+    A.no_sep = ix.nrec > 0;
+    A.max_depth = max_m + (u32)max_edits + 2;
+    return A;
+}
+
+static void approx_walk(const DeviceIndex &ix, ApproxArgs &A, bool emit, u64 npat, cudaStream_t st) {
+    const u64 chunk = walk_units_per_launch(npat, (u64)A.max_depth * 16);
     DevBuf<uint4> stack((size_t)chunk * A.max_depth, st);
     A.stack = stack.ptr;
-    for (u64 first = 0; first < npat; first += chunk) {
-        A.first = first;
-        A.count = std::min(chunk, npat - first);
-        const unsigned blocks = div_up_u(A.count * AG, 128);
-        if (ix.occ_layout == OCC_DNA32) {
-            if (emit) approx_walk_kernel<1, true><<<blocks, 128, 0, st>>>(A);
-            else approx_walk_kernel<1, false><<<blocks, 128, 0, st>>>(A);
-        } else {
-            if (emit) approx_walk_kernel<2, true><<<blocks, 128, 0, st>>>(A);
-            else approx_walk_kernel<2, false><<<blocks, 128, 0, st>>>(A);
-        }
-        KERNEL_CHECK();
-    }
-    (void)max_m;
+    run_walk(approx_walk_kernels, ix, emit, A, npat, chunk, AG, 128, st);
 }
 
 // Counting pass + scan.  d_hit_off / d_ops_off: npat + 1 entries each.  Returns (hits, ops).
@@ -385,19 +385,10 @@ void approx_count(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 
     }
     DevBuf<u32> hit_count(npat, st);
     DevBuf<u64> ops_count(npat, st);
-    ApproxArgs A{};
-    A.ov = occ_view(ix);
-    A.c_dev = ix.c_table.ptr;
-    A.len = ix.len;
-    A.sigma = ix.sigma;
-    A.pat = d_pat; A.off = d_off; A.fixed_len = fixed_len;
-    A.dtab = d_dtab;
-    A.max_edits = max_edits;
-    A.no_sep = ix.nrec > 0;
-    A.max_depth = max_m + (u32)max_edits + 2;
+    ApproxArgs A = approx_args(ix, d_pat, d_off, fixed_len, max_m, d_dtab, max_edits);
     A.hit_count = hit_count.ptr;
     A.ops_count = ops_count.ptr;
-    launch_walk(ix, A, false, npat, max_m, st);
+    approx_walk(ix, A, false, npat, st);
     approx_scan_kernel<<<1, 1024, 0, st>>>(hit_count.ptr, ops_count.ptr, npat, d_hit_off, d_ops_off);
     KERNEL_CHECK();
     u64 h[2] = {0, 0};
@@ -412,22 +403,13 @@ void approx_emit(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 f
                  const u8 *d_dtab, int max_edits, const u64 *d_hit_off, const u64 *d_ops_off, u32 *d_L, u32 *d_R,
                  u32 *d_mlen, u64 *d_hit_ops_off, char *d_ops, cudaStream_t st) {
     if (!npat) return;
-    ApproxArgs A{};
-    A.ov = occ_view(ix);
-    A.c_dev = ix.c_table.ptr;
-    A.len = ix.len;
-    A.sigma = ix.sigma;
-    A.pat = d_pat; A.off = d_off; A.fixed_len = fixed_len;
-    A.dtab = d_dtab;
-    A.max_edits = max_edits;
-    A.no_sep = ix.nrec > 0;
-    A.max_depth = max_m + (u32)max_edits + 2;
+    ApproxArgs A = approx_args(ix, d_pat, d_off, fixed_len, max_m, d_dtab, max_edits);
     A.hit_off = d_hit_off;
     A.ops_off = d_ops_off;
     A.out_L = d_L; A.out_R = d_R; A.out_mlen = d_mlen;
     A.out_ops_off = d_hit_ops_off;
     A.out_ops = d_ops;
-    launch_walk(ix, A, true, npat, max_m, st);
+    approx_walk(ix, A, true, npat, st);
 }
 
 }  // namespace b200sa

@@ -131,20 +131,17 @@ void mems_stats(const DeviceIndex &ix, const u8 *d_pat, const u64 *d_off, u32 fi
 void mems_emit(const DeviceIndex &ix, const u64 *d_off, u32 fixed_len, u64 npat, u32 min_len, const u32 *d_ms,
                const u32 *d_L, const u32 *d_R, const u64 *d_smem_off, u32 *d_start, u32 *d_len, u32 *d_sL, u32 *d_sR,
                cudaStream_t st);
-// hamming.cu: k-mismatch search on ix (the text) and rev (the reversed text).  hamming_count: hits per (pattern,
-// search) unit, scanned in place into d_unit_off (npat * (k + 1) + 1 entries); returns the hits.  hamming_emit: the
-// CSR d_pat_off (npat + 1 entries) and the hits (L, R, d), every pattern's in ascending L.
-u64 hamming_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
-                  u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st);
+// hamming.cu, levenshtein.cu: k-mismatch and edit-distance search on ix (the text) and rev (the reversed text).
+// pair_count: the (raw) hits of each (pattern, search) unit of search s, scanned in place into d_unit_off
+// (npat * (k + 1) + 1 entries); returns the (raw) hits.  hamming_emit: the CSR d_pat_off (npat + 1 entries) and the
+// hits (L, R, d), every pattern's in ascending L.  levenshtein_emit: the CSR d_pat_off and the merged hits (L, R,
+// length, d), every pattern's in ascending (L, length), into buffers of raw_hits entries; returns the merged hits.
+enum class PairSearch { HAMMING, LEVENSHTEIN };
+u64 pair_count(PairSearch s, const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
+               u32 fixed_len, u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st);
 void hamming_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
                   u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 hits, u64 *d_pat_off, u32 *d_L, u32 *d_R,
                   u32 *d_d, cudaStream_t st);
-// levenshtein.cu: edit-distance search on ix (the text) and rev (the reversed text).  levenshtein_count: raw hits per
-// (pattern, search) unit, scanned in place into d_unit_off (npat * (k + 1) + 1 entries); returns the raw hits.
-// levenshtein_emit: the CSR d_pat_off (npat + 1 entries) and the merged hits (L, R, length, d), every pattern's in
-// ascending (L, length), into buffers of raw_hits entries; returns the merged hits.
-u64 levenshtein_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
-                      u32 fixed_len, u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st);
 u64 levenshtein_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
                      u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 raw_hits, u64 *d_pat_off, u32 *d_L,
                      u32 *d_R, u32 *d_len, u32 *d_d, cudaStream_t st);

@@ -1,7 +1,8 @@
 // fm_step.cuh -- device pieces of the backward search recurrence that the exact search (fm_search.cu) and the
 // matching statistics (mems.cu) both run: the k-mer seed key, one O step of the DNA layout, and the comparison of
-// pattern symbols with the packed text that finishes a unique interval; and the bidirectional steps and the pattern
-// split of the k-mismatch and edit-distance searches (hamming.cu, levenshtein.cu).
+// pattern symbols with the packed text that finishes a unique interval; and the bidirectional steps (the children of
+// all letters, the exact child of one letter, the byte layout's running start) and the pattern split of the
+// k-mismatch and edit-distance searches (hamming.cu, levenshtein.cu).
 #pragma once
 #include "occ.cuh"
 
@@ -237,6 +238,11 @@ struct BiChildren {
     u32 x[4], w[4], y[4];  // the child of letter a at [a - 1]
 };
 
+// v[a - 1] for a letter a in 1..4
+__device__ __forceinline__ u32 pick4(const u32 (&v)[4], u32 a) {
+    return a == 1 ? v[0] : a == 2 ? v[1] : a == 3 ? v[2] : v[3];
+}
+
 // DNA layout: the children of all four letters from the one or two blocks that dna_step loads
 __device__ __forceinline__ BiChildren dna_bidi_children(const OccView &ov, const CTable5 &c5, u32 x, u32 w, u32 y) {
     const u32 e = x + w;
@@ -256,8 +262,15 @@ __device__ __forceinline__ BiChildren dna_bidi_children(const OccView &ov, const
     return ch;
 }
 
-// Byte layout, one letter at a time in ascending order: the child of letter a.  `run` is y_a on entry (start it at
-// y + bidi_sentinel) and y_{a+1} on return, so a walk over the letters costs two O lookups per letter.
+// Byte layout: y_a, the start on the other index of the child of letter a (two O lookups per letter below a)
+__device__ __forceinline__ u32 byte_bidi_run(const OccView &ov, u32 x, u32 w, u32 y, u32 a) {
+    u32 run = y + bidi_sentinel(ov, x, w);
+    for (u32 b = 1; b < a; ++b) run += occ_byte(ov, b, x + w) - occ_byte(ov, b, x);
+    return run;
+}
+
+// Byte layout, one letter at a time in ascending order: the child of letter a.  `run` is y_a on entry (byte_bidi_run)
+// and y_{a+1} on return, so a walk over the letters costs two O lookups per letter.
 __device__ __forceinline__ void byte_bidi_child(const OccView &ov, const u32 *c, u32 a, u32 x, u32 w, u32 &run,
                                                 u32 &cx, u32 &cw, u32 &cy) {
     const u32 lo = occ_byte(ov, a, x), hi = occ_byte(ov, a, x + w);
@@ -265,6 +278,22 @@ __device__ __forceinline__ void byte_bidi_child(const OccView &ov, const u32 *c,
     cw = hi - lo;
     cy = run;
     run += cw;
+}
+
+// The child of letter a alone (an exact step) on either layout; `c` is the C table (byte layout).  Without `need_y`
+// the byte layout skips the letters below a, and cy is not the child's.
+template <int LAYOUT>
+__device__ __forceinline__ void bidi_child(const OccView &ov, const CTable5 &c5, const u32 *c, u32 a, u32 x, u32 w,
+                                           u32 y, bool need_y, u32 &cx, u32 &cw, u32 &cy) {
+    if (LAYOUT == 1) {
+        const BiChildren ch = dna_bidi_children(ov, c5, x, w, y);
+        cx = pick4(ch.x, a);
+        cw = pick4(ch.w, a);
+        cy = pick4(ch.y, a);
+    } else {
+        u32 run = byte_bidi_run(ov, x, w, y, need_y ? a : 1u);
+        byte_bidi_child(ov, c, a, x, w, run, cx, cw, cy);
+    }
 }
 
 // The index a step runs on: B (the reversed text) for a right extension, F (the text) for a left one.  The two
@@ -284,11 +313,6 @@ __device__ __forceinline__ u32 part_start(u32 j, u32 qs, u32 r) { return j * qs 
 __device__ __forceinline__ u32 part_of(u32 pos, u32 qs, u32 r) {
     const u32 big = r * (qs + 1);
     return pos < big ? pos / (qs + 1) : r + (pos - big) / qs;
-}
-
-// v[a - 1] for a letter a in 1..4
-__device__ __forceinline__ u32 pick4(const u32 (&v)[4], u32 a) {
-    return a == 1 ? v[0] : a == 2 ? v[1] : a == 3 ? v[2] : v[3];
 }
 
 }  // namespace b200sa

@@ -24,35 +24,15 @@
 // [f * units + t]) only when a later child may still be viable.  The walk runs twice: a counting pass (hits per
 // unit), an exclusive scan (scan_u64), and an emitting pass that writes every hit at its final offset with the key
 // [pattern | L]; one stable radix sort of the keys (sort_pairs, locate.cu) puts every pattern's hits in ascending L,
-// and R and d follow through the permutation.
-#include "engine.h"
-#include "fm_step.cuh"
-
-#include <algorithm>
+// and R and d follow through the permutation.  The edit-distance search (levenshtein.cu) runs the same count pass and
+// emitting walk with its sort (pair_count, pair_sorted_hits, below).
+#include "walk.cuh"
 
 namespace b200sa {
 
-struct HammingArgs {
-    OccView fv, bv;        // F (the text) and B (the reversed text)
-    CTable5 c5;            // DNA layout: C table (both indices)
-    const u32 *c_dev;      // byte layout: C table (sigma entries)
-    u32 len, k;
-    const u8 *pat;
-    const u64 *off;
-    u32 fixed_len;
-    u64 first, count;      // work units [first, first + count) run in this launch; unit u = (u / (k + 1), u % (k + 1))
-    uint4 *stack;          // count * max_depth frames
-    // counting pass
-    u64 *unit_count;       // hits per unit
-    // emitting pass
-    const u64 *unit_off;   // exclusive scan of unit_count
-    u64 *key;              // per hit: pattern << 32 | L
-    u32 *val, *R, *d;      // per hit: its index, R and its distance
-};
-
 // frame: x = x, y = y, z = w, w = step | mismatches << 16 | part flag << 20 | next letter << 21
 template <int LAYOUT, bool EMIT>
-__global__ void __launch_bounds__(256) hamming_walk_kernel(HammingArgs A) {
+__global__ void __launch_bounds__(256) hamming_walk_kernel(PairArgs A) {
     __shared__ u32 c_sh[256];
     if (LAYOUT != 1) {
         for (u32 j = threadIdx.x; j < 256; j += blockDim.x) c_sh[j] = j < A.fv.sigma ? A.c_dev[j] : 0;
@@ -102,23 +82,14 @@ __global__ void __launch_bounds__(256) hamming_walk_kernel(HammingArgs A) {
                 if (a == 0 || a > nsym) return;
                 const OccView ov = index_of(right);
                 u32 nx, nw, ny = 0;
-                if (LAYOUT == 1) {
-                    if (right) {
-                        const BiChildren ch = dna_bidi_children(ov, A.c5, x, w, y);
-                        nx = pick4(ch.x, a);
-                        nw = pick4(ch.w, a);
-                        ny = pick4(ch.y, a);
-                    } else {  // (to the left the walk never turns again: y is not needed)
-                        u32 n_blk = 0;
-                        const uint2 lr = dna_step<false>(ov, A.c5, a, x, x + w, n_blk);
-                        nx = lr.x;
-                        nw = lr.y - lr.x;
-                    }
+                // (to the left the walk never turns again: y is not needed)
+                if (LAYOUT == 1 && !right) {
+                    u32 n_blk = 0;
+                    const uint2 lr = dna_step<false>(ov, A.c5, a, x, x + w, n_blk);
+                    nx = lr.x;
+                    nw = lr.y - lr.x;
                 } else {
-                    u32 run = y + bidi_sentinel(ov, x, w);
-                    if (right)
-                        for (u32 b = 1; b < a; ++b) run += occ_byte(ov, b, x + w) - occ_byte(ov, b, x);
-                    byte_bidi_child(ov, c_sh, a, x, w, run, nx, nw, ny);
+                    bidi_child<LAYOUT>(ov, A.c5, c_sh, a, x, w, y, right, nx, nw, ny);
                 }
                 if (!nw) return;
                 turn(s + 1, nx, ny);
@@ -204,8 +175,7 @@ __global__ void __launch_bounds__(256) hamming_walk_kernel(HammingArgs A) {
                     }
                 }
             } else if (ok_match || ok_miss) {
-                u32 run = y + bidi_sentinel(ov, x, w);
-                for (u32 b = 1; b < cursor; ++b) run += occ_byte(ov, b, x + w) - occ_byte(ov, b, x);
+                u32 run = byte_bidi_run(ov, x, w, y, cursor);
                 for (u32 a = cursor; a <= nsym; ++a) {
                     u32 cx, cw, cy;
                     byte_bidi_child(ov, c_sh, a, x, w, run, cx, cw, cy);
@@ -257,9 +227,13 @@ __global__ void __launch_bounds__(256) hamming_pattern_off_kernel(const u64 *__r
     if (q <= npat) pat_off[q] = unit_off[q * (k + 1)];
 }
 
-static HammingArgs hamming_args(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
-                                u32 fixed_len, u32 k) {
-    HammingArgs A{};
+WalkKernels<PairArgs> hamming_walk_kernels = {{hamming_walk_kernel<1, false>, hamming_walk_kernel<1, true>},
+                                               {hamming_walk_kernel<2, false>, hamming_walk_kernel<2, true>}};
+
+// ---- the passes both searches on an index pair share (levenshtein.cu runs them too) -----------------------------
+static PairArgs pair_args(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
+                          u32 fixed_len, u32 k) {
+    PairArgs A{};
     A.fv = occ_view(ix);
     A.bv = occ_view(rev);
     for (int j = 0; j < 8; ++j) A.c5.c[j] = ix.c_host[j];
@@ -272,42 +246,59 @@ static HammingArgs hamming_args(const DeviceIndex &ix, const DeviceIndex &rev, c
     return A;
 }
 
-static void hamming_walk(const DeviceIndex &ix, HammingArgs &A, bool emit, u64 units, u32 max_m, cudaStream_t st) {
-    // units per launch: the frame stacks of one launch stay under ~1 GiB (a walk parks at most one frame per step)
-    const u64 frame_bytes = (u64)std::max<u32>(max_m, 1) * 16;
-    u64 chunk = std::max<u64>(1024, ((u64)1 << 30) / frame_bytes);
-    chunk = std::min(chunk, units);
-    DevBuf<uint4> stack((size_t)chunk * std::max<u32>(max_m, 1), st);
+// A k-mismatch walk parks at most one 16-byte frame per step; an edit-distance walk one 20-byte frame per right node
+// depth (|Q_R| <= |P_>i| + k) and one per left node depth (|Q_L| <= |P_<i| + k).
+static void pair_walk(PairSearch s, const DeviceIndex &ix, PairArgs &A, bool emit, u64 units, u32 max_m,
+                      cudaStream_t st) {
+    const bool lev = s == PairSearch::LEVENSHTEIN;
+    const u64 frames = lev ? (u64)max_m + 2 * A.k + 2 : std::max<u32>(max_m, 1);
+    const u64 chunk = walk_units_per_launch(units, frames * (lev ? 20 : 16));
+    DevBuf<uint4> stack((size_t)(chunk * frames), st);
+    DevBuf<u32> stack_w(lev ? (size_t)(chunk * frames) : 0, st);
     A.stack = stack.ptr;
-    for (u64 first = 0; first < units; first += chunk) {
-        A.first = first;
-        A.count = std::min(chunk, units - first);
-        const unsigned blocks = div_up_u(A.count, 256);
-        if (ix.occ_layout == OCC_DNA32) {
-            if (emit) hamming_walk_kernel<1, true><<<blocks, 256, 0, st>>>(A);
-            else hamming_walk_kernel<1, false><<<blocks, 256, 0, st>>>(A);
-        } else {
-            if (emit) hamming_walk_kernel<2, true><<<blocks, 256, 0, st>>>(A);
-            else hamming_walk_kernel<2, false><<<blocks, 256, 0, st>>>(A);
-        }
-        KERNEL_CHECK();
-    }
+    A.stack_w = stack_w.ptr;
+    run_walk(lev ? levenshtein_walk_kernels : hamming_walk_kernels, ix, emit, A, units, chunk, 1, 256, st);
 }
 
-u64 hamming_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
-                  u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st) {
+u64 pair_count(PairSearch s, const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
+               u32 fixed_len, u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st) {
     const u64 units = npat * (k + 1);
     if (!units) {
         CUDA_CHECK(cudaMemsetAsync(d_unit_off, 0, 8, st));
         return 0;
     }
-    HammingArgs A = hamming_args(ix, rev, d_pat, d_off, fixed_len, k);
+    PairArgs A = pair_args(ix, rev, d_pat, d_off, fixed_len, k);
     A.unit_count = d_unit_off;
-    hamming_walk(ix, A, false, units, max_m, st);
+    pair_walk(s, ix, A, false, units, max_m, st);
     scan_u64(d_unit_off, units, st);
     u64 hits = 0;
     read_back(&hits, d_unit_off + units, 8, st);
     return hits;
+}
+
+PairHits pair_sorted_hits(PairSearch s, const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat,
+                          const u64 *d_off, u32 fixed_len, u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 hits,
+                          int key_bits, cudaStream_t st) {
+    PairHits H;
+    H.kA.alloc(hits, st);
+    H.kB.alloc(hits, st);
+    H.vA.alloc(hits, st);
+    H.vB.alloc(hits, st);
+    H.R.alloc(hits, st);
+    H.d.alloc(hits, st);
+    PairArgs A = pair_args(ix, rev, d_pat, d_off, fixed_len, k);
+    A.unit_off = d_unit_off;
+    A.key = H.kA.ptr;
+    A.val = H.vA.ptr;
+    A.R = H.R.ptr;
+    A.d = H.d.ptr;
+    pair_walk(s, ix, A, true, npat * (k + 1), max_m, st);
+    int qbits = 0;
+    while ((1ull << qbits) < npat) ++qbits;
+    u64 *kb[2] = {H.kA.ptr, H.kB.ptr};
+    u32 *vb[2] = {H.vA.ptr, H.vB.ptr};
+    sort_pairs(kb, vb, (u32)hits, key_bits + qbits, H.key, H.val, st);
+    return H;
 }
 
 void hamming_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
@@ -319,23 +310,9 @@ void hamming_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat
     if (!hits) return;
     if (hits > 0xFFFFFFFFull || npat > 0xFFFFFFFFull)
         throw std::runtime_error("hamming_emit: more than 2^32 - 1 hits or patterns in one piece");
-    DevBuf<u64> kA(hits, st), kB(hits, st);
-    DevBuf<u32> vA(hits, st), vB(hits, st), R(hits, st), d(hits, st);
-    HammingArgs A = hamming_args(ix, rev, d_pat, d_off, fixed_len, k);
-    A.unit_off = d_unit_off;
-    A.key = kA.ptr;
-    A.val = vA.ptr;
-    A.R = R.ptr;
-    A.d = d.ptr;
-    hamming_walk(ix, A, true, npat * (k + 1), max_m, st);
-    int qbits = 0;
-    while ((1ull << qbits) < npat) ++qbits;
-    u64 *kb[2] = {kA.ptr, kB.ptr};
-    u32 *vb[2] = {vA.ptr, vB.ptr};
-    u64 *skeys;
-    u32 *svals;
-    sort_pairs(kb, vb, (u32)hits, 32 + qbits, skeys, svals, st);
-    hamming_take_kernel<<<div_up_u(hits, 256), 256, 0, st>>>(skeys, svals, R.ptr, d.ptr, hits, d_L, d_R, d_d);
+    const PairHits H = pair_sorted_hits(PairSearch::HAMMING, ix, rev, d_pat, d_off, fixed_len, npat, max_m, k,
+                                        d_unit_off, hits, 32, st);
+    hamming_take_kernel<<<div_up_u(hits, 256), 256, 0, st>>>(H.key, H.val, H.R.ptr, H.d.ptr, hits, d_L, d_R, d_d);
     KERNEL_CHECK();
 }
 

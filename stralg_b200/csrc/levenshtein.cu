@@ -23,34 +23,12 @@
 // step a step on F (fm_step.cuh, bidirectional steps); at the turn x and y swap, and the left walk keeps no y.  A node
 // is parked in a stack of 20-byte frames in HBM (frame f of unit t at [f * units + t]) only when a later child may
 // still be viable.  Passes: a counting walk (raw hits per unit), scan_u64, an emitting walk that writes each raw hit
-// at its final offset, one stable radix sort of the keys (sort_pairs), a head flag per key run and its scan, and one
-// pass that writes each run's hit with its minimum distance at its merged offset; per-pattern offsets come from a
-// binary search over the merged hits' patterns.
-#include "engine.h"
-#include "fm_step.cuh"
-
-#include <algorithm>
+// at its final offset, one stable radix sort of the keys (sort_pairs) -- these as in hamming.cu (pair_count,
+// pair_sorted_hits) -- a head flag per key run and its scan, and one pass that writes each run's hit with its minimum
+// distance at its merged offset; per-pattern offsets come from a binary search over the merged hits' patterns.
+#include "walk.cuh"
 
 namespace b200sa {
-
-struct LevArgs {
-    OccView fv, bv;        // F (the text) and B (the reversed text)
-    CTable5 c5;            // DNA layout: C table (both indices)
-    const u32 *c_dev;      // byte layout: C table (sigma entries)
-    u32 len, k;
-    const u8 *pat;
-    const u64 *off;
-    u32 fixed_len;
-    u64 first, count;      // work units [first, first + count) run in this launch; unit u = (u / (k + 1), u % (k + 1))
-    uint4 *stack;          // count * max_frames frames: (x, y or |Q_R|, w, band)
-    u32 *stack_w;          // and t | cursor << 17 | left << 26 | eR << 27
-    // counting pass
-    u64 *unit_count;       // raw hits per unit
-    // emitting pass
-    const u64 *unit_off;   // exclusive scan of unit_count
-    u64 *key;              // per raw hit: pattern << 36 | L << 4 | (|Q| + k - m)
-    u32 *val, *R, *d;      // per raw hit: its index, R and its distance
-};
 
 __device__ __forceinline__ u32 band_cell(u32 band, u32 b) { return (band >> (3 * b)) & 7u; }
 
@@ -96,8 +74,10 @@ __device__ __forceinline__ u32 band_step(u32 band, const u32 (&sy)[9], u32 c, u3
     return out;
 }
 
+// frame: (x, y or |Q_R|, w, band) in stack, t | cursor << 17 | left << 26 | eR << 27 in stack_w; raw hit key:
+// pattern << 36 | L << 4 | (|Q| + k - m)
 template <int LAYOUT, bool EMIT>
-__global__ void __launch_bounds__(256) levenshtein_walk_kernel(LevArgs A) {
+__global__ void __launch_bounds__(256) levenshtein_walk_kernel(PairArgs A) {
     __shared__ u32 c_sh[256];
     if (LAYOUT != 1) {
         for (u32 j = threadIdx.x; j < 256; j += blockDim.x) c_sh[j] = j < A.fv.sigma ? A.c_dev[j] : 0;
@@ -139,16 +119,7 @@ __global__ void __launch_bounds__(256) levenshtein_walk_kernel(LevArgs A) {
                 break;
             }
             u32 cx, cw, cy;
-            if (LAYOUT == 1) {
-                const BiChildren ch = dna_bidi_children(bv, A.c5, x, w, y);
-                cx = pick4(ch.x, a);
-                cw = pick4(ch.w, a);
-                cy = pick4(ch.y, a);
-            } else {
-                u32 run = y + bidi_sentinel(bv, x, w);
-                for (u32 b = 1; b < a; ++b) run += occ_byte(bv, b, x + w) - occ_byte(bv, b, x);
-                byte_bidi_child(bv, c_sh, a, x, w, run, cx, cw, cy);
-            }
+            bidi_child<LAYOUT>(bv, A.c5, c_sh, a, x, w, y, true, cx, cw, cy);
             x = cx;
             w = cw;
             y = cy;
@@ -229,9 +200,7 @@ __global__ void __launch_bounds__(256) levenshtein_walk_kernel(LevArgs A) {
                 u32 mn0;
                 band_step(band, sy, 0, t, n, k, mn0);
                 const OccView ov = step_index(A.fv, A.bv, !left);
-                u32 run = y + bidi_sentinel(ov, x, w);
-                if (!left)
-                    for (u32 b = 1; b < cursor; ++b) run += occ_byte(ov, b, x + w) - occ_byte(ov, b, x);
+                u32 run = byte_bidi_run(ov, x, w, y, left ? 1u : cursor);
                 for (u32 a = cursor; a <= nsym; ++a) {
                     u32 cx, cw, cy, mn;
                     byte_bidi_child(ov, c_sh, a, x, w, run, cx, cw, cy);
@@ -323,61 +292,9 @@ __global__ void __launch_bounds__(256) levenshtein_pattern_off_kernel(const u32 
     pat_off[q] = lo;
 }
 
-static LevArgs levenshtein_args(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
-                                u32 fixed_len, u32 k) {
-    LevArgs A{};
-    A.fv = occ_view(ix);
-    A.bv = occ_view(rev);
-    for (int j = 0; j < 8; ++j) A.c5.c[j] = ix.c_host[j];
-    A.c_dev = ix.c_table.ptr;
-    A.len = ix.len;
-    A.k = k;
-    A.pat = d_pat;
-    A.off = d_off;
-    A.fixed_len = fixed_len;
-    return A;
-}
-
-static void levenshtein_walk(const DeviceIndex &ix, LevArgs &A, bool emit, u64 units, u32 max_m, cudaStream_t st) {
-    // a walk parks at most one frame per right node depth (|Q_R| <= |P_>i| + k) and one per left node depth
-    // (|Q_L| <= |P_<i| + k); units per launch: the frame stacks of one launch stay under ~1 GiB
-    const u64 frames = (u64)max_m + 2 * A.k + 2;
-    u64 chunk = std::max<u64>(1024, ((u64)1 << 30) / (frames * 20));
-    chunk = std::min(chunk, units);
-    DevBuf<uint4> stack((size_t)(chunk * frames), st);
-    DevBuf<u32> stack_w((size_t)(chunk * frames), st);
-    A.stack = stack.ptr;
-    A.stack_w = stack_w.ptr;
-    for (u64 first = 0; first < units; first += chunk) {
-        A.first = first;
-        A.count = std::min(chunk, units - first);
-        const unsigned blocks = div_up_u(A.count, 256);
-        if (ix.occ_layout == OCC_DNA32) {
-            if (emit) levenshtein_walk_kernel<1, true><<<blocks, 256, 0, st>>>(A);
-            else levenshtein_walk_kernel<1, false><<<blocks, 256, 0, st>>>(A);
-        } else {
-            if (emit) levenshtein_walk_kernel<2, true><<<blocks, 256, 0, st>>>(A);
-            else levenshtein_walk_kernel<2, false><<<blocks, 256, 0, st>>>(A);
-        }
-        KERNEL_CHECK();
-    }
-}
-
-u64 levenshtein_count(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off,
-                      u32 fixed_len, u64 npat, u32 max_m, u32 k, u64 *d_unit_off, cudaStream_t st) {
-    const u64 units = npat * (k + 1);
-    if (!units) {
-        CUDA_CHECK(cudaMemsetAsync(d_unit_off, 0, 8, st));
-        return 0;
-    }
-    LevArgs A = levenshtein_args(ix, rev, d_pat, d_off, fixed_len, k);
-    A.unit_count = d_unit_off;
-    levenshtein_walk(ix, A, false, units, max_m, st);
-    scan_u64(d_unit_off, units, st);
-    u64 hits = 0;
-    read_back(&hits, d_unit_off + units, 8, st);
-    return hits;
-}
+WalkKernels<PairArgs> levenshtein_walk_kernels = {
+    {levenshtein_walk_kernel<1, false>, levenshtein_walk_kernel<1, true>},
+    {levenshtein_walk_kernel<2, false>, levenshtein_walk_kernel<2, true>}};
 
 u64 levenshtein_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_pat, const u64 *d_off, u32 fixed_len,
                      u64 npat, u32 max_m, u32 k, const u64 *d_unit_off, u64 raw_hits, u64 *d_pat_off, u32 *d_L,
@@ -388,27 +305,15 @@ u64 levenshtein_emit(const DeviceIndex &ix, const DeviceIndex &rev, const u8 *d_
         if (raw_hits > 0xFFFFFFFFull || npat > ((u64)1 << 28))
             throw std::runtime_error("levenshtein_emit: more than 2^32 - 1 raw hits or 2^28 patterns in one piece");
         const u64 hits = raw_hits;
-        DevBuf<u64> kA(hits, st), kB(hits, st), flag(hits + 1, st);
-        DevBuf<u32> vA(hits, st), vB(hits, st), R(hits, st), d(hits, st), hq(hits, st);
-        LevArgs A = levenshtein_args(ix, rev, d_pat, d_off, fixed_len, k);
-        A.unit_off = d_unit_off;
-        A.key = kA.ptr;
-        A.val = vA.ptr;
-        A.R = R.ptr;
-        A.d = d.ptr;
-        levenshtein_walk(ix, A, true, npat * (k + 1), max_m, st);
-        int qbits = 0;
-        while ((1ull << qbits) < npat) ++qbits;
-        u64 *kb[2] = {kA.ptr, kB.ptr};
-        u32 *vb[2] = {vA.ptr, vB.ptr};
-        u64 *skeys;
-        u32 *svals;
-        sort_pairs(kb, vb, (u32)hits, 36 + qbits, skeys, svals, st);
-        levenshtein_head_kernel<<<div_up_u(hits, 256), 256, 0, st>>>(skeys, hits, flag.ptr);
+        DevBuf<u64> flag(hits + 1, st);
+        DevBuf<u32> hq(hits, st);
+        const PairHits H = pair_sorted_hits(PairSearch::LEVENSHTEIN, ix, rev, d_pat, d_off, fixed_len, npat, max_m, k,
+                                            d_unit_off, hits, 36, st);
+        levenshtein_head_kernel<<<div_up_u(hits, 256), 256, 0, st>>>(H.key, hits, flag.ptr);
         KERNEL_CHECK();
         scan_u64(flag.ptr, hits, st);
-        levenshtein_merge_kernel<<<div_up_u(hits, 256), 256, 0, st>>>(skeys, svals, R.ptr, d.ptr, hits, flag.ptr, d_off,
-                                                                       fixed_len, k, hq.ptr, d_L, d_R, d_len, d_d);
+        levenshtein_merge_kernel<<<div_up_u(hits, 256), 256, 0, st>>>(H.key, H.val, H.R.ptr, H.d.ptr, hits, flag.ptr,
+                                                                       d_off, fixed_len, k, hq.ptr, d_L, d_R, d_len, d_d);
         KERNEL_CHECK();
         read_back(&merged, flag.ptr + hits, 8, st);
         levenshtein_pattern_off_kernel<<<div_up_u(npat + 1, 256), 256, 0, st>>>(hq.ptr, merged, npat, d_pat_off);

@@ -323,15 +323,7 @@ class SuffixArrayIndex:
         ``rev``: index of the reversed text (the reference's RO table -> D table pruning).
         Returns dict(offsets[npat+1], L, R, match_length, cigars[list of str])."""
         lib = _lib.load()
-        pat = np.ascontiguousarray(patterns, dtype=np.uint8)
-        if offsets is not None:
-            off = np.ascontiguousarray(offsets, dtype=np.uint64)
-            npat = len(off) - 1
-            offp = _np_ptr(off)
-        else:
-            assert fixed_len > 0
-            npat = pat.size // fixed_len
-            offp = None
+        pat, _, npat, offp = self._batch(patterns, offsets, fixed_len)
         dt = None
         if d_table is not None:
             dt = np.ascontiguousarray(d_table, dtype=np.uint8)
@@ -339,25 +331,17 @@ class SuffixArrayIndex:
         err = C.c_int(0)
         r = lib.b200sa_approx_batch(self._h, rev._h if rev is not None else None, _np_ptr(dt) if dt is not None else None,
                                     _np_ptr(pat), offp, fixed_len, npat, max_edits, C.byref(err))
-        if not r:
-            raise B200saError(err.value, lib.b200sa_last_error().decode())
-        r = C.c_void_p(r)
-        try:
-            nh = int(lib.b200sa_approx_hits(r))
-            hoff = np.ctypeslib.as_array(lib.b200sa_approx_hit_offsets(r), shape=(npat + 1,)).copy()
-            if nh:
-                L = np.ctypeslib.as_array(lib.b200sa_approx_L(r), shape=(nh,)).copy()
-                R = np.ctypeslib.as_array(lib.b200sa_approx_R(r), shape=(nh,)).copy()
-                ml = np.ctypeslib.as_array(lib.b200sa_approx_match_length(r), shape=(nh,)).copy()
-                coff = np.ctypeslib.as_array(lib.b200sa_approx_cigar_offsets(r), shape=(nh + 1,))
-                raw = C.string_at(lib.b200sa_approx_cigars(r), int(coff[nh]))
-                cig = [x.decode() for x in raw.split(b"\0")[:-1]]
-            else:
-                L = R = ml = np.zeros(0, np.uint32)
-                cig = []
-        finally:
-            lib.b200sa_approx_free(r)
-        return {"offsets": hoff, "L": L, "R": R, "match_length": ml, "cigars": cig}
+
+        def cigars(r, n):
+            if not n:
+                return {"cigars": []}
+            coff = np.ctypeslib.as_array(lib.b200sa_approx_cigar_offsets(r), shape=(n + 1,))
+            raw = C.string_at(lib.b200sa_approx_cigars(r), int(coff[n]))
+            return {"cigars": [x.decode() for x in raw.split(b"\0")[:-1]]}
+
+        return self._result(r, err, npat, lib.b200sa_approx_hits, lib.b200sa_approx_hit_offsets, lib.b200sa_approx_free,
+                            (("L", lib.b200sa_approx_L), ("R", lib.b200sa_approx_R),
+                             ("match_length", lib.b200sa_approx_match_length)), cigars)
 
     # ---- matching statistics and super-maximal exact matches (include/b200sa.h) ----------------------
     @staticmethod
@@ -368,6 +352,25 @@ class SuffixArrayIndex:
             return pat, off, len(off) - 1, _np_ptr(off)
         assert fixed_len > 0
         return pat, None, pat.size // fixed_len, None
+
+    @staticmethod
+    def _result(r, err, npat, count, offsets, free, columns, more=None) -> dict:
+        """A result handle (null: the call's error, ``err``) read into dict(offsets[npat + 1], one uint32 array per
+        (name, accessor) of ``columns``, and what ``more(handle, count)`` returns), then freed."""
+        lib = _lib.load()
+        if not r:
+            raise B200saError(err.value, lib.b200sa_last_error().decode())
+        r = C.c_void_p(r)
+        try:
+            n = int(count(r))
+            out = {"offsets": np.ctypeslib.as_array(offsets(r), shape=(npat + 1,)).copy()}
+            for k, fn in columns:
+                out[k] = np.ctypeslib.as_array(fn(r), shape=(n,)).copy() if n else np.zeros(0, np.uint32)
+            if more is not None:
+                out.update(more(r, n))
+        finally:
+            free(r)
+        return out
 
     def matching_stats(self, patterns, offsets=None, fixed_len: int = 0) -> dict:
         """Per pattern symbol, laid out like ``patterns``: ms (the length of the longest substring of the pattern that
@@ -388,19 +391,9 @@ class SuffixArrayIndex:
         pat, _, npat, offp = self._batch(patterns, offsets, fixed_len)
         err = C.c_int(0)
         r = lib.b200sa_smem_batch(self._h, _np_ptr(pat), offp, fixed_len, npat, min_len, C.byref(err))
-        if not r:
-            raise B200saError(err.value, lib.b200sa_last_error().decode())
-        r = C.c_void_p(r)
-        try:
-            n = int(lib.b200sa_smem_count(r))
-            soff = np.ctypeslib.as_array(lib.b200sa_smem_offsets(r), shape=(npat + 1,)).copy()
-            cols = {}
-            for k, fn in (("start", lib.b200sa_smem_start), ("length", lib.b200sa_smem_length),
-                          ("L", lib.b200sa_smem_L), ("R", lib.b200sa_smem_R)):
-                cols[k] = np.ctypeslib.as_array(fn(r), shape=(n,)).copy() if n else np.zeros(0, np.uint32)
-        finally:
-            lib.b200sa_smem_free(r)
-        return {"offsets": soff, **cols}
+        return self._result(r, err, npat, lib.b200sa_smem_count, lib.b200sa_smem_offsets, lib.b200sa_smem_free,
+                            (("start", lib.b200sa_smem_start), ("length", lib.b200sa_smem_length),
+                             ("L", lib.b200sa_smem_L), ("R", lib.b200sa_smem_R)))
 
     # ---- k-mismatch search (include/b200sa.h: b200sa_hamming_batch) ------------------------------
     def hamming_search(self, patterns, offsets=None, fixed_len: int = 0, max_mismatches: int = 1,
@@ -415,19 +408,9 @@ class SuffixArrayIndex:
         err = C.c_int(0)
         r = lib.b200sa_hamming_batch(self._h, rev._h, _np_ptr(pat), offp, fixed_len, npat, max_mismatches,
                                      C.byref(err))
-        if not r:
-            raise B200saError(err.value, lib.b200sa_last_error().decode())
-        r = C.c_void_p(r)
-        try:
-            n = int(lib.b200sa_hamming_hits(r))
-            hoff = np.ctypeslib.as_array(lib.b200sa_hamming_offsets(r), shape=(npat + 1,)).copy()
-            cols = {}
-            for k, fn in (("L", lib.b200sa_hamming_L), ("R", lib.b200sa_hamming_R),
-                          ("mismatches", lib.b200sa_hamming_mismatches)):
-                cols[k] = np.ctypeslib.as_array(fn(r), shape=(n,)).copy() if n else np.zeros(0, np.uint32)
-        finally:
-            lib.b200sa_hamming_free(r)
-        return {"offsets": hoff, **cols}
+        return self._result(r, err, npat, lib.b200sa_hamming_hits, lib.b200sa_hamming_offsets, lib.b200sa_hamming_free,
+                            (("L", lib.b200sa_hamming_L), ("R", lib.b200sa_hamming_R),
+                             ("mismatches", lib.b200sa_hamming_mismatches)))
 
     # ---- edit-distance search (include/b200sa.h: b200sa_levenshtein_batch) -------------------------
     def levenshtein_search(self, patterns, offsets=None, fixed_len: int = 0, max_edits: int = 1,
@@ -442,19 +425,10 @@ class SuffixArrayIndex:
         err = C.c_int(0)
         r = lib.b200sa_levenshtein_batch(self._h, rev._h, _np_ptr(pat), offp, fixed_len, npat, max_edits,
                                          C.byref(err))
-        if not r:
-            raise B200saError(err.value, lib.b200sa_last_error().decode())
-        r = C.c_void_p(r)
-        try:
-            n = int(lib.b200sa_levenshtein_hits(r))
-            hoff = np.ctypeslib.as_array(lib.b200sa_levenshtein_offsets(r), shape=(npat + 1,)).copy()
-            cols = {}
-            for k, fn in (("L", lib.b200sa_levenshtein_L), ("R", lib.b200sa_levenshtein_R),
-                          ("length", lib.b200sa_levenshtein_length), ("edits", lib.b200sa_levenshtein_distance)):
-                cols[k] = np.ctypeslib.as_array(fn(r), shape=(n,)).copy() if n else np.zeros(0, np.uint32)
-        finally:
-            lib.b200sa_levenshtein_free(r)
-        return {"offsets": hoff, **cols}
+        return self._result(r, err, npat, lib.b200sa_levenshtein_hits, lib.b200sa_levenshtein_offsets,
+                            lib.b200sa_levenshtein_free,
+                            (("L", lib.b200sa_levenshtein_L), ("R", lib.b200sa_levenshtein_R),
+                             ("length", lib.b200sa_levenshtein_length), ("edits", lib.b200sa_levenshtein_distance)))
 
     # ---- sampled suffix array (SURVEY 8f rank 3) -----------------------------------------------
     def sample_sa(self, rate: int = 32, drop_sa: bool = False) -> None:

@@ -1,11 +1,10 @@
-"""Stage times of b200sa_approx_batch on a synthetic DNA index (B200SA_APPROX_DEBUG=1)."""
+"""End-to-end times of b200sa_approx_batch on a synthetic DNA index."""
 import ctypes as C
 import os
 import sys
 import time
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-os.environ["B200SA_APPROX_DEBUG"] = "1"
 import numpy as np
 import torch
 import stralg_b200
